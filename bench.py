@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the batched tracking-MPC solve path (BASELINE.json metric: tracking-MPC solves/s + p99 latency).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (mpcb_solve_batch: warm start -> linearise -> ADMM QP rounds -> outputs) over
 one batch of BASELINE config 4: the seeded Monte-Carlo set of 65,536 perturbed states / obstacle scenarios on
@@ -18,6 +18,11 @@ roofline  neither HBM nor tensor cores bound this path (SURVEY 8d): it is report
           algorithmic flops per SURVEY 8d's formula, peak measured in-process by a register-resident DFMA loop
 --impl reference   the reference's CPU algorithm (oracle port of trajectory_tracking.py solve(): SLSQP ftol=1e-3,
           maxiter=15, finite differences) on all host cores, bounded sample per step
+--dump-outputs DIR   after the timed steps, the outputs of the last timed step of the device-resident arm (what
+          mpcb_solve_batch hands its caller) as DIR/<name>.npy in float64, rank 0 only: U, Xpred, obj, status, iters,
+          cmin, and the 64-bit active-set mask as its low and high 32-bit halves.  The inputs are seeded, so two builds
+          run with the same arguments can be compared output for output.  Above 64 MB a fixed seeded sample of problems
+          is written, with its indices in sample_index.npy
 """
 import argparse
 import json
@@ -174,6 +179,28 @@ N_HANDLES = 2      # device-resident arm: batches in flight (one handle + one st
 N_HANDLES_E2E = 3  # host arm (tools/gpu_e2e_pipe.py): every output 1 / 2 / 3 / 4 handles 1.06 / 0.92 / 0.55 / 0.59 ms per batch,
                    # closed-loop form 0.71 / 0.51 / 0.44 / 0.44
 N_SETS = 8         # distinct seeded 65,536-problem sets the steps rotate over: 8 x 28 MB of inputs + outputs > 126 MB L2
+DUMP_LIMIT = 64 << 20   # bytes --dump-outputs may write (at the default batch every output fits: 24 MB)
+
+
+def dump_outputs(out, dirname):
+    """Write the device outputs of one solve_batch call as dirname/<name>.npy, float64 (exact for every field; the
+    active-set mask is split into its low and high 32-bit halves).  Returns the number of bytes written."""
+    arrs = {k: v.cpu().numpy() for k, v in out.items()}
+    act = arrs["active"].view(np.uint64)
+    arrs["active"] = np.stack([act & np.uint64(0xFFFFFFFF), act >> np.uint64(32)], axis=1)
+    arrs = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in arrs.items()}
+    B = len(arrs["obj"])
+    row = sum(a.nbytes for a in arrs.values()) // max(B, 1)
+    slack = 4096                                              # .npy headers
+    if B * row + slack > DUMP_LIMIT:
+        m = (DUMP_LIMIT - slack) // (row + 8)                  # + 8: the index of each sampled problem
+        idx = np.sort(np.random.default_rng(0).choice(B, m, replace=False))
+        arrs = {k: v[idx] for k, v in arrs.items()}
+        arrs["sample_index"] = idx.astype(np.float64)
+    os.makedirs(dirname, exist_ok=True)
+    for k, v in arrs.items():
+        np.save(os.path.join(dirname, k + ".npy"), v)
+    return sum(a.nbytes for a in arrs.values())
 
 
 def traffic_from_profile():
@@ -342,6 +369,12 @@ def run_ours(args):
     ms_dev = e0.elapsed_time(e1) / args.steps
     launches = sum(t.launch_count() for t in trackers) - launches0
     flops_step = float(np.mean([flops_set[i % N_SETS] for i in range(args.steps)]))
+    if args.dump_outputs and rank == 0:
+        # the last timed step solved set (steps - 1) % N_SETS into its output buffers; later blocks reuse outs[0]
+        k_last = (args.steps - 1) % N_SETS
+        nbytes = dump_outputs(outs[k_last], args.dump_outputs)
+        print(f"bench.py: outputs of timed step {args.steps - 1} (input set {k_last}) written to {args.dump_outputs} "
+              f"({nbytes / 1e6:.1f} MB)", file=sys.stderr)
 
     # ---- one call alone (latency of a whole batch, per-pass times), L2 flushed between calls ---------------
     flush = torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device=dev)   # > 126 MB L2
@@ -563,7 +596,12 @@ def main():
     ap.add_argument("--batch", type=int, default=BATCH)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the closed-loop / planner lines of configs 1-3 and 5")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     global _OUT
     _OUT = _quiet_stdout()
     if args.impl == "reference":

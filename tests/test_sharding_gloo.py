@@ -86,6 +86,8 @@ def test_shard_bounds_partition():
 def test_sharded_equals_unsharded_world2():
     import torch.multiprocessing as mp
     B, world = 301, 2                      # odd size: ragged shards
+    # compiles tests/hostbuild once, here, so that the two workers do not both write the library on a fresh checkout
+    P, tab, solve = _host_solver()
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = _free_port()
@@ -96,7 +98,6 @@ def test_sharded_equals_unsharded_world2():
     for p in procs:
         p.join(timeout=60)
         assert p.exitcode == 0
-    P, tab, solve = _host_solver()
     x0, obs, n = P.monte_carlo_problems(tab, B)
     ref = solve(x0, obs, n)
     got.sort(key=lambda t: t[0])
