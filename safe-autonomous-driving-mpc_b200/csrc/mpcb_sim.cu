@@ -61,7 +61,9 @@ mpcb_fsm_kernel(int B, double dt, double s_stop, const double* __restrict__ x, c
     if (sc.dynamic_obstacle) {
       if (s >= sc.obs_trigger_s && !(f & F_OBS_TRIGGERED)) f |= F_OBS_TRIGGERED | F_OBS_ACTIVE;
       if (f & F_OBS_ACTIVE) {
-        obs_s += sc.obs_v * dt;
+        // no FMA contraction: the car advances by the rounded product, as in the reference, so the obstacle the
+        // solver sees is the reference's to the bit (the rounding difference otherwise grows with every step)
+        obs_s = __dadd_rn(obs_s, __dmul_rn(sc.obs_v, dt));
         if (obs_s > sc.obs_end_s) f &= ~F_OBS_ACTIVE;
         else { o[0] = obs_s; o[1] = sc.obs_v; n = 1; car_s = obs_s; }
       }
