@@ -53,6 +53,7 @@ template <> struct ClsCfg<2> { typedef Store<SOLVE_THREADS, MPCB_CLS_MASK2, 2> S
 constexpr int cmax3(int a, int b, int c) { return a > b ? (a > c ? a : c) : (b > c ? b : c); }
 constexpr size_t CLS_SMEM = sizeof(double) * SOLVE_THREADS * cmax3(ClsCfg<0>::St::SHARED, ClsCfg<1>::St::SHARED, ClsCfg<2>::St::SHARED);
 constexpr int CLS_HDR = 4;                // class-list header: three counts, pad; then three lists of B indices each
+constexpr int CARRY_HDR = 12;             // survivor lists of the first pass: three headers of 4 ints (counts of classes 0-2, pad)
 constexpr int EVAL_THREADS = 128;
 
 // Device pointers of one solve call (mpcb_solve_batch's arguments), handed to the kernels as one block.
@@ -218,7 +219,8 @@ mpcb_solve_kernel(const __grid_constant__ DevTable T, const __grid_constant__ De
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
 mpcb_classify_kernel(int B, const int* __restrict__ idx, const int* __restrict__ n_idx, const int* __restrict__ n_obs,
-                     int* __restrict__ cls) {
+                     int* __restrict__ cls, int* __restrict__ carry_hdr) {
+  if (blockIdx.x == 0 && threadIdx.x < CARRY_HDR) carry_hdr[threadIdx.x] = 0;   // survivor lists of the first pass
   const int n_work = idx ? min(*n_idx, B) : B;
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
   const bool live = t < n_work;
@@ -248,15 +250,115 @@ __device__ __forceinline__ void load_hot_start(const SolveIO& io, int b, double 
   for (int i = 0; i < NV; ++i) Uh[i] = io.shift_start ? src[i + 2 < NV ? i + 2 : i] : src[i];
 }
 
+// ------------------------------------------------------------------------------------------------
+// Compaction of the first pass (batches of more than one wave of CTAs, see launch_solve).  Every problem runs rounds
+// 1..r0 in mpcb_solve_cls_kernel; one that is still unfinished then parks what crosses a round boundary in a slot of
+// the carry workspace and mpcb_solve_round_kernel runs each further round over the packed survivors, so that a CTA no
+// longer carries its finished lanes through the rounds its slowest problem needs.  A problem's arithmetic is the same
+// whichever kernel runs its rounds.
+// Measured on B200 (65,536 Monte-Carlo problems; survivors after rounds 2 / 3 / 4: 65,509 / 30,221 / 1,034):
+// r0 = 2 / 3 / 4 -> class kernel 178 / 239 / 284 us + round kernels 207 / 108 / 75 us, against 312 us for all rounds in
+// the class kernel; with two batches in flight 0.419 / 0.393 / 0.363 ms per step against 0.393 ms.  A round kernel over a
+// few CTAs costs about a whole round of the full kernel (its code runs cold), so r0 = 4 leaves it only the 1.6 % of the
+// problems that need round 5.  Also measured: the later rounds as tail tasks of the class kernel itself (a CTA done with
+// its own problems takes chunks of 128 survivors of a finished class from a counter): 0.362 ms at r0 = 4, the same, with
+// twice the spill code in the class kernel; at r0 = 3 most chunks fall to the last CTA of a class, 0.710 ms.
+// ------------------------------------------------------------------------------------------------
+#ifndef MPCB_CLS_ROUNDS
+#define MPCB_CLS_ROUNDS 4
+#endif
+constexpr int CLS_ROUNDS = MPCB_CLS_ROUNDS;   // rounds of the class kernel (the rest: one round kernel per round)
+
+// One carry workspace: slot-major arrays (field f of slot s at [f * cap + s], so the loads of a CTA's consecutive slots
+// coalesce).  A list of survivors is a header of per-class counts; class k's survivors occupy the slots from the class-k
+// offset of the batch's class partition on (classes with more rows first: class 2 at 0, class 1 at n2, class 0 at n2 + n1).
+enum : int { CD_U = 0, CD_X = CD_U + NV, CD_V = CD_X + NV, CD_LOV = CD_V + ROW_OBS + 2 * N_OBSROW, CD_BLO = CD_LOV + NH,
+             CD_BHI = CD_BLO + NH, CD_HIO = CD_BHI + NH, N_CD = CD_HIO + 2 * N_OBSROW };
+enum : int { CI_B = 0, CI_HINT = 1, CI_FAILS = CI_HINT + NH + 1, CI_ROUNDS, CI_ITERS, CI_STATUS, CI_FLAGS, N_CI };
+constexpr size_t CARRY_SLOT_BYTES = sizeof(double) * N_CD + sizeof(unsigned long long) + sizeof(int) * N_CI;
+
+struct Carry {
+  double* d; unsigned long long* a; int* i; int cap;
+  __host__ __device__ static Carry at(void* base, int cap) {
+    Carry c;
+    c.d = (double*)base;
+    c.a = (unsigned long long*)(c.d + (size_t)N_CD * cap);
+    c.i = (int*)(c.a + cap);
+    c.cap = cap;
+    return c;
+  }
+};
+
+// Slot of this thread in a list (warp-aggregated append to counter; every lane of the warp calls it), -1 if !pred.
+__device__ __forceinline__ int warp_append(bool pred, int* counter) {
+  const unsigned m = __ballot_sync(0xffffffffu, pred);
+  if (m == 0u) return -1;
+  const unsigned lane = threadIdx.x & 31u;
+  const int leader = __ffs(m) - 1;
+  int base = 0;
+  if ((int)lane == leader) base = atomicAdd(counter, __popc(m));
+  base = __shfl_sync(0xffffffffu, base, leader);
+  return pred ? base + __popc(m & ((1u << lane) - 1u)) : -1;
+}
+
+// What crosses a round boundary of the first pass: the iterate, the ADMM state v and the active set, the table hints, the
+// prologue's bounds, and the loop scalars (step_prev is read by the robust pass only, the rungs E by the robust ladder only).
+template <class ST>
+__device__ __forceinline__ void park(const Carry& c, int slot, int b, const Problem& pb, const ST& st, const SolveState& s) {
+  MPCB_ASSERT(slot >= 0 && slot < c.cap);
+  double* __restrict__ d = c.d + slot;
+  int* __restrict__ iv = c.i + slot;
+  const size_t n = c.cap;
+#pragma unroll
+  for (int k = 0; k < NV; ++k) { d[(CD_U + k) * n] = pb.U[k]; d[(CD_X + k) * n] = pb.x[k]; }
+#pragma unroll
+  for (int r = 0; r < ST::MROWS; ++r) d[(CD_V + r) * n] = st.v[r];
+#pragma unroll
+  for (int j = 0; j < NH; ++j) { d[(CD_LOV + j) * n] = st.lov[j]; d[(CD_BLO + j) * n] = st.blo[j]; d[(CD_BHI + j) * n] = st.bhi[j]; }
+#pragma unroll
+  for (int r = 0; r < ST::KOBS * N_OBSROW; ++r) d[(CD_HIO + r) * n] = st.hio[r];
+  c.a[slot] = pb.act_prev;
+  iv[CI_B * n] = b;
+#pragma unroll
+  for (int j = 0; j <= NH; ++j) iv[(CI_HINT + j) * n] = pb.hint[j];
+  iv[CI_FAILS * n] = s.fails;
+  iv[CI_ROUNDS * n] = s.out.rounds;
+  iv[CI_ITERS * n] = s.out.iters;
+  iv[CI_STATUS * n] = s.out.status;
+  iv[CI_FLAGS * n] = (s.infeasible ? 1 : 0) | (s.out.const_infeasible ? 2 : 0);
+}
+
+template <class ST>
+__device__ __forceinline__ void unpark(const Carry& c, int slot, Problem& pb, const ST& st, SolveState& s) {
+  MPCB_ASSERT(slot >= 0 && slot < c.cap);
+  const double* __restrict__ d = c.d + slot;
+  const int* __restrict__ iv = c.i + slot;
+  const size_t n = c.cap;
+#pragma unroll
+  for (int k = 0; k < NV; ++k) { pb.U[k] = d[(CD_U + k) * n]; pb.x[k] = d[(CD_X + k) * n]; }
+#pragma unroll
+  for (int r = 0; r < ST::MROWS; ++r) st.v[r] = d[(CD_V + r) * n];
+#pragma unroll
+  for (int j = 0; j < NH; ++j) { st.lov[j] = d[(CD_LOV + j) * n]; st.blo[j] = d[(CD_BLO + j) * n]; st.bhi[j] = d[(CD_BHI + j) * n]; }
+#pragma unroll
+  for (int r = 0; r < ST::KOBS * N_OBSROW; ++r) st.hio[r] = d[(CD_HIO + r) * n];
+  pb.act_prev = c.a[slot];
+#pragma unroll
+  for (int j = 0; j <= NH; ++j) pb.hint[j] = iv[(CI_HINT + j) * n];
+  s.fails = iv[CI_FAILS * n];
+  s.out.rounds = iv[CI_ROUNDS * n];
+  s.out.iters = iv[CI_ITERS * n];
+  s.out.status = iv[CI_STATUS * n];
+  const int f = iv[CI_FLAGS * n];
+  s.infeasible = (f & 1) != 0;
+  s.out.const_infeasible = (f & 2) != 0;
+  s.done = false; s.first = false; s.hot = false;
+  s.step_prev = 1e30;
+}
+
+// problem b's inputs (class NOBS); a thread without a problem gets a benign zero problem it never works on
 template <int NOBS>
-__device__ __forceinline__ void solve_cls_body(const DevTable& T, const DevParams& P, const SolveIO& io, const int* __restrict__ list,
-                                               int n_work, int t0, int* __restrict__ fb_list, int* __restrict__ fb_count) {
-  typedef typename ClsCfg<NOBS>::St St;
-  const int t = t0 + threadIdx.x;
-  const bool live = t < n_work;
-  const int b = live ? list[t] : 0;
-  MPCB_ASSERT(b >= 0 && b < io.n_total);
-  Problem pb;
+__device__ __forceinline__ void load_problem(const SolveIO& io, int b, bool live, Problem& pb) {
   if (live) {
 #pragma unroll
     for (int c = 0; c < 5; ++c) pb.x0[c] = io.x0[(size_t)b * 5 + c];
@@ -272,30 +374,129 @@ __device__ __forceinline__ void solve_cls_body(const DevTable& T, const DevParam
     pb.obs[0][0] = pb.obs[0][1] = pb.obs[1][0] = pb.obs[1][1] = 0.0;
     pb.n_obs = 0;
   }
+}
+
+// After a problem's last round in this kernel: park it in the next list (cont, every thread of the warp calls this),
+// or finalize it.
+template <int NOBS, class ST>
+__device__ __forceinline__ void park_or_finalize(const DevTable& T, const DevParams& P, const SolveIO& io, bool live, bool cont,
+                                                 int b, Problem& pb, const ST& st, SolveState& s, int n_work,
+                                                 const Carry& cout, int* __restrict__ cnt_out, int off,
+                                                 int* __restrict__ fb_list, int* __restrict__ fb_count) {
+  const int k = warp_append(cont, cnt_out + NOBS);
+  if (!live) return;
+  if (cont) {
+    MPCB_ASSERT(k >= 0 && k < n_work);             // a list never outgrows the one it was compacted from
+    park(cout, off + k, b, pb, st, s);
+    return;
+  }
+  const SolveOut so = solve_end<true>(P, pb, s);
+  finalize<true>(T, P, pb, so, b, io.accumulate != 0, io, fb_list, fb_count);
+}
+
+template <int NOBS>
+__device__ __forceinline__ void solve_cls_body(const DevTable& T, const DevParams& P, const SolveIO& io, const int* __restrict__ list,
+                                               int n_work, int t0, int off, int r0, const Carry& cout,
+                                               int* __restrict__ cnt_out, int* __restrict__ fb_list, int* __restrict__ fb_count) {
+  typedef typename ClsCfg<NOBS>::St St;
+  const int t = t0 + threadIdx.x;
+  const bool live = t < n_work;
+  const int b = live ? list[t] : 0;
+  MPCB_ASSERT(b >= 0 && b < io.n_total);
+  Problem pb;
+  load_problem<NOBS>(io, b, live, pb);
   extern __shared__ double solve_smem[];
   double solve_local[St::LOCAL];
   const St st(solve_smem + threadIdx.x, solve_local);
   double Uh[NV];
   const bool hot = io.U_start != nullptr;             // CTA-uniform
   if (hot && live) load_hot_start(io, b, Uh);
-  SolveOut so = solve_one<true>(T, P, pb, st, live, (hot && live) ? Uh : nullptr);
-  if (!live) return;
-  finalize<true>(T, P, pb, so, b, io.accumulate != 0, io, fb_list, fb_count);
+  SolveState s;
+  solve_start<true>(T, P, pb, st, live, (hot && live) ? Uh : nullptr, s);
+#pragma unroll 1
+  for (int round = 0; round < r0; ++round) {   // not unrolled: no FMA contraction across a round boundary
+    if (MPCB_ALL(s.done)) break;
+    solve_round<true>(T, P, pb, st, s, round);
+  }
+  park_or_finalize<NOBS>(T, P, io, live, live && !s.done && r0 < P.thread_max_rounds, b, pb, st, s, n_work, cout, cnt_out,
+                         off, fb_list, fb_count);
+}
+
+// class k's region of a list: classes with more rows first
+__device__ __forceinline__ int class_offset(const int* __restrict__ cls, int k) {
+  return k == 2 ? 0 : (k == 1 ? cls[2] : cls[2] + cls[1]);
 }
 
 __global__ void __launch_bounds__(SOLVE_THREADS, MPCB_SOLVE_CTAS)
 mpcb_solve_cls_kernel(const __grid_constant__ DevTable T, const __grid_constant__ DevParams P, int B,
-                      const __grid_constant__ SolveIO io, const int* __restrict__ cls, int* __restrict__ fb_list,
+                      const __grid_constant__ SolveIO io, const int* __restrict__ cls, int r0,
+                      const __grid_constant__ Carry cout, int* __restrict__ cnt_out, int* __restrict__ fb_list,
                       int* __restrict__ fb_count) {
   const int n2 = cls[2], n1 = cls[1], n0 = cls[0];
   const int c2 = (n2 + SOLVE_THREADS - 1) / SOLVE_THREADS, c1 = (n1 + SOLVE_THREADS - 1) / SOLVE_THREADS,
             c0 = (n0 + SOLVE_THREADS - 1) / SOLVE_THREADS;
+  const int* lists = cls + CLS_HDR;
   int blk = blockIdx.x;                                                       // CTA-uniform from here on
-  if (blk < c2) { solve_cls_body<2>(T, P, io, cls + CLS_HDR + (size_t)2 * B, n2, blk * SOLVE_THREADS, fb_list, fb_count); return; }
+  if (blk < c2) { solve_cls_body<2>(T, P, io, lists + (size_t)2 * B, n2, blk * SOLVE_THREADS, 0, r0, cout, cnt_out, fb_list, fb_count); return; }
   blk -= c2;
-  if (blk < c1) { solve_cls_body<1>(T, P, io, cls + CLS_HDR + (size_t)1 * B, n1, blk * SOLVE_THREADS, fb_list, fb_count); return; }
+  if (blk < c1) { solve_cls_body<1>(T, P, io, lists + (size_t)1 * B, n1, blk * SOLVE_THREADS, n2, r0, cout, cnt_out, fb_list, fb_count); return; }
   blk -= c1;
-  if (blk < c0) solve_cls_body<0>(T, P, io, cls + CLS_HDR, n0, blk * SOLVE_THREADS, fb_list, fb_count);
+  if (blk < c0) solve_cls_body<0>(T, P, io, lists, n0, blk * SOLVE_THREADS, n2 + n1, r0, cout, cnt_out, fb_list, fb_count);
+}
+
+#ifdef MPCB_ROUND_STATS   // development: survivors per round and class, summed over calls (tools/gpu_round_counts.py)
+__device__ unsigned long long g_round_stats[16 * 3];
+#endif
+
+// One further round of the first pass over the survivors of class NOBS listed in cin (slots off + t0 + threadIdx.x).
+template <int NOBS>
+__device__ __forceinline__ void solve_round_body(const DevTable& T, const DevParams& P, const SolveIO& io, int n_work, int t0,
+                                                 int off, const Carry& cin, const Carry& cout, int* __restrict__ cnt_out,
+                                                 int round, int* __restrict__ fb_list, int* __restrict__ fb_count) {
+  typedef typename ClsCfg<NOBS>::St St;
+  const int t = t0 + threadIdx.x;
+  const bool live = t < n_work;
+  const int slot = off + t;
+  MPCB_ASSERT(!live || (slot >= 0 && slot < cin.cap));
+  const int b = live ? cin.i[(size_t)CI_B * cin.cap + slot] : 0;
+  MPCB_ASSERT(b >= 0 && b < io.n_total);
+  Problem pb;
+  load_problem<NOBS>(io, b, live, pb);
+  extern __shared__ double solve_smem[];
+  double solve_local[St::LOCAL];
+  const St st(solve_smem + threadIdx.x, solve_local);
+  SolveState s;
+  s.out = SolveOut{MPCB_MAXITER, 0, 0, false};
+  s.done = true; s.infeasible = false; s.first = false; s.hot = false; s.fails = 0; s.step_prev = 1e30;
+  if (live) unpark(cin, slot, pb, st, s);
+  solve_round<true>(T, P, pb, st, s, round);
+  park_or_finalize<NOBS>(T, P, io, live, live && !s.done && round + 1 < P.thread_max_rounds, b, pb, st, s, n_work, cout,
+                         cnt_out, off, fb_list, fb_count);
+}
+
+// Round `round` (0-based, >= the class kernel's r0) of the first pass: 128 listed problems of one class per CTA, classes with more
+// rows first; CTAs beyond the list's counts exit at once.  Survivors go to the next list (cout, cnt_out), the others are
+// finalized as in the class kernel -- after the last round all of them.  cnt_clear: the header the next round kernel
+// appends to (read by the previous one, which has finished), zeroed here.
+__global__ void __launch_bounds__(SOLVE_THREADS, MPCB_SOLVE_CTAS)
+mpcb_solve_round_kernel(const __grid_constant__ DevTable T, const __grid_constant__ DevParams P,
+                        const __grid_constant__ SolveIO io, const int* __restrict__ cls, const int* __restrict__ cnt_in,
+                        const __grid_constant__ Carry cin, int* __restrict__ cnt_out, const __grid_constant__ Carry cout,
+                        int* __restrict__ cnt_clear, int round, int* __restrict__ fb_list, int* __restrict__ fb_count) {
+  if (blockIdx.x == 0 && threadIdx.x < 3) cnt_clear[threadIdx.x] = 0;
+  const int n2 = cnt_in[2], n1 = cnt_in[1], n0 = cnt_in[0];
+#ifdef MPCB_ROUND_STATS
+  if (blockIdx.x == 0 && threadIdx.x < 3 && round < 16) atomicAdd(&g_round_stats[3 * round + threadIdx.x], (unsigned long long)cnt_in[threadIdx.x]);
+#endif
+  MPCB_ASSERT(n2 >= 0 && n2 <= cls[2] && n1 >= 0 && n1 <= cls[1] && n0 >= 0 && n0 <= cls[0]);
+  const int c2 = (n2 + SOLVE_THREADS - 1) / SOLVE_THREADS, c1 = (n1 + SOLVE_THREADS - 1) / SOLVE_THREADS,
+            c0 = (n0 + SOLVE_THREADS - 1) / SOLVE_THREADS;
+  int blk = blockIdx.x;                                                       // CTA-uniform from here on
+  if (blk < c2) { solve_round_body<2>(T, P, io, n2, blk * SOLVE_THREADS, class_offset(cls, 2), cin, cout, cnt_out, round, fb_list, fb_count); return; }
+  blk -= c2;
+  if (blk < c1) { solve_round_body<1>(T, P, io, n1, blk * SOLVE_THREADS, class_offset(cls, 1), cin, cout, cnt_out, round, fb_list, fb_count); return; }
+  blk -= c1;
+  if (blk < c0) solve_round_body<0>(T, P, io, n0, blk * SOLVE_THREADS, class_offset(cls, 0), cin, cout, cnt_out, round, fb_list, fb_count);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -640,6 +841,7 @@ int mpcb_create(mpcb_handle* out, const mpcb_params* p, mpcb_table_handle t, int
   if ((e = cudaEventCreate(&c->ev_mid)) != cudaSuccess) return fail(cuda_fail(e, "cudaEventCreate"));
   if ((e = cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming)) != cudaSuccess) return fail(cuda_fail(e, "cudaEventCreate"));
   if ((e = cudaFuncSetAttribute(mpcb_solve_cls_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(mpcb_solve_round_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
       (e = cudaFuncSetAttribute(mpcb_solve_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SOLVE_SMEM)) != cudaSuccess ||
       (e = cudaFuncSetAttribute(mpcb_coop_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)COOP_SMEM)) != cudaSuccess ||
       (e = cudaFuncSetAttribute(mpcb_coop_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)COOP_SMEM)) != cudaSuccess)
@@ -690,8 +892,7 @@ int mpcb_destroy(mpcb_handle h) {
   }
   if (h->ev_fork) cudaEventDestroy(h->ev_fork);
   if (h->ws) cudaFree(h->ws);
-  if (h->fb) cudaFree(h->fb);
-  if (h->cls) cudaFree(h->cls);
+  if (h->fb) cudaFree(h->fb);                      // fb, cls and carry are one block
   if (h->ev0) cudaEventDestroy(h->ev0);
   if (h->ev1) cudaEventDestroy(h->ev1);
   if (h->ev_mid) cudaEventDestroy(h->ev_mid);
@@ -711,15 +912,23 @@ int mpcb_destroy(mpcb_handle h) {
 #define MPCB_HOST_CHUNKS 4
 #endif
 static const int HOST_CHUNKS = MPCB_HOST_CHUNKS;   // parts of a large host batch, dealt round-robin onto the 4 streams
+static size_t al256(size_t x) { return (x + 255) & ~(size_t)255; }
+
+// fb, cls and carry are one allocation, so that h->fb (in the graph key) stands for all three.  A part whose work list
+// starts at fb + o keeps its class-list header and three lists at cls + 3 o, and its survivor-list headers and two carry
+// workspaces at carry + 2 o CARRY_SLOT_BYTES (FB_HDR == CLS_HDR, so the slices of the parts of a chunked host call do not
+// overlap; FB_HDR carry slots hold the headers).
 static int ensure_fb(mpcb_handle h, int B) {
   if (!h->params.fast_pass || B + FB_HDR * HOST_CHUNKS <= h->fb_cap) return MPCB_OK;
-  if (h->fb) { CK(cudaFree(h->fb)); h->fb = nullptr; h->fb_cap = 0; }
-  if (h->cls) { CK(cudaFree(h->cls)); h->cls = nullptr; }
-  if (cudaMalloc(&h->fb, sizeof(int) * ((size_t)B + FB_HDR * HOST_CHUNKS)) != cudaSuccess) { cudaGetLastError(); return MPCB_ERR_NOMEM; }
-  // class lists of the first pass: a part whose work list starts at fb + o keeps its header and three lists at cls + 3 o
-  // (FB_HDR == CLS_HDR, so the slices of the parts of a chunked host call do not overlap)
-  if (cudaMalloc(&h->cls, sizeof(int) * 3 * ((size_t)B + FB_HDR * HOST_CHUNKS)) != cudaSuccess) { cudaGetLastError(); return MPCB_ERR_NOMEM; }
-  h->fb_cap = B + FB_HDR * HOST_CHUNKS;
+  if (h->fb) { CK(cudaFree(h->fb)); h->fb = nullptr; h->cls = nullptr; h->carry = nullptr; h->fb_cap = 0; }
+  const size_t cap = (size_t)B + FB_HDR * HOST_CHUNKS;
+  const size_t o_cls = al256(sizeof(int) * cap), o_carry = o_cls + al256(sizeof(int) * 3 * cap);
+  void* p = nullptr;
+  if (cudaMalloc(&p, o_carry + 2 * cap * CARRY_SLOT_BYTES) != cudaSuccess) { cudaGetLastError(); return MPCB_ERR_NOMEM; }
+  h->fb = (int*)p;
+  h->cls = (int*)((char*)p + o_cls);
+  h->carry = (char*)p + o_carry;
+  h->fb_cap = (int)cap;
   return MPCB_OK;
 }
 
@@ -762,13 +971,32 @@ static int launch_solve(mpcb_handle h, int B, const SolveIO& io_in, cudaStream_t
       // partition by obstacle count, then one CTA per 128 problems of one class (at most two partly filled CTAs more
       // than the unpartitioned grid)
       int* cls = h->cls + (fb - h->fb) * 3;                    // this part's slice: header + three lists of B
+      char* cw = h->carry + (size_t)(fb - h->fb) * 2 * CARRY_SLOT_BYTES;   // survivor-list headers, two workspaces of B
+      int* hdr = (int*)cw;                                     // headers: survivors after round r at hdr + 4 (r % 3)
+      const size_t w0 = FB_HDR * 2 * CARRY_SLOT_BYTES;
+      const Carry wk[2] = {Carry::at(cw + w0, B), Carry::at(cw + w0 + (size_t)B * CARRY_SLOT_BYTES, B)};
       CK(cudaMemsetAsync(cls, 0, sizeof(int) * CLS_HDR, st));
-      mpcb_classify_kernel<<<(B + 255) / 256, 256, 0, st>>>(B, io.idx, io.n_idx, io.n_obs, cls);
+      mpcb_classify_kernel<<<(B + 255) / 256, 256, 0, st>>>(B, io.idx, io.n_idx, io.n_obs, cls, hdr);
       CK(cudaGetLastError());
       SolveIO io1 = io;
       io1.idx = nullptr; io1.n_idx = nullptr;                  // the class lists carry the problem indices from here on
-      mpcb_solve_cls_kernel<<<grid + 2, SOLVE_THREADS, CLS_SMEM, st>>>(h->dt, h->dp, B, io1, cls, fb_list, fb_count);
+      // Compaction only pays when the batch is more than one wave of CTAs: within one wave every CTA runs at once and the
+      // pass lasts as long as its slowest CTA anyway, and a round kernel would only add its latency (closed loops).
+      const int max_rounds = h->dp.thread_max_rounds;
+      const bool compact = grid > h->n_sm * MPCB_SOLVE_CTAS;
+      const int r0 = compact ? std::min(CLS_ROUNDS, max_rounds) : max_rounds;
+      mpcb_solve_cls_kernel<<<grid + 2, SOLVE_THREADS, CLS_SMEM, st>>>(h->dt, h->dp, B, io1, cls, r0, wk[0],
+                                                                      hdr + 4 * (r0 % 3), fb_list, fb_count);
       h->launches++;
+      // the rounds after r0 over the packed survivors, one launch per round (workspaces ping-pong; each kernel zeroes
+      // the header its successor appends to)
+      for (int r = r0; r < max_rounds; ++r) {
+        const int p = (r - r0) & 1;
+        mpcb_solve_round_kernel<<<grid + 2, SOLVE_THREADS, CLS_SMEM, st>>>(h->dt, h->dp, io1, cls, hdr + 4 * (r % 3), wk[p],
+                                                                          hdr + 4 * ((r + 1) % 3), wk[p ^ 1],
+                                                                          hdr + 4 * ((r + 2) % 3), r, fb_list, fb_count);
+        h->launches++;
+      }
     }
     CK(cudaGetLastError());
     if (timed) CK(record_event(h->ev_mid, st));
@@ -841,8 +1069,6 @@ int mpcb_solve_list_internal(mpcb_handle h, int B, const int* idx, const int* n_
   io.shift_start = 1;
   return launch_solve(h, B, io, st, h->fb, true, call_uses_coop(h, B));
 }
-
-static size_t al256(size_t x) { return (x + 255) & ~(size_t)255; }
 
 // Lower edge of part c of a chunked host call, as a fraction of the batch (measured on B200, 65,536 problems: equal parts
 // 1.08 ms, 1/8 - 1/4 - 5/16 - 5/16 1.05 ms).
@@ -918,6 +1144,7 @@ static int solve_host(mpcb_handle h, int B, const double* x0, const double* obs_
                                 (unsigned long long)(size_t)h->pin, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
   for (int k = 3; k < 11; ++k) key[4] |= (unsigned long long)(up[k] != nullptr) << k;
   key[4] |= (unsigned long long)(wait ? 0 : 1) << 32;
+  key[4] |= (unsigned long long)h->fb_cap << 33;           // layout of the fb / cls / carry block
   if (!packed)
     for (int k = 0; k < 11; ++k) key[5 + k] = (unsigned long long)(size_t)up[k];
   const bool hit = g.valid && memcmp(g.key, key, sizeof(key)) == 0;
@@ -1163,6 +1390,17 @@ int mpcb_debug_coop_profile(unsigned long long* sum8, unsigned long long* max8, 
     unsigned long long z[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     CK(cudaMemcpyToSymbol(g_coop_sum, z, 64));
     CK(cudaMemcpyToSymbol(g_coop_max, z, 64));
+  }
+  return MPCB_OK;
+}
+#endif
+
+#ifdef MPCB_ROUND_STATS
+int mpcb_debug_round_counts(unsigned long long* counts48, int reset) {
+  if (counts48) CK(cudaMemcpyFromSymbol(counts48, g_round_stats, sizeof(unsigned long long) * 48));
+  if (reset) {
+    unsigned long long z[48] = {0};
+    CK(cudaMemcpyToSymbol(g_round_stats, z, sizeof(z)));
   }
   return MPCB_OK;
 }

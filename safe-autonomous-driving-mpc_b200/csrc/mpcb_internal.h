@@ -33,6 +33,7 @@ struct mpcb_ctx {
   int* fb = nullptr;          // work list(s): header (count, two cursors, pad), then indices of problems left to the second pass
   int fb_cap = 0;
   int* cls = nullptr;         // class lists of the first pass (problems by obstacle count), 3x the size of fb
+  char* carry = nullptr;      // survivor lists of the first pass and the state they carry between rounds (ensure_fb)
   cudaStream_t stream = nullptr;   // private stream of the *_host entry points
   cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_mid = nullptr;
   cudaStream_t xs[4] = {nullptr, nullptr, nullptr, nullptr};   // xs[0] == stream; one stream per part of a large host batch

@@ -707,12 +707,23 @@ MPCB_HD bool prologue(const DevTable& T, const DevParams& P, Problem& pb, const 
 // previous time step's solution shifted by one step; rows that sit on their bounds there start as active, so the first
 // segment is already a KKT solve on that active set (a vehicle waiting at a red light poses the same problem at every
 // step: certified in one or two rounds instead of being left to the robust pass every time).
+// The solve is cut into three pieces so that a kernel can stop a problem between two Gauss-Newton rounds, park what
+// crosses the round boundary (SolveState, pb.U / x / act_prev / hint, v and the prologue's bounds in the store) and go on
+// in another CTA; solve_one is their composition, which the host build, the robust pass and the evaluation kernel run.
+struct SolveState {
+  SolveOut out;
+  bool done, infeasible, first, hot;
+  int fails;
+  double step_prev;
+};
+
+// start: prologue (screens, warm start), hot start, loop scalars
 template <bool FIRST_PASS, class ST>
-MPCB_HD SolveOut solve_one(const DevTable& T, const DevParams& P, Problem& pb, const ST& st, bool live,
-                           const double* U_start = nullptr) {
-  SolveOut out{MPCB_MAXITER, 0, 0, false};
+MPCB_HD void solve_start(const DevTable& T, const DevParams& P, Problem& pb, const ST& st, bool live,
+                         const double* U_start, SolveState& s) {
+  s.out = SolveOut{MPCB_MAXITER, 0, 0, false};
   const bool screened = prologue(T, P, pb, st);
-  const bool hot = FIRST_PASS && U_start != nullptr;
+  s.hot = FIRST_PASS && U_start != nullptr;
   if (U_start) {
 #pragma unroll
     for (int i = 0; i < NV; ++i) {
@@ -720,15 +731,21 @@ MPCB_HD SolveOut solve_one(const DevTable& T, const DevParams& P, Problem& pb, c
       pb.U[i] = (i & 1) ? clipd(u, st.blo[i >> 1], st.bhi[i >> 1]) : u;
     }
   }
-  bool done = !live;
-  bool infeasible = screened;
-  out.const_infeasible = screened;
-  bool first = true;
+  s.done = !live;
+  s.infeasible = screened;
+  s.out.const_infeasible = screened;
+  s.first = true;
+  s.step_prev = 1e30;
+  s.fails = 0;
+}
+
+// one Gauss-Newton round: linearise (cold ADMM start on the first), segments, step test.  Every thread of the CTA calls it
+// (the segment votes are CTA-uniform); a thread whose problem is done only takes part in the votes.
+template <bool FIRST_PASS, class ST>
+MPCB_HD void solve_round(const DevTable& T, const DevParams& P, Problem& pb, const ST& st, SolveState& s, int round) {
   const Policy& pl = P.pol[FIRST_PASS ? 1 : 0];
-  double step_prev = 1e30;
-  int fails = 0;
-  const int max_rounds = FIRST_PASS ? P.thread_max_rounds : P.max_rounds;
   const int max_segments = FIRST_PASS ? P.thread_max_segments : pl.max_segments;
+  const bool hot = s.hot;
   // cold ADMM state at x: z = clip(A x), y = 0  ->  v = z ; all rows on the initial rung of policy m
   auto cold_start = [&](const double (&xx)[NV]) {
 #pragma unroll
@@ -746,72 +763,99 @@ MPCB_HD SolveOut solve_one(const DevTable& T, const DevParams& P, Problem& pb, c
     });
     pb.act_prev = act0;
   };
-  for (int round = 0; round < max_rounds; ++round) {
-    if (MPCB_ALL(done)) break;
-    if (!done) {
-      double cviol;
-      linearise(T, P, pb, st, cviol);
-      if (first) {
-        cold_start(pb.U);
+  if (!s.done) {
+    double cviol;
+    linearise(T, P, pb, st, cviol);
+    if (s.first) {
+      cold_start(pb.U);
 #pragma unroll
-        for (int i = 0; i < NV; ++i) pb.x[i] = pb.U[i];
-        first = false;
-      }
-      if (cviol > P.feas_tol) { infeasible = true; out.const_infeasible = true; }
-      out.rounds++;
+      for (int i = 0; i < NV; ++i) pb.x[i] = pb.U[i];
+      s.first = false;
     }
-    // inexact Gauss-Newton: a round's QP is only solved as accurately as the previous SQP step warrants
-    const double loosen = (FIRST_PASS || P.qp_forcing <= 0.0) ? 1.0
-                          : dmax(1.0, (step_prev * P.qp_forcing < P.qp_eps_loose ? step_prev * P.qp_forcing : P.qp_eps_loose) / P.eps_p);
-    const double eps_p = P.eps_p * loosen, eps_d = P.eps_d * loosen;
-    bool conv = false;                           // this round's QP closed
-    bool qdone = done;                           // nothing more to do on this round's QP (closed, certified or caps hit)
-    bool cert = false;
-    for (int seg = 0; seg < max_segments; ++seg) {
-      if (MPCB_ALL(qdone)) break;
-      if (!qdone) {
-        factor<FIRST_PASS>(P, pl, pb, st);
-        SegStats s;
-        for (int it = 0; it < pl.segment_iters - 1; ++it) admm_iter<false, false, FIRST_PASS>(P, pl, pb, st, s);
-        admm_iter<true, !FIRST_PASS, FIRST_PASS>(P, pl, pb, st, s, eps_p);
-        out.iters += pl.segment_iters;
+    if (cviol > P.feas_tol) { s.infeasible = true; s.out.const_infeasible = true; }
+    s.out.rounds++;
+  }
+  // inexact Gauss-Newton: a round's QP is only solved as accurately as the previous SQP step warrants
+  const double step_prev = s.step_prev;
+  const double loosen = (FIRST_PASS || P.qp_forcing <= 0.0) ? 1.0
+                        : dmax(1.0, (step_prev * P.qp_forcing < P.qp_eps_loose ? step_prev * P.qp_forcing : P.qp_eps_loose) / P.eps_p);
+  const double eps_p = P.eps_p * loosen, eps_d = P.eps_d * loosen;
+  bool conv = false;                           // this round's QP closed
+  bool qdone = s.done;                         // nothing more to do on this round's QP (closed, certified or caps hit)
+  bool cert = false;
+  for (int seg = 0; seg < max_segments; ++seg) {
+    if (MPCB_ALL(qdone)) break;
+    if (!qdone) {
+      factor<FIRST_PASS>(P, pl, pb, st);
+      SegStats ss;
+      for (int it = 0; it < pl.segment_iters - 1; ++it) admm_iter<false, false, FIRST_PASS>(P, pl, pb, st, ss);
+      admm_iter<true, !FIRST_PASS, FIRST_PASS>(P, pl, pb, st, ss, eps_p);
+      s.out.iters += pl.segment_iters;
 #ifdef MPCB_TRACE
-        if (getenv("MPCB_TRACE")) {
-          printf("  r%d s%d pass %d rp %.2e rd %.2e nd %.2e act %011llx E", round, seg, FIRST_PASS ? 1 : 2, s.rp, s.rd, s.nd, pb.act_prev);
-          for (int r = 0; r < M_ROWS; ++r) printf("%d", pb.E.get(r));
-          printf(" x");
-          for (int i = 0; i < NV; ++i) printf(" %.4f", pb.x[i]);
-          printf("\n");
-        }
+      if (getenv("MPCB_TRACE")) {
+        printf("  r%d s%d pass %d rp %.2e rd %.2e nd %.2e act %011llx E", round, seg, FIRST_PASS ? 1 : 2, ss.rp, ss.rd, ss.nd, pb.act_prev);
+        for (int r = 0; r < M_ROWS; ++r) printf("%d", pb.E.get(r));
+        printf(" x");
+        for (int i = 0; i < NV; ++i) printf(" %.4f", pb.x[i]);
+        printf("\n");
+      }
 #endif
-        if (s.rp <= eps_p && s.rd <= eps_d) { conv = true; qdone = true; }
-        else if (!FIRST_PASS && s.nd > 1e-9 && s.atdy <= P.eps_inf * s.nd && s.sup < -P.eps_inf * s.nd &&
-                 s.bad <= P.eps_inf * s.nd) { conv = true; cert = true; qdone = true; }
-      }
-    }
-    if (!done) {
-      double step = 0.0;
-#pragma unroll
-      for (int i = 0; i < NV; ++i) { step = dmax(step, fabs(pb.x[i] - pb.U[i])); pb.U[i] = pb.x[i]; }
-      step_prev = step;
-      if (cert) { infeasible = true; done = true; }
-      else if (conv && step < P.step_tol) { done = true; out.status = 0; }
-      else if (!conv) {
-        // first pass: a QP it cannot close goes to the robust pass (after fast_fail_rounds tolerated ones);
-        // robust pass: QPs that never close end as status 1, or 2 through the final constraint check
-        ++fails;
-        if (FIRST_PASS ? fails > P.fast_fail_rounds : fails >= P.max_fail_rounds) done = true;
-      }
+      if (ss.rp <= eps_p && ss.rd <= eps_d) { conv = true; qdone = true; }
+      else if (!FIRST_PASS && ss.nd > 1e-9 && ss.atdy <= P.eps_inf * ss.nd && ss.sup < -P.eps_inf * ss.nd &&
+               ss.bad <= P.eps_inf * ss.nd) { conv = true; cert = true; qdone = true; }
     }
   }
+  (void)round;
+  if (!s.done) {
+    double step = 0.0;
+#pragma unroll
+    for (int i = 0; i < NV; ++i) { step = dmax(step, fabs(pb.x[i] - pb.U[i])); pb.U[i] = pb.x[i]; }
+    s.step_prev = step;
+    if (cert) { s.infeasible = true; s.done = true; }
+    else if (conv && step < P.step_tol) { s.done = true; s.out.status = 0; }
+    else if (!conv) {
+      // first pass: a QP it cannot close goes to the robust pass (after fast_fail_rounds tolerated ones);
+      // robust pass: QPs that never close end as status 1, or 2 through the final constraint check
+      ++s.fails;
+      if (FIRST_PASS ? s.fails > P.fast_fail_rounds : s.fails >= P.max_fail_rounds) s.done = true;
+    }
+  }
+}
+
+// end: the infeasibility verdict and the box clip of the returned controls
+template <bool FIRST_PASS>
+MPCB_HD SolveOut solve_end(const DevParams& P, Problem& pb, const SolveState& s) {
+  SolveOut out = s.out;
   // an infeasibility verdict is final only on a point the pass actually converged to (or, in the robust pass, gave
   // up on): a first pass that could not close its QP hands the problem over whatever the screens said
-  if (infeasible && (!FIRST_PASS || out.status == 0)) out.status = 2;
+  if (s.infeasible && (!FIRST_PASS || out.status == 0)) out.status = 2;
   // the returned controls always respect the box (a no-op for converged problems; non-converged or infeasible
   // ADMM iterates may sit slightly outside).  SLSQP treats the bounds as hard in the same way.
 #pragma unroll
   for (int i = 0; i < NV; ++i) pb.U[i] = clipd(pb.U[i], P.umin[i & 1], P.umax[i & 1]);
   return out;
+}
+
+// FIRST_PASS = true : two-level policy only; a QP it cannot close ends the attempt (status MPCB_MAXITER = "not
+//                      certified"), no infeasibility verdict other than the rigorous screens.
+// FIRST_PASS = false: robust ladder with OSQP's infeasibility certificate; inexact Gauss-Newton: the QP of a round is
+//                      solved only as accurately as the previous SQP step warrants (P.qp_forcing).
+// U_start (optional): controls to start from instead of the reference's warm start (clipped to the box and to the
+// screen's pins like any start).  First pass: a HOT start -- the plan of a neighbouring problem, in the closed loop the
+// previous time step's solution shifted by one step; rows that sit on their bounds there start as active, so the first
+// segment is already a KKT solve on that active set (a vehicle waiting at a red light poses the same problem at every
+// step: certified in one or two rounds instead of being left to the robust pass every time).
+template <bool FIRST_PASS, class ST>
+MPCB_HD SolveOut solve_one(const DevTable& T, const DevParams& P, Problem& pb, const ST& st, bool live,
+                           const double* U_start = nullptr) {
+  SolveState s;
+  solve_start<FIRST_PASS>(T, P, pb, st, live, U_start, s);
+  const int max_rounds = FIRST_PASS ? P.thread_max_rounds : P.max_rounds;
+  for (int round = 0; round < max_rounds; ++round) {
+    if (MPCB_ALL(s.done)) break;
+    solve_round<FIRST_PASS>(T, P, pb, st, s, round);
+  }
+  return solve_end<FIRST_PASS>(P, pb, s);
 }
 
 }  // namespace mpcb
