@@ -34,6 +34,9 @@ typedef enum mpcb_status {
 #define MPCB_SOLVED 0       /* SQP step and QP residuals under tolerance, all constraints satisfied */
 #define MPCB_MAXITER 1      /* iteration caps hit; returned point satisfies the constraints to feas_tol */
 #define MPCB_INFEASIBLE 2   /* infeasibility certificate, or returned point violates a constraint > feas_tol */
+#define MPCB_BAD_ROUTE 3    /* routed solve: the problem's route is outside [0, n_routes); not solved */
+
+#define MPCB_MAX_ROUTES 16  /* reference-signal tables one handle can hold (mpcb_create_routes) */
 
 /* Mirrors the attributes of TrajectoryTracker.__init__ (trajectory_tracking.py:12-47) one to one, followed by
  * the solver controls of this implementation.  Fill with mpcb_default_params() first. */
@@ -113,6 +116,15 @@ int mpcb_table_raw(mpcb_table_handle t, double* ref_X, double* ref_U);   /* copi
 int mpcb_create(mpcb_handle* out, const mpcb_params* p, mpcb_table_handle t, int device);
 int mpcb_destroy(mpcb_handle h);
 
+/* Solver context over several routes: tables[0 .. n_routes-1] (1 <= n_routes <= MPCB_MAX_ROUTES, none NULL; checked
+ * before any CUDA call).  Route r of a routed call (mpcb_solve_batch_routes, mpcb_sim_create_routes) is tables[r].
+ * mpcb_create(out, p, t, device) is mpcb_create_routes(out, p, &t, 1, device).
+ * Every entry point without a route argument -- mpcb_solve_batch, the host-buffer and asynchronous entry points,
+ * mpcb_eval_batch, the planner evaluators (mpcb_hs_*), mpcb_sim_create, mpcb_check_histories -- behaves on a multi-route
+ * handle exactly as on a single-route handle of tables[0]: every problem or vehicle is on route 0. */
+int mpcb_create_routes(mpcb_handle* out, const mpcb_params* p, const mpcb_table_handle* tables, int n_routes, int device);
+int mpcb_n_routes(mpcb_handle h);   /* number of routes of the handle (1 for mpcb_create) */
+
 /* Solve B independent problems.  DEVICE pointers; asynchronous on `cuda_stream` (a cudaStream_t, may be 0).
  *   x0      [B][5]             current states [s,d,o,k,v]
  *   obs_sv  [B][MAX_OBS][2]    (s, v) per obstacle, first n_obs[b] entries used
@@ -129,6 +141,14 @@ int mpcb_destroy(mpcb_handle h);
 int mpcb_solve_batch(mpcb_handle h, int B, const double* x0, const double* obs_sv, const int* n_obs,
                      double* U_out, double* Xpred_out, double* obj_out, int* status_out, int* iters_out,
                      double* cmin_out, unsigned long long* active_out, void* cuda_stream);
+
+/* mpcb_solve_batch over several routes: problem b follows route[b] (DEVICE [B]; NULL: route 0 for every problem, bitwise
+ * identical to mpcb_solve_batch).  A problem's answer depends only on its own inputs and route, not on the routes of
+ * the other problems of the batch.  A problem whose route is outside [0, n_routes) is not solved and reads no table:
+ * status MPCB_BAD_ROUTE, U, Xpred, obj and cmin NaN, iters and active 0. */
+int mpcb_solve_batch_routes(mpcb_handle h, int B, const double* x0, const double* obs_sv, const int* n_obs,
+                            const int* route, double* U_out, double* Xpred_out, double* obj_out, int* status_out,
+                            int* iters_out, double* cmin_out, unsigned long long* active_out, void* cuda_stream);
 
 /* Same, with HOST buffers: copies inputs to the device, solves, copies results back and synchronises.
  * Pinned buffers (mpcb_host_alloc) make the copies asynchronous DMA. */
@@ -250,6 +270,10 @@ int mpcb_scenario_default(mpcb_scenario* s, int which);
  * or NULL for the reference's start [0,0,0,0,0.5] (:382).  history_steps > 0 records that many steps on the device. */
 int mpcb_sim_create(mpcb_sim_handle* out, mpcb_handle h, int B, const mpcb_scenario* scen, int n_scen,
                     const double* x_init, int history_steps);
+/* Same, vehicle b driving route[b] (HOST [B], each in [0, mpcb_n_routes(h)), else MPCB_ERR_INVALID; NULL: route 0):
+ * its reference signal, its end-of-route test s <= s_max - 1 and the s_max of its mpcb_sim_check verdict are its route's. */
+int mpcb_sim_create_routes(mpcb_sim_handle* out, mpcb_handle h, int B, const mpcb_scenario* scen, int n_scen,
+                           const int* route, const double* x_init, int history_steps);
 int mpcb_sim_destroy(mpcb_sim_handle s);
 /* n_steps closed-loop steps, asynchronous on cuda_stream (3 + the solver's launches per step, no host round trip).
  * Vehicles that have passed s_max - 1 are frozen. */

@@ -76,6 +76,9 @@ SYMBOLS = {
     "mpcb_table_knots": (C.c_int, [C.c_void_p]),
     "mpcb_create": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(Params), C.c_void_p, C.c_int]),
     "mpcb_destroy": (C.c_int, [C.c_void_p]),
+    "mpcb_create_routes": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(Params), C.POINTER(C.c_void_p), C.c_int, C.c_int]),
+    "mpcb_n_routes": (C.c_int, [C.c_void_p]),
+    "mpcb_solve_batch_routes": (C.c_int, [C.c_void_p, C.c_int] + [C.c_void_p] * 11 + [C.c_void_p]),
     "mpcb_solve_batch": (C.c_int, [C.c_void_p, C.c_int] + [C.c_void_p] * 10 + [C.c_void_p]),
     "mpcb_solve_batch_host": (C.c_int, [C.c_void_p, C.c_int] + [C.c_void_p] * 10),
     "mpcb_solve_batch_host_u0": (C.c_int, [C.c_void_p, C.c_int] + [C.c_void_p] * 6),
@@ -98,6 +101,8 @@ SYMBOLS = {
     "mpcb_hs_nodes": (C.c_int, [C.c_void_p, C.POINTER(PlannerParams), C.c_int, C.c_int] + [C.c_void_p] * 9 + [C.c_void_p]),
     "mpcb_scenario_default": (C.c_int, [C.POINTER(Scenario), C.c_int]),
     "mpcb_sim_create": (C.c_int, [C.POINTER(C.c_void_p), C.c_void_p, C.c_int, C.POINTER(Scenario), C.c_int, C.c_void_p, C.c_int]),
+    "mpcb_sim_create_routes": (C.c_int, [C.POINTER(C.c_void_p), C.c_void_p, C.c_int, C.POINTER(Scenario), C.c_int, C.c_void_p,
+                                         C.c_void_p, C.c_int]),
     "mpcb_sim_destroy": (C.c_int, [C.c_void_p]),
     "mpcb_sim_step": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
     "mpcb_sim_set_hot_start": (C.c_int, [C.c_void_p, C.c_int]),

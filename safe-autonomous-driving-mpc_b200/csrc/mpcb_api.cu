@@ -53,7 +53,9 @@ template <> struct ClsCfg<2> { typedef Store<SOLVE_THREADS, MPCB_CLS_MASK2, 2> S
 constexpr int cmax3(int a, int b, int c) { return a > b ? (a > c ? a : c) : (b > c ? b : c); }
 constexpr size_t CLS_SMEM = sizeof(double) * SOLVE_THREADS * cmax3(ClsCfg<0>::St::SHARED, ClsCfg<1>::St::SHARED, ClsCfg<2>::St::SHARED);
 constexpr int CLS_HDR = 4;                // class-list header: three counts, pad; then three lists of B indices each
-constexpr int CARRY_HDR = 12;             // survivor lists of the first pass: three headers of 4 ints (counts of classes 0-2, pad)
+constexpr int CARRY_HDR_STRIDE = 3 * MPCB_MAX_ROUTES;   // survivor-list header: counts per (class, route), [k * nr + r]
+constexpr int CARRY_HDR = 3 * CARRY_HDR_STRIDE;         // survivor lists of the first pass: three headers
+constexpr int ROUTE_CNT = 3 * MPCB_MAX_ROUTES;          // routed first pass: part sizes per (class, route), then cursors
 constexpr int EVAL_THREADS = 128;
 
 // Device pointers of one solve call (mpcb_solve_batch's arguments), handed to the kernels as one block.
@@ -67,7 +69,24 @@ struct SolveIO {
   const double* U_start;  // optional [B][10]: hot start of the first pass (closed loop: the previous step's plans, shifted
   int shift_start;        // by one step when shift_start != 0); may alias U
   int n_total;          // problems in the batch the indices refer to (bounds of the work lists; asserted in checked builds)
+  const int* route;     // optional [B]: route of each problem (mpcb_solve_batch_routes); nullptr: route 0
 };
+
+// Outputs of a problem whose route is outside the handle's tables: not solved, nothing read from any table.
+__device__ __forceinline__ void write_bad_route(const SolveIO& io, int b) {
+  const double q = nan("");
+#pragma unroll
+  for (int i = 0; i < NV; ++i) io.U[(size_t)b * NV + i] = q;
+  if (io.u0) { io.u0[(size_t)b * 2] = q; io.u0[(size_t)b * 2 + 1] = q; }
+  if (io.Xpred)
+#pragma unroll
+    for (int i = 0; i < 30; ++i) io.Xpred[(size_t)b * 30 + i] = q;
+  if (io.obj) io.obj[b] = q;
+  if (io.status) io.status[b] = MPCB_BAD_ROUTE;
+  if (io.iters) { io.iters[2 * b] = 0; io.iters[2 * b + 1] = 0; }
+  if (io.cmin) io.cmin[b] = q;
+  if (io.active) io.active[b] = 0ull;
+}
 
 // Final evaluation at U* (predict, cost, constraint rows in the reference's order), flags, outputs.  In the first pass a
 // problem that is not certified is appended to the work list of the next pass instead (fb_list == nullptr: the caller
@@ -182,14 +201,18 @@ __device__ __forceinline__ bool finalize(const DevTable& T, const DevParams& P, 
 // ------------------------------------------------------------------------------------------------
 template <bool FIRST_PASS>
 __global__ void __launch_bounds__(SOLVE_THREADS, MPCB_SOLVE_CTAS)
-mpcb_solve_kernel(const __grid_constant__ DevTable T, const __grid_constant__ DevParams P, int B,
+mpcb_solve_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ DevParams P, int B,
                   const __grid_constant__ SolveIO io, int* __restrict__ fb_list, int* __restrict__ fb_count) {
   const int* __restrict__ idx = io.idx;
   const int n_work = idx ? min(*io.n_idx, B) : B;
   if ((int)(blockIdx.x * blockDim.x) >= n_work) return;          // CTA-uniform
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
-  const bool live = t < n_work;
-  const int b = live ? (idx ? idx[t] : t) : 0;
+  const int b = t < n_work ? (idx ? idx[t] : t) : 0;
+  const int r = t < n_work ? problem_route(io.route, b, Ts.n) : 0;   // per thread
+  if (t < n_work && r < 0) write_bad_route(io, b);
+  const bool live = t < n_work && r >= 0;
+  MPCB_ASSERT(!live || r < Ts.n);
+  const DevTable& T = Ts.t[live ? r : 0];
   Problem pb;
   if (live) {
 #pragma unroll
@@ -217,30 +240,44 @@ mpcb_solve_kernel(const __grid_constant__ DevTable T, const __grid_constant__ De
 // -- the classes with more rows first, so that the longest CTAs start first -- and runs the instantiation of the solver
 // that has exactly that many obstacle slots.  A problem's answer does not depend on which CTA it lands in.
 // ------------------------------------------------------------------------------------------------
+// Slot of this thread in list `key` (warp-aggregated append to counters[key]; every lane of the warp calls it), -1 if
+// key < 0.
+__device__ __forceinline__ int warp_append_key(int key, int* counters) {
+  const unsigned m = __match_any_sync(0xffffffffu, key);
+  const unsigned lane = threadIdx.x & 31u;
+  const int leader = __ffs(m) - 1;
+  int base = 0;
+  if ((int)lane == leader && key >= 0) base = atomicAdd(counters + key, __popc(m));
+  base = __shfl_sync(0xffffffffu, base, leader);
+  return key >= 0 ? base + __popc(m & ((1u << lane) - 1u)) : -1;
+}
+
+// A routed call (nr = the handle's routes) partitions by (class, route), so that every CTA of the first pass runs on
+// one table: a count pass (cls == nullptr) counts the parts into cursor[k * nr + r]; the listing pass then appends each
+// problem to its part, which starts at the sum of the sizes pcnt of the class's earlier routes.  A single-route call
+// (nr = 1, pcnt == nullptr) lists straight into the class lists, its cursors the class-list header.  Problems whose
+// route is bad are written out here and listed nowhere.
 __global__ void __launch_bounds__(256)
-mpcb_classify_kernel(int B, const int* __restrict__ idx, const int* __restrict__ n_idx, const int* __restrict__ n_obs,
-                     int* __restrict__ cls, int* __restrict__ carry_hdr) {
-  if (blockIdx.x == 0 && threadIdx.x < CARRY_HDR) carry_hdr[threadIdx.x] = 0;   // survivor lists of the first pass
-  const int n_work = idx ? min(*n_idx, B) : B;
+mpcb_classify_kernel(int B, const __grid_constant__ SolveIO io, int n_routes, int nr, const int* __restrict__ pcnt,
+                     int* __restrict__ cursor, int* __restrict__ cls, int* __restrict__ carry_hdr) {
+  if (cls && blockIdx.x == 0)                                   // survivor lists of the first pass
+    for (int i = threadIdx.x; i < CARRY_HDR; i += blockDim.x) carry_hdr[i] = 0;
+  const int n_work = io.idx ? min(*io.n_idx, B) : B;
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
   const bool live = t < n_work;
-  const int b = live ? (idx ? idx[t] : t) : 0;
-  const int c = live ? min(max(n_obs[b], 0), 2) : -1;
-  const unsigned lane = threadIdx.x & 31u;
-#pragma unroll
-  for (int k = 0; k < 3; ++k) {
-    const unsigned m = __ballot_sync(0xffffffffu, c == k);
-    if (m == 0u) continue;
-    int base = 0;
-    const int leader = __ffs(m) - 1;
-    if ((int)lane == leader) base = atomicAdd(cls + k, __popc(m));
-    base = __shfl_sync(0xffffffffu, base, leader);
-    if (c == k) {
-      const int slot = base + __popc(m & ((1u << lane) - 1u));
-      MPCB_ASSERT(slot >= 0 && slot < B && b >= 0 && b < B);
-      cls[CLS_HDR + (size_t)k * B + slot] = b;
-    }
-  }
+  const int b = live ? (io.idx ? io.idx[t] : t) : 0;
+  const int r = live ? problem_route(io.route, b, n_routes) : -1;
+  if (cls && live && r < 0) write_bad_route(io, b);
+  const int k = min(max(io.n_obs[b], 0), 2);
+  const int key = r >= 0 ? k * nr + r : -1;
+  MPCB_ASSERT(r < nr);
+  const int slot = warp_append_key(key, cursor);
+  if (!cls || key < 0) return;
+  int off = 0;
+  if (pcnt)
+    for (int q = 0; q < r; ++q) off += pcnt[k * nr + q];
+  MPCB_ASSERT(slot >= 0 && (!pcnt || slot < pcnt[key]) && off + slot < B && b >= 0 && b < B);
+  cls[CLS_HDR + (size_t)k * B + off + slot] = b;
 }
 
 // hot start of problem b: the stored plan, optionally advanced by one step (the last step is repeated)
@@ -270,8 +307,9 @@ __device__ __forceinline__ void load_hot_start(const SolveIO& io, int b, double 
 constexpr int CLS_ROUNDS = MPCB_CLS_ROUNDS;   // rounds of the class kernel (the rest: one round kernel per round)
 
 // One carry workspace: slot-major arrays (field f of slot s at [f * cap + s], so the loads of a CTA's consecutive slots
-// coalesce).  A list of survivors is a header of per-class counts; class k's survivors occupy the slots from the class-k
-// offset of the batch's class partition on (classes with more rows first: class 2 at 0, class 1 at n2, class 0 at n2 + n1).
+// coalesce).  A list of survivors is a header of counts per (class, route) part; a part's survivors occupy the slots from
+// that part's offset in the batch's partition on (find_part: classes with more rows first, routes in order within a class;
+// single route: class 2 at 0, class 1 at n2, class 0 at n2 + n1).
 enum : int { CD_U = 0, CD_X = CD_U + NV, CD_V = CD_X + NV, CD_LOV = CD_V + ROW_OBS + 2 * N_OBSROW, CD_BLO = CD_LOV + NH,
              CD_BHI = CD_BLO + NH, CD_HIO = CD_BHI + NH, N_CD = CD_HIO + 2 * N_OBSROW };
 enum : int { CI_B = 0, CI_HINT = 1, CI_FAILS = CI_HINT + NH + 1, CI_ROUNDS, CI_ITERS, CI_STATUS, CI_FLAGS, N_CI };
@@ -299,6 +337,27 @@ __device__ __forceinline__ int warp_append(bool pred, int* counter) {
   if ((int)lane == leader) base = atomicAdd(counter, __popc(m));
   base = __shfl_sync(0xffffffffu, base, leader);
   return pred ? base + __popc(m & ((1u << lane) - 1u)) : -1;
+}
+
+// The part of a first-pass list that CTA blk works on, 128 problems per CTA.  Parts are (class, route) pairs, classes
+// with more rows first and routes in order within a class; cnt[k * nr + r] are the sizes that assign CTAs, base[.] the
+// sizes of the batch's partition, which fix where each part starts: off_cls in its class list, off in a survivor list.
+struct Part { int k, r, key, n, t0, off_cls, off; };
+__device__ __forceinline__ bool find_part(const int* __restrict__ cnt, const int* __restrict__ base, int nr, int blk, Part& p) {
+  int off = 0;
+#pragma unroll
+  for (int k = 2; k >= 0; --k) {
+    int off_cls = 0;
+    for (int r = 0; r < nr; ++r) {
+      const int key = k * nr + r, n = cnt[key];
+      const int c = (n + SOLVE_THREADS - 1) / SOLVE_THREADS;
+      if (blk < c) { p = Part{k, r, key, n, blk * SOLVE_THREADS, off_cls, off}; return true; }
+      blk -= c;
+      off += base[key];
+      off_cls += base[key];
+    }
+  }
+  return false;
 }
 
 // What crosses a round boundary of the first pass: the iterate, the ADMM state v and the active set, the table hints, the
@@ -383,7 +442,7 @@ __device__ __forceinline__ void park_or_finalize(const DevTable& T, const DevPar
                                                  int b, Problem& pb, const ST& st, SolveState& s, int n_work,
                                                  const Carry& cout, int* __restrict__ cnt_out, int off,
                                                  int* __restrict__ fb_list, int* __restrict__ fb_count) {
-  const int k = warp_append(cont, cnt_out + NOBS);
+  const int k = warp_append(cont, cnt_out);
   if (!live) return;
   if (cont) {
     MPCB_ASSERT(k >= 0 && k < n_work);             // a list never outgrows the one it was compacted from
@@ -422,26 +481,23 @@ __device__ __forceinline__ void solve_cls_body(const DevTable& T, const DevParam
                          off, fb_list, fb_count);
 }
 
-// class k's region of a list: classes with more rows first
-__device__ __forceinline__ int class_offset(const int* __restrict__ cls, int k) {
-  return k == 2 ? 0 : (k == 1 ? cls[2] : cls[2] + cls[1]);
-}
-
+// pcnt[k * nr + r]: sizes of the (class, route) parts of the class lists (nr = 1: the class-list header).  The part, and
+// with it the table, is CTA-uniform.  ROUTED = false (a single-route call, nr = 1) fixes the table at t[0] at compile
+// time: an indexed table costs the single-route first pass 1 % (see DESIGN.md 4, "Several routes on one handle").
+template <bool ROUTED>
 __global__ void __launch_bounds__(SOLVE_THREADS, MPCB_SOLVE_CTAS)
-mpcb_solve_cls_kernel(const __grid_constant__ DevTable T, const __grid_constant__ DevParams P, int B,
-                      const __grid_constant__ SolveIO io, const int* __restrict__ cls, int r0,
-                      const __grid_constant__ Carry cout, int* __restrict__ cnt_out, int* __restrict__ fb_list,
+mpcb_solve_cls_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ DevParams P, int B,
+                      const __grid_constant__ SolveIO io, const int* __restrict__ cls, const int* __restrict__ pcnt, int nr,
+                      int r0, const __grid_constant__ Carry cout, int* __restrict__ cnt_out, int* __restrict__ fb_list,
                       int* __restrict__ fb_count) {
-  const int n2 = cls[2], n1 = cls[1], n0 = cls[0];
-  const int c2 = (n2 + SOLVE_THREADS - 1) / SOLVE_THREADS, c1 = (n1 + SOLVE_THREADS - 1) / SOLVE_THREADS,
-            c0 = (n0 + SOLVE_THREADS - 1) / SOLVE_THREADS;
-  const int* lists = cls + CLS_HDR;
-  int blk = blockIdx.x;                                                       // CTA-uniform from here on
-  if (blk < c2) { solve_cls_body<2>(T, P, io, lists + (size_t)2 * B, n2, blk * SOLVE_THREADS, 0, r0, cout, cnt_out, fb_list, fb_count); return; }
-  blk -= c2;
-  if (blk < c1) { solve_cls_body<1>(T, P, io, lists + (size_t)1 * B, n1, blk * SOLVE_THREADS, n2, r0, cout, cnt_out, fb_list, fb_count); return; }
-  blk -= c1;
-  if (blk < c0) solve_cls_body<0>(T, P, io, lists, n0, blk * SOLVE_THREADS, n2 + n1, r0, cout, cnt_out, fb_list, fb_count);
+  Part p;
+  if (!find_part(pcnt, pcnt, ROUTED ? nr : 1, blockIdx.x, p)) return;       // CTA-uniform from here on
+  MPCB_ASSERT(p.r >= 0 && p.r < Ts.n && p.off_cls + p.n <= B);
+  const DevTable& T = Ts.t[ROUTED ? p.r : 0];
+  const int* list = cls + CLS_HDR + (size_t)p.k * B + p.off_cls;
+  if (p.k == 2) solve_cls_body<2>(T, P, io, list, p.n, p.t0, p.off, r0, cout, cnt_out + p.key, fb_list, fb_count);
+  else if (p.k == 1) solve_cls_body<1>(T, P, io, list, p.n, p.t0, p.off, r0, cout, cnt_out + p.key, fb_list, fb_count);
+  else solve_cls_body<0>(T, P, io, list, p.n, p.t0, p.off, r0, cout, cnt_out + p.key, fb_list, fb_count);
 }
 
 #ifdef MPCB_ROUND_STATS   // development: survivors per round and class, summed over calls (tools/gpu_round_counts.py)
@@ -478,25 +534,25 @@ __device__ __forceinline__ void solve_round_body(const DevTable& T, const DevPar
 // rows first; CTAs beyond the list's counts exit at once.  Survivors go to the next list (cout, cnt_out), the others are
 // finalized as in the class kernel -- after the last round all of them.  cnt_clear: the header the next round kernel
 // appends to (read by the previous one, which has finished), zeroed here.
+template <bool ROUTED>
 __global__ void __launch_bounds__(SOLVE_THREADS, MPCB_SOLVE_CTAS)
-mpcb_solve_round_kernel(const __grid_constant__ DevTable T, const __grid_constant__ DevParams P,
-                        const __grid_constant__ SolveIO io, const int* __restrict__ cls, const int* __restrict__ cnt_in,
-                        const __grid_constant__ Carry cin, int* __restrict__ cnt_out, const __grid_constant__ Carry cout,
-                        int* __restrict__ cnt_clear, int round, int* __restrict__ fb_list, int* __restrict__ fb_count) {
-  if (blockIdx.x == 0 && threadIdx.x < 3) cnt_clear[threadIdx.x] = 0;
-  const int n2 = cnt_in[2], n1 = cnt_in[1], n0 = cnt_in[0];
+mpcb_solve_round_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ DevParams P,
+                        const __grid_constant__ SolveIO io, const int* __restrict__ pcnt, int nr,
+                        const int* __restrict__ cnt_in, const __grid_constant__ Carry cin, int* __restrict__ cnt_out,
+                        const __grid_constant__ Carry cout, int* __restrict__ cnt_clear, int round,
+                        int* __restrict__ fb_list, int* __restrict__ fb_count) {
+  if (!ROUTED) nr = 1;
+  if (blockIdx.x == 0 && threadIdx.x < 3 * nr) cnt_clear[threadIdx.x] = 0;
 #ifdef MPCB_ROUND_STATS
-  if (blockIdx.x == 0 && threadIdx.x < 3 && round < 16) atomicAdd(&g_round_stats[3 * round + threadIdx.x], (unsigned long long)cnt_in[threadIdx.x]);
+  if (blockIdx.x == 0 && nr == 1 && threadIdx.x < 3 && round < 16) atomicAdd(&g_round_stats[3 * round + threadIdx.x], (unsigned long long)cnt_in[threadIdx.x]);
 #endif
-  MPCB_ASSERT(n2 >= 0 && n2 <= cls[2] && n1 >= 0 && n1 <= cls[1] && n0 >= 0 && n0 <= cls[0]);
-  const int c2 = (n2 + SOLVE_THREADS - 1) / SOLVE_THREADS, c1 = (n1 + SOLVE_THREADS - 1) / SOLVE_THREADS,
-            c0 = (n0 + SOLVE_THREADS - 1) / SOLVE_THREADS;
-  int blk = blockIdx.x;                                                       // CTA-uniform from here on
-  if (blk < c2) { solve_round_body<2>(T, P, io, n2, blk * SOLVE_THREADS, class_offset(cls, 2), cin, cout, cnt_out, round, fb_list, fb_count); return; }
-  blk -= c2;
-  if (blk < c1) { solve_round_body<1>(T, P, io, n1, blk * SOLVE_THREADS, class_offset(cls, 1), cin, cout, cnt_out, round, fb_list, fb_count); return; }
-  blk -= c1;
-  if (blk < c0) solve_round_body<0>(T, P, io, n0, blk * SOLVE_THREADS, class_offset(cls, 0), cin, cout, cnt_out, round, fb_list, fb_count);
+  Part p;
+  if (!find_part(cnt_in, pcnt, nr, blockIdx.x, p)) return;                  // CTA-uniform from here on
+  MPCB_ASSERT(p.n >= 0 && p.n <= pcnt[p.key] && p.r >= 0 && p.r < Ts.n);
+  const DevTable& T = Ts.t[ROUTED ? p.r : 0];
+  if (p.k == 2) solve_round_body<2>(T, P, io, p.n, p.t0, p.off, cin, cout, cnt_out + p.key, round, fb_list, fb_count);
+  else if (p.k == 1) solve_round_body<1>(T, P, io, p.n, p.t0, p.off, cin, cout, cnt_out + p.key, round, fb_list, fb_count);
+  else solve_round_body<0>(T, P, io, p.n, p.t0, p.off, cin, cout, cnt_out + p.key, round, fb_list, fb_count);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -514,7 +570,7 @@ constexpr size_t COOP_SMEM = sizeof(WarpShared) * COOP_WARPS;
 
 template <bool FIRST_PASS>
 __global__ void __launch_bounds__(COOP_WARPS * 32, COOP_CTAS)
-mpcb_coop_kernel(const __grid_constant__ DevTable T, const __grid_constant__ DevParams P, int B,
+mpcb_coop_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ DevParams P, int B,
                  const __grid_constant__ SolveIO io, int* __restrict__ fb_list, int* __restrict__ fb_count,
                  int* __restrict__ cursor) {
   extern __shared__ double coop_smem[];
@@ -529,6 +585,13 @@ mpcb_coop_kernel(const __grid_constant__ DevTable T, const __grid_constant__ Dev
     if (t >= n_work) break;
     const int b = idx ? idx[t] : t;
     MPCB_ASSERT(b >= 0 && b < B);
+    const int r = problem_route(io.route, b, Ts.n);                // warp-uniform
+    if (r < 0) {
+      if (lane == 0) write_bad_route(io, b);
+      continue;
+    }
+    MPCB_ASSERT(r < Ts.n);
+    const DevTable& T = Ts.t[r];
     __syncwarp();
     if (lane < 5) ws.pb.x0[lane] = io.x0[(size_t)b * 5 + lane];
     if (lane < 4) ws.pb.obs[lane >> 1][lane & 1] = io.obs_sv[(size_t)b * 4 + lane];
@@ -797,8 +860,53 @@ int mpcb_table_raw(mpcb_table_handle t, double* ref_X, double* ref_U) {
   return MPCB_OK;
 }
 
+// Upload one host table to the device: knots, rows, controls, the bucket index and the reciprocal segment lengths.
+// The arrays become owned by the caller's DevTable (freed by free_table) even when a later step fails.
+static int upload_table(mpcb_table_handle t, DevTable& dt) {
+  const int K = t->K, Ku = t->Ku;
+  auto up = [](void** dst, const void* src, size_t bytes) -> int {
+    if (cudaMalloc(dst, bytes) != cudaSuccess) return cuda_fail(cudaGetLastError(), "cudaMalloc");
+    const cudaError_t e = cudaMemcpy(*dst, src, bytes, cudaMemcpyHostToDevice);
+    return e == cudaSuccess ? MPCB_OK : cuda_fail(e, "cudaMemcpy");
+  };
+  // bucket index for lookups that have no previous segment to start from (first probe of the warm start, planner)
+  const int n = 4096;
+  const double s0 = t->s[0], span = t->s[K - 1] - t->s[0];
+  std::vector<int> lut(n);
+  const double scale = span > 0 ? (double)n / span : 0.0;
+  for (int b = 0; b < n; ++b) {
+    const double edge = s0 + (scale > 0 ? (double)b / scale : 0.0);
+    const int lo = (int)(std::lower_bound(t->s.begin(), t->s.end(), edge) - t->s.begin());
+    lut[b] = std::min(std::max(lo, 1), K - 1);
+  }
+  std::vector<double> sinv(K, 0.0);
+  for (int i = 1; i < K; ++i) sinv[i] = 1.0 / (t->s[i] - t->s[i - 1]);
+  dt = DevTable{};
+  dt.K = K; dt.Ku = Ku; dt.s_max = t->s_max;
+  for (int k = 0; k < 4; ++k) dt.last[k] = t->last_row[1 + k];
+  dt.lut_n = n; dt.lut_s0 = s0; dt.lut_scale = scale;
+  int rc;
+  if ((rc = up((void**)&dt.s, t->s.data(), sizeof(double) * K)) != MPCB_OK) return rc;
+  if ((rc = up((void**)&dt.y, t->y.data(), sizeof(double) * K * 4)) != MPCB_OK) return rc;
+  if ((rc = up((void**)&dt.u, t->u.data(), sizeof(double) * Ku * 2)) != MPCB_OK) return rc;
+  if ((rc = up((void**)&dt.lut, lut.data(), sizeof(int) * n)) != MPCB_OK) return rc;
+  return up((void**)&dt.sinv, sinv.data(), sizeof(double) * K);
+}
+
+static void free_table(DevTable& dt) {
+  const void* p[5] = {dt.s, dt.y, dt.u, dt.lut, dt.sinv};
+  for (const void* q : p) if (q) cudaFree(const_cast<void*>(q));
+  dt = DevTable{};
+}
+
 int mpcb_create(mpcb_handle* out, const mpcb_params* p, mpcb_table_handle t, int device) {
-  if (!out || !p || !t) return MPCB_ERR_INVALID;
+  return mpcb_create_routes(out, p, &t, 1, device);
+}
+
+int mpcb_create_routes(mpcb_handle* out, const mpcb_params* p, const mpcb_table_handle* tables, int n_routes, int device) {
+  if (!out || !p || !tables || n_routes < 1 || n_routes > MPCB_MAX_ROUTES) return MPCB_ERR_INVALID;
+  for (int r = 0; r < n_routes; ++r)
+    if (!tables[r]) return MPCB_ERR_INVALID;
   *out = nullptr;
   DevParams dp;
   int rc = derive_params(*p, dp);
@@ -820,17 +928,12 @@ int mpcb_create(mpcb_handle* out, const mpcb_params* p, mpcb_table_handle t, int
   c->n_sm = prop.multiProcessorCount;
   c->params = *p;
   c->dp = dp;
-  const int K = t->K;
-  c->K = K;
-  c->Ku = t->Ku;
   auto fail = [&](int code) { mpcb_destroy(c); return code; };
-  if (cudaMalloc(&c->d_s, sizeof(double) * K) != cudaSuccess) return fail(cuda_fail(cudaGetLastError(), "cudaMalloc"));
-  if (cudaMalloc(&c->d_y, sizeof(double) * K * 4) != cudaSuccess) return fail(cuda_fail(cudaGetLastError(), "cudaMalloc"));
-  if (cudaMalloc(&c->d_u, sizeof(double) * c->Ku * 2) != cudaSuccess) return fail(cuda_fail(cudaGetLastError(), "cudaMalloc"));
+  for (int r = 0; r < n_routes; ++r) {
+    c->dt.n = r + 1;                                              // what mpcb_destroy frees
+    if ((rc = upload_table(tables[r], c->dt.t[r])) != MPCB_OK) return fail(rc);
+  }
   cudaError_t e;
-  if ((e = cudaMemcpy(c->d_s, t->s.data(), sizeof(double) * K, cudaMemcpyHostToDevice)) != cudaSuccess) return fail(cuda_fail(e, "cudaMemcpy"));
-  if ((e = cudaMemcpy(c->d_y, t->y.data(), sizeof(double) * K * 4, cudaMemcpyHostToDevice)) != cudaSuccess) return fail(cuda_fail(e, "cudaMemcpy"));
-  if ((e = cudaMemcpy(c->d_u, t->u.data(), sizeof(double) * c->Ku * 2, cudaMemcpyHostToDevice)) != cudaSuccess) return fail(cuda_fail(e, "cudaMemcpy"));
   // streams of the host-buffer entry point: part c of a large batch runs on xs[c] with a priority that falls with c,
   // so the parts drain in order and the D2H copy of one overlaps the kernels of the next
   int prio_lo = 0, prio_hi = 0;
@@ -840,8 +943,10 @@ int mpcb_create(mpcb_handle* out, const mpcb_params* p, mpcb_table_handle t, int
   if ((e = cudaEventCreate(&c->ev1)) != cudaSuccess) return fail(cuda_fail(e, "cudaEventCreate"));
   if ((e = cudaEventCreate(&c->ev_mid)) != cudaSuccess) return fail(cuda_fail(e, "cudaEventCreate"));
   if ((e = cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming)) != cudaSuccess) return fail(cuda_fail(e, "cudaEventCreate"));
-  if ((e = cudaFuncSetAttribute(mpcb_solve_cls_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
-      (e = cudaFuncSetAttribute(mpcb_solve_round_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
+  if ((e = cudaFuncSetAttribute(mpcb_solve_cls_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(mpcb_solve_cls_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(mpcb_solve_round_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(mpcb_solve_round_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
       (e = cudaFuncSetAttribute(mpcb_solve_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SOLVE_SMEM)) != cudaSuccess ||
       (e = cudaFuncSetAttribute(mpcb_coop_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)COOP_SMEM)) != cudaSuccess ||
       (e = cudaFuncSetAttribute(mpcb_coop_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)COOP_SMEM)) != cudaSuccess)
@@ -851,48 +956,23 @@ int mpcb_create(mpcb_handle* out, const mpcb_params* p, mpcb_table_handle t, int
     if ((e = cudaStreamCreateWithPriority(&c->xs[k], cudaStreamNonBlocking, std::min(prio_lo, prio_hi + k))) != cudaSuccess) return fail(cuda_fail(e, "cudaStreamCreate"));
     if ((e = cudaEventCreateWithFlags(&c->xe[k], cudaEventDisableTiming)) != cudaSuccess) return fail(cuda_fail(e, "cudaEventCreate"));
   }
-  c->dt.s = c->d_s; c->dt.y = c->d_y; c->dt.u = c->d_u;
-  c->dt.K = K; c->dt.Ku = c->Ku; c->dt.s_max = t->s_max;
-  {
-    // bucket index for lookups that have no previous segment to start from (first probe of the warm start, planner)
-    const int n = 4096;
-    const double s0 = t->s[0], span = t->s[K - 1] - t->s[0];
-    std::vector<int> lut(n);
-    const double scale = span > 0 ? (double)n / span : 0.0;
-    for (int b = 0; b < n; ++b) {
-      const double edge = s0 + (scale > 0 ? (double)b / scale : 0.0);
-      const int lo = (int)(std::lower_bound(t->s.begin(), t->s.end(), edge) - t->s.begin());
-      lut[b] = std::min(std::max(lo, 1), K - 1);
-    }
-    if (cudaMalloc(&c->d_lut, sizeof(int) * n) != cudaSuccess) return fail(cuda_fail(cudaGetLastError(), "cudaMalloc"));
-    if ((e = cudaMemcpy(c->d_lut, lut.data(), sizeof(int) * n, cudaMemcpyHostToDevice)) != cudaSuccess) return fail(cuda_fail(e, "cudaMemcpy"));
-    c->dt.lut = c->d_lut; c->dt.lut_n = n; c->dt.lut_s0 = s0; c->dt.lut_scale = scale;
-    std::vector<double> sinv(K, 0.0);
-    for (int i = 1; i < K; ++i) sinv[i] = 1.0 / (t->s[i] - t->s[i - 1]);
-    if (cudaMalloc(&c->d_sinv, sizeof(double) * K) != cudaSuccess) return fail(cuda_fail(cudaGetLastError(), "cudaMalloc"));
-    if ((e = cudaMemcpy(c->d_sinv, sinv.data(), sizeof(double) * K, cudaMemcpyHostToDevice)) != cudaSuccess) return fail(cuda_fail(e, "cudaMemcpy"));
-    c->dt.sinv = c->d_sinv;
-  }
-  for (int k = 0; k < 4; ++k) c->dt.last[k] = t->last_row[1 + k];
   *out = c;
   return MPCB_OK;
 }
 
+int mpcb_n_routes(mpcb_handle h) { return h ? h->dt.n : MPCB_ERR_INVALID; }
+
 int mpcb_destroy(mpcb_handle h) {
   if (!h) return MPCB_ERR_INVALID;
   cudaSetDevice(h->device);
-  if (h->d_s) cudaFree(h->d_s);
-  if (h->d_y) cudaFree(h->d_y);
-  if (h->d_u) cudaFree(h->d_u);
-  if (h->d_lut) cudaFree(h->d_lut);
-  if (h->d_sinv) cudaFree(h->d_sinv);
+  for (int r = 0; r < h->dt.n; ++r) free_table(h->dt.t[r]);
   for (int k = 0; k < 2; ++k) {
     if (h->gslot[k].exec) cudaGraphExecDestroy(h->gslot[k].exec);
     if (h->gslot[k].graph) cudaGraphDestroy(h->gslot[k].graph);
   }
   if (h->ev_fork) cudaEventDestroy(h->ev_fork);
   if (h->ws) cudaFree(h->ws);
-  if (h->fb) cudaFree(h->fb);                      // fb, cls and carry are one block
+  if (h->fb) cudaFree(h->fb);                      // fb, cls, carry and route_cnt are one block
   if (h->ev0) cudaEventDestroy(h->ev0);
   if (h->ev1) cudaEventDestroy(h->ev1);
   if (h->ev_mid) cudaEventDestroy(h->ev_mid);
@@ -917,17 +997,20 @@ static size_t al256(size_t x) { return (x + 255) & ~(size_t)255; }
 // fb, cls and carry are one allocation, so that h->fb (in the graph key) stands for all three.  A part whose work list
 // starts at fb + o keeps its class-list header and three lists at cls + 3 o, and its survivor-list headers and two carry
 // workspaces at carry + 2 o CARRY_SLOT_BYTES (FB_HDR == CLS_HDR, so the slices of the parts of a chunked host call do not
-// overlap; FB_HDR carry slots hold the headers).
+// overlap; FB_HDR carry slots hold the headers).  route_cnt, at the end, serves routed calls, which are never chunked.
+static_assert(sizeof(int) * CARRY_HDR <= FB_HDR * 2 * CARRY_SLOT_BYTES, "survivor-list headers outgrow their slots");
 static int ensure_fb(mpcb_handle h, int B) {
   if (!h->params.fast_pass || B + FB_HDR * HOST_CHUNKS <= h->fb_cap) return MPCB_OK;
-  if (h->fb) { CK(cudaFree(h->fb)); h->fb = nullptr; h->cls = nullptr; h->carry = nullptr; h->fb_cap = 0; }
+  if (h->fb) { CK(cudaFree(h->fb)); h->fb = nullptr; h->cls = nullptr; h->carry = nullptr; h->route_cnt = nullptr; h->fb_cap = 0; }
   const size_t cap = (size_t)B + FB_HDR * HOST_CHUNKS;
-  const size_t o_cls = al256(sizeof(int) * cap), o_carry = o_cls + al256(sizeof(int) * 3 * cap);
+  const size_t o_cls = al256(sizeof(int) * cap), o_carry = o_cls + al256(sizeof(int) * 3 * cap),
+               o_route = o_carry + al256(2 * cap * CARRY_SLOT_BYTES);
   void* p = nullptr;
-  if (cudaMalloc(&p, o_carry + 2 * cap * CARRY_SLOT_BYTES) != cudaSuccess) { cudaGetLastError(); return MPCB_ERR_NOMEM; }
+  if (cudaMalloc(&p, o_route + sizeof(int) * 2 * ROUTE_CNT) != cudaSuccess) { cudaGetLastError(); return MPCB_ERR_NOMEM; }
   h->fb = (int*)p;
   h->cls = (int*)((char*)p + o_cls);
   h->carry = (char*)p + o_carry;
+  h->route_cnt = (int*)((char*)p + o_route);
   h->fb_cap = (int)cap;
   return MPCB_OK;
 }
@@ -968,15 +1051,29 @@ static int launch_solve(mpcb_handle h, int B, const SolveIO& io_in, cudaStream_t
       const int g1 = std::min((B + COOP_WARPS - 1) / COOP_WARPS, h->n_sm * COOP_CTAS);
       mpcb_coop_kernel<true><<<g1, COOP_WARPS * 32, COOP_SMEM, st>>>(h->dt, h->dp, B, io, fb_list, fb_count, fb + 1);
     } else {
-      // partition by obstacle count, then one CTA per 128 problems of one class (at most two partly filled CTAs more
-      // than the unpartitioned grid)
+      // partition by obstacle count -- and route, in a routed call -- then one CTA per 128 problems of one part (at most
+      // one partly filled CTA per part more than the unpartitioned grid)
       int* cls = h->cls + (fb - h->fb) * 3;                    // this part's slice: header + three lists of B
       char* cw = h->carry + (size_t)(fb - h->fb) * 2 * CARRY_SLOT_BYTES;   // survivor-list headers, two workspaces of B
-      int* hdr = (int*)cw;                                     // headers: survivors after round r at hdr + 4 (r % 3)
+      int* hdr = (int*)cw;                                     // headers: survivors after round r at hdr + CARRY_HDR_STRIDE (r % 3)
       const size_t w0 = FB_HDR * 2 * CARRY_SLOT_BYTES;
       const Carry wk[2] = {Carry::at(cw + w0, B), Carry::at(cw + w0 + (size_t)B * CARRY_SLOT_BYTES, B)};
-      CK(cudaMemsetAsync(cls, 0, sizeof(int) * CLS_HDR, st));
-      mpcb_classify_kernel<<<(B + 255) / 256, 256, 0, st>>>(B, io.idx, io.n_idx, io.n_obs, cls, hdr);
+      const int n_routes = h->dt.n;
+      const int* pcnt = cls;                                   // part sizes: the class-list header ...
+      int nr = 1;
+      if (io.route) {                                          // ... or, routed, counted per (class, route) first
+        if (fb != h->fb) return MPCB_ERR_INVALID;              // (routed calls are never chunked)
+        pcnt = h->route_cnt;
+        nr = n_routes;
+        CK(cudaMemsetAsync(h->route_cnt, 0, sizeof(int) * 2 * ROUTE_CNT, st));
+        mpcb_classify_kernel<<<(B + 255) / 256, 256, 0, st>>>(B, io, n_routes, nr, nullptr, h->route_cnt, nullptr, hdr);
+        CK(cudaGetLastError());
+        h->launches++;
+        mpcb_classify_kernel<<<(B + 255) / 256, 256, 0, st>>>(B, io, n_routes, nr, pcnt, h->route_cnt + ROUTE_CNT, cls, hdr);
+      } else {
+        CK(cudaMemsetAsync(cls, 0, sizeof(int) * CLS_HDR, st));
+        mpcb_classify_kernel<<<(B + 255) / 256, 256, 0, st>>>(B, io, n_routes, 1, nullptr, cls, cls, hdr);
+      }
       CK(cudaGetLastError());
       SolveIO io1 = io;
       io1.idx = nullptr; io1.n_idx = nullptr;                  // the class lists carry the problem indices from here on
@@ -985,16 +1082,19 @@ static int launch_solve(mpcb_handle h, int B, const SolveIO& io_in, cudaStream_t
       const int max_rounds = h->dp.thread_max_rounds;
       const bool compact = grid > h->n_sm * MPCB_SOLVE_CTAS;
       const int r0 = compact ? std::min(CLS_ROUNDS, max_rounds) : max_rounds;
-      mpcb_solve_cls_kernel<<<grid + 2, SOLVE_THREADS, CLS_SMEM, st>>>(h->dt, h->dp, B, io1, cls, r0, wk[0],
-                                                                      hdr + 4 * (r0 % 3), fb_list, fb_count);
+      const int grid1 = grid + 3 * nr - 1;
+      const auto cls_kernel = io.route ? mpcb_solve_cls_kernel<true> : mpcb_solve_cls_kernel<false>;
+      const auto round_kernel = io.route ? mpcb_solve_round_kernel<true> : mpcb_solve_round_kernel<false>;
+      cls_kernel<<<grid1, SOLVE_THREADS, CLS_SMEM, st>>>(h->dt, h->dp, B, io1, cls, pcnt, nr, r0, wk[0],
+                                                         hdr + CARRY_HDR_STRIDE * (r0 % 3), fb_list, fb_count);
       h->launches++;
       // the rounds after r0 over the packed survivors, one launch per round (workspaces ping-pong; each kernel zeroes
       // the header its successor appends to)
       for (int r = r0; r < max_rounds; ++r) {
         const int p = (r - r0) & 1;
-        mpcb_solve_round_kernel<<<grid + 2, SOLVE_THREADS, CLS_SMEM, st>>>(h->dt, h->dp, io1, cls, hdr + 4 * (r % 3), wk[p],
-                                                                          hdr + 4 * ((r + 1) % 3), wk[p ^ 1],
-                                                                          hdr + 4 * ((r + 2) % 3), r, fb_list, fb_count);
+        round_kernel<<<grid1, SOLVE_THREADS, CLS_SMEM, st>>>(h->dt, h->dp, io1, pcnt, nr, hdr + CARRY_HDR_STRIDE * (r % 3), wk[p],
+                                                             hdr + CARRY_HDR_STRIDE * ((r + 1) % 3), wk[p ^ 1],
+                                                             hdr + CARRY_HDR_STRIDE * ((r + 2) % 3), r, fb_list, fb_count);
         h->launches++;
       }
     }
@@ -1040,29 +1140,40 @@ static SolveIO make_io(const double* x0, const double* obs_sv, const int* n_obs,
   io.x0 = x0; io.obs_sv = obs_sv; io.n_obs = n_obs; io.U = U_out; io.Xpred = Xpred_out; io.obj = obj_out;
   io.status = status_out; io.iters = iters_out; io.cmin = cmin_out; io.active = active_out; io.u0 = u0_out;
   io.idx = nullptr; io.n_idx = nullptr; io.accumulate = 0; io.n_total = 0; io.U_start = nullptr; io.shift_start = 0;
+  io.route = nullptr;
   return io;
 }
 
 int mpcb_solve_batch(mpcb_handle h, int B, const double* x0, const double* obs_sv, const int* n_obs, double* U_out,
                      double* Xpred_out, double* obj_out, int* status_out, int* iters_out, double* cmin_out,
                      unsigned long long* active_out, void* cuda_stream) {
+  return mpcb_solve_batch_routes(h, B, x0, obs_sv, n_obs, nullptr, U_out, Xpred_out, obj_out, status_out, iters_out,
+                                 cmin_out, active_out, cuda_stream);
+}
+
+int mpcb_solve_batch_routes(mpcb_handle h, int B, const double* x0, const double* obs_sv, const int* n_obs,
+                            const int* route, double* U_out, double* Xpred_out, double* obj_out, int* status_out,
+                            int* iters_out, double* cmin_out, unsigned long long* active_out, void* cuda_stream) {
   if (!h || B < 0 || (B > 0 && (!x0 || !obs_sv || !n_obs || !U_out))) return MPCB_ERR_INVALID;
   if ((((size_t)U_out) | ((size_t)Xpred_out)) & 15u) return MPCB_ERR_INVALID;      // rows are written with 128-bit stores
   if (B == 0) return MPCB_OK;
   CK(cudaSetDevice(h->device));
   int rc = ensure_fb(h, B);
   if (rc != MPCB_OK) return rc;
-  return launch_solve(h, B, make_io(x0, obs_sv, n_obs, U_out, Xpred_out, obj_out, status_out, iters_out, cmin_out, active_out),
-                      (cudaStream_t)cuda_stream, h->fb, true, call_uses_coop(h, B));
+  SolveIO io = make_io(x0, obs_sv, n_obs, U_out, Xpred_out, obj_out, status_out, iters_out, cmin_out, active_out);
+  io.route = route;
+  return launch_solve(h, B, io, (cudaStream_t)cuda_stream, h->fb, true, call_uses_coop(h, B));
 }
 
 // Solve the problems idx[0 .. *n_idx - 1] of a batch of B (both on the device; the closed loop's list of vehicles that
 // are still driving).  Outputs of the other problems are left untouched.
 int mpcb_solve_list_internal(mpcb_handle h, int B, const int* idx, const int* n_idx, const double* x0, const double* obs_sv,
-                             const int* n_obs, double* U_out, int* status_out, cudaStream_t st, const double* U_start) {
+                             const int* n_obs, const int* route, double* U_out, int* status_out, cudaStream_t st,
+                             const double* U_start) {
   int rc = ensure_fb(h, B);
   if (rc != MPCB_OK) return rc;
   SolveIO io = make_io(x0, obs_sv, n_obs, U_out, nullptr, nullptr, status_out, nullptr, nullptr, nullptr);
+  io.route = route;
   io.idx = idx;
   io.n_idx = n_idx;
   io.U_start = U_start;          // closed loop: the previous step's plans (U_out itself), advanced by one step
@@ -1319,7 +1430,7 @@ int mpcb_eval_batch(mpcb_handle h, int B, const double* x0, const double* U, con
   if (B == 0) return MPCB_OK;
   CK(cudaSetDevice(h->device));
   const int grid = (B + EVAL_THREADS - 1) / EVAL_THREADS;
-  mpcb_eval_kernel<<<grid, EVAL_THREADS, 0, (cudaStream_t)cuda_stream>>>(h->dt, h->dp, B, x0, U, obs_sv, n_obs,
+  mpcb_eval_kernel<<<grid, EVAL_THREADS, 0, (cudaStream_t)cuda_stream>>>(h->dt.t[0], h->dp, B, x0, U, obs_sv, n_obs,
                                                                        Xpred_out, cost_out, cons_out, Jr_out, warm_out);
   CK(cudaGetLastError());
   h->launches++;

@@ -66,6 +66,24 @@ struct DevTable {
   const double* sinv;
 };
 
+#ifndef MPCB_MAX_ROUTES
+#define MPCB_MAX_ROUTES 16   // include/mpcb200.h
+#endif
+// The tables of a handle, handed to the kernels as one grid-constant parameter: a problem on route r runs on t[r].
+struct DevTables {
+  DevTable t[MPCB_MAX_ROUTES];
+  int n;
+};
+static_assert(sizeof(DevTables) <= 2048, "DevTables must stay well inside the 4 KB a kernel's parameters may take");
+
+// Route of problem b: route[b] (route == nullptr: 0 for every problem), or -1 when route[b] is outside [0, n).  Every
+// kernel that reads a caller's route array goes through here, so no route from outside the library becomes a table index.
+MPCB_HD int problem_route(const int* __restrict__ route, int b, int n) {
+  if (!route) return 0;
+  const int r = route[b];
+  return (r >= 0 && r < n) ? r : -1;
+}
+
 // Step-size policy of the ADMM machinery (mpcb_solver.cuh).
 struct Policy {
   double lad[MAXRUNG];        // step-size ladder

@@ -20,13 +20,7 @@ struct mpcb_ctx {
   int n_sm = 148;
   mpcb_params params;
   mpcb::DevParams dp;
-  mpcb::DevTable dt;
-  int K, Ku;
-  double* d_s = nullptr;
-  double* d_y = nullptr;
-  double* d_u = nullptr;
-  int* d_lut = nullptr;
-  double* d_sinv = nullptr;
+  mpcb::DevTables dt = {};     // one table per route (mpcb_create_routes); dt.t[r]'s arrays are owned by the context
   // workspace for the host-buffer entry points
   void* ws = nullptr;
   size_t ws_bytes = 0;
@@ -34,6 +28,7 @@ struct mpcb_ctx {
   int fb_cap = 0;
   int* cls = nullptr;         // class lists of the first pass (problems by obstacle count), 3x the size of fb
   char* carry = nullptr;      // survivor lists of the first pass and the state they carry between rounds (ensure_fb)
+  int* route_cnt = nullptr;   // routed first pass: sizes of its (class, route) parts and their cursors (ensure_fb)
   cudaStream_t stream = nullptr;   // private stream of the *_host entry points
   cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_mid = nullptr;
   cudaStream_t xs[4] = {nullptr, nullptr, nullptr, nullptr};   // xs[0] == stream; one stream per part of a large host batch
@@ -57,7 +52,8 @@ struct mpcb_ctx {
   cudaEvent_t ev_fork = nullptr;
 };
 
-// Solve the problems idx[0 .. *n_idx - 1] (device list) of a batch of B on stream st; used by the device closed loop.
+// Solve the problems idx[0 .. *n_idx - 1] (device list) of a batch of B on stream st, problem b on route[b] (nullptr:
+// route 0); used by the device closed loop.
 extern "C" int mpcb_solve_list_internal(mpcb_handle h, int B, const int* idx, const int* n_idx, const double* x0,
-                                        const double* obs_sv, const int* n_obs, double* U_out, int* status_out,
-                                        cudaStream_t st, const double* U_start);
+                                        const double* obs_sv, const int* n_obs, const int* route, double* U_out,
+                                        int* status_out, cudaStream_t st, const double* U_start);

@@ -188,7 +188,7 @@ int mpcb_hs_eval(mpcb_handle h, const mpcb_planner_params* p, int n_chunks, int 
   const int grid = (n_int + HS_INTERVALS - 1) / HS_INTERVALS;
   auto launch = [&](auto kern, size_t smem) -> int {
     CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   // per device
-    kern<<<grid, HS_THREADS, smem, st>>>(h->dt, d, n_int, N, z, lam, defect, jac, hess);
+    kern<<<grid, HS_THREADS, smem, st>>>(h->dt.t[0], d, n_int, N, z, lam, defect, jac, hess);
     return MPCB_OK;
   };
   const size_t per = sizeof(double) * HS_INTERVALS;

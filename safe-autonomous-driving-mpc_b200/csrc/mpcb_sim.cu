@@ -27,9 +27,22 @@ struct DevScenario {          // per vehicle, mirrors ObstaclesFSM.__init__ (:28
 
 enum { F_OBS_ACTIVE = 1, F_OBS_TRIGGERED = 2, F_TL_GREEN = 4, F_TL_WAITING = 8 };
 
+// Table of vehicle b's route (route == nullptr: route 0).  The routes of a simulation are checked when it is created.
+__device__ __forceinline__ const DevTable& vehicle_table(const DevTables& Ts, const int* __restrict__ route, int b) {
+  const int r = problem_route(route, b, Ts.n);
+  MPCB_ASSERT(r >= 0 && r < Ts.n);
+  return Ts.t[r < 0 ? 0 : r];
+}
+
+// loop condition (:395): still driving while s <= s_max - 1 of the vehicle's route
+__device__ __forceinline__ double stop_s(const DevTables& Ts, const int* __restrict__ route, int b) {
+  return vehicle_table(Ts, route, b).s_max - 1.0;
+}
+
 // ObstaclesFSM.update for every vehicle that is still driving (:330-374); car first, then light (:349, :362)
 __global__ void __launch_bounds__(128)
-mpcb_fsm_kernel(int B, double dt, double s_stop, const double* __restrict__ x, const DevScenario* __restrict__ scen,
+mpcb_fsm_kernel(const __grid_constant__ DevTables Ts, const int* __restrict__ route, int B, double dt,
+                const double* __restrict__ x, const DevScenario* __restrict__ scen,
                 double* __restrict__ fsm_f, int* __restrict__ fsm_i, int* __restrict__ alive,
                 double* __restrict__ obs_sv, int* __restrict__ n_obs, int rec_t, double* __restrict__ hist_obs,
                 int* __restrict__ hist_tl, int* __restrict__ alive_idx, int* __restrict__ alive_cnt,
@@ -38,7 +51,7 @@ mpcb_fsm_kernel(int B, double dt, double s_stop, const double* __restrict__ x, c
   if (b == 0) *next_cnt = 0;                                 // the other counter of the pair: next step's list length
   const bool in = b < B;
   const double s = in ? x[(size_t)b * 5] : 0.0, v = in ? x[(size_t)b * 5 + 4] : 0.0;
-  const int live = (in && s <= s_stop) ? 1 : 0;              // loop condition (:395), evaluated before the step
+  const int live = (in && s <= stop_s(Ts, route, b)) ? 1 : 0;   // loop condition (:395), evaluated before the step
   // list of the vehicles still driving: the solve of this step runs over the list, not over all B (one atomic per warp;
   // the order of the list does not matter, every problem is solved on its own and written to its own slot)
   {
@@ -94,7 +107,7 @@ mpcb_fsm_kernel(int B, double dt, double s_stop, const double* __restrict__ x, c
 
 // plant step (:404-406) for the vehicles that were alive at the start of the step
 __global__ void __launch_bounds__(128)
-mpcb_plant_kernel(const __grid_constant__ DevTable T, int B, double dt, double* __restrict__ x,
+mpcb_plant_kernel(const __grid_constant__ DevTables Ts, const int* __restrict__ route, int B, double dt, double* __restrict__ x,
                   const double* __restrict__ U, const int* __restrict__ status, const int* __restrict__ alive,
                   int* __restrict__ steps, int* __restrict__ n_unsolved, int rec_t, double* __restrict__ hist_x,
                   double* __restrict__ hist_u, int* __restrict__ hist_status) {
@@ -114,7 +127,7 @@ mpcb_plant_kernel(const __grid_constant__ DevTable T, int B, double dt, double* 
   }
   if (!live) return;
   double val[4], slope[4];
-  lookup_state(T, xs[0], val, slope);                        // k_ref = get_state(current_s)[3]  (:404)
+  lookup_state(vehicle_table(Ts, route, b), xs[0], val, slope);   // k_ref = get_state(current_s)[3]  (:404)
   const double kref = val[2];
   const double s = xs[0], o = xs[2], k = xs[3], v = xs[4];
   // x + dt * [v, v o, v (k - k_ref), u1, u2]   (:50-67, :406); no FMA contraction: same rounding as numpy
@@ -127,9 +140,10 @@ mpcb_plant_kernel(const __grid_constant__ DevTable T, int B, double dt, double* 
   if (status[b] != MPCB_SOLVED) n_unsolved[b] += 1;
 }
 
-__global__ void mpcb_count_alive_kernel(int B, double s_stop, const double* __restrict__ x, int* __restrict__ count) {
+__global__ void mpcb_count_alive_kernel(const __grid_constant__ DevTables Ts, const int* __restrict__ route, int B,
+                                        const double* __restrict__ x, int* __restrict__ count) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
-  const int live = (b < B && x[(size_t)b * 5] <= s_stop) ? 1 : 0;
+  const int live = (b < B && x[(size_t)b * 5] <= stop_s(Ts, route, b)) ? 1 : 0;
   const unsigned m = __ballot_sync(0xffffffffu, live);
   if ((threadIdx.x & 31) == 0 && m) atomicAdd(count, __popc(m));
 }
@@ -137,10 +151,12 @@ __global__ void mpcb_count_alive_kernel(int B, double s_stop, const double* __re
 // trajectory_tracking_check (sanity_checks.py:79-184) for every vehicle at once, on the recorded histories; one thread
 // per vehicle, coalesced over vehicles.  Verdict bits (1 = passed): 0 destination reached (:98-103), 1 stayed on road
 // (:106-111), 2 steering within limits +-0.1 (:121-125), 3 acceleration within limits (:127-131), 4 moving obstacle
-// avoided, gap >= 1 m (:142-164), 5 red light respected (:167-181), 6 history covers the whole drive.
+// avoided, gap >= 1 m (:142-164), 5 red light respected (:167-181), 6 history covers the whole drive.  route == nullptr:
+// every vehicle's route is s_total long; else vehicle b's route's s_max.
 // (The reference's CPU-time item :134-139 is a property of the host, not of the trajectory; it is not evaluated here.)
 __global__ void __launch_bounds__(128)
-mpcb_sim_check_kernel(int B, int n_rec, double s_total, double u1_min, double u1_max, double u2_min, double u2_max,
+mpcb_sim_check_kernel(const __grid_constant__ DevTables Ts, const int* __restrict__ route, int B, int n_rec,
+                      double s_total, double u1_min, double u1_max, double u2_min, double u2_max,
                       const double* __restrict__ x_final, const int* __restrict__ steps,
                       const DevScenario* __restrict__ scen, const double* __restrict__ hist_x,
                       const double* __restrict__ hist_u, const double* __restrict__ hist_obs,
@@ -165,7 +181,8 @@ mpcb_sim_check_kernel(int B, int n_rec, double s_total, double u1_min, double u1
   }
   const double s_final = x_final[(size_t)b * 5];
   int v = 0;
-  if (!(s_final < s_total - 1.0)) v |= 1;
+  const double s_end = route ? vehicle_table(Ts, route, b).s_max : s_total;
+  if (!(s_final < s_end - 1.0)) v |= 1;
   if (!(max_dev > lateral)) v |= 2;
   if (!(u1lo < u1_min - tol || u1hi > u1_max + tol)) v |= 4;
   if (!(u2lo < u2_min - tol || u2hi > u2_max + tol)) v |= 8;
@@ -188,7 +205,8 @@ struct mpcb_sim {
   mpcb_handle h;
   int B, cap, t;              // vehicles, history capacity (steps), steps recorded so far
   int hot_start = 0;          // first pass of step t > 0 starts from step t - 1's plans advanced by one step (mpcb_sim_set_hot_start)
-  double dt, s_stop;
+  double dt;
+  int* route = nullptr;       // route of each vehicle (device); nullptr: all on route 0
   DevScenario* scen = nullptr;
   double *x = nullptr, *fsm_f = nullptr, *obs_sv = nullptr, *U = nullptr;
   int *fsm_i = nullptr, *alive = nullptr, *n_obs = nullptr, *status = nullptr, *steps = nullptr, *n_unsolved = nullptr,
@@ -219,7 +237,7 @@ int mpcb_scenario_default(mpcb_scenario* s, int which) {
 int mpcb_sim_destroy(mpcb_sim_handle s) {
   if (!s) return MPCB_ERR_INVALID;
   cudaSetDevice(s->h->device);
-  void* ptrs[] = {s->scen, s->x, s->fsm_f, s->obs_sv, s->U, s->fsm_i, s->alive, s->n_obs, s->status, s->steps,
+  void* ptrs[] = {s->route, s->scen, s->x, s->fsm_f, s->obs_sv, s->U, s->fsm_i, s->alive, s->n_obs, s->status, s->steps,
                   s->n_unsolved, s->count, s->hist_x, s->hist_u, s->hist_obs, s->hist_status, s->hist_tl, s->alive_idx,
                   s->alive_cnt, s->d_verdict, s->d_metrics};
   for (void* p : ptrs) if (p) cudaFree(p);
@@ -229,14 +247,21 @@ int mpcb_sim_destroy(mpcb_sim_handle s) {
 
 int mpcb_sim_create(mpcb_sim_handle* out, mpcb_handle h, int B, const mpcb_scenario* scen, int n_scen,
                     const double* x_init, int history_steps) {
+  return mpcb_sim_create_routes(out, h, B, scen, n_scen, nullptr, x_init, history_steps);
+}
+
+int mpcb_sim_create_routes(mpcb_sim_handle* out, mpcb_handle h, int B, const mpcb_scenario* scen, int n_scen,
+                           const int* route, const double* x_init, int history_steps) {
   if (!out || !h || B < 1 || !scen || (n_scen != 1 && n_scen != B) || history_steps < 0) return MPCB_ERR_INVALID;
+  if (route)
+    for (int b = 0; b < B; ++b)
+      if (route[b] < 0 || route[b] >= h->dt.n) return MPCB_ERR_INVALID;
   *out = nullptr;
   CK(cudaSetDevice(h->device));
   mpcb_sim* s = new (std::nothrow) mpcb_sim();
   if (!s) return MPCB_ERR_NOMEM;
   s->h = h; s->B = B; s->cap = history_steps; s->t = 0;
   s->dt = h->params.dt;
-  s->s_stop = h->dt.s_max - 1.0;                                        // :395
   auto fail = [&](int code) { mpcb_sim_destroy(s); return code; };
   const size_t nb = (size_t)B;
 #define SIM_ALLOC(ptr, bytes) if (cudaMalloc((void**)&(ptr), (bytes)) != cudaSuccess) { cudaGetLastError(); return fail(MPCB_ERR_NOMEM); }
@@ -245,6 +270,7 @@ int mpcb_sim_create(mpcb_sim_handle* out, mpcb_handle h, int B, const mpcb_scena
   SIM_ALLOC(s->fsm_i, nb * 4); SIM_ALLOC(s->alive, nb * 4); SIM_ALLOC(s->n_obs, nb * 4); SIM_ALLOC(s->status, nb * 4);
   SIM_ALLOC(s->steps, nb * 4); SIM_ALLOC(s->n_unsolved, nb * 4); SIM_ALLOC(s->count, 4);
   SIM_ALLOC(s->alive_idx, nb * 4); SIM_ALLOC(s->alive_cnt, 8);
+  if (route) SIM_ALLOC(s->route, nb * 4);
   if (history_steps > 0) {
     SIM_ALLOC(s->d_verdict, nb * 4); SIM_ALLOC(s->d_metrics, nb * 32);
     const size_t nt = (size_t)history_steps * nb;
@@ -264,6 +290,7 @@ int mpcb_sim_create(mpcb_sim_handle* out, mpcb_handle h, int B, const mpcb_scena
     hf[b * 2 + 1] = 0.0;
   }
   cudaError_t e;
+  if (route && (e = cudaMemcpy(s->route, route, nb * 4, cudaMemcpyHostToDevice)) != cudaSuccess) return fail(cuda_fail(e, "cudaMemcpy"));
   if ((e = cudaMemcpy(s->scen, hs.data(), nb * sizeof(DevScenario), cudaMemcpyHostToDevice)) != cudaSuccess) return fail(cuda_fail(e, "cudaMemcpy"));
   if ((e = cudaMemcpy(s->x, hx.data(), nb * 40, cudaMemcpyHostToDevice)) != cudaSuccess) return fail(cuda_fail(e, "cudaMemcpy"));
   if ((e = cudaMemcpy(s->fsm_f, hf.data(), nb * 16, cudaMemcpyHostToDevice)) != cudaSuccess) return fail(cuda_fail(e, "cudaMemcpy"));
@@ -285,15 +312,15 @@ int mpcb_sim_step(mpcb_sim_handle s, int n_steps, void* cuda_stream) {
   for (int k = 0; k < n_steps; ++k) {
     const int rec = (s->t < s->cap) ? s->t : -1;
     int* cnt = s->alive_cnt + (s->t & 1);
-    mpcb_fsm_kernel<<<grid, 128, 0, st>>>(s->B, s->dt, s->s_stop, s->x, s->scen, s->fsm_f, s->fsm_i, s->alive, s->obs_sv,
+    mpcb_fsm_kernel<<<grid, 128, 0, st>>>(s->h->dt, s->route, s->B, s->dt, s->x, s->scen, s->fsm_f, s->fsm_i, s->alive, s->obs_sv,
                                           s->n_obs, rec, s->hist_obs, s->hist_tl, s->alive_idx, cnt,
                                           s->alive_cnt + ((s->t + 1) & 1));
     CK(cudaGetLastError());
     // the solve runs over the list of vehicles still driving (arrived vehicles are frozen and cost nothing)
-    int rc = mpcb_solve_list_internal(s->h, s->B, s->alive_idx, cnt, s->x, s->obs_sv, s->n_obs, s->U, s->status, st,
-                                      (s->hot_start && s->t > 0) ? s->U : nullptr);
+    int rc = mpcb_solve_list_internal(s->h, s->B, s->alive_idx, cnt, s->x, s->obs_sv, s->n_obs, s->route, s->U, s->status,
+                                      st, (s->hot_start && s->t > 0) ? s->U : nullptr);
     if (rc != MPCB_OK) return rc;
-    mpcb_plant_kernel<<<grid, 128, 0, st>>>(s->h->dt, s->B, s->dt, s->x, s->U, s->status, s->alive, s->steps,
+    mpcb_plant_kernel<<<grid, 128, 0, st>>>(s->h->dt, s->route, s->B, s->dt, s->x, s->U, s->status, s->alive, s->steps,
                                             s->n_unsolved, rec, s->hist_x, s->hist_u, s->hist_status);
     CK(cudaGetLastError());
     s->h->launches += 2;
@@ -313,7 +340,7 @@ int mpcb_sim_alive(mpcb_sim_handle s, int* n_alive, void* cuda_stream) {
   CK(cudaSetDevice(s->h->device));
   cudaStream_t st = (cudaStream_t)cuda_stream;
   CK(cudaMemsetAsync(s->count, 0, 4, st));
-  mpcb_count_alive_kernel<<<(s->B + 127) / 128, 128, 0, st>>>(s->B, s->s_stop, s->x, s->count);
+  mpcb_count_alive_kernel<<<(s->B + 127) / 128, 128, 0, st>>>(s->h->dt, s->route, s->B, s->x, s->count);
   CK(cudaGetLastError());
   CK(cudaMemcpyAsync(n_alive, s->count, 4, cudaMemcpyDeviceToHost, st));
   CK(cudaStreamSynchronize(st));
@@ -339,7 +366,7 @@ int mpcb_sim_check(mpcb_sim_handle s, int* verdict, double* metrics, void* cuda_
   const size_t nb = (size_t)s->B;
   const mpcb_params& p = s->h->params;
   const int nt = s->t < s->cap ? s->t : s->cap;
-  mpcb_sim_check_kernel<<<(s->B + 127) / 128, 128, 0, st>>>(s->B, nt, s->h->dt.s_max, p.u_min[0], p.u_max[0], p.u_min[1],
+  mpcb_sim_check_kernel<<<(s->B + 127) / 128, 128, 0, st>>>(s->h->dt, s->route, s->B, nt, s->h->dt.t[0].s_max, p.u_min[0], p.u_max[0], p.u_min[1],
                                                            p.u_max[1], s->x, s->steps, s->scen, s->hist_x, s->hist_u,
                                                            s->hist_obs, s->hist_tl, s->d_verdict, s->d_metrics);
   CK(cudaGetLastError());
@@ -381,7 +408,7 @@ int mpcb_check_histories(mpcb_handle h, int B, int T, double s_total, const mpcb
     int* d_v = (int*)(d + off[7]);
     double* d_m = (double*)(d + off[7] + ((nb * 4 + 255) & ~(size_t)255));
     // (the metrics block sits behind the verdicts inside the last region: re-derive its offset so both are aligned)
-    mpcb_sim_check_kernel<<<(B + 127) / 128, 128, 0, st>>>(B, T, s_total, p.u_min[0], p.u_max[0], p.u_min[1], p.u_max[1],
+    mpcb_sim_check_kernel<<<(B + 127) / 128, 128, 0, st>>>(h->dt, nullptr, B, T, s_total, p.u_min[0], p.u_max[0], p.u_min[1], p.u_max[1],
                                                           (const double*)(d + off[1]), (const int*)(d + off[2]),
                                                           (const DevScenario*)(d + off[0]), (const double*)(d + off[3]),
                                                           (const double*)(d + off[4]), (const double*)(d + off[5]),

@@ -67,10 +67,11 @@ def check_histories(tracker, s_total, scenarios, x_final, steps, hist_x, hist_u,
 
 
 class BatchedSimulation:
-    def __init__(self, tracker, scenarios, B=None, x_init=None, history_steps=0, hot_start=False):
+    def __init__(self, tracker, scenarios, B=None, x_init=None, history_steps=0, hot_start=False, route=None):
         """tracker: BatchedTracker; scenarios: one Scenario (shared) or a list of B; x_init: [B,5] or None for the
         reference's start state.  hot_start: from its second step on a vehicle's solve starts from its previous plan
-        advanced by one step (mpcb_sim_set_hot_start) instead of the reference's table-based warm start."""
+        advanced by one step (mpcb_sim_set_hot_start) instead of the reference's table-based warm start.
+        route: one int or an int array [B], vehicle b driving ``tracker.routes[route[b]]`` (None: route 0)."""
         self._lib = tracker._lib
         self._t = tracker
         scen = list(scenarios) if isinstance(scenarios, (list, tuple)) else [scenarios]
@@ -80,9 +81,19 @@ class BatchedSimulation:
         xi = None
         if x_init is not None:
             xi = np.ascontiguousarray(x_init, dtype=np.float64).reshape(B, 5)
+        rt = None
+        if route is not None:
+            rt = np.asarray(route)
+            if rt.ndim == 0:
+                rt = np.full(B, rt)
+            if not np.issubdtype(rt.dtype, np.integer) or rt.shape != (B,):
+                raise ValueError(f"route must be one int or an int array of shape ({B},)")
+            rt = np.ascontiguousarray(rt, dtype=np.int32)
         h = C.c_void_p()
-        check(self._lib.mpcb_sim_create(C.byref(h), tracker._need(), int(B), arr, len(scen),
-                                        _dp(xi) if xi is not None else None, int(history_steps)), "mpcb_sim_create")
+        check(self._lib.mpcb_sim_create_routes(C.byref(h), tracker._need(), int(B), arr, len(scen),
+                                               _dp(rt) if rt is not None else None,
+                                               _dp(xi) if xi is not None else None, int(history_steps)),
+              "mpcb_sim_create_routes")
         self._h = h
         self.B = int(B)
         self.history_steps = int(history_steps)

@@ -108,11 +108,20 @@ class BatchedTracker:
     """Drop-in for the reference's TrajectoryTracker, running on one B200.
 
     Same attributes as trajectory_tracking.py:12-47; ``solve`` has the reference's signature and return
-    tuple so the object can be passed to the reference's own ``run_simulation``."""
+    tuple so the object can be passed to the reference's own ``run_simulation``.
 
-    STATUS_SOLVED, STATUS_MAXITER, STATUS_INFEASIBLE = 0, 1, 2
+    ``X_ref`` may also be a sequence of up to ``MAX_ROUTES`` loaders: the tracker then holds one route per loader
+    (``routes``, ``n_routes``), ``solve_batch(..., route=)`` and ``BatchedSimulation(..., route=)`` pick a route per
+    problem or vehicle, and every other call runs on route 0.  ``X_ref`` is then the first loader."""
+
+    STATUS_SOLVED, STATUS_MAXITER, STATUS_INFEASIBLE, STATUS_BAD_ROUTE = 0, 1, 2, 3
+    MAX_ROUTES = 16
 
     def __init__(self, X_ref=None, device=0, **solver_overrides):
+        routes = tuple(X_ref) if isinstance(X_ref, (list, tuple)) else ((X_ref,) if X_ref is not None else ())
+        if isinstance(X_ref, (list, tuple)) and not 1 <= len(routes) <= self.MAX_ROUTES:
+            raise ValueError(f"a tracker holds 1 to {self.MAX_ROUTES} routes, got {len(routes)}")
+        X_ref = routes[0] if routes else None
         lib = _lib.load()
         self._lib = lib
         p = TrackerParams()
@@ -123,6 +132,8 @@ class BatchedTracker:
             setattr(p, k, v)
         self.params = p
         self.X_ref = X_ref
+        self.routes = routes
+        self.n_routes = len(routes)
         # attributes of the reference object (read by run_simulation, sanity checks, plots)
         self.dt = p.dt
         self.N = p.N
@@ -137,9 +148,14 @@ class BatchedTracker:
         self.safe_lane_margin = p.safe_lane_margin
         self.device = device
         self._h = None
-        if X_ref is not None:
+        if len(routes) == 1:
             h = C.c_void_p()
             check(lib.mpcb_create(C.byref(h), C.byref(p), X_ref._h, int(device)), "mpcb_create")
+            self._h = h
+        elif routes:
+            h = C.c_void_p()
+            tabs = (C.c_void_p * len(routes))(*[L._h for L in routes])
+            check(lib.mpcb_create_routes(C.byref(h), C.byref(p), tabs, len(routes), int(device)), "mpcb_create_routes")
             self._h = h
         self._pin = {}
         self.last_status = None
@@ -247,12 +263,16 @@ class BatchedTracker:
     def wait(self):
         check(self._lib.mpcb_wait(self._need()), "mpcb_wait")
 
-    def solve_batch(self, x0, obs_sv, n_obs, out=None, stream=None):
+    def solve_batch(self, x0, obs_sv, n_obs, out=None, stream=None, route=None):
         """Device tensors in, device tensors out (torch used only for memory + stream hand-off).
-        Asynchronous on ``stream`` (default: torch's current stream)."""
+        Asynchronous on ``stream`` (default: torch's current stream).  ``route``: device int32 tensor [B], problem b on
+        ``routes[route[b]]`` (None: route 0); a problem whose route is out of range gets ``STATUS_BAD_ROUTE`` and NaN."""
         import torch
-        h = self._need()
         B = x0.shape[0]
+        if route is not None and not (isinstance(route, torch.Tensor) and route.dtype == torch.int32
+                                      and tuple(route.shape) == (B,) and route.is_contiguous()):
+            raise ValueError(f"route must be a contiguous int32 tensor of shape ({B},)")
+        h = self._need()
         dev = x0.device
         assert x0.dtype == torch.float64 and obs_sv.dtype == torch.float64 and n_obs.dtype == torch.int32
         assert x0.is_contiguous() and obs_sv.is_contiguous() and n_obs.is_contiguous()
@@ -265,10 +285,11 @@ class BatchedTracker:
                        cmin=torch.empty((B,), dtype=torch.float64, device=dev),
                        active=torch.empty((B,), dtype=torch.int64, device=dev))
         st = torch.cuda.current_stream(dev).cuda_stream if stream is None else stream
-        check(self._lib.mpcb_solve_batch(h, B, x0.data_ptr(), obs_sv.data_ptr(), n_obs.data_ptr(),
-                                         out["U"].data_ptr(), out["Xpred"].data_ptr(), out["obj"].data_ptr(),
-                                         out["status"].data_ptr(), out["iters"].data_ptr(), out["cmin"].data_ptr(),
-                                         out["active"].data_ptr(), C.c_void_p(st)), "mpcb_solve_batch")
+        check(self._lib.mpcb_solve_batch_routes(h, B, x0.data_ptr(), obs_sv.data_ptr(), n_obs.data_ptr(),
+                                                route.data_ptr() if route is not None else None,
+                                                out["U"].data_ptr(), out["Xpred"].data_ptr(), out["obj"].data_ptr(),
+                                                out["status"].data_ptr(), out["iters"].data_ptr(), out["cmin"].data_ptr(),
+                                                out["active"].data_ptr(), C.c_void_p(st)), "mpcb_solve_batch_routes")
         return out
 
     def eval_batch(self, x0, U, obs_sv, n_obs):
