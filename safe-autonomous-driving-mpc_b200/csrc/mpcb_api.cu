@@ -52,11 +52,18 @@ template <> struct ClsCfg<1> { typedef Store<SOLVE_THREADS, MPCB_CLS_MASK1, 1> S
 template <> struct ClsCfg<2> { typedef Store<SOLVE_THREADS, MPCB_CLS_MASK2, 2> St; };
 constexpr int cmax3(int a, int b, int c) { return a > b ? (a > c ? a : c) : (b > c ? b : c); }
 constexpr size_t CLS_SMEM = sizeof(double) * SOLVE_THREADS * cmax3(ClsCfg<0>::St::SHARED, ClsCfg<1>::St::SHARED, ClsCfg<2>::St::SHARED);
-constexpr int CLS_HDR = 4;                // class-list header: three counts, pad; then three lists of B indices each
-constexpr int CARRY_HDR_STRIDE = 3 * MPCB_MAX_ROUTES;   // survivor-list header: counts per (class, route), [k * nr + r]
-constexpr int CARRY_HDR = 3 * CARRY_HDR_STRIDE;         // survivor lists of the first pass: three headers
-constexpr int ROUTE_CNT = 3 * MPCB_MAX_ROUTES;          // routed first pass: part sizes per (class, route), then cursors
 constexpr int EVAL_THREADS = 128;
+
+// Counts and cursors of one part of a solve call (the whole call, or one part of a chunked host call; the lists they
+// count are laid out by part_view).  The call zeroes them before its first kernel.  The first pass is partitioned into
+// (class, route) parts, counted at [k * nr + r] (nr = 1 on a single-route call).
+struct PartLists {
+  int n_robust;                       // problems listed for the robust pass
+  int cursor[2];                      // work cursors of the warp-per-problem kernels: first pass, robust pass
+  int part[3 * MPCB_MAX_ROUTES];      // part sizes of the class lists
+  int fill[3 * MPCB_MAX_ROUTES];      // listing cursors of a routed call (its count pass fills part)
+  int surv[3][3 * MPCB_MAX_ROUTES];   // survivors of the first pass after round r, at surv[r % 3]
+};
 
 // Device pointers of one solve call (mpcb_solve_batch's arguments), handed to the kernels as one block.
 struct SolveIO {
@@ -89,12 +96,11 @@ __device__ __forceinline__ void write_bad_route(const SolveIO& io, int b) {
 }
 
 // Final evaluation at U* (predict, cost, constraint rows in the reference's order), flags, outputs.  In the first pass a
-// problem that is not certified is appended to the work list of the next pass instead (fb_list == nullptr: the caller
-// goes on itself); its iteration counts are still recorded, the next pass adds its own.  Returns "written out".
+// problem that is not certified is appended to the robust pass's list instead (robust, counted in hdr->n_robust); its
+// iteration counts are still recorded, the robust pass adds its own.  Returns "written out".
 template <bool FIRST_PASS>
 __device__ __forceinline__ bool finalize(const DevTable& T, const DevParams& P, const Problem& pb, const SolveOut& so, int b,
-                                         bool accumulate, const SolveIO& io, int* __restrict__ fb_list,
-                                         int* __restrict__ fb_count) {
+                                         bool accumulate, const SolveIO& io, PartLists* hdr, int* __restrict__ robust) {
   double* __restrict__ U_out = io.U;
   double* __restrict__ Xpred_out = io.Xpred;
   double* __restrict__ obj_out = io.obj;
@@ -102,16 +108,14 @@ __device__ __forceinline__ bool finalize(const DevTable& T, const DevParams& P, 
   int* __restrict__ iters_out = io.iters;
   double* __restrict__ cmin_out = io.cmin;
   unsigned long long* __restrict__ active_out = io.active;
+  if (iters_out) {
+    if (accumulate) { iters_out[2 * b] += so.rounds; iters_out[2 * b + 1] += so.iters; }     // work of both passes
+    else { iters_out[2 * b] = so.rounds; iters_out[2 * b + 1] = so.iters; }
+  }
   auto defer = [&]() {
-    if (fb_list) {
-      const int slot = atomicAdd(fb_count, 1);
-      MPCB_ASSERT(slot >= 0 && slot < io.n_total && b >= 0 && b < io.n_total);
-      fb_list[slot] = b;
-    }
-    if (iters_out) {
-      if (accumulate) { iters_out[2 * b] += so.rounds; iters_out[2 * b + 1] += so.iters; }
-      else { iters_out[2 * b] = so.rounds; iters_out[2 * b + 1] = so.iters; }
-    }
+    const int slot = atomicAdd(&hdr->n_robust, 1);
+    MPCB_ASSERT(slot >= 0 && slot < io.n_total && b >= 0 && b < io.n_total);
+    robust[slot] = b;
   };
   if (FIRST_PASS && so.status == MPCB_MAXITER) {                   // not certified: leave it to the next pass
     defer();
@@ -184,25 +188,39 @@ __device__ __forceinline__ bool finalize(const DevTable& T, const DevParams& P, 
   }
   if (obj_out) obj_out[b] = cost;
   if (status_out) status_out[b] = status;
-  if (iters_out) {
-    if (accumulate) { iters_out[2 * b] += so.rounds; iters_out[2 * b + 1] += so.iters; }     // work of both passes
-    else { iters_out[2 * b] = so.rounds; iters_out[2 * b + 1] = so.iters; }
-  }
   if (cmin_out) cmin_out[b] = cmin;
   if (active_out) active_out[b] = act;
   return true;
 }
 
+// problem b's inputs (class NOBS); a thread without a problem gets a benign zero problem it never works on
+template <int NOBS>
+__device__ __forceinline__ void load_problem(const SolveIO& io, int b, bool live, Problem& pb) {
+  if (live) {
+#pragma unroll
+    for (int c = 0; c < 5; ++c) pb.x0[c] = io.x0[(size_t)b * 5 + c];
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      pb.obs[k][0] = (k < NOBS) ? io.obs_sv[(size_t)b * 4 + 2 * k] : 0.0;
+      pb.obs[k][1] = (k < NOBS) ? io.obs_sv[(size_t)b * 4 + 2 * k + 1] : 0.0;
+    }
+    pb.n_obs = NOBS;
+  } else {
+#pragma unroll
+    for (int c = 0; c < 5; ++c) pb.x0[c] = 0.0;
+    pb.obs[0][0] = pb.obs[0][1] = pb.obs[1][0] = pb.obs[1][1] = 0.0;
+    pb.n_obs = 0;
+  }
+}
+
 // ------------------------------------------------------------------------------------------------
-// Solve kernel: one thread per problem, CTA-uniform loop control.
+// Solve kernel: one thread per problem, CTA-uniform loop control, every problem written out (the robust pass with
+// coop_pass2 = 0, and the only pass with fast_pass = 0).
 //   work list   idx == nullptr: problems 0..B-1;  else problems idx[0 .. *n_idx - 1] (second pass)
-//   FIRST_PASS  problems this pass cannot certify (iteration caps hit, or a verdict only the robust pass may give)
-//               are appended to fb_list / fb_count instead of being written out.
 // ------------------------------------------------------------------------------------------------
-template <bool FIRST_PASS>
 __global__ void __launch_bounds__(SOLVE_THREADS, MPCB_SOLVE_CTAS)
 mpcb_solve_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ DevParams P, int B,
-                  const __grid_constant__ SolveIO io, int* __restrict__ fb_list, int* __restrict__ fb_count) {
+                  const __grid_constant__ SolveIO io) {
   const int* __restrict__ idx = io.idx;
   const int n_work = idx ? min(*io.n_idx, B) : B;
   if ((int)(blockIdx.x * blockDim.x) >= n_work) return;          // CTA-uniform
@@ -214,24 +232,14 @@ mpcb_solve_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ 
   MPCB_ASSERT(!live || r < Ts.n);
   const DevTable& T = Ts.t[live ? r : 0];
   Problem pb;
-  if (live) {
-#pragma unroll
-    for (int c = 0; c < 5; ++c) pb.x0[c] = io.x0[(size_t)b * 5 + c];
-#pragma unroll
-    for (int k = 0; k < 2; ++k) { pb.obs[k][0] = io.obs_sv[(size_t)b * 4 + 2 * k]; pb.obs[k][1] = io.obs_sv[(size_t)b * 4 + 2 * k + 1]; }
-    pb.n_obs = min(max(io.n_obs[b], 0), 2);
-  } else {
-#pragma unroll
-    for (int c = 0; c < 5; ++c) pb.x0[c] = 0.0;
-    pb.obs[0][0] = pb.obs[0][1] = pb.obs[1][0] = pb.obs[1][1] = 0.0;
-    pb.n_obs = 0;
-  }
+  load_problem<2>(io, b, live, pb);
+  if (live) pb.n_obs = min(max(io.n_obs[b], 0), 2);
   extern __shared__ double solve_smem[];
   double solve_local[SolveStore::LOCAL > 0 ? SolveStore::LOCAL : 1];
   const SolveStore st(solve_smem + threadIdx.x, solve_local);
-  SolveOut so = solve_one<FIRST_PASS>(T, P, pb, st, live);
+  SolveOut so = solve_one<false>(T, P, pb, st, live);
   if (!live) return;
-  finalize<FIRST_PASS>(T, P, pb, so, b, io.accumulate != 0, io, fb_list, fb_count);
+  finalize<false>(T, P, pb, so, b, io.accumulate != 0, io, nullptr, nullptr);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -252,16 +260,15 @@ __device__ __forceinline__ int warp_append_key(int key, int* counters) {
   return key >= 0 ? base + __popc(m & ((1u << lane) - 1u)) : -1;
 }
 
-// A routed call (nr = the handle's routes) partitions by (class, route), so that every CTA of the first pass runs on
-// one table: a count pass (cls == nullptr) counts the parts into cursor[k * nr + r]; the listing pass then appends each
-// problem to its part, which starts at the sum of the sizes pcnt of the class's earlier routes.  A single-route call
-// (nr = 1, pcnt == nullptr) lists straight into the class lists, its cursors the class-list header.  Problems whose
-// route is bad are written out here and listed nowhere.
+// A routed call (io.route, nr = the handle's routes) partitions by (class, route), so that every CTA of the first pass
+// runs on one table: a count pass (cls == nullptr) counts the parts into hdr->part; the listing pass then appends each
+// problem to its part, which starts at the sum of the sizes of the class's earlier routes, through the cursors
+// hdr->fill.  A single-route call (nr = 1) lists straight into the class lists, counting them in hdr->part.  Problems
+// whose route is bad are written out here and listed nowhere.
 __global__ void __launch_bounds__(256)
-mpcb_classify_kernel(int B, const __grid_constant__ SolveIO io, int n_routes, int nr, const int* __restrict__ pcnt,
-                     int* __restrict__ cursor, int* __restrict__ cls, int* __restrict__ carry_hdr) {
-  if (cls && blockIdx.x == 0)                                   // survivor lists of the first pass
-    for (int i = threadIdx.x; i < CARRY_HDR; i += blockDim.x) carry_hdr[i] = 0;
+mpcb_classify_kernel(int B, const __grid_constant__ SolveIO io, int n_routes, int nr, PartLists* __restrict__ hdr,
+                     int* __restrict__ cls) {
+  const bool fill = io.route && cls;
   const int n_work = io.idx ? min(*io.n_idx, B) : B;
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
   const bool live = t < n_work;
@@ -271,13 +278,13 @@ mpcb_classify_kernel(int B, const __grid_constant__ SolveIO io, int n_routes, in
   const int k = min(max(io.n_obs[b], 0), 2);
   const int key = r >= 0 ? k * nr + r : -1;
   MPCB_ASSERT(r < nr);
-  const int slot = warp_append_key(key, cursor);
+  const int slot = warp_append_key(key, fill ? hdr->fill : hdr->part);
   if (!cls || key < 0) return;
   int off = 0;
-  if (pcnt)
-    for (int q = 0; q < r; ++q) off += pcnt[k * nr + q];
-  MPCB_ASSERT(slot >= 0 && (!pcnt || slot < pcnt[key]) && off + slot < B && b >= 0 && b < B);
-  cls[CLS_HDR + (size_t)k * B + off + slot] = b;
+  if (fill)
+    for (int q = 0; q < r; ++q) off += hdr->part[k * nr + q];
+  MPCB_ASSERT(slot >= 0 && (!fill || slot < hdr->part[key]) && off + slot < B && b >= 0 && b < B);
+  cls[(size_t)k * B + off + slot] = b;
 }
 
 // hot start of problem b: the stored plan, optionally advanced by one step (the last step is repeated)
@@ -307,9 +314,9 @@ __device__ __forceinline__ void load_hot_start(const SolveIO& io, int b, double 
 constexpr int CLS_ROUNDS = MPCB_CLS_ROUNDS;   // rounds of the class kernel (the rest: one round kernel per round)
 
 // One carry workspace: slot-major arrays (field f of slot s at [f * cap + s], so the loads of a CTA's consecutive slots
-// coalesce).  A list of survivors is a header of counts per (class, route) part; a part's survivors occupy the slots from
-// that part's offset in the batch's partition on (find_part: classes with more rows first, routes in order within a class;
-// single route: class 2 at 0, class 1 at n2, class 0 at n2 + n1).
+// coalesce).  A list of survivors is a row of PartLists::surv, counts per (class, route) part; a part's survivors
+// occupy the slots from that part's offset in the batch's partition on (find_part: classes with more rows first, routes
+// in order within a class; single route: class 2 at 0, class 1 at n2, class 0 at n2 + n1).
 enum : int { CD_U = 0, CD_X = CD_U + NV, CD_V = CD_X + NV, CD_LOV = CD_V + ROW_OBS + 2 * N_OBSROW, CD_BLO = CD_LOV + NH,
              CD_BHI = CD_BLO + NH, CD_HIO = CD_BHI + NH, N_CD = CD_HIO + 2 * N_OBSROW };
 enum : int { CI_B = 0, CI_HINT = 1, CI_FAILS = CI_HINT + NH + 1, CI_ROUNDS, CI_ITERS, CI_STATUS, CI_FLAGS, N_CI };
@@ -326,18 +333,6 @@ struct Carry {
     return c;
   }
 };
-
-// Slot of this thread in a list (warp-aggregated append to counter; every lane of the warp calls it), -1 if !pred.
-__device__ __forceinline__ int warp_append(bool pred, int* counter) {
-  const unsigned m = __ballot_sync(0xffffffffu, pred);
-  if (m == 0u) return -1;
-  const unsigned lane = threadIdx.x & 31u;
-  const int leader = __ffs(m) - 1;
-  int base = 0;
-  if ((int)lane == leader) base = atomicAdd(counter, __popc(m));
-  base = __shfl_sync(0xffffffffu, base, leader);
-  return pred ? base + __popc(m & ((1u << lane) - 1u)) : -1;
-}
 
 // The part of a first-pass list that CTA blk works on, 128 problems per CTA.  Parts are (class, route) pairs, classes
 // with more rows first and routes in order within a class; cnt[k * nr + r] are the sizes that assign CTAs, base[.] the
@@ -415,33 +410,13 @@ __device__ __forceinline__ void unpark(const Carry& c, int slot, Problem& pb, co
   s.step_prev = 1e30;
 }
 
-// problem b's inputs (class NOBS); a thread without a problem gets a benign zero problem it never works on
-template <int NOBS>
-__device__ __forceinline__ void load_problem(const SolveIO& io, int b, bool live, Problem& pb) {
-  if (live) {
-#pragma unroll
-    for (int c = 0; c < 5; ++c) pb.x0[c] = io.x0[(size_t)b * 5 + c];
-#pragma unroll
-    for (int k = 0; k < 2; ++k) {
-      pb.obs[k][0] = (k < NOBS) ? io.obs_sv[(size_t)b * 4 + 2 * k] : 0.0;
-      pb.obs[k][1] = (k < NOBS) ? io.obs_sv[(size_t)b * 4 + 2 * k + 1] : 0.0;
-    }
-    pb.n_obs = NOBS;
-  } else {
-#pragma unroll
-    for (int c = 0; c < 5; ++c) pb.x0[c] = 0.0;
-    pb.obs[0][0] = pb.obs[0][1] = pb.obs[1][0] = pb.obs[1][1] = 0.0;
-    pb.n_obs = 0;
-  }
-}
-
-// After a problem's last round in this kernel: park it in the next list (cont, every thread of the warp calls this),
-// or finalize it.
+// After a problem's last round in this kernel: park it in the next list (cont, every thread of the warp calls this;
+// cnt_out counts the survivors of its part), or finalize it.
 template <int NOBS, class ST>
 __device__ __forceinline__ void park_or_finalize(const DevTable& T, const DevParams& P, const SolveIO& io, bool live, bool cont,
                                                  int b, Problem& pb, const ST& st, SolveState& s, int n_work,
-                                                 const Carry& cout, int* __restrict__ cnt_out, int off,
-                                                 int* __restrict__ fb_list, int* __restrict__ fb_count) {
+                                                 const Carry& cout, int* __restrict__ cnt_out, int off, PartLists* hdr,
+                                                 int* __restrict__ robust) {
   const int k = warp_append(cont, cnt_out);
   if (!live) return;
   if (cont) {
@@ -450,13 +425,13 @@ __device__ __forceinline__ void park_or_finalize(const DevTable& T, const DevPar
     return;
   }
   const SolveOut so = solve_end<true>(P, pb, s);
-  finalize<true>(T, P, pb, so, b, io.accumulate != 0, io, fb_list, fb_count);
+  finalize<true>(T, P, pb, so, b, io.accumulate != 0, io, hdr, robust);
 }
 
 template <int NOBS>
 __device__ __forceinline__ void solve_cls_body(const DevTable& T, const DevParams& P, const SolveIO& io, const int* __restrict__ list,
                                                int n_work, int t0, int off, int r0, const Carry& cout,
-                                               int* __restrict__ cnt_out, int* __restrict__ fb_list, int* __restrict__ fb_count) {
+                                               int* __restrict__ cnt_out, PartLists* hdr, int* __restrict__ robust) {
   typedef typename ClsCfg<NOBS>::St St;
   const int t = t0 + threadIdx.x;
   const bool live = t < n_work;
@@ -478,26 +453,27 @@ __device__ __forceinline__ void solve_cls_body(const DevTable& T, const DevParam
     solve_round<true>(T, P, pb, st, s, round);
   }
   park_or_finalize<NOBS>(T, P, io, live, live && !s.done && r0 < P.thread_max_rounds, b, pb, st, s, n_work, cout, cnt_out,
-                         off, fb_list, fb_count);
+                         off, hdr, robust);
 }
 
-// pcnt[k * nr + r]: sizes of the (class, route) parts of the class lists (nr = 1: the class-list header).  The part, and
-// with it the table, is CTA-uniform.  ROUTED = false (a single-route call, nr = 1) fixes the table at t[0] at compile
-// time: an indexed table costs the single-route first pass 1 % (see DESIGN.md 4, "Several routes on one handle").
+// Rounds 1..r0 over the class lists cls (class k at cls + k B), cut into the parts hdr->part; survivors go to the list
+// hdr->surv[r0 % 3].  The part, and with it the table, is CTA-uniform.  ROUTED = false (a single-route call, nr = 1)
+// fixes the table at t[0] at compile time: an indexed table costs the single-route first pass 1 % (see DESIGN.md 4,
+// "Several routes on one handle").
 template <bool ROUTED>
 __global__ void __launch_bounds__(SOLVE_THREADS, MPCB_SOLVE_CTAS)
 mpcb_solve_cls_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ DevParams P, int B,
-                      const __grid_constant__ SolveIO io, const int* __restrict__ cls, const int* __restrict__ pcnt, int nr,
-                      int r0, const __grid_constant__ Carry cout, int* __restrict__ cnt_out, int* __restrict__ fb_list,
-                      int* __restrict__ fb_count) {
+                      const __grid_constant__ SolveIO io, PartLists* hdr, const int* __restrict__ cls, int nr, int r0,
+                      const __grid_constant__ Carry cout, int* __restrict__ robust) {
   Part p;
-  if (!find_part(pcnt, pcnt, ROUTED ? nr : 1, blockIdx.x, p)) return;       // CTA-uniform from here on
+  if (!find_part(hdr->part, hdr->part, ROUTED ? nr : 1, blockIdx.x, p)) return;       // CTA-uniform from here on
   MPCB_ASSERT(p.r >= 0 && p.r < Ts.n && p.off_cls + p.n <= B);
   const DevTable& T = Ts.t[ROUTED ? p.r : 0];
-  const int* list = cls + CLS_HDR + (size_t)p.k * B + p.off_cls;
-  if (p.k == 2) solve_cls_body<2>(T, P, io, list, p.n, p.t0, p.off, r0, cout, cnt_out + p.key, fb_list, fb_count);
-  else if (p.k == 1) solve_cls_body<1>(T, P, io, list, p.n, p.t0, p.off, r0, cout, cnt_out + p.key, fb_list, fb_count);
-  else solve_cls_body<0>(T, P, io, list, p.n, p.t0, p.off, r0, cout, cnt_out + p.key, fb_list, fb_count);
+  const int* list = cls + (size_t)p.k * B + p.off_cls;
+  int* cnt_out = hdr->surv[r0 % 3] + p.key;
+  if (p.k == 2) solve_cls_body<2>(T, P, io, list, p.n, p.t0, p.off, r0, cout, cnt_out, hdr, robust);
+  else if (p.k == 1) solve_cls_body<1>(T, P, io, list, p.n, p.t0, p.off, r0, cout, cnt_out, hdr, robust);
+  else solve_cls_body<0>(T, P, io, list, p.n, p.t0, p.off, r0, cout, cnt_out, hdr, robust);
 }
 
 #ifdef MPCB_ROUND_STATS   // development: survivors per round and class, summed over calls (tools/gpu_round_counts.py)
@@ -508,7 +484,7 @@ __device__ unsigned long long g_round_stats[16 * 3];
 template <int NOBS>
 __device__ __forceinline__ void solve_round_body(const DevTable& T, const DevParams& P, const SolveIO& io, int n_work, int t0,
                                                  int off, const Carry& cin, const Carry& cout, int* __restrict__ cnt_out,
-                                                 int round, int* __restrict__ fb_list, int* __restrict__ fb_count) {
+                                                 int round, PartLists* hdr, int* __restrict__ robust) {
   typedef typename ClsCfg<NOBS>::St St;
   const int t = t0 + threadIdx.x;
   const bool live = t < n_work;
@@ -527,32 +503,33 @@ __device__ __forceinline__ void solve_round_body(const DevTable& T, const DevPar
   if (live) unpark(cin, slot, pb, st, s);
   solve_round<true>(T, P, pb, st, s, round);
   park_or_finalize<NOBS>(T, P, io, live, live && !s.done && round + 1 < P.thread_max_rounds, b, pb, st, s, n_work, cout,
-                         cnt_out, off, fb_list, fb_count);
+                         cnt_out, off, hdr, robust);
 }
 
 // Round `round` (0-based, >= the class kernel's r0) of the first pass: 128 listed problems of one class per CTA, classes with more
-// rows first; CTAs beyond the list's counts exit at once.  Survivors go to the next list (cout, cnt_out), the others are
-// finalized as in the class kernel -- after the last round all of them.  cnt_clear: the header the next round kernel
-// appends to (read by the previous one, which has finished), zeroed here.
+// rows first; CTAs beyond the list's counts exit at once.  The survivors of the previous round are counted in
+// hdr->surv[round % 3] and parked in cin; survivors of this round go to hdr->surv[(round + 1) % 3] and cout, the others
+// are finalized as in the class kernel -- after the last round all of them.  hdr->surv[(round + 2) % 3], which the next
+// round kernel appends to (read by the previous one, which has finished), is zeroed here.
 template <bool ROUTED>
 __global__ void __launch_bounds__(SOLVE_THREADS, MPCB_SOLVE_CTAS)
 mpcb_solve_round_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ DevParams P,
-                        const __grid_constant__ SolveIO io, const int* __restrict__ pcnt, int nr,
-                        const int* __restrict__ cnt_in, const __grid_constant__ Carry cin, int* __restrict__ cnt_out,
-                        const __grid_constant__ Carry cout, int* __restrict__ cnt_clear, int round,
-                        int* __restrict__ fb_list, int* __restrict__ fb_count) {
+                        const __grid_constant__ SolveIO io, PartLists* hdr, int nr, const __grid_constant__ Carry cin,
+                        const __grid_constant__ Carry cout, int round, int* __restrict__ robust) {
   if (!ROUTED) nr = 1;
-  if (blockIdx.x == 0 && threadIdx.x < 3 * nr) cnt_clear[threadIdx.x] = 0;
+  const int* cnt_in = hdr->surv[round % 3];
+  int* cnt_out = hdr->surv[(round + 1) % 3];
+  if (blockIdx.x == 0 && threadIdx.x < 3 * nr) hdr->surv[(round + 2) % 3][threadIdx.x] = 0;
 #ifdef MPCB_ROUND_STATS
   if (blockIdx.x == 0 && nr == 1 && threadIdx.x < 3 && round < 16) atomicAdd(&g_round_stats[3 * round + threadIdx.x], (unsigned long long)cnt_in[threadIdx.x]);
 #endif
   Part p;
-  if (!find_part(cnt_in, pcnt, nr, blockIdx.x, p)) return;                  // CTA-uniform from here on
-  MPCB_ASSERT(p.n >= 0 && p.n <= pcnt[p.key] && p.r >= 0 && p.r < Ts.n);
+  if (!find_part(cnt_in, hdr->part, nr, blockIdx.x, p)) return;             // CTA-uniform from here on
+  MPCB_ASSERT(p.n >= 0 && p.n <= hdr->part[p.key] && p.r >= 0 && p.r < Ts.n);
   const DevTable& T = Ts.t[ROUTED ? p.r : 0];
-  if (p.k == 2) solve_round_body<2>(T, P, io, p.n, p.t0, p.off, cin, cout, cnt_out + p.key, round, fb_list, fb_count);
-  else if (p.k == 1) solve_round_body<1>(T, P, io, p.n, p.t0, p.off, cin, cout, cnt_out + p.key, round, fb_list, fb_count);
-  else solve_round_body<0>(T, P, io, p.n, p.t0, p.off, cin, cout, cnt_out + p.key, round, fb_list, fb_count);
+  if (p.k == 2) solve_round_body<2>(T, P, io, p.n, p.t0, p.off, cin, cout, cnt_out + p.key, round, hdr, robust);
+  else if (p.k == 1) solve_round_body<1>(T, P, io, p.n, p.t0, p.off, cin, cout, cnt_out + p.key, round, hdr, robust);
+  else solve_round_body<0>(T, P, io, p.n, p.t0, p.off, cin, cout, cnt_out + p.key, round, hdr, robust);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -565,14 +542,12 @@ constexpr int COOP_WARPS = 4;
 #define MPCB_COOP_CTAS 2
 #endif
 constexpr int COOP_CTAS = MPCB_COOP_CTAS;   // CTAs per SM the kernel is compiled for
-constexpr int FB_HDR = 4;               // work-list header: count, cursor of the first pass, cursor of the second, pad
 constexpr size_t COOP_SMEM = sizeof(WarpShared) * COOP_WARPS;
 
 template <bool FIRST_PASS>
 __global__ void __launch_bounds__(COOP_WARPS * 32, COOP_CTAS)
 mpcb_coop_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ DevParams P, int B,
-                 const __grid_constant__ SolveIO io, int* __restrict__ fb_list, int* __restrict__ fb_count,
-                 int* __restrict__ cursor) {
+                 const __grid_constant__ SolveIO io, PartLists* hdr, int* __restrict__ robust) {
   extern __shared__ double coop_smem[];
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   WarpShared& ws = reinterpret_cast<WarpShared*>(coop_smem)[wid];
@@ -580,7 +555,7 @@ mpcb_coop_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ D
   const int n_work = idx ? min(*io.n_idx, B) : B;
   for (;;) {
     int t = 0;
-    if (lane == 0) t = atomicAdd(cursor, 1);
+    if (lane == 0) t = atomicAdd(&hdr->cursor[FIRST_PASS ? 0 : 1], 1);
     t = __shfl_sync(0xffffffffu, t, 0);
     if (t >= n_work) break;
     const int b = idx ? idx[t] : t;
@@ -605,7 +580,7 @@ mpcb_coop_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ D
       __syncwarp();
     }
     const SolveOut so = coop_solve<FIRST_PASS>(T, P, ws, lane, FIRST_PASS && io.U_start != nullptr);
-    if (lane == 0) finalize<FIRST_PASS>(T, P, ws.pb, so, b, io.accumulate != 0, io, fb_list, fb_count);
+    if (lane == 0) finalize<FIRST_PASS>(T, P, ws.pb, so, b, io.accumulate != 0, io, hdr, robust);
     __syncwarp();
   }
 }
@@ -947,7 +922,7 @@ int mpcb_create_routes(mpcb_handle* out, const mpcb_params* p, const mpcb_table_
       (e = cudaFuncSetAttribute(mpcb_solve_cls_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
       (e = cudaFuncSetAttribute(mpcb_solve_round_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
       (e = cudaFuncSetAttribute(mpcb_solve_round_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
-      (e = cudaFuncSetAttribute(mpcb_solve_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SOLVE_SMEM)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(mpcb_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SOLVE_SMEM)) != cudaSuccess ||
       (e = cudaFuncSetAttribute(mpcb_coop_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)COOP_SMEM)) != cudaSuccess ||
       (e = cudaFuncSetAttribute(mpcb_coop_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)COOP_SMEM)) != cudaSuccess)
     return fail(cuda_fail(e, "cudaFuncSetAttribute"));
@@ -972,7 +947,7 @@ int mpcb_destroy(mpcb_handle h) {
   }
   if (h->ev_fork) cudaEventDestroy(h->ev_fork);
   if (h->ws) cudaFree(h->ws);
-  if (h->fb) cudaFree(h->fb);                      // fb, cls, carry and route_cnt are one block
+  if (h->lists) cudaFree(h->lists);
   if (h->ev0) cudaEventDestroy(h->ev0);
   if (h->ev1) cudaEventDestroy(h->ev1);
   if (h->ev_mid) cudaEventDestroy(h->ev_mid);
@@ -994,25 +969,43 @@ int mpcb_destroy(mpcb_handle h) {
 static const int HOST_CHUNKS = MPCB_HOST_CHUNKS;   // parts of a large host batch, dealt round-robin onto the 4 streams
 static size_t al256(size_t x) { return (x + 255) & ~(size_t)255; }
 
-// fb, cls and carry are one allocation, so that h->fb (in the graph key) stands for all three.  A part whose work list
-// starts at fb + o keeps its class-list header and three lists at cls + 3 o, and its survivor-list headers and two carry
-// workspaces at carry + 2 o CARRY_SLOT_BYTES (FB_HDR == CLS_HDR, so the slices of the parts of a chunked host call do not
-// overlap; FB_HDR carry slots hold the headers).  route_cnt, at the end, serves routed calls, which are never chunked.
-static_assert(sizeof(int) * CARRY_HDR <= FB_HDR * 2 * CARRY_SLOT_BYTES, "survivor-list headers outgrow their slots");
-static int ensure_fb(mpcb_handle h, int B) {
-  if (!h->params.fast_pass || B + FB_HDR * HOST_CHUNKS <= h->fb_cap) return MPCB_OK;
-  if (h->fb) { CK(cudaFree(h->fb)); h->fb = nullptr; h->cls = nullptr; h->carry = nullptr; h->route_cnt = nullptr; h->fb_cap = 0; }
-  const size_t cap = (size_t)B + FB_HDR * HOST_CHUNKS;
-  const size_t o_cls = al256(sizeof(int) * cap), o_carry = o_cls + al256(sizeof(int) * 3 * cap),
-               o_route = o_carry + al256(2 * cap * CARRY_SLOT_BYTES);
-  void* p = nullptr;
-  if (cudaMalloc(&p, o_route + sizeof(int) * 2 * ROUTE_CNT) != cudaSuccess) { cudaGetLastError(); return MPCB_ERR_NOMEM; }
-  h->fb = (int*)p;
-  h->cls = (int*)((char*)p + o_cls);
-  h->carry = (char*)p + o_carry;
-  h->route_cnt = (int*)((char*)p + o_route);
-  h->fb_cap = (int)cap;
+// The lists of a handle are one block of capacity cap, so that its address and cap (in the graph key) stand for all of
+// them.  Its regions, each 256-byte aligned: the headers PartLists[HOST_CHUNKS], the robust pass's list (cap ints), the
+// class lists (3 cap ints) and the carry workspace (2 cap slots).  lists_offset(k, cap): offset of region k (4: size).
+static size_t lists_offset(int k, size_t cap) {
+  const size_t bytes[4] = {sizeof(PartLists) * HOST_CHUNKS, sizeof(int) * cap, sizeof(int) * 3 * cap,
+                           2 * cap * CARRY_SLOT_BYTES};
+  size_t o = 0;
+  for (int i = 0; i < k; ++i) o += al256(bytes[i]);
+  return o;
+}
+
+static int ensure_lists(mpcb_handle h, int B) {
+  if (!h->params.fast_pass || B <= h->lists_cap) return MPCB_OK;
+  if (h->lists) { CK(cudaFree(h->lists)); h->lists = nullptr; h->lists_cap = 0; }
+  if (cudaMalloc((void**)&h->lists, lists_offset(4, B)) != cudaSuccess) { cudaGetLastError(); return MPCB_ERR_NOMEM; }
+  h->lists_cap = B;
   return MPCB_OK;
+}
+
+// What part c of a call, problems [lo, lo + n) of the block's capacity, works with: header c, the robust list from lo,
+// its three class lists of n from 3 lo, and its two carry workspaces of n slots from slot 2 lo.  The parts of a chunked
+// host call cover disjoint problems, so their lists do not overlap.
+struct PartView {
+  PartLists* hdr;
+  int* robust;      // problems left to the robust pass
+  int* cls;         // class k at cls + k n
+  Carry wk[2];      // ping-pong survivor workspaces of the first pass
+};
+
+static PartView part_view(mpcb_handle h, int c, size_t lo, size_t n) {
+  if (!h->lists) return PartView{};                      // fast_pass = 0: one pass, no lists
+  const size_t cap = h->lists_cap;
+  int* robust = (int*)(h->lists + lists_offset(1, cap)) + lo;
+  int* cls = (int*)(h->lists + lists_offset(2, cap)) + 3 * lo;
+  char* carry = h->lists + lists_offset(3, cap) + 2 * lo * CARRY_SLOT_BYTES;
+  return PartView{(PartLists*)h->lists + c, robust, cls,
+                  {Carry::at(carry, (int)n), Carry::at(carry + n * CARRY_SLOT_BYTES, (int)n)}};
 }
 
 // Timing events: inside a stream capture a plain cudaEventRecord does not become a node of the graph (the event would be
@@ -1029,51 +1022,36 @@ static cudaError_t record_event(cudaEvent_t ev, cudaStream_t st) {
 // call keep the shape of the whole call and host and device entry points agree bit for bit).
 static bool call_uses_coop(mpcb_handle h, int B_total) { return h->params.fast_pass && B_total <= h->params.coop_max_batch; }
 
-// Enqueue the solve of B problems on `st`.  fb = [count, cursor, cursor, pad, idx[B]] (device ints) for the two-pass scheme.
+// Enqueue the solve of B problems on `st`, with the lists of v (part_view) for the two-pass scheme.
 // timed: bracket the passes with the handle's events (single-stream callers only).
 // use_coop: first pass one warp per problem (call_uses_coop of the WHOLE call).  part: one part of a chunked host call
 // (second-pass grid sized for the expected leftovers, so that the parts do not queue whole grids of idle CTAs behind
 // each other's first passes); otherwise the second pass gets the full persistent grid -- a closed-loop step near a stop
 // line leaves a fifth of its problems to it, not the 1.4 % of the Monte-Carlo set.
-static int launch_solve(mpcb_handle h, int B, const SolveIO& io_in, cudaStream_t st, int* fb, bool timed, bool use_coop,
-                        bool part = false) {
+static int launch_solve(mpcb_handle h, int B, const SolveIO& io_in, cudaStream_t st, const PartView& v, bool timed,
+                        bool use_coop, bool part = false) {
   const int grid = (B + SOLVE_THREADS - 1) / SOLVE_THREADS;
   SolveIO io = io_in;
   io.n_total = B;
   h->last_shape = (h->params.fast_pass && use_coop) ? 1 : 0;
   if (timed) CK(record_event(h->ev0, st));
   if (h->params.fast_pass) {
-    int* fb_count = fb;
-    int* fb_list = fb + FB_HDR;
-    CK(cudaMemsetAsync(fb, 0, sizeof(int) * FB_HDR, st));
+    CK(cudaMemsetAsync(v.hdr, 0, sizeof(PartLists), st));
     if (use_coop) {
       // small batch: too few problems to fill the GPU with one thread each -> one warp per problem, for latency
       const int g1 = std::min((B + COOP_WARPS - 1) / COOP_WARPS, h->n_sm * COOP_CTAS);
-      mpcb_coop_kernel<true><<<g1, COOP_WARPS * 32, COOP_SMEM, st>>>(h->dt, h->dp, B, io, fb_list, fb_count, fb + 1);
+      mpcb_coop_kernel<true><<<g1, COOP_WARPS * 32, COOP_SMEM, st>>>(h->dt, h->dp, B, io, v.hdr, v.robust);
     } else {
-      // partition by obstacle count -- and route, in a routed call -- then one CTA per 128 problems of one part (at most
-      // one partly filled CTA per part more than the unpartitioned grid)
-      int* cls = h->cls + (fb - h->fb) * 3;                    // this part's slice: header + three lists of B
-      char* cw = h->carry + (size_t)(fb - h->fb) * 2 * CARRY_SLOT_BYTES;   // survivor-list headers, two workspaces of B
-      int* hdr = (int*)cw;                                     // headers: survivors after round r at hdr + CARRY_HDR_STRIDE (r % 3)
-      const size_t w0 = FB_HDR * 2 * CARRY_SLOT_BYTES;
-      const Carry wk[2] = {Carry::at(cw + w0, B), Carry::at(cw + w0 + (size_t)B * CARRY_SLOT_BYTES, B)};
+      // partition by obstacle count -- and route, in a routed call, whose parts are counted first -- then one CTA per
+      // 128 problems of one part (at most one partly filled CTA per part more than the unpartitioned grid)
       const int n_routes = h->dt.n;
-      const int* pcnt = cls;                                   // part sizes: the class-list header ...
-      int nr = 1;
-      if (io.route) {                                          // ... or, routed, counted per (class, route) first
-        if (fb != h->fb) return MPCB_ERR_INVALID;              // (routed calls are never chunked)
-        pcnt = h->route_cnt;
-        nr = n_routes;
-        CK(cudaMemsetAsync(h->route_cnt, 0, sizeof(int) * 2 * ROUTE_CNT, st));
-        mpcb_classify_kernel<<<(B + 255) / 256, 256, 0, st>>>(B, io, n_routes, nr, nullptr, h->route_cnt, nullptr, hdr);
+      const int nr = io.route ? n_routes : 1;
+      if (io.route) {
+        mpcb_classify_kernel<<<(B + 255) / 256, 256, 0, st>>>(B, io, n_routes, nr, v.hdr, nullptr);
         CK(cudaGetLastError());
         h->launches++;
-        mpcb_classify_kernel<<<(B + 255) / 256, 256, 0, st>>>(B, io, n_routes, nr, pcnt, h->route_cnt + ROUTE_CNT, cls, hdr);
-      } else {
-        CK(cudaMemsetAsync(cls, 0, sizeof(int) * CLS_HDR, st));
-        mpcb_classify_kernel<<<(B + 255) / 256, 256, 0, st>>>(B, io, n_routes, 1, nullptr, cls, cls, hdr);
       }
+      mpcb_classify_kernel<<<(B + 255) / 256, 256, 0, st>>>(B, io, n_routes, nr, v.hdr, v.cls);
       CK(cudaGetLastError());
       SolveIO io1 = io;
       io1.idx = nullptr; io1.n_idx = nullptr;                  // the class lists carry the problem indices from here on
@@ -1085,16 +1063,13 @@ static int launch_solve(mpcb_handle h, int B, const SolveIO& io_in, cudaStream_t
       const int grid1 = grid + 3 * nr - 1;
       const auto cls_kernel = io.route ? mpcb_solve_cls_kernel<true> : mpcb_solve_cls_kernel<false>;
       const auto round_kernel = io.route ? mpcb_solve_round_kernel<true> : mpcb_solve_round_kernel<false>;
-      cls_kernel<<<grid1, SOLVE_THREADS, CLS_SMEM, st>>>(h->dt, h->dp, B, io1, cls, pcnt, nr, r0, wk[0],
-                                                         hdr + CARRY_HDR_STRIDE * (r0 % 3), fb_list, fb_count);
+      cls_kernel<<<grid1, SOLVE_THREADS, CLS_SMEM, st>>>(h->dt, h->dp, B, io1, v.hdr, v.cls, nr, r0, v.wk[0], v.robust);
       h->launches++;
       // the rounds after r0 over the packed survivors, one launch per round (workspaces ping-pong; each kernel zeroes
-      // the header its successor appends to)
+      // the survivor count its successor appends to)
       for (int r = r0; r < max_rounds; ++r) {
         const int p = (r - r0) & 1;
-        round_kernel<<<grid1, SOLVE_THREADS, CLS_SMEM, st>>>(h->dt, h->dp, io1, pcnt, nr, hdr + CARRY_HDR_STRIDE * (r % 3), wk[p],
-                                                             hdr + CARRY_HDR_STRIDE * ((r + 1) % 3), wk[p ^ 1],
-                                                             hdr + CARRY_HDR_STRIDE * ((r + 2) % 3), r, fb_list, fb_count);
+        round_kernel<<<grid1, SOLVE_THREADS, CLS_SMEM, st>>>(h->dt, h->dp, io1, v.hdr, nr, v.wk[p], v.wk[p ^ 1], r, v.robust);
         h->launches++;
       }
     }
@@ -1102,25 +1077,25 @@ static int launch_solve(mpcb_handle h, int B, const SolveIO& io_in, cudaStream_t
     if (timed) CK(record_event(h->ev_mid, st));
     // second pass over whatever the first did not certify
     SolveIO io2 = io;
-    io2.idx = fb_list;
-    io2.n_idx = fb_count;
+    io2.idx = v.robust;
+    io2.n_idx = &v.hdr->n_robust;
     io2.accumulate = 1;
     if (h->params.coop_pass2) {
       // one warp per problem: the leftovers are few and hard, what matters is their latency
       const int full = std::min(h->n_sm * COOP_CTAS, (B + COOP_WARPS - 1) / COOP_WARPS);
       const int g2 = (part && !use_coop) ? std::min(full, std::max(16, (B + 63) / 64)) : full;
-      mpcb_coop_kernel<false><<<g2, COOP_WARPS * 32, COOP_SMEM, st>>>(h->dt, h->dp, B, io2, nullptr, nullptr, fb + 2);
+      mpcb_coop_kernel<false><<<g2, COOP_WARPS * 32, COOP_SMEM, st>>>(h->dt, h->dp, B, io2, v.hdr, v.robust);
     } else {
       // thread per problem; CTAs beyond the list length exit at once (one warp per CTA when the working set is
       // thread-local: the few leftover warps then never wait for each other)
       const int t2 = (MPCB_STORE_MASK == 0) ? 32 : SOLVE_THREADS;
-      mpcb_solve_kernel<false><<<(B + t2 - 1) / t2, t2, SOLVE_SMEM, st>>>(h->dt, h->dp, B, io2, nullptr, nullptr);
+      mpcb_solve_kernel<<<(B + t2 - 1) / t2, t2, SOLVE_SMEM, st>>>(h->dt, h->dp, B, io2);
     }
     CK(cudaGetLastError());
     h->launches += 2;
   } else {
     if (timed) CK(record_event(h->ev_mid, st));
-    mpcb_solve_kernel<false><<<grid, SOLVE_THREADS, SOLVE_SMEM, st>>>(h->dt, h->dp, B, io, nullptr, nullptr);
+    mpcb_solve_kernel<<<grid, SOLVE_THREADS, SOLVE_SMEM, st>>>(h->dt, h->dp, B, io);
     CK(cudaGetLastError());
     h->launches++;
   }
@@ -1128,7 +1103,7 @@ static int launch_solve(mpcb_handle h, int B, const SolveIO& io_in, cudaStream_t
     CK(record_event(h->ev1, st));
     h->timed = true;
     h->pass_timed = true;
-    h->fb_last = fb;
+    h->lists_last = v.hdr;
   }
   return MPCB_OK;
 }
@@ -1158,11 +1133,11 @@ int mpcb_solve_batch_routes(mpcb_handle h, int B, const double* x0, const double
   if ((((size_t)U_out) | ((size_t)Xpred_out)) & 15u) return MPCB_ERR_INVALID;      // rows are written with 128-bit stores
   if (B == 0) return MPCB_OK;
   CK(cudaSetDevice(h->device));
-  int rc = ensure_fb(h, B);
+  int rc = ensure_lists(h, B);
   if (rc != MPCB_OK) return rc;
   SolveIO io = make_io(x0, obs_sv, n_obs, U_out, Xpred_out, obj_out, status_out, iters_out, cmin_out, active_out);
   io.route = route;
-  return launch_solve(h, B, io, (cudaStream_t)cuda_stream, h->fb, true, call_uses_coop(h, B));
+  return launch_solve(h, B, io, (cudaStream_t)cuda_stream, part_view(h, 0, 0, B), true, call_uses_coop(h, B));
 }
 
 // Solve the problems idx[0 .. *n_idx - 1] of a batch of B (both on the device; the closed loop's list of vehicles that
@@ -1170,7 +1145,7 @@ int mpcb_solve_batch_routes(mpcb_handle h, int B, const double* x0, const double
 int mpcb_solve_list_internal(mpcb_handle h, int B, const int* idx, const int* n_idx, const double* x0, const double* obs_sv,
                              const int* n_obs, const int* route, double* U_out, int* status_out, cudaStream_t st,
                              const double* U_start) {
-  int rc = ensure_fb(h, B);
+  int rc = ensure_lists(h, B);
   if (rc != MPCB_OK) return rc;
   SolveIO io = make_io(x0, obs_sv, n_obs, U_out, nullptr, nullptr, status_out, nullptr, nullptr, nullptr);
   io.route = route;
@@ -1178,7 +1153,7 @@ int mpcb_solve_list_internal(mpcb_handle h, int B, const int* idx, const int* n_
   io.n_idx = n_idx;
   io.U_start = U_start;          // closed loop: the previous step's plans (U_out itself), advanced by one step
   io.shift_start = 1;
-  return launch_solve(h, B, io, st, h->fb, true, call_uses_coop(h, B));
+  return launch_solve(h, B, io, st, part_view(h, 0, 0, B), true, call_uses_coop(h, B));
 }
 
 // Lower edge of part c of a chunked host call, as a fraction of the batch (measured on B200, 65,536 problems: equal parts
@@ -1225,7 +1200,7 @@ static int solve_host(mpcb_handle h, int B, const double* x0, const double* obs_
     if (cudaMalloc(&h->ws, total) != cudaSuccess) { cudaGetLastError(); return MPCB_ERR_NOMEM; }
     h->ws_bytes = total;
   }
-  int rc = ensure_fb(h, B);
+  int rc = ensure_lists(h, B);
   if (rc != MPCB_OK) return rc;
   char* w = (char*)h->ws;
   double* dU = (double*)(w + o_U);
@@ -1251,11 +1226,11 @@ static int solve_host(mpcb_handle h, int B, const double* x0, const double* obs_
   // everything the enqueued work depends on: batch size, which outputs are wanted, the library's own buffers, and
   // (chunked path: the copies go straight from / to the caller's arrays) the caller's pointers
   const void* up[11] = {x0, obs_sv, n_obs, U_out, Xpred_out, obj_out, status_out, iters_out, cmin_out, active_out, u0_out};
-  unsigned long long key[16] = {(unsigned long long)B, (unsigned long long)(size_t)h->ws, (unsigned long long)(size_t)h->fb,
+  unsigned long long key[16] = {(unsigned long long)B, (unsigned long long)(size_t)h->ws, (unsigned long long)(size_t)h->lists,
                                 (unsigned long long)(size_t)h->pin, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
   for (int k = 3; k < 11; ++k) key[4] |= (unsigned long long)(up[k] != nullptr) << k;
   key[4] |= (unsigned long long)(wait ? 0 : 1) << 32;
-  key[4] |= (unsigned long long)h->fb_cap << 33;           // layout of the fb / cls / carry block
+  key[4] |= (unsigned long long)h->lists_cap << 33;        // layout of the list block
   if (!packed)
     for (int k = 0; k < 11; ++k) key[5 + k] = (unsigned long long)(size_t)up[k];
   const bool hit = g.valid && memcmp(g.key, key, sizeof(key)) == 0;
@@ -1285,7 +1260,7 @@ static int solve_host(mpcb_handle h, int B, const double* x0, const double* obs_
       char* p = (char*)h->pin;
       CK(cudaMemcpyAsync(w, p, o_U, cudaMemcpyHostToDevice, s0));
       int r = launch_solve(h, B, make_io((double*)(w + o_x0), (double*)(w + o_obs), (int*)(w + o_n), dU, dX, dobj, dst, dit, dcm,
-                                         dac, du0), s0, h->fb, true, use_coop);
+                                         dac, du0), s0, part_view(h, 0, 0, nb), true, use_coop);
       if (r != MPCB_OK) return r;
       // results: one copy of the whole output region, or -- closed-loop form -- the three small blocks only
       if (U_out) CK(cudaMemcpyAsync(p + o_U, w + o_U, total - o_U, cudaMemcpyDeviceToHost, s0));
@@ -1320,7 +1295,7 @@ static int solve_host(mpcb_handle h, int B, const double* x0, const double* obs_
                                    dX ? dX + lo * 30 : nullptr, dobj ? dobj + lo : nullptr, dst ? dst + lo : nullptr,
                                    dit ? dit + lo * 2 : nullptr, dcm ? dcm + lo : nullptr, dac ? dac + lo : nullptr,
                                    du0 ? du0 + lo * 2 : nullptr),
-                           st, h->fb + lo + FB_HDR * c, false, use_coop, nparts > 1);
+                           st, part_view(h, c, lo, n), false, use_coop, nparts > 1);
       if (r != MPCB_OK) return r;
       if (U_out) CK(cudaMemcpyAsync(U_out + lo * 10, dU + lo * 10, n * 80, cudaMemcpyDeviceToHost, st));
       if (u0_out) CK(cudaMemcpyAsync(u0_out + lo * 2, du0 + lo * 2, n * 16, cudaMemcpyDeviceToHost, st));
@@ -1370,7 +1345,7 @@ static int solve_host(mpcb_handle h, int B, const double* x0, const double* obs_
     h->launches += g.launches;
     h->timed = true;           // mpcb_last_kernel_ms: chunked path = device span of the whole call (copies included)
     h->pass_timed = packed;    // packed path: the graph's own event-record nodes (ev0, ev_mid, ev1) fire on every replay
-    h->fb_last = h->fb;
+    h->lists_last = part_view(h, 0, 0, nb).hdr;
   } else {
     if (!packed) CK(cudaEventRecord(h->ev0, s0));
     rc = enqueue();
@@ -1488,7 +1463,8 @@ int mpcb_last_pass_ms(mpcb_handle h, float* first_ms, float* second_ms, int* n_s
   if (second_ms) *second_ms = b;
   if (n_second) {
     *n_second = 0;
-    if (h->params.fast_pass && h->fb_last) CK(cudaMemcpy(n_second, h->fb_last, sizeof(int), cudaMemcpyDeviceToHost));
+    if (h->params.fast_pass && h->lists_last)
+      CK(cudaMemcpy(n_second, &h->lists_last->n_robust, sizeof(int), cudaMemcpyDeviceToHost));
   }
   return MPCB_OK;
 }

@@ -84,6 +84,20 @@ MPCB_HD int problem_route(const int* __restrict__ route, int b, int n) {
   return (r >= 0 && r < n) ? r : -1;
 }
 
+#ifdef __CUDACC__
+// Slot of this thread in a list (warp-aggregated append to counter; every lane of the warp calls it), -1 if !pred.
+__device__ __forceinline__ int warp_append(bool pred, int* counter) {
+  const unsigned m = __ballot_sync(0xffffffffu, pred);
+  if (m == 0u) return -1;
+  const unsigned lane = threadIdx.x & 31u;
+  const int leader = __ffs(m) - 1;
+  int base = 0;
+  if ((int)lane == leader) base = atomicAdd(counter, __popc(m));
+  base = __shfl_sync(0xffffffffu, base, leader);
+  return pred ? base + __popc(m & ((1u << lane) - 1u)) : -1;
+}
+#endif
+
 // Step-size policy of the ADMM machinery (mpcb_solver.cuh).
 struct Policy {
   double lad[MAXRUNG];        // step-size ladder

@@ -9,6 +9,8 @@
 extern thread_local char g_cuda_err[512];
 int cuda_fail(cudaError_t e, const char* where);
 
+namespace mpcb { struct PartLists; }
+
 #define CK(call)                                        \
   do {                                                  \
     cudaError_t e_ = (call);                            \
@@ -24,18 +26,15 @@ struct mpcb_ctx {
   // workspace for the host-buffer entry points
   void* ws = nullptr;
   size_t ws_bytes = 0;
-  int* fb = nullptr;          // work list(s): header (count, two cursors, pad), then indices of problems left to the second pass
-  int fb_cap = 0;
-  int* cls = nullptr;         // class lists of the first pass (problems by obstacle count), 3x the size of fb
-  char* carry = nullptr;      // survivor lists of the first pass and the state they carry between rounds (ensure_fb)
-  int* route_cnt = nullptr;   // routed first pass: sizes of its (class, route) parts and their cursors (ensure_fb)
+  char* lists = nullptr;      // work lists of the solve passes and the state the first pass carries (ensure_lists)
+  int lists_cap = 0;          // problems they hold
   cudaStream_t stream = nullptr;   // private stream of the *_host entry points
   cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_mid = nullptr;
   cudaStream_t xs[4] = {nullptr, nullptr, nullptr, nullptr};   // xs[0] == stream; one stream per part of a large host batch
   cudaEvent_t xe[4] = {nullptr, nullptr, nullptr, nullptr};
   void* pin = nullptr;             // pinned staging block of the packed small-batch path
   size_t pin_bytes = 0;
-  int* fb_last = nullptr;          // list used by the last timed solve
+  mpcb::PartLists* lists_last = nullptr;   // header of the last timed solve
   bool timed = false;
   bool pass_timed = false;
   int last_shape = 0;              // first pass of the last solve: 0 thread per problem, 1 warp per problem

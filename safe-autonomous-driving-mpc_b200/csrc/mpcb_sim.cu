@@ -54,14 +54,8 @@ mpcb_fsm_kernel(const __grid_constant__ DevTables Ts, const int* __restrict__ ro
   const int live = (in && s <= stop_s(Ts, route, b)) ? 1 : 0;   // loop condition (:395), evaluated before the step
   // list of the vehicles still driving: the solve of this step runs over the list, not over all B (one atomic per warp;
   // the order of the list does not matter, every problem is solved on its own and written to its own slot)
-  {
-    const unsigned m = __ballot_sync(0xffffffffu, live);
-    const int lane = threadIdx.x & 31;
-    int base = 0;
-    if (lane == 0 && m) base = atomicAdd(alive_cnt, __popc(m));
-    base = __shfl_sync(0xffffffffu, base, 0);
-    if (live) alive_idx[base + __popc(m & ((1u << lane) - 1u))] = b;
-  }
+  const int slot = warp_append(live, alive_cnt);
+  if (live) alive_idx[slot] = b;
   if (!in) return;
   alive[b] = live;
   int n = 0;
