@@ -962,12 +962,7 @@ int mpcb_destroy(mpcb_handle h) {
 }
 
 // ---- solve ---------------------------------------------------------------------------------------
-// fallback-list storage for a batch of B problems split into up to HOST_CHUNKS independently launched parts
-#ifndef MPCB_HOST_CHUNKS
-#define MPCB_HOST_CHUNKS 4
-#endif
-static const int HOST_CHUNKS = MPCB_HOST_CHUNKS;   // parts of a large host batch, dealt round-robin onto the 4 streams
-static size_t al256(size_t x) { return (x + 255) & ~(size_t)255; }
+static const int HOST_CHUNKS = 4;   // parts of a large host batch, one per stream xs[c]
 
 // The lists of a handle are one block of capacity cap, so that its address and cap (in the graph key) stand for all of
 // them.  Its regions, each 256-byte aligned: the headers PartLists[HOST_CHUNKS], the robust pass's list (cap ints), the
@@ -975,9 +970,9 @@ static size_t al256(size_t x) { return (x + 255) & ~(size_t)255; }
 static size_t lists_offset(int k, size_t cap) {
   const size_t bytes[4] = {sizeof(PartLists) * HOST_CHUNKS, sizeof(int) * cap, sizeof(int) * 3 * cap,
                            2 * cap * CARRY_SLOT_BYTES};
-  size_t o = 0;
-  for (int i = 0; i < k; ++i) o += al256(bytes[i]);
-  return o;
+  size_t off[5];
+  region_offsets(bytes, 4, off);
+  return off[k];
 }
 
 static int ensure_lists(mpcb_handle h, int B) {
@@ -1108,17 +1103,6 @@ static int launch_solve(mpcb_handle h, int B, const SolveIO& io_in, cudaStream_t
   return MPCB_OK;
 }
 
-static SolveIO make_io(const double* x0, const double* obs_sv, const int* n_obs, double* U_out, double* Xpred_out,
-                       double* obj_out, int* status_out, int* iters_out, double* cmin_out, unsigned long long* active_out,
-                       double* u0_out = nullptr) {
-  SolveIO io;
-  io.x0 = x0; io.obs_sv = obs_sv; io.n_obs = n_obs; io.U = U_out; io.Xpred = Xpred_out; io.obj = obj_out;
-  io.status = status_out; io.iters = iters_out; io.cmin = cmin_out; io.active = active_out; io.u0 = u0_out;
-  io.idx = nullptr; io.n_idx = nullptr; io.accumulate = 0; io.n_total = 0; io.U_start = nullptr; io.shift_start = 0;
-  io.route = nullptr;
-  return io;
-}
-
 int mpcb_solve_batch(mpcb_handle h, int B, const double* x0, const double* obs_sv, const int* n_obs, double* U_out,
                      double* Xpred_out, double* obj_out, int* status_out, int* iters_out, double* cmin_out,
                      unsigned long long* active_out, void* cuda_stream) {
@@ -1135,8 +1119,10 @@ int mpcb_solve_batch_routes(mpcb_handle h, int B, const double* x0, const double
   CK(cudaSetDevice(h->device));
   int rc = ensure_lists(h, B);
   if (rc != MPCB_OK) return rc;
-  SolveIO io = make_io(x0, obs_sv, n_obs, U_out, Xpred_out, obj_out, status_out, iters_out, cmin_out, active_out);
-  io.route = route;
+  SolveIO io{};
+  io.x0 = x0; io.obs_sv = obs_sv; io.n_obs = n_obs; io.route = route;
+  io.U = U_out; io.Xpred = Xpred_out; io.obj = obj_out; io.status = status_out; io.iters = iters_out; io.cmin = cmin_out;
+  io.active = active_out;
   return launch_solve(h, B, io, (cudaStream_t)cuda_stream, part_view(h, 0, 0, B), true, call_uses_coop(h, B));
 }
 
@@ -1147,8 +1133,8 @@ int mpcb_solve_list_internal(mpcb_handle h, int B, const int* idx, const int* n_
                              const double* U_start) {
   int rc = ensure_lists(h, B);
   if (rc != MPCB_OK) return rc;
-  SolveIO io = make_io(x0, obs_sv, n_obs, U_out, nullptr, nullptr, status_out, nullptr, nullptr, nullptr);
-  io.route = route;
+  SolveIO io{};
+  io.x0 = x0; io.obs_sv = obs_sv; io.n_obs = n_obs; io.route = route; io.U = U_out; io.status = status_out;
   io.idx = idx;
   io.n_idx = n_idx;
   io.U_start = U_start;          // closed loop: the previous step's plans (U_out itself), advanced by one step
@@ -1156,31 +1142,42 @@ int mpcb_solve_list_internal(mpcb_handle h, int B, const int* idx, const int* n_
   return launch_solve(h, B, io, st, part_view(h, 0, 0, B), true, call_uses_coop(h, B));
 }
 
-// Lower edge of part c of a chunked host call, as a fraction of the batch (measured on B200, 65,536 problems: equal parts
-// 1.08 ms, 1/8 - 1/4 - 5/16 - 5/16 1.05 ms).
-static double part_edge(int c) {
-  static double edges[17];
-  static bool init = false;
-  if (!init) {
-    for (int k = 0; k <= HOST_CHUNKS; ++k) edges[k] = (double)k / HOST_CHUNKS;
-    if (HOST_CHUNKS == 4) { edges[1] = 0.125; edges[2] = 0.375; edges[3] = 0.6875; }   // small first part: its results start
-                                                                                       // the device-to-host stream earlier
-#ifdef MPCB_DEV
-    if (const char* e = getenv("MPCB_HOST_SPLIT")) {     // development builds only: "e1,e2,.." overrides the inner edges
-      int k = 1;
-      while (*e && k < HOST_CHUNKS) { edges[k++] = atof(e); while (*e && *e != ',') ++e; if (*e == ',') ++e; }
-    }
-#endif
-    init = true;
-  }
-  return edges[c];
+// Lower edges of the parts of a chunked host call, as fractions of the batch: a small first part starts the
+// device-to-host stream earlier (measured on B200, 65,536 problems: equal parts 1.08 ms, 1/8 - 1/4 - 5/16 - 5/16 1.05 ms).
+static const double HOST_EDGES[HOST_CHUNKS + 1] = {0.0, 0.125, 0.375, 0.6875, 1.0};
+
+// The per-problem arrays of a host call, inputs first, in the order the chunked path copies them, and their bytes per
+// problem.  The workspace and staging layout, the copies and the graph key are all derived from this table.
+enum HostArray { HA_X0, HA_OBS, HA_NOBS, HA_U, HA_U0, HA_XPRED, HA_OBJ, HA_STATUS, HA_ITERS, HA_CMIN, HA_ACTIVE, N_HA };
+static const size_t HA_BYTES[N_HA] = {40, 32, 4, 80, 16, 240, 8, 4, 8, 8, 8};
+
+// Layout of a host call of n problems, in the device workspace and in the pinned staging block alike: array a at
+// off[a] (the inputs one contiguous block from 0, the outputs one from off[HA_U]), off[N_HA] bytes in all.
+static void host_layout(size_t n, size_t (&off)[N_HA + 1]) {
+  size_t bytes[N_HA];
+  for (int a = 0; a < N_HA; ++a) bytes[a] = n * HA_BYTES[a];
+  region_offsets(bytes, N_HA, off);
+}
+
+// The device arrays of problems lo.. of a host call in the workspace w: the inputs and U always (the kernels write U
+// whether or not the caller asked for it), every other output only when the caller passed an array for it (up[a]).
+static SolveIO host_io(char* w, const size_t* off, void* const* up, size_t lo) {
+  void* d[N_HA];
+  for (int a = 0; a < N_HA; ++a) d[a] = (a <= HA_U || up[a]) ? w + off[a] + lo * HA_BYTES[a] : nullptr;
+  SolveIO io{};
+  io.x0 = (const double*)d[HA_X0]; io.obs_sv = (const double*)d[HA_OBS]; io.n_obs = (const int*)d[HA_NOBS];
+  io.U = (double*)d[HA_U]; io.u0 = (double*)d[HA_U0]; io.Xpred = (double*)d[HA_XPRED]; io.obj = (double*)d[HA_OBJ];
+  io.status = (int*)d[HA_STATUS]; io.iters = (int*)d[HA_ITERS]; io.cmin = (double*)d[HA_CMIN];
+  io.active = (unsigned long long*)d[HA_ACTIVE];
+  return io;
 }
 
 // Host-buffer entry points.  Small batches (the reference's B = 1 call in particular) go through one packed pinned
-// staging block: one H2D copy, the two launches, one D2H copy.  Large batches are cut into HOST_CHUNKS parts on as many
-// streams, each part copying straight from / to the caller's arrays, so that the H2D of one part, the kernels of
-// another and the D2H of a third overlap (PCIe is full duplex) and the latency tails of the parts' robust passes overlap
-// each other.  U_out may be NULL when u0_out is given (the closed-loop form: only U*[0] and the flags come back).
+// staging block: one H2D copy of the inputs, the two launches, then one D2H copy of the whole output region when U is
+// wanted, else one copy per wanted output (the closed-loop form: U*[0] and the flags only).  Large batches are cut into
+// HOST_CHUNKS parts on as many streams, each part copying straight from / to the caller's arrays, so that the H2D of one
+// part, the kernels of another and the D2H of a third overlap (PCIe is full duplex) and the latency tails of the parts'
+// robust passes overlap each other.  U_out may be NULL when u0_out is given; any other output may be NULL.
 static const int HOST_PACKED_MAX = 2048;
 
 static int solve_host(mpcb_handle h, int B, const double* x0, const double* obs_sv, const int* n_obs,
@@ -1190,62 +1187,50 @@ static int solve_host(mpcb_handle h, int B, const double* x0, const double* obs_
   if (B == 0) return MPCB_OK;
   CK(cudaSetDevice(h->device));
   const size_t nb = (size_t)B;
-  // one layout for both paths; inputs first, outputs after (each block contiguous)
-  const size_t o_x0 = 0, o_obs = o_x0 + al256(nb * 40), o_n = o_obs + al256(nb * 32), o_U = o_n + al256(nb * 4),
-               o_X = o_U + al256(nb * 80), o_obj = o_X + al256(nb * 240), o_st = o_obj + al256(nb * 8),
-               o_it = o_st + al256(nb * 4), o_cm = o_it + al256(nb * 8), o_ac = o_cm + al256(nb * 8),
-               o_u0 = o_ac + al256(nb * 8), total = o_u0 + al256(nb * 16);
-  if (total > h->ws_bytes) {
+  void* const up[N_HA] = {(void*)x0, (void*)obs_sv, (void*)n_obs, U_out, u0_out, Xpred_out, obj_out, status_out,
+                          iters_out, cmin_out, active_out};
+  size_t off[N_HA + 1];
+  host_layout(nb, off);
+  if (off[N_HA] > h->ws_bytes) {
     if (h->ws) { cudaFree(h->ws); h->ws = nullptr; h->ws_bytes = 0; }
-    if (cudaMalloc(&h->ws, total) != cudaSuccess) { cudaGetLastError(); return MPCB_ERR_NOMEM; }
-    h->ws_bytes = total;
+    if (cudaMalloc(&h->ws, off[N_HA]) != cudaSuccess) { cudaGetLastError(); return MPCB_ERR_NOMEM; }
+    h->ws_bytes = off[N_HA];
   }
   int rc = ensure_lists(h, B);
   if (rc != MPCB_OK) return rc;
-  char* w = (char*)h->ws;
-  double* dU = (double*)(w + o_U);
-  double* dX = Xpred_out ? (double*)(w + o_X) : nullptr;
-  double* dobj = obj_out ? (double*)(w + o_obj) : nullptr;
-  int* dst = status_out ? (int*)(w + o_st) : nullptr;
-  int* dit = iters_out ? (int*)(w + o_it) : nullptr;
-  double* dcm = cmin_out ? (double*)(w + o_cm) : nullptr;
-  unsigned long long* dac = active_out ? (unsigned long long*)(w + o_ac) : nullptr;
-  double* du0 = u0_out ? (double*)(w + o_u0) : nullptr;
   const bool use_coop = call_uses_coop(h, B);
+  const bool packed = B <= HOST_PACKED_MAX;
+  if (packed && !h->pin) {                                 // sized once, for the largest packed batch
+    size_t pmax[N_HA + 1];
+    host_layout(HOST_PACKED_MAX, pmax);
+    if (cudaHostAlloc(&h->pin, pmax[N_HA], cudaHostAllocDefault) != cudaSuccess) { cudaGetLastError(); return MPCB_ERR_NOMEM; }
+  }
+  char* w = (char*)h->ws;
+  char* p = (char*)h->pin;
+  auto at = [&](char* base, int a, size_t lo) { return base + off[a] + lo * HA_BYTES[a]; };   // workspace or staging
+  auto user = [&](int a, size_t lo) { return (char*)up[a] + lo * HA_BYTES[a]; };              // caller's array
 
   // ---- graph replay / capture bookkeeping --------------------------------------------------------------------
-  const bool packed = B <= HOST_PACKED_MAX;
-  if (packed && total > h->pin_bytes) {
-    if (h->pin) { cudaFreeHost(h->pin); h->pin = nullptr; h->pin_bytes = 0; }
-    size_t want = total;
-    { const size_t nmax = HOST_PACKED_MAX; want = std::max(want, (size_t)(al256(nmax * 40) + al256(nmax * 32) + 2 * al256(nmax * 4) + al256(nmax * 80) + al256(nmax * 240) + 4 * al256(nmax * 8) + al256(nmax * 16))); }
-    if (cudaHostAlloc(&h->pin, want, cudaHostAllocDefault) != cudaSuccess) { cudaGetLastError(); return MPCB_ERR_NOMEM; }
-    h->pin_bytes = want;
-  }
   mpcb_ctx::GraphSlot& g = h->gslot[packed ? 0 : 1];
   // everything the enqueued work depends on: batch size, which outputs are wanted, the library's own buffers, and
   // (chunked path: the copies go straight from / to the caller's arrays) the caller's pointers
-  const void* up[11] = {x0, obs_sv, n_obs, U_out, Xpred_out, obj_out, status_out, iters_out, cmin_out, active_out, u0_out};
   unsigned long long key[16] = {(unsigned long long)B, (unsigned long long)(size_t)h->ws, (unsigned long long)(size_t)h->lists,
                                 (unsigned long long)(size_t)h->pin, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-  for (int k = 3; k < 11; ++k) key[4] |= (unsigned long long)(up[k] != nullptr) << k;
+  for (int a = HA_U; a < N_HA; ++a) key[4] |= (unsigned long long)(up[a] != nullptr) << a;
   key[4] |= (unsigned long long)(wait ? 0 : 1) << 32;
   key[4] |= (unsigned long long)h->lists_cap << 33;        // layout of the list block
   if (!packed)
-    for (int k = 0; k < 11; ++k) key[5 + k] = (unsigned long long)(size_t)up[k];
+    for (int a = 0; a < N_HA; ++a) key[5 + a] = (unsigned long long)(size_t)up[a];
   const bool hit = g.valid && memcmp(g.key, key, sizeof(key)) == 0;
   bool capture = false;
   if (!hit) {
     capture = g.have_last && memcmp(g.last, key, sizeof(key)) == 0;     // second call in a row with these buffers
-#ifdef MPCB_DEV
-    if (getenv("MPCB_NO_GRAPH")) capture = false;
-#endif
     if (capture && !packed) {
       // a graph replays the copies asynchronously: only for page-locked caller buffers
-      for (int k = 0; k < 11 && capture; ++k) {
-        if (!up[k]) continue;
-        cudaPointerAttributes at;
-        if (cudaPointerGetAttributes(&at, up[k]) != cudaSuccess || at.type != cudaMemoryTypeHost) { cudaGetLastError(); capture = false; }
+      for (int a = 0; a < N_HA && capture; ++a) {
+        if (!up[a]) continue;
+        cudaPointerAttributes pa;
+        if (cudaPointerGetAttributes(&pa, up[a]) != cudaSuccess || pa.type != cudaMemoryTypeHost) { cudaGetLastError(); capture = false; }
       }
     }
     memcpy(g.last, key, sizeof(key));
@@ -1257,18 +1242,13 @@ static int solve_host(mpcb_handle h, int B, const double* x0, const double* obs_
   // event-record nodes, see record_event)
   auto enqueue = [&]() -> int {
     if (packed) {
-      char* p = (char*)h->pin;
-      CK(cudaMemcpyAsync(w, p, o_U, cudaMemcpyHostToDevice, s0));
-      int r = launch_solve(h, B, make_io((double*)(w + o_x0), (double*)(w + o_obs), (int*)(w + o_n), dU, dX, dobj, dst, dit, dcm,
-                                         dac, du0), s0, part_view(h, 0, 0, nb), true, use_coop);
+      CK(cudaMemcpyAsync(w, p, off[HA_U], cudaMemcpyHostToDevice, s0));
+      int r = launch_solve(h, B, host_io(w, off, up, 0), s0, part_view(h, 0, 0, nb), true, use_coop);
       if (r != MPCB_OK) return r;
-      // results: one copy of the whole output region, or -- closed-loop form -- the three small blocks only
-      if (U_out) CK(cudaMemcpyAsync(p + o_U, w + o_U, total - o_U, cudaMemcpyDeviceToHost, s0));
-      else {
-        CK(cudaMemcpyAsync(p + o_u0, w + o_u0, nb * 16, cudaMemcpyDeviceToHost, s0));
-        if (status_out) CK(cudaMemcpyAsync(p + o_st, w + o_st, nb * 4, cudaMemcpyDeviceToHost, s0));
-        if (obj_out) CK(cudaMemcpyAsync(p + o_obj, w + o_obj, nb * 8, cudaMemcpyDeviceToHost, s0));
-      }
+      if (U_out) CK(cudaMemcpyAsync(at(p, HA_U, 0), at(w, HA_U, 0), off[N_HA] - off[HA_U], cudaMemcpyDeviceToHost, s0));
+      else
+        for (int a = HA_U + 1; a < N_HA; ++a)
+          if (up[a]) CK(cudaMemcpyAsync(at(p, a, 0), at(w, a, 0), nb * HA_BYTES[a], cudaMemcpyDeviceToHost, s0));
       return MPCB_OK;
     }
     // chunked, one stream per part
@@ -1276,49 +1256,29 @@ static int solve_host(mpcb_handle h, int B, const double* x0, const double* obs_
     // so that the device-to-host copy of the first half runs under the kernels of the second, else the batch as one part
     // (measured on B200 with three handles in flight, 65,536 problems: every output 1 / 2 / 3 / 4 parts 0.92 / 0.55 / 0.93 /
     // 0.90 ms per batch; closed-loop form 1 / 2 parts 0.44 / 0.47 ms)
-    int nparts = wait ? HOST_CHUNKS : (Xpred_out ? 2 : 1);
-#ifdef MPCB_DEV
-    if (!wait && getenv("MPCB_ASYNC_PARTS")) nparts = std::min(HOST_CHUNKS, std::max(1, atoi(getenv("MPCB_ASYNC_PARTS"))));
-#endif
+    const int nparts = wait ? HOST_CHUNKS : (Xpred_out ? 2 : 1);
+    auto edge = [&](int k) { return nparts == HOST_CHUNKS ? HOST_EDGES[k] : (double)k / nparts; };
     CK(cudaEventRecord(h->ev_fork, s0));
     for (int c = 0; c < nparts; ++c) {
-      auto edge = [&](int k) { return nparts == HOST_CHUNKS ? part_edge(k) : (double)k / nparts; };
       const size_t lo = (size_t)(nb * edge(c)), hi = (c + 1 == nparts) ? nb : (size_t)(nb * edge(c + 1)), n = hi - lo;
       if (n == 0) continue;
-      cudaStream_t st = h->xs[c % 4];
-      if (c > 0 && c < 4) CK(cudaStreamWaitEvent(st, h->ev_fork, 0));
-      CK(cudaMemcpyAsync(w + o_x0 + lo * 40, x0 + lo * 5, n * 40, cudaMemcpyHostToDevice, st));
-      CK(cudaMemcpyAsync(w + o_obs + lo * 32, obs_sv + lo * 4, n * 32, cudaMemcpyHostToDevice, st));
-      CK(cudaMemcpyAsync(w + o_n + lo * 4, n_obs + lo, n * 4, cudaMemcpyHostToDevice, st));
-      int r = launch_solve(h, (int)n,
-                           make_io((double*)(w + o_x0) + lo * 5, (double*)(w + o_obs) + lo * 4, (int*)(w + o_n) + lo, dU + lo * 10,
-                                   dX ? dX + lo * 30 : nullptr, dobj ? dobj + lo : nullptr, dst ? dst + lo : nullptr,
-                                   dit ? dit + lo * 2 : nullptr, dcm ? dcm + lo : nullptr, dac ? dac + lo : nullptr,
-                                   du0 ? du0 + lo * 2 : nullptr),
-                           st, part_view(h, c, lo, n), false, use_coop, nparts > 1);
+      cudaStream_t st = h->xs[c];
+      if (c > 0) CK(cudaStreamWaitEvent(st, h->ev_fork, 0));
+      for (int a = 0; a < HA_U; ++a) CK(cudaMemcpyAsync(at(w, a, lo), user(a, lo), n * HA_BYTES[a], cudaMemcpyHostToDevice, st));
+      int r = launch_solve(h, (int)n, host_io(w, off, up, lo), st, part_view(h, c, lo, n), false, use_coop, nparts > 1);
       if (r != MPCB_OK) return r;
-      if (U_out) CK(cudaMemcpyAsync(U_out + lo * 10, dU + lo * 10, n * 80, cudaMemcpyDeviceToHost, st));
-      if (u0_out) CK(cudaMemcpyAsync(u0_out + lo * 2, du0 + lo * 2, n * 16, cudaMemcpyDeviceToHost, st));
-      if (Xpred_out) CK(cudaMemcpyAsync(Xpred_out + lo * 30, dX + lo * 30, n * 240, cudaMemcpyDeviceToHost, st));
-      if (obj_out) CK(cudaMemcpyAsync(obj_out + lo, dobj + lo, n * 8, cudaMemcpyDeviceToHost, st));
-      if (status_out) CK(cudaMemcpyAsync(status_out + lo, dst + lo, n * 4, cudaMemcpyDeviceToHost, st));
-      if (iters_out) CK(cudaMemcpyAsync(iters_out + lo * 2, dit + lo * 2, n * 8, cudaMemcpyDeviceToHost, st));
-      if (cmin_out) CK(cudaMemcpyAsync(cmin_out + lo, dcm + lo, n * 8, cudaMemcpyDeviceToHost, st));
-      if (active_out) CK(cudaMemcpyAsync(active_out + lo, dac + lo, n * 8, cudaMemcpyDeviceToHost, st));
+      for (int a = HA_U; a < N_HA; ++a)
+        if (up[a]) CK(cudaMemcpyAsync(user(a, lo), at(w, a, lo), n * HA_BYTES[a], cudaMemcpyDeviceToHost, st));
     }
-    for (int c = 1; c < 4 && c < nparts; ++c) {   // join
+    for (int c = 1; c < nparts; ++c) {   // join
       CK(cudaEventRecord(h->xe[c], h->xs[c]));
       CK(cudaStreamWaitEvent(s0, h->xe[c], 0));
     }
     return MPCB_OK;
   };
 
-  if (packed) {
-    char* p = (char*)h->pin;
-    memcpy(p + o_x0, x0, nb * 40);
-    memcpy(p + o_obs, obs_sv, nb * 32);
-    memcpy(p + o_n, n_obs, nb * 4);
-  }
+  if (packed)
+    for (int a = 0; a < HA_U; ++a) memcpy(at(p, a, 0), up[a], nb * HA_BYTES[a]);
   if (capture) {
     // capture this call's work (nothing executes yet), instantiate, and fall through to the replay
     if (g.exec) { cudaGraphExecDestroy(g.exec); g.exec = nullptr; }
@@ -1338,37 +1298,29 @@ static int solve_host(mpcb_handle h, int B, const double* x0, const double* obs_
     h->launches = l0;
     if (!ok) cudaGetLastError();              // capture not possible here: enqueue directly below
   }
+  // mpcb_last_kernel_ms: chunked path = device span of the whole call (copies included); the packed path records its
+  // per-pass events in launch_solve
+  if (!packed) CK(cudaEventRecord(h->ev0, s0));
   if (g.valid && memcmp(g.key, key, sizeof(key)) == 0) {
-    if (!packed) CK(cudaEventRecord(h->ev0, s0));
     CK(cudaGraphLaunch(g.exec, s0));
-    if (!packed) CK(cudaEventRecord(h->ev1, s0));
     h->launches += g.launches;
-    h->timed = true;           // mpcb_last_kernel_ms: chunked path = device span of the whole call (copies included)
-    h->pass_timed = packed;    // packed path: the graph's own event-record nodes (ev0, ev_mid, ev1) fire on every replay
-    h->lists_last = part_view(h, 0, 0, nb).hdr;
-  } else {
-    if (!packed) CK(cudaEventRecord(h->ev0, s0));
-    rc = enqueue();
-    if (rc != MPCB_OK) return rc;
-    if (!packed) {
-      CK(cudaEventRecord(h->ev1, s0));
-      h->timed = true;
-      h->pass_timed = false;
+    if (packed) {              // the graph's own event-record nodes (ev0, ev_mid, ev1) fire on every replay
+      h->timed = h->pass_timed = true;
+      h->lists_last = part_view(h, 0, 0, nb).hdr;
     }
+  } else if ((rc = enqueue()) != MPCB_OK) {
+    return rc;
+  }
+  if (!packed) {
+    CK(cudaEventRecord(h->ev1, s0));
+    h->timed = true;
+    h->pass_timed = false;
   }
   if (!wait && !packed) return MPCB_OK;      // asynchronous form: mpcb_wait() synchronises (small batches complete here)
   CK(cudaStreamSynchronize(s0));
-  if (packed) {
-    char* p = (char*)h->pin;
-    if (U_out) memcpy(U_out, p + o_U, nb * 80);
-    if (u0_out) memcpy(u0_out, p + o_u0, nb * 16);
-    if (Xpred_out) memcpy(Xpred_out, p + o_X, nb * 240);
-    if (obj_out) memcpy(obj_out, p + o_obj, nb * 8);
-    if (status_out) memcpy(status_out, p + o_st, nb * 4);
-    if (iters_out) memcpy(iters_out, p + o_it, nb * 8);
-    if (cmin_out) memcpy(cmin_out, p + o_cm, nb * 8);
-    if (active_out) memcpy(active_out, p + o_ac, nb * 8);
-  }
+  if (packed)
+    for (int a = HA_U; a < N_HA; ++a)
+      if (up[a]) memcpy(up[a], at(p, a, 0), nb * HA_BYTES[a]);
   return MPCB_OK;
 }
 

@@ -17,6 +17,13 @@ namespace mpcb { struct PartLists; }
     if (e_ != cudaSuccess) return cuda_fail(e_, #call); \
   } while (0)
 
+// Regions of bytes[0 .. n-1] bytes back to back in one allocation, each 256-byte aligned: region k at off[k], off[n]
+// bytes in all.
+inline void region_offsets(const size_t* bytes, int n, size_t* off) {
+  off[0] = 0;
+  for (int k = 0; k < n; ++k) off[k + 1] = off[k] + ((bytes[k] + 255) & ~(size_t)255);
+}
+
 struct mpcb_ctx {
   int device;
   int n_sm = 148;
@@ -33,7 +40,6 @@ struct mpcb_ctx {
   cudaStream_t xs[4] = {nullptr, nullptr, nullptr, nullptr};   // xs[0] == stream; one stream per part of a large host batch
   cudaEvent_t xe[4] = {nullptr, nullptr, nullptr, nullptr};
   void* pin = nullptr;             // pinned staging block of the packed small-batch path
-  size_t pin_bytes = 0;
   mpcb::PartLists* lists_last = nullptr;   // header of the last timed solve
   bool timed = false;
   bool pass_timed = false;

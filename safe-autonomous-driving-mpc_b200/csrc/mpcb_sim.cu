@@ -387,21 +387,20 @@ int mpcb_check_histories(mpcb_handle h, int B, int T, double s_total, const mpcb
     hs[b] = DevScenario{c.obs_trigger_s, c.obs_start_s, c.obs_v, c.obs_end_s, c.tl_pos, c.tl_trigger_s,
                         c.tl_stop_duration, c.dynamic_obstacle, c.traffic_light};
   }
-  const size_t sz[8] = {nb * sizeof(DevScenario), nb * 40, nb * 4, nt * 40, nt * 16, nt * 8, nt * 4, ((nb * 4 + 255) & ~(size_t)255) + nb * 32};
+  // one allocation: the seven inputs, then the verdicts and the metrics
+  const size_t sz[9] = {nb * sizeof(DevScenario), nb * 40, nb * 4, nt * 40, nt * 16, nt * 8, nt * 4, nb * 4, nb * 32};
   const void* src[7] = {hs.data(), x_final, steps, hist_x, hist_u, hist_obs, hist_tl};
-  size_t off[9];
-  off[0] = 0;
-  for (int k = 0; k < 8; ++k) off[k + 1] = off[k] + ((sz[k] + 255) & ~(size_t)255);
+  size_t off[10];
+  region_offsets(sz, 9, off);
   char* d = nullptr;
-  if (cudaMalloc((void**)&d, off[8]) != cudaSuccess) { cudaGetLastError(); return MPCB_ERR_NOMEM; }
+  if (cudaMalloc((void**)&d, off[9]) != cudaSuccess) { cudaGetLastError(); return MPCB_ERR_NOMEM; }
   cudaStream_t st = h->stream;
   cudaError_t e = cudaSuccess;
   for (int k = 0; k < 7 && e == cudaSuccess; ++k) e = cudaMemcpyAsync(d + off[k], src[k], sz[k], cudaMemcpyHostToDevice, st);
   if (e == cudaSuccess) {
     const mpcb_params& p = h->params;
     int* d_v = (int*)(d + off[7]);
-    double* d_m = (double*)(d + off[7] + ((nb * 4 + 255) & ~(size_t)255));
-    // (the metrics block sits behind the verdicts inside the last region: re-derive its offset so both are aligned)
+    double* d_m = (double*)(d + off[8]);
     mpcb_sim_check_kernel<<<(B + 127) / 128, 128, 0, st>>>(h->dt, nullptr, B, T, s_total, p.u_min[0], p.u_max[0], p.u_min[1], p.u_max[1],
                                                           (const double*)(d + off[1]), (const int*)(d + off[2]),
                                                           (const DevScenario*)(d + off[0]), (const double*)(d + off[3]),

@@ -409,8 +409,9 @@ def test_closed_loop_form_of_the_host_entry(gpu_trackers, port_tables):
 
 def test_asynchronous_host_entry_with_batches_in_flight(gpu_trackers, port_tables):
     """mpcb_solve_batch_host_async / mpcb_wait with three handles in flight (the form bench.py's e2e arm uses): every
-    batch comes back bit-identical to the synchronous call on the same problems -- every output and the closed-loop form
-    (U*[0] + status), first calls, captured call and graph replays, with the input buffers rewritten between rounds."""
+    batch comes back bit-identical to the synchronous call on the same problems -- every output, the closed-loop form
+    (U*[0] + status) and U*[0] with every output but U, first calls, captured call and graph replays, with the input
+    buffers rewritten between rounds; then the same three output sets for a small batch (packed staging path)."""
     import safe_autonomous_driving_mpc_b200 as M
     from oracle import tracker_port as P
     L, T = gpu_trackers[3]
@@ -421,9 +422,10 @@ def test_asynchronous_host_entry_with_batches_in_flight(gpu_trackers, port_table
     full_spec = dict(U=((B, 5, 2), np.float64), Xpred=((B, 6, 5), np.float64), obj=((B,), np.float64),
                      status=((B,), np.int32), iters=((B, 2), np.int32), cmin=((B,), np.float64), active=((B,), np.uint64))
     cl_spec = dict(u0=((B, 2), np.float64), status=((B,), np.int32))
+    mixed_spec = dict(u0=((B, 2), np.float64), **{k: v for k, v in full_spec.items() if k != "U"})
     refs = [{k: v.copy() for k, v in T.solve_batch_host(x0[j * B:(j + 1) * B], obs[j * B:(j + 1) * B], n[j * B:(j + 1) * B]).items()}
             for j in range(2 * nh)]
-    for spec in (full_spec, cl_spec):
+    for spec in (full_spec, cl_spec, mixed_spec):
         bufs = [dict(x0=PB((B, 5), np.float64), obs=PB((B, 2, 2), np.float64), n=PB((B,), np.int32)) for _ in range(nh)]
         outs = [{k: PB(shp, dt) for k, (shp, dt) in spec.items()} for _ in range(nh)]
         for rnd in range(4):                                   # 0 direct, 1 captured, 2.. replayed; data alternates
@@ -441,9 +443,14 @@ def test_asynchronous_host_entry_with_batches_in_flight(gpu_trackers, port_table
                 for kk, o in outs[k].items():
                     want = refs[j]["U"][:, 0, :] if kk == "u0" else refs[j][kk]
                     assert np.array_equal(o.array, want), (kk, rnd, k)
-    # small batches complete inside the call (packed staging path)
-    o = dict(u0=np.zeros((5, 2)), status=np.zeros(5, np.int32))
-    Ts[0].solve_batch_host_async(x0[:5].copy(), obs[:5].copy(), n[:5].copy(), o)
-    small = T.solve_batch_host(x0[:5], obs[:5], n[:5])        # same execution shape (one warp per problem)
-    assert np.array_equal(o["u0"], small["U"][:, 0, :]) and np.array_equal(o["status"], small["status"])
-    Ts[0].wait()
+    # small batches complete inside the call (packed staging path): first, captured and replayed call of each output
+    # set, every call on other problems than the one before, so that stale staging memory cannot pass for an answer
+    for i, spec in enumerate((full_spec, cl_spec, mixed_spec)):
+        for rnd in range(3):
+            sl = slice(5 * (3 * i + rnd), 5 * (3 * i + rnd) + 5)
+            o = {k: np.zeros((5,) + shp[1:], dt) for k, (shp, dt) in spec.items()}
+            Ts[0].solve_batch_host_async(x0[sl].copy(), obs[sl].copy(), n[sl].copy(), o)
+            small = T.solve_batch_host(x0[sl], obs[sl], n[sl])    # same execution shape (one warp per problem)
+            for k, a in o.items():
+                assert np.array_equal(a, small["U"][:, 0, :] if k == "u0" else small[k]), (k, i, rnd)
+            Ts[0].wait()

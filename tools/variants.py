@@ -11,8 +11,6 @@ VARIANTS = {
     "T64_C4_M5": ["MPCB_SOLVE_THREADS=64", "MPCB_SOLVE_CTAS=4", "MPCB_STORE_MASK=5"],
     "T32_C8_M7": ["MPCB_SOLVE_THREADS=32", "MPCB_SOLVE_CTAS=8", "MPCB_STORE_MASK=7"],
     "T32_C9_M5": ["MPCB_SOLVE_THREADS=32", "MPCB_SOLVE_CTAS=9", "MPCB_STORE_MASK=5"],
-    "HC1": ["MPCB_HOST_CHUNKS=1"], "HC2": ["MPCB_HOST_CHUNKS=2"], "HC3": ["MPCB_HOST_CHUNKS=3"], "HC4": ["MPCB_HOST_CHUNKS=4"],
-    "HC6": ["MPCB_HOST_CHUNKS=6"], "HC8": ["MPCB_HOST_CHUNKS=8"],
     "T128_C1_M189": ["MPCB_SOLVE_THREADS=128", "MPCB_SOLVE_CTAS=1", "MPCB_STORE_MASK=189"],
     "T64_C2_M189": ["MPCB_SOLVE_THREADS=64", "MPCB_SOLVE_CTAS=2", "MPCB_STORE_MASK=189"],
     "T96_C1_M191": ["MPCB_SOLVE_THREADS=96", "MPCB_SOLVE_CTAS=1", "MPCB_STORE_MASK=191"],
