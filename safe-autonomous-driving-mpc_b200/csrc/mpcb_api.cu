@@ -46,10 +46,33 @@ constexpr size_t SOLVE_SMEM = sizeof(double) * SolveStore::SHARED * SOLVE_THREAD
 #ifndef MPCB_CLS_MASK2
 #define MPCB_CLS_MASK2 7u
 #endif
+// The one-segment instantiations (thread_max_segments = 1, the default caps) also keep the factor -- and, for the
+// classes with obstacles, D and O -- in tensor memory (MPCB_CLS_TMASK*, a second mask beside MPCB_CLS_MASK*; see
+// tmem_cols_alloc for the budget) and do not store H.
+#ifndef MPCB_CLS_TMASK0
+#define MPCB_CLS_TMASK0 16u
+#endif
+#ifndef MPCB_CLS_TMASK1
+#define MPCB_CLS_TMASK1 (8u | 16u)
+#endif
+#ifndef MPCB_CLS_TMASK2
+#define MPCB_CLS_TMASK2 (8u | 16u)
+#endif
 template <int NOBS> struct ClsCfg;
-template <> struct ClsCfg<0> { typedef Store<SOLVE_THREADS, MPCB_CLS_MASK0, 0> St; };
-template <> struct ClsCfg<1> { typedef Store<SOLVE_THREADS, MPCB_CLS_MASK1, 1> St; };
-template <> struct ClsCfg<2> { typedef Store<SOLVE_THREADS, MPCB_CLS_MASK2, 2> St; };
+template <> struct ClsCfg<0> {
+  typedef Store<SOLVE_THREADS, MPCB_CLS_MASK0, 0> St;
+  typedef Store<SOLVE_THREADS, MPCB_CLS_MASK0, 0, MPCB_CLS_TMASK0, 64u> StOne;
+};
+template <> struct ClsCfg<1> {
+  typedef Store<SOLVE_THREADS, MPCB_CLS_MASK1, 1> St;
+  typedef Store<SOLVE_THREADS, MPCB_CLS_MASK1, 1, MPCB_CLS_TMASK1, 64u> StOne;
+};
+template <> struct ClsCfg<2> {
+  typedef Store<SOLVE_THREADS, MPCB_CLS_MASK2, 2> St;
+  typedef Store<SOLVE_THREADS, MPCB_CLS_MASK2, 2, MPCB_CLS_TMASK2, 64u> StOne;
+};
+template <int NOBS, bool ONESEG> using ClsStore = typename std::conditional<ONESEG, typename ClsCfg<NOBS>::StOne,
+                                                                           typename ClsCfg<NOBS>::St>::type;
 constexpr int cmax3(int a, int b, int c) { return a > b ? (a > c ? a : c) : (b > c ? b : c); }
 constexpr size_t CLS_SMEM = sizeof(double) * SOLVE_THREADS * cmax3(ClsCfg<0>::St::SHARED, ClsCfg<1>::St::SHARED, ClsCfg<2>::St::SHARED);
 constexpr int EVAL_THREADS = 128;
@@ -428,11 +451,12 @@ __device__ __forceinline__ void park_or_finalize(const DevTable& T, const DevPar
   finalize<true>(T, P, pb, so, b, io.accumulate != 0, io, hdr, robust);
 }
 
-template <int NOBS>
+template <int NOBS, bool ONESEG>
 __device__ __forceinline__ void solve_cls_body(const DevTable& T, const DevParams& P, const SolveIO& io, const int* __restrict__ list,
                                                int n_work, int t0, int off, int r0, const Carry& cout,
-                                               int* __restrict__ cnt_out, PartLists* hdr, int* __restrict__ robust) {
-  typedef typename ClsCfg<NOBS>::St St;
+                                               int* __restrict__ cnt_out, PartLists* hdr, int* __restrict__ robust,
+                                               uint32_t tm) {
+  typedef ClsStore<NOBS, ONESEG> St;
   const int t = t0 + threadIdx.x;
   const bool live = t < n_work;
   const int b = live ? list[t] : 0;
@@ -441,7 +465,7 @@ __device__ __forceinline__ void solve_cls_body(const DevTable& T, const DevParam
   load_problem<NOBS>(io, b, live, pb);
   extern __shared__ double solve_smem[];
   double solve_local[St::LOCAL];
-  const St st(solve_smem + threadIdx.x, solve_local);
+  const St st(solve_smem + threadIdx.x, solve_local, tm);
   double Uh[NV];
   const bool hot = io.U_start != nullptr;             // CTA-uniform
   if (hot && live) load_hot_start(io, b, Uh);
@@ -450,17 +474,47 @@ __device__ __forceinline__ void solve_cls_body(const DevTable& T, const DevParam
 #pragma unroll 1
   for (int round = 0; round < r0; ++round) {   // not unrolled: no FMA contraction across a round boundary
     if (MPCB_ALL(s.done)) break;
-    solve_round<true>(T, P, pb, st, s, round);
+    solve_round<true, ONESEG>(T, P, pb, st, s, round);
   }
   park_or_finalize<NOBS>(T, P, io, live, live && !s.done && r0 < P.thread_max_rounds, b, pb, st, s, n_work, cout, cnt_out,
                          off, hdr, robust);
+}
+
+// Tensor memory of a one-segment class or round CTA.  Warp 0 allocates (tcgen05.alloc writes the address to shared
+// memory) and, after the CTA's last barrier, deallocates; CTAs that find no work return before allocating, and nothing
+// returns in between.  Budget: 255 registers x 128 threads cap these kernels at two CTAs per SM, whichever streams
+// they come from, and no other kernel uses tensor memory, so 2 x 256 columns never exceed the SM's 512 and the
+// allocation never waits.  (Should a change lower the register count so that a third CTA fits, its alloc would block
+// until one of the two before it deallocates, not fail.)
+constexpr int TMEM_COLS = 256;
+static_assert(ClsCfg<0>::StOne::TMEM_COLS <= TMEM_COLS && ClsCfg<1>::StOne::TMEM_COLS <= TMEM_COLS &&
+              ClsCfg<2>::StOne::TMEM_COLS <= TMEM_COLS, "one-segment store exceeds its tensor-memory allocation");
+static_assert(SOLVE_THREADS == 128, "32x32b tensor-memory access: warp w of the CTA owns TMEM lanes 32w .. 32w + 31");
+__device__ __forceinline__ uint32_t tmem_cols_alloc(uint32_t* slot) {
+  if (threadIdx.x < 32) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
+                 :: "r"((uint32_t)__cvta_generic_to_shared(slot)), "n"(TMEM_COLS) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  }
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  return *slot + ((threadIdx.x & ~31u) << 16);          // this warp's lanes (address: lane << 16 | column)
+}
+__device__ __forceinline__ void tmem_cols_free(const uint32_t* slot) {
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  if (threadIdx.x < 32) {
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(*slot), "n"(TMEM_COLS) : "memory");
+  }
 }
 
 // Rounds 1..r0 over the class lists cls (class k at cls + k B), cut into the parts hdr->part; survivors go to the list
 // hdr->surv[r0 % 3].  The part, and with it the table, is CTA-uniform.  ROUTED = false (a single-route call, nr = 1)
 // fixes the table at t[0] at compile time: an indexed table costs the single-route first pass 1 % (see DESIGN.md 4,
 // "Several routes on one handle").
-template <bool ROUTED>
+template <bool ROUTED, bool ONESEG>
 __global__ void __launch_bounds__(SOLVE_THREADS, MPCB_SOLVE_CTAS)
 mpcb_solve_cls_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ DevParams P, int B,
                       const __grid_constant__ SolveIO io, PartLists* hdr, const int* __restrict__ cls, int nr, int r0,
@@ -471,9 +525,12 @@ mpcb_solve_cls_kernel(const __grid_constant__ DevTables Ts, const __grid_constan
   const DevTable& T = Ts.t[ROUTED ? p.r : 0];
   const int* list = cls + (size_t)p.k * B + p.off_cls;
   int* cnt_out = hdr->surv[r0 % 3] + p.key;
-  if (p.k == 2) solve_cls_body<2>(T, P, io, list, p.n, p.t0, p.off, r0, cout, cnt_out, hdr, robust);
-  else if (p.k == 1) solve_cls_body<1>(T, P, io, list, p.n, p.t0, p.off, r0, cout, cnt_out, hdr, robust);
-  else solve_cls_body<0>(T, P, io, list, p.n, p.t0, p.off, r0, cout, cnt_out, hdr, robust);
+  __shared__ uint32_t tm_slot;
+  const uint32_t tm = ONESEG ? tmem_cols_alloc(&tm_slot) : 0u;
+  if (p.k == 2) solve_cls_body<2, ONESEG>(T, P, io, list, p.n, p.t0, p.off, r0, cout, cnt_out, hdr, robust, tm);
+  else if (p.k == 1) solve_cls_body<1, ONESEG>(T, P, io, list, p.n, p.t0, p.off, r0, cout, cnt_out, hdr, robust, tm);
+  else solve_cls_body<0, ONESEG>(T, P, io, list, p.n, p.t0, p.off, r0, cout, cnt_out, hdr, robust, tm);
+  if (ONESEG) tmem_cols_free(&tm_slot);
 }
 
 #ifdef MPCB_ROUND_STATS   // development: survivors per round and class, summed over calls (tools/gpu_round_counts.py)
@@ -481,11 +538,11 @@ __device__ unsigned long long g_round_stats[16 * 3];
 #endif
 
 // One further round of the first pass over the survivors of class NOBS listed in cin (slots off + t0 + threadIdx.x).
-template <int NOBS>
+template <int NOBS, bool ONESEG>
 __device__ __forceinline__ void solve_round_body(const DevTable& T, const DevParams& P, const SolveIO& io, int n_work, int t0,
                                                  int off, const Carry& cin, const Carry& cout, int* __restrict__ cnt_out,
-                                                 int round, PartLists* hdr, int* __restrict__ robust) {
-  typedef typename ClsCfg<NOBS>::St St;
+                                                 int round, PartLists* hdr, int* __restrict__ robust, uint32_t tm) {
+  typedef ClsStore<NOBS, ONESEG> St;
   const int t = t0 + threadIdx.x;
   const bool live = t < n_work;
   const int slot = off + t;
@@ -496,12 +553,26 @@ __device__ __forceinline__ void solve_round_body(const DevTable& T, const DevPar
   load_problem<NOBS>(io, b, live, pb);
   extern __shared__ double solve_smem[];
   double solve_local[St::LOCAL];
-  const St st(solve_smem + threadIdx.x, solve_local);
+  const St st(solve_smem + threadIdx.x, solve_local, tm);
   SolveState s;
   s.out = SolveOut{MPCB_MAXITER, 0, 0, false};
   s.done = true; s.infeasible = false; s.first = false; s.hot = false; s.fails = 0; s.step_prev = 1e30;
-  if (live) unpark(cin, slot, pb, st, s);
-  solve_round<true>(T, P, pb, st, s, round);
+  if (live) {
+    unpark(cin, slot, pb, st, s);
+  } else if (ONESEG) {   // an empty lane runs the round with its warp (solve_round): a benign problem at rest
+#pragma unroll
+    for (int k = 0; k < NV; ++k) { pb.U[k] = 0.0; pb.x[k] = 0.0; }
+#pragma unroll
+    for (int r = 0; r < St::MROWS; ++r) st.v[r] = 0.0;
+#pragma unroll
+    for (int j = 0; j < NH; ++j) { st.lov[j] = -BIG; st.blo[j] = P.umin[1]; st.bhi[j] = P.umax[1]; }
+#pragma unroll
+    for (int r = 0; r < NOBS * N_OBSROW; ++r) st.hio[r] = BIG;
+#pragma unroll
+    for (int j = 0; j <= NH; ++j) pb.hint[j] = 1;
+    pb.act_prev = 0ull;
+  }
+  solve_round<true, ONESEG>(T, P, pb, st, s, round);
   park_or_finalize<NOBS>(T, P, io, live, live && !s.done && round + 1 < P.thread_max_rounds, b, pb, st, s, n_work, cout,
                          cnt_out, off, hdr, robust);
 }
@@ -511,7 +582,7 @@ __device__ __forceinline__ void solve_round_body(const DevTable& T, const DevPar
 // hdr->surv[round % 3] and parked in cin; survivors of this round go to hdr->surv[(round + 1) % 3] and cout, the others
 // are finalized as in the class kernel -- after the last round all of them.  hdr->surv[(round + 2) % 3], which the next
 // round kernel appends to (read by the previous one, which has finished), is zeroed here.
-template <bool ROUTED>
+template <bool ROUTED, bool ONESEG>
 __global__ void __launch_bounds__(SOLVE_THREADS, MPCB_SOLVE_CTAS)
 mpcb_solve_round_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ DevParams P,
                         const __grid_constant__ SolveIO io, PartLists* hdr, int nr, const __grid_constant__ Carry cin,
@@ -527,9 +598,12 @@ mpcb_solve_round_kernel(const __grid_constant__ DevTables Ts, const __grid_const
   if (!find_part(cnt_in, hdr->part, nr, blockIdx.x, p)) return;             // CTA-uniform from here on
   MPCB_ASSERT(p.n >= 0 && p.n <= hdr->part[p.key] && p.r >= 0 && p.r < Ts.n);
   const DevTable& T = Ts.t[ROUTED ? p.r : 0];
-  if (p.k == 2) solve_round_body<2>(T, P, io, p.n, p.t0, p.off, cin, cout, cnt_out + p.key, round, hdr, robust);
-  else if (p.k == 1) solve_round_body<1>(T, P, io, p.n, p.t0, p.off, cin, cout, cnt_out + p.key, round, hdr, robust);
-  else solve_round_body<0>(T, P, io, p.n, p.t0, p.off, cin, cout, cnt_out + p.key, round, hdr, robust);
+  __shared__ uint32_t tm_slot;
+  const uint32_t tm = ONESEG ? tmem_cols_alloc(&tm_slot) : 0u;
+  if (p.k == 2) solve_round_body<2, ONESEG>(T, P, io, p.n, p.t0, p.off, cin, cout, cnt_out + p.key, round, hdr, robust, tm);
+  else if (p.k == 1) solve_round_body<1, ONESEG>(T, P, io, p.n, p.t0, p.off, cin, cout, cnt_out + p.key, round, hdr, robust, tm);
+  else solve_round_body<0, ONESEG>(T, P, io, p.n, p.t0, p.off, cin, cout, cnt_out + p.key, round, hdr, robust, tm);
+  if (ONESEG) tmem_cols_free(&tm_slot);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -918,10 +992,14 @@ int mpcb_create_routes(mpcb_handle* out, const mpcb_params* p, const mpcb_table_
   if ((e = cudaEventCreate(&c->ev1)) != cudaSuccess) return fail(cuda_fail(e, "cudaEventCreate"));
   if ((e = cudaEventCreate(&c->ev_mid)) != cudaSuccess) return fail(cuda_fail(e, "cudaEventCreate"));
   if ((e = cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming)) != cudaSuccess) return fail(cuda_fail(e, "cudaEventCreate"));
-  if ((e = cudaFuncSetAttribute(mpcb_solve_cls_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
-      (e = cudaFuncSetAttribute(mpcb_solve_cls_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
-      (e = cudaFuncSetAttribute(mpcb_solve_round_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
-      (e = cudaFuncSetAttribute(mpcb_solve_round_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
+  if ((e = cudaFuncSetAttribute(mpcb_solve_cls_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(mpcb_solve_cls_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(mpcb_solve_cls_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(mpcb_solve_cls_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(mpcb_solve_round_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(mpcb_solve_round_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(mpcb_solve_round_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(mpcb_solve_round_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLS_SMEM)) != cudaSuccess ||
       (e = cudaFuncSetAttribute(mpcb_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SOLVE_SMEM)) != cudaSuccess ||
       (e = cudaFuncSetAttribute(mpcb_coop_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)COOP_SMEM)) != cudaSuccess ||
       (e = cudaFuncSetAttribute(mpcb_coop_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)COOP_SMEM)) != cudaSuccess)
@@ -1056,8 +1134,12 @@ static int launch_solve(mpcb_handle h, int B, const SolveIO& io_in, cudaStream_t
       const bool compact = grid > h->n_sm * MPCB_SOLVE_CTAS;
       const int r0 = compact ? std::min(CLS_ROUNDS, max_rounds) : max_rounds;
       const int grid1 = grid + 3 * nr - 1;
-      const auto cls_kernel = io.route ? mpcb_solve_cls_kernel<true> : mpcb_solve_cls_kernel<false>;
-      const auto round_kernel = io.route ? mpcb_solve_round_kernel<true> : mpcb_solve_round_kernel<false>;
+      // one segment per round (the default caps): the instantiations that keep their factor in tensor memory
+      const bool one = h->dp.thread_max_segments == 1;
+      const auto cls_kernel = io.route ? (one ? mpcb_solve_cls_kernel<true, true> : mpcb_solve_cls_kernel<true, false>)
+                                       : (one ? mpcb_solve_cls_kernel<false, true> : mpcb_solve_cls_kernel<false, false>);
+      const auto round_kernel = io.route ? (one ? mpcb_solve_round_kernel<true, true> : mpcb_solve_round_kernel<true, false>)
+                                         : (one ? mpcb_solve_round_kernel<false, true> : mpcb_solve_round_kernel<false, false>);
       cls_kernel<<<grid1, SOLVE_THREADS, CLS_SMEM, st>>>(h->dt, h->dp, B, io1, v.hdr, v.cls, nr, r0, v.wk[0], v.robust);
       h->launches++;
       // the rounds after r0 over the packed survivors, one launch per round (workspaces ping-pong; each kernel zeroes

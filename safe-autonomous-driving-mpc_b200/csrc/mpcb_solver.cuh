@@ -24,8 +24,9 @@
 // Data placement: a compile-time mask (MPCB_STORE_MASK) says which per-thread arrays live in a strided store (shared
 // memory on the GPU: element i of thread t at base[i * CTA + t], conflict free) -- by default the per-row vectors v,
 // rho and the obstacle bounds -- and which stay thread-private (registers / local memory): D, O, the 10x10 factor, H,
-// q and the iterate.
+// q and the iterate.  The one-segment first pass also puts the factor and D, O in tensor memory (TCol below).
 #pragma once
+#include <stdint.h>
 #include <type_traits>
 
 #include "mpcb200.h"
@@ -69,37 +70,131 @@ struct LCol {          // thread-private, plain: registers / local memory, place
   double* p;
   MPCB_HD double& operator[](int i) const { return p[i]; }
 };
-template <bool SHARED, int S> struct ColSel { typedef Col<S> type; };
-template <int S> struct ColSel<false, S> { typedef LCol type; };
+// Tensor memory (first-pass class and round kernels): a column kind with no references, because tcgen05.ld is
+// asynchronous.  Shape 32x32b maps TMEM lane t of the warp's sub-partition to lane t of the warp, so the columns are
+// thread-private; double i of a TCol sits in its columns 2i (low word) and 2i + 1 (high word).  Every access is a block
+// load (tcgen05.ld, then tcgen05.wait::ld before the values are used) or a block store, and is .sync.aligned: the whole
+// warp must execute it together (see solve_round's one-segment path).  a: TMEM address of this warp's lanes and of the
+// array's first column.
+struct TCol { uint32_t a; };
+template <class C> struct IsTmem : std::false_type {};
+template <> struct IsTmem<TCol> : std::true_type {};
 
-// Per-thread working set.  MASK says which array groups sit in the strided (shared-memory) part, the rest lives in
-// a thread-private buffer of LOCAL doubles (registers / local memory, placement left to the compiler):
+#if defined(__CUDA_ARCH__)
+__device__ __forceinline__ void tmem_converged() {
+  __syncwarp();
+  MPCB_ASSERT(__activemask() == 0xffffffffu);
+}
+#define MPCB_TLD_ASM(N, REGS, ...)                                                                                     \
+  asm volatile("{\n\ttcgen05.ld.sync.aligned.32x32b.x" #N ".b32 " REGS ", [%" #N "];\n\ttcgen05.wait::ld.sync.aligned;\n}" \
+               : __VA_ARGS__ : "r"(a) : "memory")
+template <int N> __device__ __forceinline__ void tmem_ld(uint32_t a, uint32_t (&r)[N]);
+template <> __device__ __forceinline__ void tmem_ld<2>(uint32_t a, uint32_t (&r)[2]) {
+  MPCB_TLD_ASM(2, "{%0, %1}", "=r"(r[0]), "=r"(r[1]));
+}
+template <> __device__ __forceinline__ void tmem_ld<4>(uint32_t a, uint32_t (&r)[4]) {
+  MPCB_TLD_ASM(4, "{%0, %1, %2, %3}", "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]));
+}
+template <> __device__ __forceinline__ void tmem_ld<8>(uint32_t a, uint32_t (&r)[8]) {
+  MPCB_TLD_ASM(8, "{%0, %1, %2, %3, %4, %5, %6, %7}", "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]),
+               "=r"(r[5]), "=r"(r[6]), "=r"(r[7]));
+}
+template <> __device__ __forceinline__ void tmem_ld<16>(uint32_t a, uint32_t (&r)[16]) {
+  MPCB_TLD_ASM(16, "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}", "=r"(r[0]), "=r"(r[1]),
+               "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
+               "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]));
+}
+#undef MPCB_TLD_ASM
+__device__ __forceinline__ void tmem_st2(uint32_t a, double x) {   // one double; completed by tmem_wait_st
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x2.b32 [%0], {%1, %2};"
+               :: "r"(a), "r"(__double2loint(x)), "r"(__double2hiint(x)) : "memory");
+}
+__device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+
+// chunk of 2 * W columns at double i + k of c into x[k .. k + W)
+template <int W, int NMAX>
+__device__ __forceinline__ void tload_chunk(const TCol& c, int i, int k, double (&x)[NMAX]) {
+  uint32_t r[2 * W];
+  tmem_ld<2 * W>(c.a + 2 * (i + k), r);
+#pragma unroll
+  for (int m = 0; m < W; ++m)
+    if (k + m < NMAX) x[k + m] = __hiloint2double((int)r[2 * m + 1], (int)r[2 * m]);
+}
+// x[0 .. n) = doubles i .. i + n of c (n <= NMAX <= 15, a compile-time constant once the caller's loops are unrolled)
+template <int NMAX>
+__device__ __forceinline__ void tload(const TCol& c, int i, int n, double (&x)[NMAX]) {
+  static_assert(NMAX <= 15, "chunks of 8, 4, 2, 1 doubles");
+  tmem_converged();
+  int k = 0;
+  if (n - k >= 8) { tload_chunk<8>(c, i, k, x); k += 8; }
+  if (n - k >= 4) { tload_chunk<4>(c, i, k, x); k += 4; }
+  if (n - k >= 2) { tload_chunk<2>(c, i, k, x); k += 2; }
+  if (n - k >= 1) tload_chunk<1>(c, i, k, x);
+}
+// doubles i .. i + n of c = x[0 .. n); the caller ends its stores with tmem_wait_st before anything reads them
+template <int NMAX>
+__device__ __forceinline__ void tstore(const TCol& c, int i, int n, const double (&x)[NMAX]) {
+  tmem_converged();
+#pragma unroll
+  for (int m = 0; m < NMAX; ++m)
+    if (m < n) tmem_st2(c.a + 2 * (i + m), x[m]);
+}
+#else
+// the host never places an array in tensor memory (ColSel below); these only keep the discarded branches well formed
+template <int NMAX> inline void tload(const TCol&, int, int, double (&)[NMAX]) {}
+template <int NMAX> inline void tstore(const TCol&, int, int, const double (&)[NMAX]) {}
+inline void tmem_wait_st() {}
+#endif
+
+// placement of an array group: 0 thread-private, 1 shared, 2 tensor memory, 3 not stored
+template <int KIND, int S> struct ColSel { typedef Col<S> type; };
+template <int S> struct ColSel<0, S> { typedef LCol type; };
+template <int S> struct ColSel<3, S> { typedef LCol type; };
+#if defined(__CUDA_ARCH__)
+template <int S> struct ColSel<2, S> { typedef TCol type; };
+#else
+template <int S> struct ColSel<2, S> { typedef LCol type; };
+#endif
+
+// Per-thread working set.  MASK says which array groups sit in the strided (shared-memory) part, TMASK which sit in
+// tensor memory (device only), NONE which are not stored at all; the rest lives in a thread-private buffer of LOCAL
+// doubles (registers / local memory, placement left to the compiler):
 //   bit 0  v        [41] ADMM state                      bit 4  L, rdiag   [55+10] factor of K
 //   bit 1  rho      [41] step sizes                      bit 5  q, lane_c  [10+8]
 //   bit 2  hio      [18] obstacle-row bounds             bit 6  H          [55]
 //   bit 3  D, O     [20+20] lane sensitivities           bit 7  lane_inrm, lov, blo, bhi  [8+5+5+5]
+// In tensor memory, L holds the factor column by column: column j at fcol(j) is rdiag[j], then L[j+1..9][j] (55 doubles
+// in all; rdiag is not a separate array there).  Only bits 3 and 4 can go to tensor memory, only bit 6 (H, which the
+// one-segment first pass hands from linearise to factor in registers) can be left out.
 // MASK = 0: host build, evaluation kernel, cooperative kernel (S must be 1).
 // NOBS: how many obstacle slots the problems of this instantiation can have (0, 1 or 2).  The thread-per-problem first
 // pass runs one instantiation per obstacle count (the batch is partitioned by n_obs first, mpcb_api.cu): a problem
 // without obstacles walks 23 rows instead of 41 and keeps 46 instead of 100 doubles of row state, so more of its
 // working set fits in shared memory.  Rows keep their numbers; the slots k >= NOBS simply do not exist.
-template <int S, unsigned MASK, int NOBS = 2>
+__host__ __device__ constexpr int fcol(int j) { return j * NV - j * (j - 1) / 2; }
+template <int S, unsigned MASK, int NOBS = 2, unsigned TMASK = 0u, unsigned NONE = 0u>
 struct Store {
+  static_assert((MASK & TMASK) == 0u && ((MASK | TMASK) & NONE) == 0u, "one placement per array group");
+  static_assert((TMASK & ~(8u | 16u)) == 0u && (NONE & ~64u) == 0u, "only D, O, L, rdiag go to tensor memory, only H can be left out");
   static constexpr int KOBS = NOBS;
   static constexpr int MROWS = ROW_OBS + N_OBSROW * NOBS;
-  template <int BIT> using G = typename ColSel<((MASK >> BIT) & 1u) != 0, S>::type;
+  MPCB_HD static constexpr int kind(int bit) {
+    return ((NONE >> bit) & 1u) ? 3 : ((TMASK >> bit) & 1u) ? 2 : ((MASK >> bit) & 1u) ? 1 : 0;
+  }
+  template <int BIT> using G = typename ColSel<kind(BIT), S>::type;
   static constexpr int size_of(int bit) {
     return bit == 0 ? MROWS : bit == 1 ? MROWS : bit == 2 ? NOBS * N_OBSROW : bit == 3 ? 2 * N_DO : bit == 4 ? NTRI + NV
          : bit == 5 ? NV + N_LANE : bit == 6 ? NTRI : N_LANE + 3 * NH;
   }
-  static constexpr int shared_doubles() {
+  static constexpr int doubles_of(int k) {
     int n = 0;
-    for (int b = 0; b < 8; ++b) if ((MASK >> b) & 1u) n += size_of(b);
+    for (int b = 0; b < 8; ++b) if (kind(b) == k) n += (k == 2 && b == 4) ? NTRI : size_of(b);
     return n;
   }
   static constexpr int TOTAL = 2 * MROWS + NOBS * N_OBSROW + 2 * N_DO + NTRI + NV + NV + N_LANE + NTRI + N_LANE + 3 * NH;
-  static constexpr int SHARED = shared_doubles();
-  static constexpr int LOCAL = (TOTAL - SHARED) > 0 ? (TOTAL - SHARED) : 1;
+  static constexpr int SHARED = doubles_of(1);
+  static constexpr int TMEM_COLS = 2 * doubles_of(2);   // 32-bit columns
+  static constexpr int LOCAL = doubles_of(0) > 0 ? doubles_of(0) : 1;
   G<0> v;
   G<1> rho;
   G<2> hio;         // upper bounds of the obstacle rows (BIG: row absent or dropped)
@@ -108,18 +203,26 @@ struct Store {
   G<5> q, lane_c;   // lane_c: row value offset (d_j + alpha o_j)(U) - a.U
   G<6> H;
   G<7> lane_inrm, lov, blo, bhi;   // lov: lower bound of the speed rows; blo/bhi: per-problem box of the accelerations
-  // sh: this thread's first element of the strided part; lo: thread-private buffer of LOCAL doubles
-  MPCB_HD Store(double* sh, double* lo) {
-    auto take = [&](auto& c, bool shared, int n) {
-      typedef decltype(c.p) P;
-      if (shared) { c.p = (P)sh; sh += n * S; } else { c.p = (P)lo; lo += n; }
+  // sh: this thread's first element of the strided part; lo: thread-private buffer of LOCAL doubles; tm: TMEM address of
+  // this warp's lanes and of the first column the store may use (TMEM_COLS of them)
+  MPCB_HD Store(double* sh, double* lo, uint32_t tm = 0u) {
+    auto take = [&](auto& c, int k, int n) {
+      if constexpr (IsTmem<std::decay_t<decltype(c)>>::value) {
+        c.a = tm; tm += 2 * n;
+      } else {
+        typedef decltype(c.p) P;
+        if (k == 1) { c.p = (P)sh; sh += n * S; }
+        else if (k == 3) c.p = nullptr;
+        else { c.p = (P)lo; lo += n; }
+      }
     };
-    take(v, MASK & 1u, MROWS); take(rho, MASK & 2u, MROWS); take(hio, MASK & 4u, NOBS * N_OBSROW);
-    take(D, MASK & 8u, N_DO); take(O, MASK & 8u, N_DO);
-    take(L, MASK & 16u, NTRI); take(rdiag, MASK & 16u, NV);
-    take(q, MASK & 32u, NV); take(lane_c, MASK & 32u, N_LANE);
-    take(H, MASK & 64u, NTRI);
-    take(lane_inrm, MASK & 128u, N_LANE); take(lov, MASK & 128u, NH); take(blo, MASK & 128u, NH); take(bhi, MASK & 128u, NH);
+    (void)tm;
+    take(v, kind(0), MROWS); take(rho, kind(1), MROWS); take(hio, kind(2), NOBS * N_OBSROW);
+    take(D, kind(3), N_DO); take(O, kind(3), N_DO);
+    take(L, kind(4), NTRI); take(rdiag, kind(4), kind(4) == 2 ? 0 : NV);
+    take(q, kind(5), NV); take(lane_c, kind(5), N_LANE);
+    take(H, kind(6), NTRI);
+    take(lane_inrm, kind(7), N_LANE); take(lov, kind(7), NH); take(blo, kind(7), NH); take(bhi, kind(7), NH);
   }
 };
 
@@ -216,10 +319,13 @@ MPCB_HD void lane_rows(const DevParams& P, Problem& pb, const ST& st, const doub
   constexpr int L = 2 * (J - 1);
   constexpr int o = doff(J - 2);
   double dU = 0.0, oU = 0.0, dd = 0.0, dox = 0.0, oo = 0.0;
+  if constexpr (IsTmem<decltype(st.D)>::value) { tstore(st.D, o, L, dD); tstore(st.O, o, L, dO); }
 #pragma unroll
   for (int c = 0; c < L; ++c) {
-    st.D[o + c] = dD[c];
-    st.O[o + c] = dO[c];
+    if constexpr (!IsTmem<decltype(st.D)>::value) {
+      st.D[o + c] = dD[c];
+      st.O[o + c] = dO[c];
+    }
     dU = fma(dD[c], pb.U[c], dU);
     oU = fma(dO[c], pb.U[c], oU);
     dd = fma(dD[c], dD[c], dd);
@@ -235,10 +341,11 @@ MPCB_HD void lane_rows(const DevParams& P, Problem& pb, const ST& st, const doub
   }
 }
 
+// H: the Gauss-Newton Hessian, left in the caller's registers (the one-segment first pass factors it straight away)
 template <class ST>
-MPCB_HD void linearise(const DevTable& T, const DevParams& P, Problem& pb, const ST& st, double& const_viol) {
+MPCB_HD void linearise(const DevTable& T, const DevParams& P, Problem& pb, const ST& st, double& const_viol,
+                       double (&H)[NTRI]) {
   const double h = P.h;
-  double H[NTRI];
 #pragma unroll
   for (int i = 0; i < NTRI; ++i) H[i] = 0.0;
 #pragma unroll
@@ -312,9 +419,16 @@ MPCB_HD void linearise(const DevTable& T, const DevParams& P, Problem& pb, const
     for (int j = 0; j < NV; ++j) acc = fma(-H[i >= j ? tri(i, j) : tri(j, i)], pb.U[j], acc);
     st.q[i] = acc;
   }
+  if constexpr (IsTmem<decltype(st.D)>::value) tmem_wait_st();   // D, O complete before the first read
+  const_viol = cv;
+}
+
+template <class ST>
+MPCB_HD void linearise(const DevTable& T, const DevParams& P, Problem& pb, const ST& st, double& const_viol) {
+  double H[NTRI];
+  linearise(T, P, pb, st, const_viol, H);
 #pragma unroll
   for (int i = 0; i < NTRI; ++i) st.H[i] = H[i];
-  const_viol = cv;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -332,10 +446,21 @@ MPCB_HD void for_rows(const DevParams& P, const Problem& pb, const ST& st, const
 #pragma unroll
   for (int jj = 0; jj < 4; ++jj) {
     double dj = 0.0, oj = 0.0;
+    if constexpr (IsTmem<decltype(st.D)>::value) {
+      double Db[8], Ob[8];
+      tload(st.D, doff(jj), 2 * (jj + 1), Db);
+      tload(st.O, doff(jj), 2 * (jj + 1), Ob);
 #pragma unroll
-    for (int c = 0; c < 2 * (jj + 1); ++c) {
-      dj = fma(st.D[doff(jj) + c], x[c], dj);
-      oj = fma(st.O[doff(jj) + c], x[c], oj);
+      for (int c = 0; c < 2 * (jj + 1); ++c) {
+        dj = fma(Db[c], x[c], dj);
+        oj = fma(Ob[c], x[c], oj);
+      }
+    } else {
+#pragma unroll
+      for (int c = 0; c < 2 * (jj + 1); ++c) {
+        dj = fma(st.D[doff(jj) + c], x[c], dj);
+        oj = fma(st.O[doff(jj) + c], x[c], oj);
+      }
     }
     f(ROW_LANE + 2 * jj, dj, -P.sld - st.lane_c[2 * jj], P.sld - st.lane_c[2 * jj], RowKind<0>{});
     f(ROW_LANE + 2 * jj + 1, fma(P.alpha_lane[2], oj, dj), -P.sld - st.lane_c[2 * jj + 1],
@@ -381,9 +506,18 @@ struct AtAcc {
         w0 = w;
       } else {
         const double wD = w0 + w, wO = P.alpha_lane[2] * w;
+        if constexpr (IsTmem<decltype(st.D)>::value) {
+          double Db[8], Ob[8];
+          tload(st.D, doff(jj), 2 * (jj + 1), Db);
+          tload(st.O, doff(jj), 2 * (jj + 1), Ob);
 #pragma unroll
-        for (int c = 0; c < NV; ++c)
-          if (c < 2 * (jj + 1)) out[c] = fma(st.D[doff(jj) + c], wD, fma(st.O[doff(jj) + c], wO, out[c]));
+          for (int c = 0; c < 8; ++c)
+            if (c < 2 * (jj + 1)) out[c] = fma(Db[c], wD, fma(Ob[c], wO, out[c]));
+        } else {
+#pragma unroll
+          for (int c = 0; c < NV; ++c)
+            if (c < 2 * (jj + 1)) out[c] = fma(st.D[doff(jj) + c], wD, fma(st.O[doff(jj) + c], wO, out[c]));
+        }
       }
     } else if (r < ROW_OBS) {
       Tv[r - ROW_V] += w;
@@ -417,8 +551,9 @@ struct AtAcc {
 // TWO: the two-level policy (two rungs, no hysteresis, inactive rows drop at once).  Under it a row's rung after a
 // check is simply "was active in that check", i.e. the rung vector IS the bit mask act_prev: no 4-bit rung fields to
 // read, modify and write back, and the two step sizes are selected, not looked up.
+// K: the Gauss-Newton Hessian H on entry (st.H is not read), overwritten.
 template <bool TWO, class ST>
-MPCB_HD void factor(const DevParams& P, const Policy& pl, Problem& pb, const ST& st) {
+MPCB_HD void factor(const DevParams& P, const Policy& pl, Problem& pb, const ST& st, double (&K)[NTRI]) {
   const double h = P.h;
   // step sizes of this factorisation
   const double lad0 = pl.lad[0], lad1 = pl.lad[1];
@@ -442,9 +577,6 @@ MPCB_HD void factor(const DevParams& P, const Policy& pl, Problem& pb, const ST&
       }
     }
   }
-  double K[NTRI];
-#pragma unroll
-  for (int i = 0; i < NTRI; ++i) K[i] = st.H[i];
 #pragma unroll
   for (int i = 0; i < NV; ++i) K[tri(i, i)] += st.rho[i];
   // lane rows of step j:  rho0 D D' + rho1 (D + wb O)(D + wb O)' = D (r0 D + r1 O)' + O (r1 D + r2 O)'
@@ -453,14 +585,28 @@ MPCB_HD void factor(const DevParams& P, const Policy& pl, Problem& pb, const ST&
     const double rho0 = st.rho[ROW_LANE + 2 * jj], rho1 = st.rho[ROW_LANE + 2 * jj + 1];
     const double wb = P.alpha_lane[2];
     const double r0 = rho0 + rho1, r1 = rho1 * wb, r2 = rho1 * wb * wb;
+    auto rank2 = [&](const auto& Dc, const auto& Oc) {
 #pragma unroll
-    for (int i = 0; i < 2 * (jj + 1); ++i) {
-      const double Di = st.D[doff(jj) + i], Oi = st.O[doff(jj) + i];
-      const double p = r0 * Di + r1 * Oi;
-      const double t = r1 * Di + r2 * Oi;
+      for (int i = 0; i < 2 * (jj + 1); ++i) {
+        const double Di = Dc[doff(jj) + i], Oi = Oc[doff(jj) + i];
+        const double p = r0 * Di + r1 * Oi;
+        const double t = r1 * Di + r2 * Oi;
 #pragma unroll
-      for (int j = 0; j <= i; ++j)
-        K[tri(i, j)] = fma(p, st.D[doff(jj) + j], fma(t, st.O[doff(jj) + j], K[tri(i, j)]));
+        for (int j = 0; j <= i; ++j)
+          K[tri(i, j)] = fma(p, Dc[doff(jj) + j], fma(t, Oc[doff(jj) + j], K[tri(i, j)]));
+      }
+    };
+    if constexpr (IsTmem<decltype(st.D)>::value) {
+      double Db[8], Ob[8];   // indexed from doff(jj) like the store
+      tload(st.D, doff(jj), 2 * (jj + 1), Db);
+      tload(st.O, doff(jj), 2 * (jj + 1), Ob);
+      struct Block {
+        const double* p; int o;
+        MPCB_HD double operator[](int e) const { return p[e - o]; }
+      };
+      rank2(Block{Db, doff(jj)}, Block{Ob, doff(jj)});
+    } else {
+      rank2(st.D, st.O);
     }
   }
   // constant-coefficient rows act on the b entries only: Kb[i][k] += sum_r rho_r c_r[i] c_r[k]
@@ -495,7 +641,7 @@ MPCB_HD void factor(const DevParams& P, const Policy& pl, Problem& pb, const ST&
     for (int k = 0; k < j; ++k) d = fma(-K[tri(j, k)], K[tri(j, k)], d);
     const double rs = rsqrt(d);
     K[tri(j, j)] = d * rs;
-    st.rdiag[j] = rs;
+    if constexpr (!IsTmem<decltype(st.L)>::value) st.rdiag[j] = rs;
 #pragma unroll
     for (int i = j + 1; i < NV; ++i) {
       double s = K[tri(i, j)];
@@ -503,25 +649,65 @@ MPCB_HD void factor(const DevParams& P, const Policy& pl, Problem& pb, const ST&
       for (int k = 0; k < j; ++k) s = fma(-K[tri(i, k)], K[tri(j, k)], s);
       K[tri(i, j)] = s * rs;
     }
-  }
+    if constexpr (IsTmem<decltype(st.L)>::value) {   // column j as chol_solve reads it: rdiag[j], L[j+1..9][j]
+      double col[NV];
+      col[0] = rs;
 #pragma unroll
-  for (int i = 0; i < NTRI; ++i) st.L[i] = K[i];
+      for (int i = j + 1; i < NV; ++i) col[i - j] = K[tri(i, j)];
+      tstore(st.L, fcol(j), NV - j, col);
+    }
+  }
+  if constexpr (IsTmem<decltype(st.L)>::value) {
+    tmem_wait_st();
+  } else {
+#pragma unroll
+    for (int i = 0; i < NTRI; ++i) st.L[i] = K[i];
+  }
+}
+
+template <bool TWO, class ST>
+MPCB_HD void factor(const DevParams& P, const Policy& pl, Problem& pb, const ST& st) {
+  double K[NTRI];
+#pragma unroll
+  for (int i = 0; i < NTRI; ++i) K[i] = st.H[i];
+  factor<TWO>(P, pl, pb, st, K);
 }
 
 // x = K^-1 r through the factor (column-oriented substitutions: independent updates after every pivot)
 template <class ST>
 MPCB_HD void chol_solve(const ST& st, double (&r)[NV], double (&x)[NV]) {
+  if constexpr (IsTmem<decltype(st.L)>::value) {
+    // one column block per pivot; the back substitution reads column i of L to finish x[i], which applies the same
+    // updates to r[i] in the same order (j = 9 down to i + 1) as the row updates below
 #pragma unroll
-  for (int j = 0; j < NV; ++j) {
-    r[j] *= st.rdiag[j];
+    for (int j = 0; j < NV; ++j) {
+      double c[NV];
+      tload(st.L, fcol(j), NV - j, c);
+      r[j] *= c[0];
 #pragma unroll
-    for (int i = j + 1; i < NV; ++i) r[i] = fma(-st.L[tri(i, j)], r[j], r[i]);
-  }
+      for (int i = j + 1; i < NV; ++i) r[i] = fma(-c[i - j], r[j], r[i]);
+    }
 #pragma unroll
-  for (int j = NV - 1; j >= 0; --j) {
-    x[j] = r[j] * st.rdiag[j];
+    for (int i = NV - 1; i >= 0; --i) {
+      double c[NV];
+      tload(st.L, fcol(i), NV - i, c);
 #pragma unroll
-    for (int i = 0; i < j; ++i) r[i] = fma(-st.L[tri(j, i)], x[j], r[i]);
+      for (int j = NV - 1; j > i; --j) r[i] = fma(-c[j - i], x[j], r[i]);
+      x[i] = r[i] * c[0];
+    }
+  } else {
+#pragma unroll
+    for (int j = 0; j < NV; ++j) {
+      r[j] *= st.rdiag[j];
+#pragma unroll
+      for (int i = j + 1; i < NV; ++i) r[i] = fma(-st.L[tri(i, j)], r[j], r[i]);
+    }
+#pragma unroll
+    for (int j = NV - 1; j >= 0; --j) {
+      x[j] = r[j] * st.rdiag[j];
+#pragma unroll
+      for (int i = 0; i < j; ++i) r[i] = fma(-st.L[tri(j, i)], x[j], r[i]);
+    }
   }
 }
 
@@ -741,8 +927,14 @@ MPCB_HD void solve_start(const DevTable& T, const DevParams& P, Problem& pb, con
 
 // one Gauss-Newton round: linearise (cold ADMM start on the first), segments, step test.  Every thread of the CTA calls it
 // (the segment votes are CTA-uniform); a thread whose problem is done only takes part in the votes.
-template <bool FIRST_PASS, class ST>
+// ONESEG (first pass at thread_max_segments = 1, the only path whose store may sit in tensor memory): the round is one
+// segment, so linearise hands H to factor in registers, and every lane of a warp that has an unfinished problem runs
+// the round's arithmetic -- warp-convergent, as tcgen05.ld / st require -- while only lanes with an unfinished problem
+// keep what it yields in pb.U and s (a finished lane's pb.x, act_prev, hints and store are scratch from then on: what is
+// written out depends on pb.U and s alone).  A warp whose problems are all done skips the round as a whole.
+template <bool FIRST_PASS, bool ONESEG = false, class ST>
 MPCB_HD void solve_round(const DevTable& T, const DevParams& P, Problem& pb, const ST& st, SolveState& s, int round) {
+  static_assert(!ONESEG || FIRST_PASS, "the one-segment round is the first pass's");
   const Policy& pl = P.pol[FIRST_PASS ? 1 : 0];
   const int max_segments = FIRST_PASS ? P.thread_max_segments : pl.max_segments;
   const bool hot = s.hot;
@@ -763,46 +955,72 @@ MPCB_HD void solve_round(const DevTable& T, const DevParams& P, Problem& pb, con
     });
     pb.act_prev = act0;
   };
-  if (!s.done) {
-    double cviol;
-    linearise(T, P, pb, st, cviol);
+  auto start_round = [&](double cviol) {
     if (s.first) {
       cold_start(pb.U);
 #pragma unroll
       for (int i = 0; i < NV; ++i) pb.x[i] = pb.U[i];
       s.first = false;
     }
-    if (cviol > P.feas_tol) { s.infeasible = true; s.out.const_infeasible = true; }
-    s.out.rounds++;
-  }
-  // inexact Gauss-Newton: a round's QP is only solved as accurately as the previous SQP step warrants
-  const double step_prev = s.step_prev;
-  const double loosen = (FIRST_PASS || P.qp_forcing <= 0.0) ? 1.0
-                        : dmax(1.0, (step_prev * P.qp_forcing < P.qp_eps_loose ? step_prev * P.qp_forcing : P.qp_eps_loose) / P.eps_p);
-  const double eps_p = P.eps_p * loosen, eps_d = P.eps_d * loosen;
+    if (!s.done) {
+      if (cviol > P.feas_tol) { s.infeasible = true; s.out.const_infeasible = true; }
+      s.out.rounds++;
+    }
+  };
   bool conv = false;                           // this round's QP closed
-  bool qdone = s.done;                         // nothing more to do on this round's QP (closed, certified or caps hit)
   bool cert = false;
-  for (int seg = 0; seg < max_segments; ++seg) {
-    if (MPCB_ALL(qdone)) break;
-    if (!qdone) {
-      factor<FIRST_PASS>(P, pl, pb, st);
-      SegStats ss;
-      for (int it = 0; it < pl.segment_iters - 1; ++it) admm_iter<false, false, FIRST_PASS>(P, pl, pb, st, ss);
-      admm_iter<true, !FIRST_PASS, FIRST_PASS>(P, pl, pb, st, ss, eps_p);
-      s.out.iters += pl.segment_iters;
-#ifdef MPCB_TRACE
-      if (getenv("MPCB_TRACE")) {
-        printf("  r%d s%d pass %d rp %.2e rd %.2e nd %.2e act %011llx E", round, seg, FIRST_PASS ? 1 : 2, ss.rp, ss.rd, ss.nd, pb.act_prev);
-        for (int r = 0; r < M_ROWS; ++r) printf("%d", pb.E.get(r));
-        printf(" x");
-        for (int i = 0; i < NV; ++i) printf(" %.4f", pb.x[i]);
-        printf("\n");
-      }
+  if constexpr (ONESEG) {
+#if defined(__CUDA_ARCH__)
+    const bool work = __any_sync(0xffffffffu, !s.done);   // warp-uniform
+#else
+    const bool work = !s.done;
 #endif
-      if (ss.rp <= eps_p && ss.rd <= eps_d) { conv = true; qdone = true; }
-      else if (!FIRST_PASS && ss.nd > 1e-9 && ss.atdy <= P.eps_inf * ss.nd && ss.sup < -P.eps_inf * ss.nd &&
-               ss.bad <= P.eps_inf * ss.nd) { conv = true; cert = true; qdone = true; }
+    if (work) {
+      double H[NTRI], cviol;
+      linearise(T, P, pb, st, cviol, H);
+      start_round(cviol);
+      factor<true>(P, pl, pb, st, H);
+      SegStats ss;
+      for (int it = 0; it < pl.segment_iters - 1; ++it) admm_iter<false, false, true>(P, pl, pb, st, ss);
+      admm_iter<true, false, true>(P, pl, pb, st, ss, P.eps_p);
+      if (!s.done) {
+        s.out.iters += pl.segment_iters;
+        conv = ss.rp <= P.eps_p && ss.rd <= P.eps_d;
+      }
+    }
+  } else {
+    if (!s.done) {
+      double cviol;
+      linearise(T, P, pb, st, cviol);
+      start_round(cviol);
+    }
+    // inexact Gauss-Newton: a round's QP is only solved as accurately as the previous SQP step warrants
+    const double step_prev = s.step_prev;
+    const double loosen = (FIRST_PASS || P.qp_forcing <= 0.0) ? 1.0
+                          : dmax(1.0, (step_prev * P.qp_forcing < P.qp_eps_loose ? step_prev * P.qp_forcing : P.qp_eps_loose) / P.eps_p);
+    const double eps_p = P.eps_p * loosen, eps_d = P.eps_d * loosen;
+    bool qdone = s.done;                         // nothing more to do on this round's QP (closed, certified or caps hit)
+    for (int seg = 0; seg < max_segments; ++seg) {
+      if (MPCB_ALL(qdone)) break;
+      if (!qdone) {
+        factor<FIRST_PASS>(P, pl, pb, st);
+        SegStats ss;
+        for (int it = 0; it < pl.segment_iters - 1; ++it) admm_iter<false, false, FIRST_PASS>(P, pl, pb, st, ss);
+        admm_iter<true, !FIRST_PASS, FIRST_PASS>(P, pl, pb, st, ss, eps_p);
+        s.out.iters += pl.segment_iters;
+#ifdef MPCB_TRACE
+        if (getenv("MPCB_TRACE")) {
+          printf("  r%d s%d pass %d rp %.2e rd %.2e nd %.2e act %011llx E", round, seg, FIRST_PASS ? 1 : 2, ss.rp, ss.rd, ss.nd, pb.act_prev);
+          for (int r = 0; r < M_ROWS; ++r) printf("%d", pb.E.get(r));
+          printf(" x");
+          for (int i = 0; i < NV; ++i) printf(" %.4f", pb.x[i]);
+          printf("\n");
+        }
+#endif
+        if (ss.rp <= eps_p && ss.rd <= eps_d) { conv = true; qdone = true; }
+        else if (!FIRST_PASS && ss.nd > 1e-9 && ss.atdy <= P.eps_inf * ss.nd && ss.sup < -P.eps_inf * ss.nd &&
+                 ss.bad <= P.eps_inf * ss.nd) { conv = true; cert = true; qdone = true; }
+      }
     }
   }
   (void)round;
