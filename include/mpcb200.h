@@ -275,7 +275,8 @@ int mpcb_sim_create(mpcb_sim_handle* out, mpcb_handle h, int B, const mpcb_scena
 int mpcb_sim_create_routes(mpcb_sim_handle* out, mpcb_handle h, int B, const mpcb_scenario* scen, int n_scen,
                            const int* route, const double* x_init, int history_steps);
 int mpcb_sim_destroy(mpcb_sim_handle s);
-/* n_steps closed-loop steps, asynchronous on cuda_stream (3 + the solver's launches per step, no host round trip).
+/* n_steps closed-loop steps, asynchronous on cuda_stream (3 + the solver's launches per step, no host round trip; with
+ * following on, 2 more plus the kernels of two radix sorts).
  * Vehicles that have passed s_max - 1 are frozen. */
 int mpcb_sim_step(mpcb_sim_handle s, int n_steps, void* cuda_stream);
 /* Hot start (off by default): from its second step on, a vehicle's first pass starts from its previous plan advanced by
@@ -283,6 +284,28 @@ int mpcb_sim_step(mpcb_sim_handle s, int n_steps, void* cuda_stream);
  * sit on their bounds there taken as active.  The problem solved is the same and so is its converged answer; what changes
  * is how often the robust pass is needed (a vehicle waiting at a red light poses the same problem a hundred steps in a row). */
 int mpcb_sim_set_hot_start(mpcb_sim_handle s, int on);
+/* Following (off by default; on = 1 takes effect from the next step, on = 0 switches it off and ignores follow_range):
+ * the vehicles see each other.  At the start of every step, from the states the loop condition is evaluated on:
+ *   - a leader is a vehicle still driving on the same route (an arrived vehicle has left the route);
+ *   - the vehicles of a route are ordered by (s, index); the leader of b is the next vehicle in that order when
+ *     s_leader - s_b <= follow_range, else b has none;
+ *   - the FSM runs per vehicle as before, lights included; the car slot of the obstacle set takes the nearer (smaller s)
+ *     of the scripted car, when the FSM reports one, and the leader, at (s, v) of the leader at the start of the step;
+ *     on a tie the scripted car.  The light stays after the car slot, so n_obs <= MPCB_MAX_OBS.
+ * Hot start and routes work unchanged.  With following off, every entry point behaves as without this call.
+ * follow_range must be positive and finite (else MPCB_ERR_INVALID before any CUDA call); B <= 2^27.  The first call with
+ * on = 1 allocates the sort workspace and the leader histories (synchronises the device's default stream).
+ * mpcb_launch_count counts the two kernels following adds per step, not the kernels of its two radix sorts. */
+int mpcb_sim_set_follow(mpcb_sim_handle s, int on, double follow_range);
+/* Leaders of the first history_steps steps, HOST outputs (any may be NULL): hist_lead_idx [n_recorded][B] (-1: none),
+ * hist_lead_sv [n_recorded][B][2] its (s, v) at the start of the step (NaN: none).  -1 / NaN also mark steps where the
+ * vehicle had arrived and steps taken with following off. */
+int mpcb_sim_follow_history(mpcb_sim_handle s, int* n_recorded, int* hist_lead_idx, double* hist_lead_sv,
+                            void* cuda_stream);
+/* Gap to the leader over the recorded steps (needs history_steps > 0, else MPCB_ERR_INVALID): min_gap [B] HOST (may be
+ * NULL) = min of s_leader - s (1e30 for a vehicle that never had a leader), ok [B] HOST = min_gap >= 1 m (the reference's
+ * safety distance of its moving-obstacle check, sanity_checks.py:142-164). */
+int mpcb_sim_follow_check(mpcb_sim_handle s, int* ok, double* min_gap, void* cuda_stream);
 /* number of vehicles still driving (synchronises the stream) */
 int mpcb_sim_alive(mpcb_sim_handle s, int* n_alive, void* cuda_stream);
 /* HOST outputs (any may be NULL): current states [B][5], steps driven [B], steps whose solve was not MPCB_SOLVED [B] */

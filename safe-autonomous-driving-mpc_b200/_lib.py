@@ -106,7 +106,10 @@ SYMBOLS = {
     "mpcb_sim_destroy": (C.c_int, [C.c_void_p]),
     "mpcb_sim_step": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
     "mpcb_sim_set_hot_start": (C.c_int, [C.c_void_p, C.c_int]),
-    "mpcb_sim_alive": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.c_void_p]),
+    "mpcb_sim_set_follow": (C.c_int, [C.c_void_p, C.c_int, C.c_double]),
+    "mpcb_sim_follow_history": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mpcb_sim_follow_check": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mpcb_sim_alive":(C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.c_void_p]),
     "mpcb_sim_state": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mpcb_sim_check": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mpcb_check_histories": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_double, C.POINTER(Scenario)] + [C.c_void_p] * 8),

@@ -6,13 +6,16 @@
 //
 // One simulation object holds B vehicles (each with its own scenario constants and FSM state).  A step is three
 // launches on one stream -- FSM kernel -> mpcb_solve_batch -> plant kernel -- with no host round trip, so a
-// Monte-Carlo of whole drives never leaves the GPU; histories are recorded into device buffers when asked for.
+// Monte-Carlo of whole drives never leaves the GPU; histories are recorded into device buffers when asked for.  With
+// following on (mpcb_sim_set_follow), a key kernel, two radix sorts and a leader kernel come first.
 #include <cuda_runtime.h>
 #include <math.h>
 #include <string.h>
 
 #include <new>
 #include <vector>
+
+#include <cub/device/device_radix_sort.cuh>
 
 #include "mpcb200.h"
 #include "mpcb_internal.h"
@@ -39,14 +42,70 @@ __device__ __forceinline__ double stop_s(const DevTables& Ts, const int* __restr
   return vehicle_table(Ts, route, b).s_max - 1.0;
 }
 
-// ObstaclesFSM.update for every vehicle that is still driving (:330-374); car first, then light (:349, :362)
+// ---- following (mpcb_sim_set_follow): the nearest vehicle ahead on the same route is a moving obstacle ---------------
+// Each step, before the FSM kernel and from the states the loop condition is evaluated on, the vehicles are ordered by
+// (driving, route, s, b): the key kernel writes an order-preserving 64-bit key of s and a 32-bit tag (route key << 27 | b,
+// route key MPCB_MAX_ROUTES for a vehicle that is not driving), a stable radix sort by the s key carries the tags, and a
+// stable sort of the tags by their route bits groups them by route.  Both sorts are stable and the input is in index
+// order, so equal positions are ordered by index.  The leader of b is the next tag of its route segment, if it is within
+// follow_range.
+constexpr int FOLLOW_IDX_BITS = 27;                     // vehicles of a following simulation: < 2^27
+constexpr unsigned FOLLOW_IDX_MASK = (1u << FOLLOW_IDX_BITS) - 1u;
+constexpr int FOLLOW_ROUTE_BITS = 5;                    // route keys 0 .. MPCB_MAX_ROUTES (= not driving)
+static_assert(MPCB_MAX_ROUTES < (1 << FOLLOW_ROUTE_BITS), "route key does not fit its bits");
+static_assert(FOLLOW_IDX_BITS + FOLLOW_ROUTE_BITS == 32, "tag layout");
+
+__global__ void __launch_bounds__(128)
+mpcb_follow_key_kernel(const __grid_constant__ DevTables Ts, const int* __restrict__ route, int B,
+                       const double* __restrict__ x, unsigned long long* __restrict__ key, unsigned* __restrict__ tag) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  const double s = x[(size_t)b * 5] + 0.0;              // -0.0 -> +0.0: equal positions get equal keys
+  const bool live = s <= stop_s(Ts, route, b);          // loop condition (:395), as the FSM kernel evaluates it
+  const unsigned long long u = (unsigned long long)__double_as_longlong(s);
+  key[b] = (u >> 63) ? ~u : (u | (1ull << 63));         // order-preserving: unsigned order of keys = order of s
+  const unsigned r = live ? (unsigned)problem_route(route, b, Ts.n) : (unsigned)MPCB_MAX_ROUTES;
+  MPCB_ASSERT(r <= (unsigned)MPCB_MAX_ROUTES);
+  tag[b] = (r << FOLLOW_IDX_BITS) | (unsigned)b;
+}
+
+// over the sorted tags: lead_idx[b] (-1: none) and lead_sv[b] = (s, v) of the leader (NaN: none)
+__global__ void __launch_bounds__(128)
+mpcb_follow_leader_kernel(int B, double range, const double* __restrict__ x, const unsigned* __restrict__ sorted,
+                          int* __restrict__ lead_idx, double* __restrict__ lead_sv) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= B) return;
+  const unsigned t = sorted[i];
+  const int b = (int)(t & FOLLOW_IDX_MASK);
+  const unsigned r = t >> FOLLOW_IDX_BITS;
+  MPCB_ASSERT(b < B && r <= (unsigned)MPCB_MAX_ROUTES);
+  int lead = -1;
+  double ls = nan(""), lv = nan("");
+  if (r < (unsigned)MPCB_MAX_ROUTES && i + 1 < B) {
+    const unsigned tn = sorted[i + 1];
+    if ((tn >> FOLLOW_IDX_BITS) == r) {
+      const int j = (int)(tn & FOLLOW_IDX_MASK);
+      MPCB_ASSERT(j < B && j != b);
+      const double sj = x[(size_t)j * 5];
+      if (sj - x[(size_t)b * 5] <= range) { lead = j; ls = sj; lv = x[(size_t)j * 5 + 4]; }
+    }
+  }
+  lead_idx[b] = lead;
+  lead_sv[2 * b] = ls;
+  lead_sv[2 * b + 1] = lv;
+}
+
+// ObstaclesFSM.update for every vehicle that is still driving (:330-374); car first, then light (:349, :362).
+// lead_sv != nullptr (following on): the car slot takes the nearer of the scripted car and the leader (lead_idx /
+// lead_sv of mpcb_follow_leader_kernel), which is recorded into hist_lead_idx / hist_lead_sv.
 __global__ void __launch_bounds__(128)
 mpcb_fsm_kernel(const __grid_constant__ DevTables Ts, const int* __restrict__ route, int B, double dt,
                 const double* __restrict__ x, const DevScenario* __restrict__ scen,
                 double* __restrict__ fsm_f, int* __restrict__ fsm_i, int* __restrict__ alive,
                 double* __restrict__ obs_sv, int* __restrict__ n_obs, int rec_t, double* __restrict__ hist_obs,
                 int* __restrict__ hist_tl, int* __restrict__ alive_idx, int* __restrict__ alive_cnt,
-                int* __restrict__ next_cnt) {
+                int* __restrict__ next_cnt, const int* __restrict__ lead_idx, const double* __restrict__ lead_sv,
+                int* __restrict__ hist_lead_idx, double* __restrict__ hist_lead_sv) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b == 0) *next_cnt = 0;                                 // the other counter of the pair: next step's list length
   const bool in = b < B;
@@ -75,6 +134,13 @@ mpcb_fsm_kernel(const __grid_constant__ DevTables Ts, const int* __restrict__ ro
         else { o[0] = obs_s; o[1] = sc.obs_v; n = 1; car_s = obs_s; }
       }
     }
+    if (lead_sv) {
+      // the car slot holds the nearer of the scripted car and the leader (tie: the scripted car).  On a single-lane
+      // route the farther car is behind the nearer one, and the nearer car is itself constrained by it, so keeping
+      // clear of the nearer one is enough; one car slot keeps n_obs <= MPCB_MAX_OBS with the light after it.
+      const double ls = lead_sv[2 * b];
+      if (!isnan(ls) && !(n == 1 && o[0] <= ls)) { o[0] = ls; o[1] = lead_sv[2 * b + 1]; n = 1; }
+    }
     if (sc.traffic_light && !(f & F_TL_GREEN)) {
       const double gap = sc.tl_pos - s;
       if (0.0 < gap && gap < sc.tl_trigger_s) {
@@ -96,6 +162,14 @@ mpcb_fsm_kernel(const __grid_constant__ DevTables Ts, const int* __restrict__ ro
   if (hist_obs && rec_t >= 0) {
     hist_obs[(size_t)rec_t * B + b] = car_s;                 // position of the moving car, NaN when absent
     hist_tl[(size_t)rec_t * B + b] = live ? ((f & F_TL_GREEN) ? 1 : 0) : -1;   // light colour returned by update()
+  }
+  if (lead_sv && hist_lead_idx && rec_t >= 0) {             // leader of this step; -1 / NaN: none or arrived
+    const size_t i = (size_t)rec_t * B + b;
+    const int lead = live ? lead_idx[b] : -1;
+    MPCB_ASSERT(lead >= -1 && lead < B);
+    hist_lead_idx[i] = lead;
+    hist_lead_sv[2 * i] = lead >= 0 ? lead_sv[2 * b] : nan("");
+    hist_lead_sv[2 * i + 1] = lead >= 0 ? lead_sv[2 * b + 1] : nan("");
   }
 }
 
@@ -191,6 +265,25 @@ mpcb_sim_check_kernel(const __grid_constant__ DevTables Ts, const int* __restric
   metrics[(size_t)b * 4 + 3] = (double)steps[b];
 }
 
+// the check of item 4 (gap >= 1 m, sanity_checks.py:142-164) against the recorded leaders: min over the recorded steps
+// of s_leader - s (BIG if never had a leader) and ok = that gap >= 1 m
+__global__ void __launch_bounds__(128)
+mpcb_follow_check_kernel(int B, int n_rec, const int* __restrict__ steps, const double* __restrict__ hist_x,
+                         const double* __restrict__ hist_lead_sv, int* __restrict__ ok, double* __restrict__ min_gap) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  const int n = min(steps[b], n_rec);
+  const double safety = 1.0;
+  double g = BIG;
+  for (int t = 0; t < n; ++t) {
+    const size_t i = (size_t)t * B + b;
+    const double ls = hist_lead_sv[2 * i];
+    if (!isnan(ls)) g = fmin(g, ls - hist_x[i * 5]);
+  }
+  ok[b] = g < safety ? 0 : 1;
+  min_gap[b] = g;
+}
+
 }  // namespace mpcb
 
 using namespace mpcb;
@@ -210,6 +303,19 @@ struct mpcb_sim {
   double* d_metrics = nullptr;
   double *hist_x = nullptr, *hist_u = nullptr, *hist_obs = nullptr;
   int *hist_status = nullptr, *hist_tl = nullptr;
+  // following (mpcb_sim_set_follow); the buffers are allocated the first time it is switched on
+  int follow = 0;
+  double follow_range = 0.0;
+  unsigned long long* f_key = nullptr;   // [2][B]: s keys, then sorted
+  unsigned* f_tag = nullptr;             // [3][B]: tags, sorted by s, then by route
+  void* f_temp = nullptr;                // radix-sort workspace, sized for B
+  size_t f_temp_bytes = 0;
+  int* lead_idx = nullptr;               // [B] leader of this step (-1: none)
+  double* lead_sv = nullptr;             // [B][2] its (s, v) (NaN: none)
+  int* hist_lead_idx = nullptr;          // [cap][B], -1 where not recorded
+  double* hist_lead_sv = nullptr;        // [cap][B][2], NaN where not recorded
+  int* d_follow_ok = nullptr;            // outputs of mpcb_sim_follow_check
+  double* d_min_gap = nullptr;
 };
 
 extern "C" {
@@ -233,7 +339,8 @@ int mpcb_sim_destroy(mpcb_sim_handle s) {
   cudaSetDevice(s->h->device);
   void* ptrs[] = {s->route, s->scen, s->x, s->fsm_f, s->obs_sv, s->U, s->fsm_i, s->alive, s->n_obs, s->status, s->steps,
                   s->n_unsolved, s->count, s->hist_x, s->hist_u, s->hist_obs, s->hist_status, s->hist_tl, s->alive_idx,
-                  s->alive_cnt, s->d_verdict, s->d_metrics};
+                  s->alive_cnt, s->d_verdict, s->d_metrics, s->f_key, s->f_tag, s->f_temp, s->lead_idx, s->lead_sv,
+                  s->hist_lead_idx, s->hist_lead_sv, s->d_follow_ok, s->d_min_gap};
   for (void* p : ptrs) if (p) cudaFree(p);
   delete s;
   return MPCB_OK;
@@ -306,9 +413,23 @@ int mpcb_sim_step(mpcb_sim_handle s, int n_steps, void* cuda_stream) {
   for (int k = 0; k < n_steps; ++k) {
     const int rec = (s->t < s->cap) ? s->t : -1;
     int* cnt = s->alive_cnt + (s->t & 1);
+    if (s->follow) {                                         // leaders of this step, from the states before it
+      const size_t nb = (size_t)s->B;
+      mpcb_follow_key_kernel<<<grid, 128, 0, st>>>(s->h->dt, s->route, s->B, s->x, s->f_key, s->f_tag);
+      CK(cudaGetLastError());
+      size_t tb = s->f_temp_bytes;
+      CK(cub::DeviceRadixSort::SortPairs(s->f_temp, tb, s->f_key, s->f_key + nb, s->f_tag, s->f_tag + nb, s->B, 0, 64, st));
+      tb = s->f_temp_bytes;
+      CK(cub::DeviceRadixSort::SortKeys(s->f_temp, tb, s->f_tag + nb, s->f_tag + 2 * nb, s->B, FOLLOW_IDX_BITS, 32, st));
+      mpcb_follow_leader_kernel<<<grid, 128, 0, st>>>(s->B, s->follow_range, s->x, s->f_tag + 2 * nb, s->lead_idx,
+                                                      s->lead_sv);
+      CK(cudaGetLastError());
+      s->h->launches += 2;                                   // the radix sorts' own kernels are not counted
+    }
     mpcb_fsm_kernel<<<grid, 128, 0, st>>>(s->h->dt, s->route, s->B, s->dt, s->x, s->scen, s->fsm_f, s->fsm_i, s->alive, s->obs_sv,
                                           s->n_obs, rec, s->hist_obs, s->hist_tl, s->alive_idx, cnt,
-                                          s->alive_cnt + ((s->t + 1) & 1));
+                                          s->alive_cnt + ((s->t + 1) & 1), s->lead_idx,
+                                          s->follow ? s->lead_sv : nullptr, s->hist_lead_idx, s->hist_lead_sv);
     CK(cudaGetLastError());
     // the solve runs over the list of vehicles still driving (arrived vehicles are frozen and cost nothing)
     int rc = mpcb_solve_list_internal(s->h, s->B, s->alive_idx, cnt, s->x, s->obs_sv, s->n_obs, s->route, s->U, s->status,
@@ -326,6 +447,88 @@ int mpcb_sim_step(mpcb_sim_handle s, int n_steps, void* cuda_stream) {
 int mpcb_sim_set_hot_start(mpcb_sim_handle s, int on) {
   if (!s) return MPCB_ERR_INVALID;
   s->hot_start = on ? 1 : 0;
+  return MPCB_OK;
+}
+
+int mpcb_sim_set_follow(mpcb_sim_handle s, int on, double follow_range) {
+  if (!s) return MPCB_ERR_INVALID;
+  if (!on) { s->follow = 0; return MPCB_OK; }
+  if (!(follow_range > 0.0) || !isfinite(follow_range) || (unsigned)s->B > FOLLOW_IDX_MASK + 1u) return MPCB_ERR_INVALID;
+  if (!s->f_key) {
+    CK(cudaSetDevice(s->h->device));
+    const size_t nb = (size_t)s->B;
+    size_t t1 = 0, t2 = 0;
+    CK(cub::DeviceRadixSort::SortPairs(nullptr, t1, (unsigned long long*)nullptr, (unsigned long long*)nullptr,
+                                       (unsigned*)nullptr, (unsigned*)nullptr, s->B, 0, 64));
+    CK(cub::DeviceRadixSort::SortKeys(nullptr, t2, (unsigned*)nullptr, (unsigned*)nullptr, s->B, FOLLOW_IDX_BITS, 32));
+    const size_t temp = t1 > t2 ? t1 : t2;
+    const size_t nt = (size_t)s->cap * nb;
+    bool ok = cudaMalloc((void**)&s->f_key, nb * 16) == cudaSuccess && cudaMalloc((void**)&s->f_tag, nb * 12) == cudaSuccess &&
+              cudaMalloc(&s->f_temp, temp) == cudaSuccess && cudaMalloc((void**)&s->lead_idx, nb * 4) == cudaSuccess &&
+              cudaMalloc((void**)&s->lead_sv, nb * 16) == cudaSuccess;
+    if (ok && nt > 0)
+      ok = cudaMalloc((void**)&s->hist_lead_idx, nt * 4) == cudaSuccess &&
+           cudaMalloc((void**)&s->hist_lead_sv, nt * 16) == cudaSuccess &&
+           cudaMalloc((void**)&s->d_follow_ok, nb * 4) == cudaSuccess && cudaMalloc((void**)&s->d_min_gap, nb * 8) == cudaSuccess;
+    if (!ok) {
+      cudaGetLastError();
+      void* ptrs[] = {s->f_key, s->f_tag, s->f_temp, s->lead_idx, s->lead_sv, s->hist_lead_idx, s->hist_lead_sv,
+                      s->d_follow_ok, s->d_min_gap};
+      for (void* p : ptrs) if (p) cudaFree(p);
+      s->f_key = nullptr; s->f_tag = nullptr; s->f_temp = nullptr; s->lead_idx = nullptr; s->lead_sv = nullptr;
+      s->hist_lead_idx = nullptr; s->hist_lead_sv = nullptr; s->d_follow_ok = nullptr; s->d_min_gap = nullptr;
+      return MPCB_ERR_NOMEM;
+    }
+    s->f_temp_bytes = temp;
+    // rows of steps taken with following off stay -1 / NaN (all-ones bytes: int -1, a double NaN)
+    if (nt > 0) {
+      CK(cudaMemset(s->hist_lead_idx, 0xff, nt * 4));
+      CK(cudaMemset(s->hist_lead_sv, 0xff, nt * 16));
+      CK(cudaStreamSynchronize(0));
+    }
+  }
+  s->follow = 1;
+  s->follow_range = follow_range;
+  return MPCB_OK;
+}
+
+int mpcb_sim_follow_history(mpcb_sim_handle s, int* n_recorded, int* hist_lead_idx, double* hist_lead_sv,
+                            void* cuda_stream) {
+  if (!s) return MPCB_ERR_INVALID;
+  const int nt = s->t < s->cap ? s->t : s->cap;
+  if (n_recorded) *n_recorded = nt;
+  const size_t n = (size_t)nt * s->B;
+  if (n == 0 || (!hist_lead_idx && !hist_lead_sv)) return MPCB_OK;
+  if (!s->hist_lead_idx) {                                   // following never switched on: nothing recorded
+    if (hist_lead_idx) for (size_t i = 0; i < n; ++i) hist_lead_idx[i] = -1;
+    if (hist_lead_sv) for (size_t i = 0; i < 2 * n; ++i) hist_lead_sv[i] = nan("");
+    return MPCB_OK;
+  }
+  CK(cudaSetDevice(s->h->device));
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  if (hist_lead_idx) CK(cudaMemcpyAsync(hist_lead_idx, s->hist_lead_idx, n * 4, cudaMemcpyDeviceToHost, st));
+  if (hist_lead_sv) CK(cudaMemcpyAsync(hist_lead_sv, s->hist_lead_sv, n * 16, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  return MPCB_OK;
+}
+
+int mpcb_sim_follow_check(mpcb_sim_handle s, int* ok, double* min_gap, void* cuda_stream) {
+  if (!s || !ok || s->cap < 1) return MPCB_ERR_INVALID;
+  const size_t nb = (size_t)s->B;
+  if (!s->hist_lead_sv) {                                    // following never switched on: no leader, ever
+    for (size_t b = 0; b < nb; ++b) { ok[b] = 1; if (min_gap) min_gap[b] = BIG; }
+    return MPCB_OK;
+  }
+  CK(cudaSetDevice(s->h->device));
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  const int nt = s->t < s->cap ? s->t : s->cap;
+  mpcb_follow_check_kernel<<<(s->B + 127) / 128, 128, 0, st>>>(s->B, nt, s->steps, s->hist_x, s->hist_lead_sv,
+                                                               s->d_follow_ok, s->d_min_gap);
+  CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(ok, s->d_follow_ok, nb * 4, cudaMemcpyDeviceToHost, st));
+  if (min_gap) CK(cudaMemcpyAsync(min_gap, s->d_min_gap, nb * 8, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  s->h->launches += 1;
   return MPCB_OK;
 }
 

@@ -66,14 +66,26 @@ def check_histories(tracker, s_total, scenarios, x_final, steps, hist_x, hist_u,
     return _verdict_dict(v, m)
 
 
+def _follow_range(r):
+    r = float(r)
+    if not (np.isfinite(r) and r > 0.0):
+        raise ValueError(f"follow_range must be positive and finite, got {r!r}")
+    return r
+
+
 class BatchedSimulation:
-    def __init__(self, tracker, scenarios, B=None, x_init=None, history_steps=0, hot_start=False, route=None):
+    def __init__(self, tracker, scenarios, B=None, x_init=None, history_steps=0, hot_start=False, route=None,
+                 follow_range=None):
         """tracker: BatchedTracker; scenarios: one Scenario (shared) or a list of B; x_init: [B,5] or None for the
         reference's start state.  hot_start: from its second step on a vehicle's solve starts from its previous plan
         advanced by one step (mpcb_sim_set_hot_start) instead of the reference's table-based warm start.
-        route: one int or an int array [B], vehicle b driving ``tracker.routes[route[b]]`` (None: route 0)."""
+        route: one int or an int array [B], vehicle b driving ``tracker.routes[route[b]]`` (None: route 0).
+        follow_range: None (off) or a positive distance: the nearest vehicle ahead on the same route within that
+        distance is a moving obstacle (``set_follow``)."""
         self._lib = tracker._lib
         self._t = tracker
+        if follow_range is not None:
+            follow_range = _follow_range(follow_range)
         scen = list(scenarios) if isinstance(scenarios, (list, tuple)) else [scenarios]
         if B is None:
             B = len(scen) if len(scen) > 1 else (len(x_init) if x_init is not None else 1)
@@ -99,6 +111,8 @@ class BatchedSimulation:
         self.history_steps = int(history_steps)
         if hot_start:
             check(self._lib.mpcb_sim_set_hot_start(h, 1), "mpcb_sim_set_hot_start")
+        if follow_range is not None:
+            self.set_follow(follow_range)
 
     def __del__(self):
         h = getattr(self, "_h", None)
@@ -127,6 +141,35 @@ class BatchedSimulation:
         hs = np.empty((T, B), np.int32); ht = np.empty((T, B), np.int32)
         check(self._lib.mpcb_sim_history(self._h, C.byref(n), _dp(hx), _dp(hu), _dp(ho), _dp(hs), _dp(ht), None))
         return dict(x=hx, u=hu, obs_s=ho, status=hs, tl=ht)
+
+    def set_follow(self, follow_range):
+        """Following from the next step on (mpcb_sim_set_follow): at the start of every step the nearest vehicle still
+        driving ahead on the same route, ordered by (s, index), is vehicle b's leader when it is at most
+        ``follow_range`` metres ahead; the nearer of the leader and the scripted car takes the car slot of b's obstacle
+        set.  None switches following off."""
+        if follow_range is None:
+            check(self._lib.mpcb_sim_set_follow(self._h, 0, 0.0), "mpcb_sim_set_follow")
+            return
+        check(self._lib.mpcb_sim_set_follow(self._h, 1, _follow_range(follow_range)), "mpcb_sim_set_follow")
+
+    def follow_history(self):
+        """Leaders of the recorded steps: lead [T,B] (vehicle index, -1: none, arrived, or following off), lead_s and
+        lead_v [T,B] (the leader's s and v at the start of the step, NaN where lead is -1)."""
+        n = C.c_int()
+        check(self._lib.mpcb_sim_follow_history(self._h, C.byref(n), None, None, None), "mpcb_sim_follow_history")
+        T, B = n.value, self.B
+        li = np.empty((T, B), np.int32)
+        sv = np.empty((T, B, 2))
+        check(self._lib.mpcb_sim_follow_history(self._h, C.byref(n), _dp(li), _dp(sv), None), "mpcb_sim_follow_history")
+        return dict(lead=li, lead_s=sv[..., 0], lead_v=sv[..., 1])
+
+    def follow_check(self):
+        """Gap to the leader over the recorded steps: min_gap [B] (1e30 if never had a leader) and ok [B] = gap >= 1 m,
+        the reference's moving-obstacle safety distance (sanity_checks.py:142-164)."""
+        ok = np.empty(self.B, np.int32)
+        g = np.empty(self.B)
+        check(self._lib.mpcb_sim_follow_check(self._h, _dp(ok), _dp(g), None), "mpcb_sim_follow_check")
+        return dict(ok=ok.astype(bool), min_gap=g)
 
     CHECKS = CHECKS
 
