@@ -13,6 +13,7 @@
 #include <string.h>
 
 #include <new>
+#include <type_traits>
 #include <vector>
 
 #include <cub/device/device_radix_sort.cuh>
@@ -27,6 +28,117 @@ struct DevScenario {          // per vehicle, mirrors ObstaclesFSM.__init__ (:28
   double tl_pos, tl_trigger_s, tl_stop_duration;
   int dynamic_obstacle, traffic_light;
 };
+
+// The device arrays of a simulation, in four groups: the loop state and the histories are one block made at create,
+// following and its histories one block made by the first mpcb_sim_set_follow(on).  The layout of a block, every copy
+// and every fill is derived from SIM_BYTES.
+enum SimRegion {
+  R_SCEN, R_X, R_FSM_F, R_OBS_SV, R_U, R_FSM_I, R_ALIVE, R_N_OBS, R_STATUS, R_STEPS, R_N_UNSOLVED, R_ALIVE_IDX,
+  R_ALIVE_CNT, R_COUNT, R_ROUTE,                                                         // loop state
+  R_HIST_X, R_HIST_U, R_HIST_OBS, R_HIST_STATUS, R_HIST_TL, R_VERDICT, R_METRICS,         // histories
+  R_F_KEY, R_F_TAG, R_F_TEMP, R_LEAD_IDX, R_LEAD_SV,                                      // following
+  R_HIST_LEAD_IDX, R_HIST_LEAD_SV, R_FOLLOW_OK, R_MIN_GAP,                                // following histories
+  N_SIM
+};
+constexpr unsigned sim_span(int lo, int hi) { return ((1u << hi) - 1u) & ~((1u << lo) - 1u); }   // regions lo .. hi-1
+constexpr unsigned SIM_LOOP = sim_span(R_SCEN, R_ROUTE);          // R_ROUTE only on a routed simulation
+constexpr unsigned SIM_HIST = sim_span(R_HIST_X, R_F_KEY);
+constexpr unsigned SIM_FOLLOW = sim_span(R_F_KEY, R_HIST_LEAD_IDX);
+constexpr unsigned SIM_FOLLOW_HIST = sim_span(R_HIST_LEAD_IDX, N_SIM);
+static_assert(N_SIM < 32, "regions are selected by the bits of an unsigned");
+
+enum SimPer { PER_VEHICLE, PER_STEP, FIXED };   // bytes per vehicle, per vehicle and recorded step, or in all
+struct SimBytes { SimPer per; size_t bytes; };
+static const SimBytes SIM_BYTES[N_SIM] = {
+  /* scen          */ {PER_VEHICLE, sizeof(DevScenario)},
+  /* x             */ {PER_VEHICLE, 5 * 8},
+  /* fsm_f         */ {PER_VEHICLE, 2 * 8},      // car position, light timer
+  /* obs_sv        */ {PER_VEHICLE, 4 * 8},
+  /* U             */ {PER_VEHICLE, NV * 8},
+  /* fsm_i         */ {PER_VEHICLE, 4},
+  /* alive         */ {PER_VEHICLE, 4},
+  /* n_obs         */ {PER_VEHICLE, 4},
+  /* status        */ {PER_VEHICLE, 4},
+  /* steps         */ {PER_VEHICLE, 4},
+  /* n_unsolved    */ {PER_VEHICLE, 4},
+  /* alive_idx     */ {PER_VEHICLE, 4},          // list of the vehicles still driving
+  /* alive_cnt     */ {FIXED, 2 * 4},            // its length, double-buffered
+  /* count         */ {FIXED, 4},                // mpcb_sim_alive
+  /* route         */ {PER_VEHICLE, 4},
+  /* hist_x        */ {PER_STEP, 5 * 8},         // [cap][B][5]
+  /* hist_u        */ {PER_STEP, 2 * 8},
+  /* hist_obs      */ {PER_STEP, 8},
+  /* hist_status   */ {PER_STEP, 4},
+  /* hist_tl       */ {PER_STEP, 4},
+  /* verdict       */ {PER_VEHICLE, 4},          // mpcb_sim_check
+  /* metrics       */ {PER_VEHICLE, 4 * 8},
+  /* f_key         */ {PER_VEHICLE, 2 * 8},      // [2][B]: s keys, then sorted
+  /* f_tag         */ {PER_VEHICLE, 3 * 4},      // [3][B]: tags, sorted by s, then by route
+  /* f_temp        */ {FIXED, 0},                // radix-sort workspace: its size query's bytes (sim_layout)
+  /* lead_idx      */ {PER_VEHICLE, 4},          // leader of this step (-1: none)
+  /* lead_sv       */ {PER_VEHICLE, 2 * 8},      // its (s, v) (NaN: none)
+  /* hist_lead_idx */ {PER_STEP, 4},             // -1 where not recorded
+  /* hist_lead_sv  */ {PER_STEP, 2 * 8},         // NaN where not recorded
+  /* follow_ok     */ {PER_VEHICLE, 4},          // mpcb_sim_follow_check
+  /* min_gap       */ {PER_VEHICLE, 8},
+};
+
+// Bytes of region r for B vehicles and T recorded steps (R_F_TEMP: see sim_layout).
+static size_t sim_bytes(int r, size_t B, size_t T) {
+  const SimBytes& s = SIM_BYTES[r];
+  return s.bytes * (s.per == PER_VEHICLE ? B : s.per == PER_STEP ? T * B : 1);
+}
+
+// Layout of the regions in mask of a simulation of B vehicles and T recorded steps, with a radix-sort workspace of temp
+// bytes: region r at off[r] (no bytes when it is not in mask), off[N_SIM] bytes in all.  Each region starts on 256
+// bytes, which also keeps U 16-byte aligned for the solve's 128-bit stores into it.
+static void sim_layout(size_t B, size_t T, unsigned mask, size_t temp, size_t (&off)[N_SIM + 1]) {
+  size_t bytes[N_SIM];
+  for (int r = 0; r < N_SIM; ++r) bytes[r] = !((mask >> r) & 1u) ? 0 : r == R_F_TEMP ? temp : sim_bytes(r, B, T);
+  region_offsets(bytes, N_SIM, off);
+}
+
+// The device arrays of a simulation (nullptr: not allocated), handed to its kernels as one grid-constant parameter.  The
+// kernels bind the arrays they use to __restrict__ locals (the qualifier is not honoured on struct members): the
+// read-only ones then load through the non-coherent path.
+struct SimArrays {
+  DevScenario* scen; double* x; double* fsm_f; double* obs_sv; double* U;
+  int* fsm_i; int* alive; int* n_obs; int* status; int* steps; int* n_unsolved; int* alive_idx; int* alive_cnt;
+  int* count; int* route;
+  double* hist_x; double* hist_u; double* hist_obs; int* hist_status; int* hist_tl; int* verdict; double* metrics;
+  unsigned long long* f_key; unsigned* f_tag; void* f_temp; int* lead_idx; double* lead_sv;
+  int* hist_lead_idx; double* hist_lead_sv; int* follow_ok; double* min_gap;
+};
+
+// One block holding the regions in mask, laid out by sim_layout; points their arrays in d into it and leaves the others.
+// nullptr (and no error left pending) when it cannot be allocated.
+static char* sim_alloc(SimArrays& d, size_t B, size_t T, unsigned mask, size_t temp, size_t (&off)[N_SIM + 1]) {
+  sim_layout(B, T, mask, temp, off);
+  char* base = nullptr;
+  if (cudaMalloc((void**)&base, off[N_SIM]) != cudaSuccess) { cudaGetLastError(); return nullptr; }
+  auto at = [&](auto*& p, int r) {
+    if ((mask >> r) & 1u) p = (std::remove_reference_t<decltype(p)>)(base + off[r]);
+  };
+  at(d.scen, R_SCEN); at(d.x, R_X); at(d.fsm_f, R_FSM_F); at(d.obs_sv, R_OBS_SV); at(d.U, R_U);
+  at(d.fsm_i, R_FSM_I); at(d.alive, R_ALIVE); at(d.n_obs, R_N_OBS); at(d.status, R_STATUS); at(d.steps, R_STEPS);
+  at(d.n_unsolved, R_N_UNSOLVED); at(d.alive_idx, R_ALIVE_IDX); at(d.alive_cnt, R_ALIVE_CNT); at(d.count, R_COUNT);
+  at(d.route, R_ROUTE);
+  at(d.hist_x, R_HIST_X); at(d.hist_u, R_HIST_U); at(d.hist_obs, R_HIST_OBS); at(d.hist_status, R_HIST_STATUS);
+  at(d.hist_tl, R_HIST_TL); at(d.verdict, R_VERDICT); at(d.metrics, R_METRICS);
+  at(d.f_key, R_F_KEY); at(d.f_tag, R_F_TAG); at(d.f_temp, R_F_TEMP); at(d.lead_idx, R_LEAD_IDX);
+  at(d.lead_sv, R_LEAD_SV);
+  at(d.hist_lead_idx, R_HIST_LEAD_IDX); at(d.hist_lead_sv, R_HIST_LEAD_SV); at(d.follow_ok, R_FOLLOW_OK);
+  at(d.min_gap, R_MIN_GAP);
+  return base;
+}
+
+// The read-only arrays of the fsm, plant and count kernels are read with __ldg: the compiler takes this non-coherent
+// path by itself for __restrict__ kernel parameters, but in these three kernels not for the restrict-qualified locals.
+__device__ __forceinline__ DevScenario ldg(const DevScenario* p) {
+  return DevScenario{__ldg(&p->obs_trigger_s), __ldg(&p->obs_start_s), __ldg(&p->obs_v), __ldg(&p->obs_end_s),
+                     __ldg(&p->tl_pos), __ldg(&p->tl_trigger_s), __ldg(&p->tl_stop_duration),
+                     __ldg(&p->dynamic_obstacle), __ldg(&p->traffic_light)};
+}
 
 enum { F_OBS_ACTIVE = 1, F_OBS_TRIGGERED = 2, F_TL_GREEN = 4, F_TL_WAITING = 8 };
 
@@ -56,8 +168,11 @@ static_assert(MPCB_MAX_ROUTES < (1 << FOLLOW_ROUTE_BITS), "route key does not fi
 static_assert(FOLLOW_IDX_BITS + FOLLOW_ROUTE_BITS == 32, "tag layout");
 
 __global__ void __launch_bounds__(128)
-mpcb_follow_key_kernel(const __grid_constant__ DevTables Ts, const int* __restrict__ route, int B,
-                       const double* __restrict__ x, unsigned long long* __restrict__ key, unsigned* __restrict__ tag) {
+mpcb_follow_key_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ SimArrays sim, int B) {
+  const int* __restrict__ route = sim.route;
+  const double* __restrict__ x = sim.x;
+  unsigned long long* __restrict__ key = sim.f_key;
+  unsigned* __restrict__ tag = sim.f_tag;
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
   const double s = x[(size_t)b * 5] + 0.0;              // -0.0 -> +0.0: equal positions get equal keys
@@ -69,10 +184,13 @@ mpcb_follow_key_kernel(const __grid_constant__ DevTables Ts, const int* __restri
   tag[b] = (r << FOLLOW_IDX_BITS) | (unsigned)b;
 }
 
-// over the sorted tags: lead_idx[b] (-1: none) and lead_sv[b] = (s, v) of the leader (NaN: none)
+// over the sorted tags (f_tag + 2 B): lead_idx[b] (-1: none) and lead_sv[b] = (s, v) of the leader (NaN: none)
 __global__ void __launch_bounds__(128)
-mpcb_follow_leader_kernel(int B, double range, const double* __restrict__ x, const unsigned* __restrict__ sorted,
-                          int* __restrict__ lead_idx, double* __restrict__ lead_sv) {
+mpcb_follow_leader_kernel(const __grid_constant__ SimArrays sim, int B, double range) {
+  const double* __restrict__ x = sim.x;
+  const unsigned* __restrict__ sorted = sim.f_tag + 2 * (size_t)B;
+  int* __restrict__ lead_idx = sim.lead_idx;
+  double* __restrict__ lead_sv = sim.lead_sv;
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= B) return;
   const unsigned t = sorted[i];
@@ -96,20 +214,31 @@ mpcb_follow_leader_kernel(int B, double range, const double* __restrict__ x, con
 }
 
 // ObstaclesFSM.update for every vehicle that is still driving (:330-374); car first, then light (:349, :362).
-// lead_sv != nullptr (following on): the car slot takes the nearer of the scripted car and the leader (lead_idx /
-// lead_sv of mpcb_follow_leader_kernel), which is recorded into hist_lead_idx / hist_lead_sv.
+// alive_cnt / next_cnt: this step's and the next step's counter of the pair sim.alive_cnt.  With following on, the car
+// slot takes the nearer of the scripted car and the leader (lead_idx / lead_sv of mpcb_follow_leader_kernel), which is
+// recorded into hist_lead_idx / hist_lead_sv.
 __global__ void __launch_bounds__(128)
-mpcb_fsm_kernel(const __grid_constant__ DevTables Ts, const int* __restrict__ route, int B, double dt,
-                const double* __restrict__ x, const DevScenario* __restrict__ scen,
-                double* __restrict__ fsm_f, int* __restrict__ fsm_i, int* __restrict__ alive,
-                double* __restrict__ obs_sv, int* __restrict__ n_obs, int rec_t, double* __restrict__ hist_obs,
-                int* __restrict__ hist_tl, int* __restrict__ alive_idx, int* __restrict__ alive_cnt,
-                int* __restrict__ next_cnt, const int* __restrict__ lead_idx, const double* __restrict__ lead_sv,
-                int* __restrict__ hist_lead_idx, double* __restrict__ hist_lead_sv) {
+mpcb_fsm_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ SimArrays sim, int B, double dt, int rec_t,
+                int* __restrict__ alive_cnt, int* __restrict__ next_cnt, int follow) {
+  const int* __restrict__ route = sim.route;
+  const double* __restrict__ x = sim.x;
+  const DevScenario* __restrict__ scen = sim.scen;
+  double* __restrict__ fsm_f = sim.fsm_f;
+  int* __restrict__ fsm_i = sim.fsm_i;
+  int* __restrict__ alive = sim.alive;
+  double* __restrict__ obs_sv = sim.obs_sv;
+  int* __restrict__ n_obs = sim.n_obs;
+  double* __restrict__ hist_obs = sim.hist_obs;
+  int* __restrict__ hist_tl = sim.hist_tl;
+  int* __restrict__ alive_idx = sim.alive_idx;
+  const int* __restrict__ lead_idx = sim.lead_idx;
+  const double* __restrict__ lead_sv = follow ? sim.lead_sv : nullptr;
+  int* __restrict__ hist_lead_idx = sim.hist_lead_idx;
+  double* __restrict__ hist_lead_sv = sim.hist_lead_sv;
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b == 0) *next_cnt = 0;                                 // the other counter of the pair: next step's list length
   const bool in = b < B;
-  const double s = in ? x[(size_t)b * 5] : 0.0, v = in ? x[(size_t)b * 5 + 4] : 0.0;
+  const double s = in ? __ldg(x + (size_t)b * 5) : 0.0, v = in ? __ldg(x + (size_t)b * 5 + 4) : 0.0;
   const int live = (in && s <= stop_s(Ts, route, b)) ? 1 : 0;   // loop condition (:395), evaluated before the step
   // list of the vehicles still driving: the solve of this step runs over the list, not over all B (one atomic per warp;
   // the order of the list does not matter, every problem is solved on its own and written to its own slot)
@@ -122,7 +251,7 @@ mpcb_fsm_kernel(const __grid_constant__ DevTables Ts, const int* __restrict__ ro
   double car_s = nan("");
   int f = fsm_i[b];
   if (live) {
-    const DevScenario sc = scen[b];
+    const DevScenario sc = ldg(scen + b);
     double obs_s = fsm_f[2 * b], timer = fsm_f[2 * b + 1];
     if (sc.dynamic_obstacle) {
       if (s >= sc.obs_trigger_s && !(f & F_OBS_TRIGGERED)) f |= F_OBS_TRIGGERED | F_OBS_ACTIVE;
@@ -138,8 +267,8 @@ mpcb_fsm_kernel(const __grid_constant__ DevTables Ts, const int* __restrict__ ro
       // the car slot holds the nearer of the scripted car and the leader (tie: the scripted car).  On a single-lane
       // route the farther car is behind the nearer one, and the nearer car is itself constrained by it, so keeping
       // clear of the nearer one is enough; one car slot keeps n_obs <= MPCB_MAX_OBS with the light after it.
-      const double ls = lead_sv[2 * b];
-      if (!isnan(ls) && !(n == 1 && o[0] <= ls)) { o[0] = ls; o[1] = lead_sv[2 * b + 1]; n = 1; }
+      const double ls = __ldg(lead_sv + 2 * b);
+      if (!isnan(ls) && !(n == 1 && o[0] <= ls)) { o[0] = ls; o[1] = __ldg(lead_sv + 2 * b + 1); n = 1; }
     }
     if (sc.traffic_light && !(f & F_TL_GREEN)) {
       const double gap = sc.tl_pos - s;
@@ -165,33 +294,41 @@ mpcb_fsm_kernel(const __grid_constant__ DevTables Ts, const int* __restrict__ ro
   }
   if (lead_sv && hist_lead_idx && rec_t >= 0) {             // leader of this step; -1 / NaN: none or arrived
     const size_t i = (size_t)rec_t * B + b;
-    const int lead = live ? lead_idx[b] : -1;
+    const int lead = live ? __ldg(lead_idx + b) : -1;
     MPCB_ASSERT(lead >= -1 && lead < B);
     hist_lead_idx[i] = lead;
-    hist_lead_sv[2 * i] = lead >= 0 ? lead_sv[2 * b] : nan("");
-    hist_lead_sv[2 * i + 1] = lead >= 0 ? lead_sv[2 * b + 1] : nan("");
+    hist_lead_sv[2 * i] = lead >= 0 ? __ldg(lead_sv + 2 * b) : nan("");
+    hist_lead_sv[2 * i + 1] = lead >= 0 ? __ldg(lead_sv + 2 * b + 1) : nan("");
   }
 }
 
 // plant step (:404-406) for the vehicles that were alive at the start of the step
 __global__ void __launch_bounds__(128)
-mpcb_plant_kernel(const __grid_constant__ DevTables Ts, const int* __restrict__ route, int B, double dt, double* __restrict__ x,
-                  const double* __restrict__ U, const int* __restrict__ status, const int* __restrict__ alive,
-                  int* __restrict__ steps, int* __restrict__ n_unsolved, int rec_t, double* __restrict__ hist_x,
-                  double* __restrict__ hist_u, int* __restrict__ hist_status) {
+mpcb_plant_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ SimArrays sim, int B, double dt,
+                  int rec_t) {
+  const int* __restrict__ route = sim.route;
+  double* __restrict__ x = sim.x;
+  const double* __restrict__ U = sim.U;
+  const int* __restrict__ status = sim.status;
+  const int* __restrict__ alive = sim.alive;
+  int* __restrict__ steps = sim.steps;
+  int* __restrict__ n_unsolved = sim.n_unsolved;
+  double* __restrict__ hist_x = sim.hist_x;
+  double* __restrict__ hist_u = sim.hist_u;
+  int* __restrict__ hist_status = sim.hist_status;
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
-  const int live = alive[b];
+  const int live = __ldg(alive + b);
   double xs[5];
 #pragma unroll
   for (int c = 0; c < 5; ++c) xs[c] = x[(size_t)b * 5 + c];
-  const double u1 = U[(size_t)b * NV], u2 = U[(size_t)b * NV + 1];
+  const double u1 = __ldg(U + (size_t)b * NV), u2 = __ldg(U + (size_t)b * NV + 1);
   if (hist_x && rec_t >= 0) {                                // state and control of THIS step (before the update)
 #pragma unroll
     for (int c = 0; c < 5; ++c) hist_x[((size_t)rec_t * B + b) * 5 + c] = live ? xs[c] : nan("");
     hist_u[((size_t)rec_t * B + b) * 2] = live ? u1 : nan("");
     hist_u[((size_t)rec_t * B + b) * 2 + 1] = live ? u2 : nan("");
-    hist_status[(size_t)rec_t * B + b] = live ? status[b] : -1;
+    hist_status[(size_t)rec_t * B + b] = live ? __ldg(status + b) : -1;
   }
   if (!live) return;
   double val[4], slope[4];
@@ -205,13 +342,16 @@ mpcb_plant_kernel(const __grid_constant__ DevTables Ts, const int* __restrict__ 
   x[(size_t)b * 5 + 3] = __dadd_rn(k, __dmul_rn(dt, u1));
   x[(size_t)b * 5 + 4] = __dadd_rn(v, __dmul_rn(dt, u2));
   steps[b] += 1;
-  if (status[b] != MPCB_SOLVED) n_unsolved[b] += 1;
+  if (__ldg(status + b) != MPCB_SOLVED) n_unsolved[b] += 1;
 }
 
-__global__ void mpcb_count_alive_kernel(const __grid_constant__ DevTables Ts, const int* __restrict__ route, int B,
-                                        const double* __restrict__ x, int* __restrict__ count) {
+__global__ void mpcb_count_alive_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ SimArrays sim,
+                                        int B) {
+  const int* __restrict__ route = sim.route;
+  const double* __restrict__ x = sim.x;
+  int* __restrict__ count = sim.count;
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
-  const int live = (b < B && x[(size_t)b * 5] <= stop_s(Ts, route, b)) ? 1 : 0;
+  const int live = (b < B && __ldg(x + (size_t)b * 5) <= stop_s(Ts, route, b)) ? 1 : 0;
   const unsigned m = __ballot_sync(0xffffffffu, live);
   if ((threadIdx.x & 31) == 0 && m) atomicAdd(count, __popc(m));
 }
@@ -223,12 +363,18 @@ __global__ void mpcb_count_alive_kernel(const __grid_constant__ DevTables Ts, co
 // every vehicle's route is s_total long; else vehicle b's route's s_max.
 // (The reference's CPU-time item :134-139 is a property of the host, not of the trajectory; it is not evaluated here.)
 __global__ void __launch_bounds__(128)
-mpcb_sim_check_kernel(const __grid_constant__ DevTables Ts, const int* __restrict__ route, int B, int n_rec,
-                      double s_total, double u1_min, double u1_max, double u2_min, double u2_max,
-                      const double* __restrict__ x_final, const int* __restrict__ steps,
-                      const DevScenario* __restrict__ scen, const double* __restrict__ hist_x,
-                      const double* __restrict__ hist_u, const double* __restrict__ hist_obs,
-                      const int* __restrict__ hist_tl, int* __restrict__ verdict, double* __restrict__ metrics) {
+mpcb_sim_check_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ SimArrays sim, int B, int n_rec,
+                      double s_total, double u1_min, double u1_max, double u2_min, double u2_max) {
+  const int* __restrict__ route = sim.route;
+  const double* __restrict__ x_final = sim.x;
+  const int* __restrict__ steps = sim.steps;
+  const DevScenario* __restrict__ scen = sim.scen;
+  const double* __restrict__ hist_x = sim.hist_x;
+  const double* __restrict__ hist_u = sim.hist_u;
+  const double* __restrict__ hist_obs = sim.hist_obs;
+  const int* __restrict__ hist_tl = sim.hist_tl;
+  int* __restrict__ verdict = sim.verdict;
+  double* __restrict__ metrics = sim.metrics;
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
   const DevScenario sc = scen[b];
@@ -268,8 +414,12 @@ mpcb_sim_check_kernel(const __grid_constant__ DevTables Ts, const int* __restric
 // the check of item 4 (gap >= 1 m, sanity_checks.py:142-164) against the recorded leaders: min over the recorded steps
 // of s_leader - s (BIG if never had a leader) and ok = that gap >= 1 m
 __global__ void __launch_bounds__(128)
-mpcb_follow_check_kernel(int B, int n_rec, const int* __restrict__ steps, const double* __restrict__ hist_x,
-                         const double* __restrict__ hist_lead_sv, int* __restrict__ ok, double* __restrict__ min_gap) {
+mpcb_follow_check_kernel(const __grid_constant__ SimArrays sim, int B, int n_rec) {
+  const int* __restrict__ steps = sim.steps;
+  const double* __restrict__ hist_x = sim.hist_x;
+  const double* __restrict__ hist_lead_sv = sim.hist_lead_sv;
+  int* __restrict__ ok = sim.follow_ok;
+  double* __restrict__ min_gap = sim.min_gap;
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
   const int n = min(steps[b], n_rec);
@@ -293,30 +443,32 @@ struct mpcb_sim {
   int B, cap, t;              // vehicles, history capacity (steps), steps recorded so far
   int hot_start = 0;          // first pass of step t > 0 starts from step t - 1's plans advanced by one step (mpcb_sim_set_hot_start)
   double dt;
-  int* route = nullptr;       // route of each vehicle (device); nullptr: all on route 0
-  DevScenario* scen = nullptr;
-  double *x = nullptr, *fsm_f = nullptr, *obs_sv = nullptr, *U = nullptr;
-  int *fsm_i = nullptr, *alive = nullptr, *n_obs = nullptr, *status = nullptr, *steps = nullptr, *n_unsolved = nullptr,
-      *count = nullptr;
-  int *alive_idx = nullptr, *alive_cnt = nullptr;   // list of the vehicles still driving; its length, double-buffered
-  int* d_verdict = nullptr;                         // outputs of mpcb_sim_check (allocated with the histories)
-  double* d_metrics = nullptr;
-  double *hist_x = nullptr, *hist_u = nullptr, *hist_obs = nullptr;
-  int *hist_status = nullptr, *hist_tl = nullptr;
-  // following (mpcb_sim_set_follow); the buffers are allocated the first time it is switched on
+  SimArrays d = {};           // the device arrays: loop state and histories in block[0] (made at create), following and
+  char* block[2] = {};        // its histories in block[1] (made the first time following is switched on)
+  // following (mpcb_sim_set_follow)
   int follow = 0;
   double follow_range = 0.0;
-  unsigned long long* f_key = nullptr;   // [2][B]: s keys, then sorted
-  unsigned* f_tag = nullptr;             // [3][B]: tags, sorted by s, then by route
-  void* f_temp = nullptr;                // radix-sort workspace, sized for B
-  size_t f_temp_bytes = 0;
-  int* lead_idx = nullptr;               // [B] leader of this step (-1: none)
-  double* lead_sv = nullptr;             // [B][2] its (s, v) (NaN: none)
-  int* hist_lead_idx = nullptr;          // [cap][B], -1 where not recorded
-  double* hist_lead_sv = nullptr;        // [cap][B][2], NaN where not recorded
-  int* d_follow_ok = nullptr;            // outputs of mpcb_sim_follow_check
-  double* d_min_gap = nullptr;
+  size_t f_temp_bytes = 0;    // bytes of d.f_temp
 };
+
+static DevScenario to_dev_scenario(const mpcb_scenario& c) {
+  return DevScenario{c.obs_trigger_s, c.obs_start_s, c.obs_v, c.obs_end_s, c.tl_pos, c.tl_trigger_s,
+                     c.tl_stop_duration, c.dynamic_obstacle, c.traffic_light};
+}
+
+// The checks on the first n_rec recorded steps of d, on stream st; the verdicts (and the metrics, when metrics is given)
+// are copied to the caller's arrays.
+static cudaError_t launch_check(mpcb_handle h, const SimArrays& d, int B, int n_rec, double s_total, int* verdict,
+                                double* metrics, cudaStream_t st) {
+  const mpcb_params& p = h->params;
+  mpcb_sim_check_kernel<<<(B + 127) / 128, 128, 0, st>>>(h->dt, d, B, n_rec, s_total, p.u_min[0], p.u_max[0], p.u_min[1],
+                                                        p.u_max[1]);
+  cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess) e = cudaMemcpyAsync(verdict, d.verdict, sim_bytes(R_VERDICT, B, 0), cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess && metrics)
+    e = cudaMemcpyAsync(metrics, d.metrics, sim_bytes(R_METRICS, B, 0), cudaMemcpyDeviceToHost, st);
+  return e;
+}
 
 extern "C" {
 
@@ -337,11 +489,7 @@ int mpcb_scenario_default(mpcb_scenario* s, int which) {
 int mpcb_sim_destroy(mpcb_sim_handle s) {
   if (!s) return MPCB_ERR_INVALID;
   cudaSetDevice(s->h->device);
-  void* ptrs[] = {s->route, s->scen, s->x, s->fsm_f, s->obs_sv, s->U, s->fsm_i, s->alive, s->n_obs, s->status, s->steps,
-                  s->n_unsolved, s->count, s->hist_x, s->hist_u, s->hist_obs, s->hist_status, s->hist_tl, s->alive_idx,
-                  s->alive_cnt, s->d_verdict, s->d_metrics, s->f_key, s->f_tag, s->f_temp, s->lead_idx, s->lead_sv,
-                  s->hist_lead_idx, s->hist_lead_sv, s->d_follow_ok, s->d_min_gap};
-  for (void* p : ptrs) if (p) cudaFree(p);
+  for (char* p : s->block) if (p) cudaFree(p);
   delete s;
   return MPCB_OK;
 }
@@ -363,44 +511,31 @@ int mpcb_sim_create_routes(mpcb_sim_handle* out, mpcb_handle h, int B, const mpc
   if (!s) return MPCB_ERR_NOMEM;
   s->h = h; s->B = B; s->cap = history_steps; s->t = 0;
   s->dt = h->params.dt;
-  auto fail = [&](int code) { mpcb_sim_destroy(s); return code; };
   const size_t nb = (size_t)B;
-#define SIM_ALLOC(ptr, bytes) if (cudaMalloc((void**)&(ptr), (bytes)) != cudaSuccess) { cudaGetLastError(); return fail(MPCB_ERR_NOMEM); }
-  SIM_ALLOC(s->scen, nb * sizeof(DevScenario));
-  SIM_ALLOC(s->x, nb * 40); SIM_ALLOC(s->fsm_f, nb * 16); SIM_ALLOC(s->obs_sv, nb * 32); SIM_ALLOC(s->U, nb * 80);
-  SIM_ALLOC(s->fsm_i, nb * 4); SIM_ALLOC(s->alive, nb * 4); SIM_ALLOC(s->n_obs, nb * 4); SIM_ALLOC(s->status, nb * 4);
-  SIM_ALLOC(s->steps, nb * 4); SIM_ALLOC(s->n_unsolved, nb * 4); SIM_ALLOC(s->count, 4);
-  SIM_ALLOC(s->alive_idx, nb * 4); SIM_ALLOC(s->alive_cnt, 8);
-  if (route) SIM_ALLOC(s->route, nb * 4);
-  if (history_steps > 0) {
-    SIM_ALLOC(s->d_verdict, nb * 4); SIM_ALLOC(s->d_metrics, nb * 32);
-    const size_t nt = (size_t)history_steps * nb;
-    SIM_ALLOC(s->hist_x, nt * 40); SIM_ALLOC(s->hist_u, nt * 16); SIM_ALLOC(s->hist_obs, nt * 8);
-    SIM_ALLOC(s->hist_status, nt * 4); SIM_ALLOC(s->hist_tl, nt * 4);
-  }
-#undef SIM_ALLOC
+  const unsigned mask = SIM_LOOP | (route ? 1u << R_ROUTE : 0u) | (history_steps > 0 ? SIM_HIST : 0u);
+  size_t off[N_SIM + 1];
+  if (!(s->block[0] = sim_alloc(s->d, nb, (size_t)history_steps, mask, 0, off))) { delete s; return MPCB_ERR_NOMEM; }
+  auto fail = [&](int code) { mpcb_sim_destroy(s); return code; };
   std::vector<DevScenario> hs(nb);
   std::vector<double> hx(nb * 5), hf(nb * 2);
   for (size_t b = 0; b < nb; ++b) {
     const mpcb_scenario& c = scen[n_scen == 1 ? 0 : b];
-    hs[b] = DevScenario{c.obs_trigger_s, c.obs_start_s, c.obs_v, c.obs_end_s, c.tl_pos, c.tl_trigger_s,
-                        c.tl_stop_duration, c.dynamic_obstacle, c.traffic_light};
+    hs[b] = to_dev_scenario(c);
     if (x_init) for (int k = 0; k < 5; ++k) hx[b * 5 + k] = x_init[b * 5 + k];
     else { hx[b * 5] = hx[b * 5 + 1] = hx[b * 5 + 2] = hx[b * 5 + 3] = 0.0; hx[b * 5 + 4] = 0.5; }   // :382
     hf[b * 2] = c.obs_start_s;                                          // obs_s = obs_start_s (:297)
     hf[b * 2 + 1] = 0.0;
   }
+  // start values, synchronous on the default stream: from the host, then zeros
+  const struct { int r; const void* src; } start[] = {{R_ROUTE, route}, {R_SCEN, hs.data()}, {R_X, hx.data()},
+                                                      {R_FSM_F, hf.data()}};
+  char* base = s->block[0];
   cudaError_t e;
-  if (route && (e = cudaMemcpy(s->route, route, nb * 4, cudaMemcpyHostToDevice)) != cudaSuccess) return fail(cuda_fail(e, "cudaMemcpy"));
-  if ((e = cudaMemcpy(s->scen, hs.data(), nb * sizeof(DevScenario), cudaMemcpyHostToDevice)) != cudaSuccess) return fail(cuda_fail(e, "cudaMemcpy"));
-  if ((e = cudaMemcpy(s->x, hx.data(), nb * 40, cudaMemcpyHostToDevice)) != cudaSuccess) return fail(cuda_fail(e, "cudaMemcpy"));
-  if ((e = cudaMemcpy(s->fsm_f, hf.data(), nb * 16, cudaMemcpyHostToDevice)) != cudaSuccess) return fail(cuda_fail(e, "cudaMemcpy"));
-  if ((e = cudaMemset(s->fsm_i, 0, nb * 4)) != cudaSuccess) return fail(cuda_fail(e, "cudaMemset"));
-  if ((e = cudaMemset(s->steps, 0, nb * 4)) != cudaSuccess) return fail(cuda_fail(e, "cudaMemset"));
-  if ((e = cudaMemset(s->n_unsolved, 0, nb * 4)) != cudaSuccess) return fail(cuda_fail(e, "cudaMemset"));
-  if ((e = cudaMemset(s->alive_cnt, 0, 8)) != cudaSuccess) return fail(cuda_fail(e, "cudaMemset"));
-  if ((e = cudaMemset(s->status, 0, nb * 4)) != cudaSuccess) return fail(cuda_fail(e, "cudaMemset"));
-  if ((e = cudaMemset(s->U, 0, nb * 80)) != cudaSuccess) return fail(cuda_fail(e, "cudaMemset"));
+  for (const auto& c : start)
+    if (c.src && (e = cudaMemcpy(base + off[c.r], c.src, sim_bytes(c.r, nb, 0), cudaMemcpyHostToDevice)) != cudaSuccess)
+      return fail(cuda_fail(e, "cudaMemcpy"));
+  for (int r : {R_FSM_I, R_STEPS, R_N_UNSOLVED, R_ALIVE_CNT, R_STATUS, R_U})
+    if ((e = cudaMemset(base + off[r], 0, sim_bytes(r, nb, 0))) != cudaSuccess) return fail(cuda_fail(e, "cudaMemset"));
   *out = s;
   return MPCB_OK;
 }
@@ -409,34 +544,30 @@ int mpcb_sim_step(mpcb_sim_handle s, int n_steps, void* cuda_stream) {
   if (!s || n_steps < 0) return MPCB_ERR_INVALID;
   CK(cudaSetDevice(s->h->device));
   cudaStream_t st = (cudaStream_t)cuda_stream;
+  const SimArrays& d = s->d;
   const int grid = (s->B + 127) / 128;
   for (int k = 0; k < n_steps; ++k) {
     const int rec = (s->t < s->cap) ? s->t : -1;
-    int* cnt = s->alive_cnt + (s->t & 1);
+    int* cnt = d.alive_cnt + (s->t & 1);
     if (s->follow) {                                         // leaders of this step, from the states before it
       const size_t nb = (size_t)s->B;
-      mpcb_follow_key_kernel<<<grid, 128, 0, st>>>(s->h->dt, s->route, s->B, s->x, s->f_key, s->f_tag);
+      mpcb_follow_key_kernel<<<grid, 128, 0, st>>>(s->h->dt, d, s->B);
       CK(cudaGetLastError());
       size_t tb = s->f_temp_bytes;
-      CK(cub::DeviceRadixSort::SortPairs(s->f_temp, tb, s->f_key, s->f_key + nb, s->f_tag, s->f_tag + nb, s->B, 0, 64, st));
+      CK(cub::DeviceRadixSort::SortPairs(d.f_temp, tb, d.f_key, d.f_key + nb, d.f_tag, d.f_tag + nb, s->B, 0, 64, st));
       tb = s->f_temp_bytes;
-      CK(cub::DeviceRadixSort::SortKeys(s->f_temp, tb, s->f_tag + nb, s->f_tag + 2 * nb, s->B, FOLLOW_IDX_BITS, 32, st));
-      mpcb_follow_leader_kernel<<<grid, 128, 0, st>>>(s->B, s->follow_range, s->x, s->f_tag + 2 * nb, s->lead_idx,
-                                                      s->lead_sv);
+      CK(cub::DeviceRadixSort::SortKeys(d.f_temp, tb, d.f_tag + nb, d.f_tag + 2 * nb, s->B, FOLLOW_IDX_BITS, 32, st));
+      mpcb_follow_leader_kernel<<<grid, 128, 0, st>>>(d, s->B, s->follow_range);
       CK(cudaGetLastError());
       s->h->launches += 2;                                   // the radix sorts' own kernels are not counted
     }
-    mpcb_fsm_kernel<<<grid, 128, 0, st>>>(s->h->dt, s->route, s->B, s->dt, s->x, s->scen, s->fsm_f, s->fsm_i, s->alive, s->obs_sv,
-                                          s->n_obs, rec, s->hist_obs, s->hist_tl, s->alive_idx, cnt,
-                                          s->alive_cnt + ((s->t + 1) & 1), s->lead_idx,
-                                          s->follow ? s->lead_sv : nullptr, s->hist_lead_idx, s->hist_lead_sv);
+    mpcb_fsm_kernel<<<grid, 128, 0, st>>>(s->h->dt, d, s->B, s->dt, rec, cnt, d.alive_cnt + ((s->t + 1) & 1), s->follow);
     CK(cudaGetLastError());
     // the solve runs over the list of vehicles still driving (arrived vehicles are frozen and cost nothing)
-    int rc = mpcb_solve_list_internal(s->h, s->B, s->alive_idx, cnt, s->x, s->obs_sv, s->n_obs, s->route, s->U, s->status,
-                                      st, (s->hot_start && s->t > 0) ? s->U : nullptr);
+    int rc = mpcb_solve_list_internal(s->h, s->B, d.alive_idx, cnt, d.x, d.obs_sv, d.n_obs, d.route, d.U, d.status, st,
+                                      (s->hot_start && s->t > 0) ? d.U : nullptr);
     if (rc != MPCB_OK) return rc;
-    mpcb_plant_kernel<<<grid, 128, 0, st>>>(s->h->dt, s->route, s->B, s->dt, s->x, s->U, s->status, s->alive, s->steps,
-                                            s->n_unsolved, rec, s->hist_x, s->hist_u, s->hist_status);
+    mpcb_plant_kernel<<<grid, 128, 0, st>>>(s->h->dt, d, s->B, s->dt, rec);
     CK(cudaGetLastError());
     s->h->launches += 2;
     s->t += 1;
@@ -454,36 +585,22 @@ int mpcb_sim_set_follow(mpcb_sim_handle s, int on, double follow_range) {
   if (!s) return MPCB_ERR_INVALID;
   if (!on) { s->follow = 0; return MPCB_OK; }
   if (!(follow_range > 0.0) || !isfinite(follow_range) || (unsigned)s->B > FOLLOW_IDX_MASK + 1u) return MPCB_ERR_INVALID;
-  if (!s->f_key) {
+  if (!s->block[1]) {
     CK(cudaSetDevice(s->h->device));
-    const size_t nb = (size_t)s->B;
+    const size_t nb = (size_t)s->B, T = (size_t)s->cap;
     size_t t1 = 0, t2 = 0;
     CK(cub::DeviceRadixSort::SortPairs(nullptr, t1, (unsigned long long*)nullptr, (unsigned long long*)nullptr,
                                        (unsigned*)nullptr, (unsigned*)nullptr, s->B, 0, 64));
     CK(cub::DeviceRadixSort::SortKeys(nullptr, t2, (unsigned*)nullptr, (unsigned*)nullptr, s->B, FOLLOW_IDX_BITS, 32));
     const size_t temp = t1 > t2 ? t1 : t2;
-    const size_t nt = (size_t)s->cap * nb;
-    bool ok = cudaMalloc((void**)&s->f_key, nb * 16) == cudaSuccess && cudaMalloc((void**)&s->f_tag, nb * 12) == cudaSuccess &&
-              cudaMalloc(&s->f_temp, temp) == cudaSuccess && cudaMalloc((void**)&s->lead_idx, nb * 4) == cudaSuccess &&
-              cudaMalloc((void**)&s->lead_sv, nb * 16) == cudaSuccess;
-    if (ok && nt > 0)
-      ok = cudaMalloc((void**)&s->hist_lead_idx, nt * 4) == cudaSuccess &&
-           cudaMalloc((void**)&s->hist_lead_sv, nt * 16) == cudaSuccess &&
-           cudaMalloc((void**)&s->d_follow_ok, nb * 4) == cudaSuccess && cudaMalloc((void**)&s->d_min_gap, nb * 8) == cudaSuccess;
-    if (!ok) {
-      cudaGetLastError();
-      void* ptrs[] = {s->f_key, s->f_tag, s->f_temp, s->lead_idx, s->lead_sv, s->hist_lead_idx, s->hist_lead_sv,
-                      s->d_follow_ok, s->d_min_gap};
-      for (void* p : ptrs) if (p) cudaFree(p);
-      s->f_key = nullptr; s->f_tag = nullptr; s->f_temp = nullptr; s->lead_idx = nullptr; s->lead_sv = nullptr;
-      s->hist_lead_idx = nullptr; s->hist_lead_sv = nullptr; s->d_follow_ok = nullptr; s->d_min_gap = nullptr;
+    size_t off[N_SIM + 1];
+    if (!(s->block[1] = sim_alloc(s->d, nb, T, SIM_FOLLOW | (T > 0 ? SIM_FOLLOW_HIST : 0u), temp, off)))
       return MPCB_ERR_NOMEM;
-    }
     s->f_temp_bytes = temp;
     // rows of steps taken with following off stay -1 / NaN (all-ones bytes: int -1, a double NaN)
-    if (nt > 0) {
-      CK(cudaMemset(s->hist_lead_idx, 0xff, nt * 4));
-      CK(cudaMemset(s->hist_lead_sv, 0xff, nt * 16));
+    if (T > 0) {
+      CK(cudaMemset(s->d.hist_lead_idx, 0xff, sim_bytes(R_HIST_LEAD_IDX, nb, T)));
+      CK(cudaMemset(s->d.hist_lead_sv, 0xff, sim_bytes(R_HIST_LEAD_SV, nb, T)));
       CK(cudaStreamSynchronize(0));
     }
   }
@@ -499,15 +616,16 @@ int mpcb_sim_follow_history(mpcb_sim_handle s, int* n_recorded, int* hist_lead_i
   if (n_recorded) *n_recorded = nt;
   const size_t n = (size_t)nt * s->B;
   if (n == 0 || (!hist_lead_idx && !hist_lead_sv)) return MPCB_OK;
-  if (!s->hist_lead_idx) {                                   // following never switched on: nothing recorded
+  if (!s->d.hist_lead_idx) {                                 // following never switched on: nothing recorded
     if (hist_lead_idx) for (size_t i = 0; i < n; ++i) hist_lead_idx[i] = -1;
     if (hist_lead_sv) for (size_t i = 0; i < 2 * n; ++i) hist_lead_sv[i] = nan("");
     return MPCB_OK;
   }
   CK(cudaSetDevice(s->h->device));
   cudaStream_t st = (cudaStream_t)cuda_stream;
-  if (hist_lead_idx) CK(cudaMemcpyAsync(hist_lead_idx, s->hist_lead_idx, n * 4, cudaMemcpyDeviceToHost, st));
-  if (hist_lead_sv) CK(cudaMemcpyAsync(hist_lead_sv, s->hist_lead_sv, n * 16, cudaMemcpyDeviceToHost, st));
+  const auto D2H = cudaMemcpyDeviceToHost;
+  if (hist_lead_idx) CK(cudaMemcpyAsync(hist_lead_idx, s->d.hist_lead_idx, sim_bytes(R_HIST_LEAD_IDX, s->B, nt), D2H, st));
+  if (hist_lead_sv) CK(cudaMemcpyAsync(hist_lead_sv, s->d.hist_lead_sv, sim_bytes(R_HIST_LEAD_SV, s->B, nt), D2H, st));
   CK(cudaStreamSynchronize(st));
   return MPCB_OK;
 }
@@ -515,18 +633,17 @@ int mpcb_sim_follow_history(mpcb_sim_handle s, int* n_recorded, int* hist_lead_i
 int mpcb_sim_follow_check(mpcb_sim_handle s, int* ok, double* min_gap, void* cuda_stream) {
   if (!s || !ok || s->cap < 1) return MPCB_ERR_INVALID;
   const size_t nb = (size_t)s->B;
-  if (!s->hist_lead_sv) {                                    // following never switched on: no leader, ever
+  if (!s->d.hist_lead_sv) {                                  // following never switched on: no leader, ever
     for (size_t b = 0; b < nb; ++b) { ok[b] = 1; if (min_gap) min_gap[b] = BIG; }
     return MPCB_OK;
   }
   CK(cudaSetDevice(s->h->device));
   cudaStream_t st = (cudaStream_t)cuda_stream;
   const int nt = s->t < s->cap ? s->t : s->cap;
-  mpcb_follow_check_kernel<<<(s->B + 127) / 128, 128, 0, st>>>(s->B, nt, s->steps, s->hist_x, s->hist_lead_sv,
-                                                               s->d_follow_ok, s->d_min_gap);
+  mpcb_follow_check_kernel<<<(s->B + 127) / 128, 128, 0, st>>>(s->d, s->B, nt);
   CK(cudaGetLastError());
-  CK(cudaMemcpyAsync(ok, s->d_follow_ok, nb * 4, cudaMemcpyDeviceToHost, st));
-  if (min_gap) CK(cudaMemcpyAsync(min_gap, s->d_min_gap, nb * 8, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(ok, s->d.follow_ok, sim_bytes(R_FOLLOW_OK, nb, 0), cudaMemcpyDeviceToHost, st));
+  if (min_gap) CK(cudaMemcpyAsync(min_gap, s->d.min_gap, sim_bytes(R_MIN_GAP, nb, 0), cudaMemcpyDeviceToHost, st));
   CK(cudaStreamSynchronize(st));
   s->h->launches += 1;
   return MPCB_OK;
@@ -536,10 +653,10 @@ int mpcb_sim_alive(mpcb_sim_handle s, int* n_alive, void* cuda_stream) {
   if (!s || !n_alive) return MPCB_ERR_INVALID;
   CK(cudaSetDevice(s->h->device));
   cudaStream_t st = (cudaStream_t)cuda_stream;
-  CK(cudaMemsetAsync(s->count, 0, 4, st));
-  mpcb_count_alive_kernel<<<(s->B + 127) / 128, 128, 0, st>>>(s->h->dt, s->route, s->B, s->x, s->count);
+  CK(cudaMemsetAsync(s->d.count, 0, sim_bytes(R_COUNT, 0, 0), st));
+  mpcb_count_alive_kernel<<<(s->B + 127) / 128, 128, 0, st>>>(s->h->dt, s->d, s->B);
   CK(cudaGetLastError());
-  CK(cudaMemcpyAsync(n_alive, s->count, 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(n_alive, s->d.count, sim_bytes(R_COUNT, 0, 0), cudaMemcpyDeviceToHost, st));
   CK(cudaStreamSynchronize(st));
   return MPCB_OK;
 }
@@ -549,9 +666,10 @@ int mpcb_sim_state(mpcb_sim_handle s, double* x, int* steps, int* n_unsolved, vo
   CK(cudaSetDevice(s->h->device));
   cudaStream_t st = (cudaStream_t)cuda_stream;
   const size_t nb = (size_t)s->B;
-  if (x) CK(cudaMemcpyAsync(x, s->x, nb * 40, cudaMemcpyDeviceToHost, st));
-  if (steps) CK(cudaMemcpyAsync(steps, s->steps, nb * 4, cudaMemcpyDeviceToHost, st));
-  if (n_unsolved) CK(cudaMemcpyAsync(n_unsolved, s->n_unsolved, nb * 4, cudaMemcpyDeviceToHost, st));
+  const auto D2H = cudaMemcpyDeviceToHost;
+  if (x) CK(cudaMemcpyAsync(x, s->d.x, sim_bytes(R_X, nb, 0), D2H, st));
+  if (steps) CK(cudaMemcpyAsync(steps, s->d.steps, sim_bytes(R_STEPS, nb, 0), D2H, st));
+  if (n_unsolved) CK(cudaMemcpyAsync(n_unsolved, s->d.n_unsolved, sim_bytes(R_N_UNSOLVED, nb, 0), D2H, st));
   CK(cudaStreamSynchronize(st));
   return MPCB_OK;
 }
@@ -560,15 +678,8 @@ int mpcb_sim_check(mpcb_sim_handle s, int* verdict, double* metrics, void* cuda_
   if (!s || !verdict || s->cap < 1) return MPCB_ERR_INVALID;
   CK(cudaSetDevice(s->h->device));
   cudaStream_t st = (cudaStream_t)cuda_stream;
-  const size_t nb = (size_t)s->B;
-  const mpcb_params& p = s->h->params;
   const int nt = s->t < s->cap ? s->t : s->cap;
-  mpcb_sim_check_kernel<<<(s->B + 127) / 128, 128, 0, st>>>(s->h->dt, s->route, s->B, nt, s->h->dt.t[0].s_max, p.u_min[0], p.u_max[0], p.u_min[1],
-                                                           p.u_max[1], s->x, s->steps, s->scen, s->hist_x, s->hist_u,
-                                                           s->hist_obs, s->hist_tl, s->d_verdict, s->d_metrics);
-  CK(cudaGetLastError());
-  CK(cudaMemcpyAsync(verdict, s->d_verdict, nb * 4, cudaMemcpyDeviceToHost, st));
-  if (metrics) CK(cudaMemcpyAsync(metrics, s->d_metrics, nb * 32, cudaMemcpyDeviceToHost, st));
+  CK(launch_check(s->h, s->d, s->B, nt, s->h->dt.t[0].s_max, verdict, metrics, st));
   CK(cudaStreamSynchronize(st));
   s->h->launches += 1;
   return MPCB_OK;
@@ -583,38 +694,26 @@ int mpcb_check_histories(mpcb_handle h, int B, int T, double s_total, const mpcb
   if (!h || B < 1 || T < 1 || !scen || !x_final || !steps || !hist_x || !hist_u || !hist_obs || !hist_tl || !verdict)
     return MPCB_ERR_INVALID;
   CK(cudaSetDevice(h->device));
-  const size_t nb = (size_t)B, nt = (size_t)T * nb;
+  const size_t nb = (size_t)B;
   std::vector<DevScenario> hs(nb);
-  for (size_t b = 0; b < nb; ++b) {
-    const mpcb_scenario& c = scen[b];
-    hs[b] = DevScenario{c.obs_trigger_s, c.obs_start_s, c.obs_v, c.obs_end_s, c.tl_pos, c.tl_trigger_s,
-                        c.tl_stop_duration, c.dynamic_obstacle, c.traffic_light};
-  }
-  // one allocation: the seven inputs, then the verdicts and the metrics
-  const size_t sz[9] = {nb * sizeof(DevScenario), nb * 40, nb * 4, nt * 40, nt * 16, nt * 8, nt * 4, nb * 4, nb * 32};
-  const void* src[7] = {hs.data(), x_final, steps, hist_x, hist_u, hist_obs, hist_tl};
-  size_t off[10];
-  region_offsets(sz, 9, off);
-  char* d = nullptr;
-  if (cudaMalloc((void**)&d, off[9]) != cudaSuccess) { cudaGetLastError(); return MPCB_ERR_NOMEM; }
+  for (size_t b = 0; b < nb; ++b) hs[b] = to_dev_scenario(scen[b]);
+  // one block laid out as a simulation's: the caller's arrays (x_final in x), the verdicts and the metrics
+  const struct { int r; const void* src; } in[] = {{R_SCEN, hs.data()}, {R_X, x_final}, {R_STEPS, steps},
+                                                   {R_HIST_X, hist_x}, {R_HIST_U, hist_u}, {R_HIST_OBS, hist_obs},
+                                                   {R_HIST_TL, hist_tl}};
+  unsigned mask = 1u << R_VERDICT | 1u << R_METRICS;
+  for (const auto& c : in) mask |= 1u << c.r;
+  SimArrays d = {};
+  size_t off[N_SIM + 1];
+  char* base = sim_alloc(d, nb, (size_t)T, mask, 0, off);
+  if (!base) return MPCB_ERR_NOMEM;
   cudaStream_t st = h->stream;
   cudaError_t e = cudaSuccess;
-  for (int k = 0; k < 7 && e == cudaSuccess; ++k) e = cudaMemcpyAsync(d + off[k], src[k], sz[k], cudaMemcpyHostToDevice, st);
-  if (e == cudaSuccess) {
-    const mpcb_params& p = h->params;
-    int* d_v = (int*)(d + off[7]);
-    double* d_m = (double*)(d + off[8]);
-    mpcb_sim_check_kernel<<<(B + 127) / 128, 128, 0, st>>>(h->dt, nullptr, B, T, s_total, p.u_min[0], p.u_max[0], p.u_min[1], p.u_max[1],
-                                                          (const double*)(d + off[1]), (const int*)(d + off[2]),
-                                                          (const DevScenario*)(d + off[0]), (const double*)(d + off[3]),
-                                                          (const double*)(d + off[4]), (const double*)(d + off[5]),
-                                                          (const int*)(d + off[6]), d_v, d_m);
-    e = cudaGetLastError();
-    if (e == cudaSuccess) e = cudaMemcpyAsync(verdict, d_v, nb * 4, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess && metrics) e = cudaMemcpyAsync(metrics, d_m, nb * 32, cudaMemcpyDeviceToHost, st);
-  }
+  for (const auto& c : in)
+    if (e == cudaSuccess) e = cudaMemcpyAsync(base + off[c.r], c.src, sim_bytes(c.r, nb, T), cudaMemcpyHostToDevice, st);
+  if (e == cudaSuccess) e = launch_check(h, d, B, T, s_total, verdict, metrics, st);
   if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-  cudaFree(d);
+  cudaFree(base);
   if (e != cudaSuccess) return cuda_fail(e, "mpcb_check_histories");
   h->launches += 1;
   return MPCB_OK;
@@ -627,13 +726,12 @@ int mpcb_sim_history(mpcb_sim_handle s, int* n_recorded, double* hist_x, double*
   cudaStream_t st = (cudaStream_t)cuda_stream;
   const int nt = s->t < s->cap ? s->t : s->cap;
   if (n_recorded) *n_recorded = nt;
-  const size_t n = (size_t)nt * s->B;
-  if (n > 0) {
-    if (hist_x) CK(cudaMemcpyAsync(hist_x, s->hist_x, n * 40, cudaMemcpyDeviceToHost, st));
-    if (hist_u) CK(cudaMemcpyAsync(hist_u, s->hist_u, n * 16, cudaMemcpyDeviceToHost, st));
-    if (hist_obs) CK(cudaMemcpyAsync(hist_obs, s->hist_obs, n * 8, cudaMemcpyDeviceToHost, st));
-    if (hist_status) CK(cudaMemcpyAsync(hist_status, s->hist_status, n * 4, cudaMemcpyDeviceToHost, st));
-    if (hist_tl) CK(cudaMemcpyAsync(hist_tl, s->hist_tl, n * 4, cudaMemcpyDeviceToHost, st));
+  if (nt > 0) {
+    const struct { int r; void* dst; const void* src; } out[] = {
+        {R_HIST_X, hist_x, s->d.hist_x}, {R_HIST_U, hist_u, s->d.hist_u}, {R_HIST_OBS, hist_obs, s->d.hist_obs},
+        {R_HIST_STATUS, hist_status, s->d.hist_status}, {R_HIST_TL, hist_tl, s->d.hist_tl}};
+    for (const auto& c : out)
+      if (c.dst) CK(cudaMemcpyAsync(c.dst, c.src, sim_bytes(c.r, s->B, nt), cudaMemcpyDeviceToHost, st));
   }
   CK(cudaStreamSynchronize(st));
   return MPCB_OK;

@@ -16,58 +16,20 @@ car position, the light colour) lets every step of every vehicle be replayed on 
 Four staggered fleets on trajectory2, each vehicle with its own start and scenario constants, car and light switched on
 and off independently: 3,500 vehicles (more than coop_max_batch = 3,072: thread-per-problem first pass, class kernels
 fed from the list of vehicles still driving) and 600 vehicles (warp-per-problem first pass), each cold and hot-started.
-The replay helpers are checked without a GPU against the reference's own closed-loop logs (tests/golden/closed_loop_*),
+The replay helpers (closed_loop_oracle) are checked without a GPU against the reference's own closed-loop logs (tests/golden/closed_loop_*),
 so that a failure on the GPU cannot come from the replay itself."""
 import numpy as np
 import pytest
 
+from closed_loop_oracle import fsm_replay, k_ref, plant_step
 from conftest import golden
-from oracle import sqp_admm_model as A
 from oracle import tracker_port as P
-
-DT = P.DT
 
 # name: (vehicles, hot start, seed of the fleet)
 FLEETS = {"bulk_cold": (3500, False, 31), "bulk_hot": (3500, True, 31),
           "small_cold": (600, False, 32), "small_hot": (600, True, 32)}
 MAX_STEPS = 1200      # the longest drive of these fleets is well below; 1,200 x 3,500 recorded steps are ~300 MB
 CHUNK = 100           # steps enqueued between looks at the fleet
-
-
-# --------------------------------------------------------------------------------------------------------------------
-# replay helpers (numpy / oracle only)
-# --------------------------------------------------------------------------------------------------------------------
-def fsm_replay(fsm, s, v):
-    """Drive an oracle FSM over recorded states (s[t], v[t]): the obstacle set the solver of step t sees (obs_sv [k,2,2],
-    unused slots 0, car first; n_obs [k]), the position of the moving car (NaN when there is none) and the light colour
-    (1 green, 0 red), as ObstacleFSMPort.update returns them."""
-    k = len(s)
-    obs_sv = np.zeros((k, 2, 2))
-    n_obs = np.zeros(k, np.int32)
-    car = np.full(k, np.nan)
-    green = np.zeros(k, np.int32)
-    for t, (st, vt) in enumerate(zip(np.asarray(s).tolist(), np.asarray(v).tolist())):
-        act, colour = fsm.update(DT, st, vt)
-        for j, o in enumerate(act):
-            obs_sv[t, j] = (o["s"], o["v"])
-            if o["type"] == "car":
-                car[t] = o["s"]
-        n_obs[t] = len(act)
-        green[t] = colour == "GREEN"
-    return obs_sv, n_obs, car, green
-
-
-def k_ref(tab, s):
-    """get_state(s)[3] (trajectory_loader.py:86-93), vectorised; s >= s_max gives the last knot's curvature."""
-    return A.lookup(tab, s)[0][..., 2]
-
-
-def plant_step(tab, x, u):
-    """x + DT * dynamics(x, u, k_ref(s)) (trajectory_tracking.py:50-67, :404-406) over leading axes, in the reference's
-    operation order."""
-    s, o, k, v = x[..., 0], x[..., 2], x[..., 3], x[..., 4]
-    f = np.stack([v, v * o, v * (k - k_ref(tab, s)), u[..., 0], u[..., 1]], axis=-1)
-    return x + DT * f
 
 
 # --------------------------------------------------------------------------------------------------------------------

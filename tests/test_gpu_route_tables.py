@@ -27,12 +27,12 @@ import functools
 import numpy as np
 import pytest
 
+from closed_loop_oracle import DT, leaders, plant_step
 from conftest import VARIANTS, golden, traj_path
 from oracle import planner_port as Q
 from oracle import sqp_admm_model as A
 from oracle import tracker_port as P
 
-DT = P.DT
 FN_TOL = 1e-12
 LUT_N = 4096                       # buckets of the device's cold-lookup index (upload_table, mpcb_api.cu)
 WAVE = 148 * 2 * 128               # problems of one wave of the first pass on a B200 (148 SMs x 2 CTAs x 128)
@@ -643,17 +643,6 @@ def test_planner_whole_route_equals_the_base_route(name, trackers):
 # --------------------------------------------------------------------------------------------------------------------
 # 6. closed loop on routes that are not committed
 # --------------------------------------------------------------------------------------------------------------------
-def k_ref(tab, s):
-    return A.lookup(tab, s)[0][..., 2]
-
-
-def plant_step(tab, x, u):
-    """x + DT * dynamics(x, u, k_ref(s)) (trajectory_tracking.py:50-67, :404-406), in the reference's operation order."""
-    s, o, k, v = x[..., 0], x[..., 2], x[..., 3], x[..., 4]
-    f = np.stack([v, v * o, v * (k - k_ref(tab, s)), u[..., 0], u[..., 1]], axis=-1)
-    return x + DT * f
-
-
 CL_FLEETS = {"dense_traj2": (3500, 51), "repaired_equal": (600, 52)}
 CL_MAX_STEPS = 1200
 
@@ -766,7 +755,6 @@ def test_sixteen_route_fleet_follows_the_numpy_leader_rule(routed16):
     """A following fleet over all sixteen routes, with vehicles on route 15 (the last slot) and vehicles that arrive:
     the recorded leaders equal the numpy rule at every step."""
     import safe_autonomous_driving_mpc_b200 as M
-    from test_gpu_sim_follow import leaders
     TR = M.BatchedTracker(routed16)
     B, n_steps, rng_range = 640, 150, 10.0
     route = (np.arange(B) % 16).astype(np.int32)

@@ -217,3 +217,50 @@ def test_hot_start_drives_the_same_closed_loop(i, gpu_trackers):
     # for 70 steps in a row, and what an infeasible problem returns depends on the path the solver took (SURVEY 4.4-4:
     # flags only there); the two loops rejoin behind the light
     assert dx[:, 1].max() <= 5e-4 and dx[:, 2].max() <= 5e-4 and dx[:, 4].max() <= 0.05 and dx[:, 0].max() <= 0.1, dx.max(axis=0)
+
+
+def test_failed_create_and_destroy_leave_no_device_memory_behind(gpu_trackers):
+    """A simulation whose histories cannot be allocated (100,000 vehicles x 10^7 recorded steps, some 70 TB) is refused
+    with MPCB_ERR_NOMEM (-3) and holds no device memory; a created, following, stepped and destroyed simulation gives all
+    of its device memory back; a simulation created afterwards steps as usual.  The driver keeps freed pages of small
+    allocations for reuse and returns them when an allocation fails, so every reading of free memory is taken right
+    after a refused create, with the garbage collector off."""
+    import ctypes as C
+    import gc
+    import torch
+    import safe_autonomous_driving_mpc_b200 as M
+    L, T = gpu_trackers[2]
+    sc = M.make_scenario(2)
+    x_init = np.array([L.get_state(s) for s in (100.0, 104.0, 300.0, 303.0)])
+    x_init[:, 4] = np.maximum(x_init[:, 4], 0.5)
+
+    def following_run():
+        sim = M.BatchedSimulation(T, sc, x_init=x_init, history_steps=16, follow_range=10.0)
+        sim.step(8)
+        lead = sim.follow_history()["lead"]
+        del sim
+        return lead
+
+    def free_after_refused_create():
+        h = C.c_void_p()
+        rc = T._lib.mpcb_sim_create_routes(C.byref(h), T._need(), 100_000, (M._lib.Scenario * 1)(sc), 1, None, None,
+                                           10_000_000)
+        assert rc == -3 and not h.value
+        torch.cuda.synchronize()
+        return torch.cuda.mem_get_info()[0]
+
+    # once before measuring: the handle's solve workspace and the modules of the kernels are loaded on first use
+    assert (following_run() >= 0).any()
+    gc.collect()
+    gc.disable()
+    try:
+        free0 = free_after_refused_create()
+        assert free_after_refused_create() == free0
+        assert (following_run() >= 0).any()
+        assert free_after_refused_create() == free0
+    finally:
+        gc.enable()
+    sim = M.BatchedSimulation(T, sc, x_init=x_init, history_steps=8)
+    sim.step(8)
+    x, steps, _ = sim.state()
+    assert np.all(steps == 8) and np.all(np.isfinite(x)) and np.all(x[:, 0] > x_init[:, 0])

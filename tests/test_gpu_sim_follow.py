@@ -12,79 +12,20 @@ obstacle.
   4. following off (never switched on, or switched on and off before the first step) is today's loop bit for bit, with
      the same launch count; switched on halfway, the loop is the off loop up to that step;
   5. argument checks.
-The helpers are checked without a GPU on hand-made cases."""
+The leader and merge rules (closed_loop_oracle) are checked without a GPU on hand-made cases."""
 import ctypes as C
 
 import numpy as np
 import pytest
 
+from closed_loop_oracle import fsm_replay, leaders, merge, plant_step
 from conftest import traj_path
-from oracle import sqp_admm_model as A
 from oracle import tracker_port as P
 
-DT = P.DT
-
 
 # --------------------------------------------------------------------------------------------------------------------
-# helpers (numpy / oracle only)
+# the helpers on hand-made cases (no GPU)
 # --------------------------------------------------------------------------------------------------------------------
-def leaders(x, live, route, follow_range):
-    """The leader rule for one step: x [B,5] states at the start of the step, live [B] still driving, route [B].
-    Returns lead [B] (-1: none) and lead_sv [B,2] (NaN: none)."""
-    B = len(x)
-    s = x[:, 0]
-    lead = np.full(B, -1, np.int64)
-    for r in np.unique(route[live]):
-        idx = np.flatnonzero(live & (route == r))
-        order = idx[np.lexsort((idx, s[idx]))]           # by s, then by index
-        a, b = order[:-1], order[1:]
-        near = s[b] - s[a] <= follow_range
-        lead[a[near]] = b[near]
-    sv = np.full((B, 2), np.nan)
-    has = lead >= 0
-    sv[has] = x[lead[has]][:, [0, 4]]
-    return lead, sv
-
-
-def merge(obs_sv, n_obs, car, lead_sv):
-    """The FSM's obstacle set (car first when present, then the light; unused slots 0) with the leader merged into the
-    car slot: the nearer of scripted car and leader, the scripted car on a tie.  Leading axes are arbitrary."""
-    obs_sv, n_obs = obs_sv.copy(), n_obs.copy()
-    ls = lead_sv[..., 0]
-    has_car = ~np.isnan(car)
-    take = ~np.isnan(ls) & ~(has_car & (car <= ls))
-    shift = take & ~has_car                              # no car: the light (if any) moves behind the leader
-    obs_sv[..., 1, :] = np.where(shift[..., None], obs_sv[..., 0, :], obs_sv[..., 1, :])
-    obs_sv[..., 0, :] = np.where(take[..., None], lead_sv, obs_sv[..., 0, :])
-    n_obs = n_obs + shift
-    return obs_sv, n_obs.astype(np.int32)
-
-
-def fsm_replay(fsm, s, v):
-    """Oracle FSM over recorded (s[t], v[t]): obstacle sets [k,2,2] (car first, unused slots 0), n_obs [k], car position
-    [k] (NaN: none)."""
-    k = len(s)
-    obs_sv = np.zeros((k, 2, 2))
-    n_obs = np.zeros(k, np.int32)
-    car = np.full(k, np.nan)
-    for t, (st, vt) in enumerate(zip(np.asarray(s).tolist(), np.asarray(v).tolist())):
-        act, _colour = fsm.update(DT, st, vt)
-        for j, o in enumerate(act):
-            obs_sv[t, j] = (o["s"], o["v"])
-            if o["type"] == "car":
-                car[t] = o["s"]
-        n_obs[t] = len(act)
-    return obs_sv, n_obs, car
-
-
-def plant_step(tab, x, u):
-    """x + DT * dynamics(x, u, k_ref(s)) (trajectory_tracking.py:50-67, :404-406) in the reference's operation order."""
-    s, o, k, v = x[..., 0], x[..., 2], x[..., 3], x[..., 4]
-    kr = A.lookup(tab, s)[0][..., 2]
-    f = np.stack([v, v * o, v * (k - kr), u[..., 0], u[..., 1]], axis=-1)
-    return x + DT * f
-
-
 def test_leader_rule_on_hand_made_cases():
     """Order by (s, index), ties to the higher index, the range filter, routes apart, arrived vehicles nobody's
     leader and without one."""
@@ -233,7 +174,7 @@ def test_in_loop_solves_see_the_merged_obstacles(fleet):
     for b in range(B):
         k = int(min(F["steps"][b], N_STEPS))
         fsm = P.ObstacleFSMPort(bool(F["dyn"][b]), bool(F["tl"][b]), **F["consts"][b])
-        obs_sv[:k, b], n_obs[:k, b], car[:k, b] = fsm_replay(fsm, h["x"][:k, b, 0], h["x"][:k, b, 4])
+        obs_sv[:k, b], n_obs[:k, b], car[:k, b], _green = fsm_replay(fsm, h["x"][:k, b, 0], h["x"][:k, b, 4])
     assert np.array_equal(h["obs_s"], car, equal_nan=True)
     lead_sv = np.stack([ld["lead_s"], ld["lead_v"]], axis=-1)
     obs_m, n_m = merge(obs_sv, n_obs, car, lead_sv)
@@ -311,7 +252,7 @@ def test_platoon_host_loop_equals_device_loop(gpu_trackers, port_tables):
         n = np.zeros(B, np.int32)
         car = np.full(B, np.nan)
         for b in np.flatnonzero(live):
-            o, m, c = fsm_replay(fsms[b], x[b:b + 1, 0], x[b:b + 1, 4])
+            o, m, c, _green = fsm_replay(fsms[b], x[b:b + 1, 0], x[b:b + 1, 4])
             obs[b], n[b], car[b] = o[0], m[0], c[0]
         obs, n = merge(obs, n, car, lsv)
         r = T.solve_batch_host(x, obs, n)
