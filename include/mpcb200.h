@@ -306,6 +306,33 @@ int mpcb_sim_follow_history(mpcb_sim_handle s, int* n_recorded, int* hist_lead_i
  * NULL) = min of s_leader - s (1e30 for a vehicle that never had a leader), ok [B] HOST = min_gap >= 1 m (the reference's
  * safety distance of its moving-obstacle check, sanity_checks.py:142-164). */
 int mpcb_sim_follow_check(mpcb_sim_handle s, int* ok, double* min_gap, void* cuda_stream);
+/* Seeded Gaussian disturbances (off by default), in three independent channels.  For vehicle b at step t (steps since
+ * mpcb_sim_create, the counter the histories use), id = first_id + b, z standard normals:
+ *   - measurement: the solve sees x_meas = x + sigma_meas * z_m (per component).  The FSM, the loop condition, following
+ *     and the plant use the true x; obstacles are not perturbed;
+ *   - actuation: the plant applies u = U*[0] + sigma_act * z_a, not clipped; the history keeps the commanded U*[0], so
+ *     mpcb_sim_check's steering and acceleration items judge the controller;
+ *   - process: x' = Euler step(x, u) + sigma_proc * z_p, added every step.  Vehicles that have arrived stay frozen.
+ * A component whose sigma is 0 is left untouched (nothing is added).  With every sigma 0 noise is off and every entry
+ * point behaves as without this call, bit for bit, with the same launches; with the measurement sigmas all 0 the solve
+ * reads the true state.  Additions and products are rounded separately (no fused multiply-add), so that a replay of the
+ * recorded values gives the same bits.
+ * Generator: z depends only on (seed, id, t, channel, component), not on B, on how the steps are split between calls, on
+ * the execution shape or on which other channels are on.  Philox4x32-10 with key (seed & 0xffffffff, seed >> 32) and
+ * counter (t, id, j, 0), j = 0..2 measurement, 3 actuation, 4..6 process; component i of a channel is output i mod 2 of
+ * call j_first + i / 2.  A call's words x, y, z, w give W1 = x << 32 | y and W2 = z << 32 | w, u = ((W >> 11) + 0.5) 2^-53
+ * each, and Box-Muller: rho = sqrt(-2 ln u1), output 0 = rho cos(2 pi u2), output 1 = rho sin(2 pi u2).  first_id lets a
+ * shard of a fleet (vehicles lo .. hi-1, first_id = lo) draw exactly the whole fleet's noise.
+ * sigma_meas [5], sigma_act [2], sigma_proc [5]: HOST, NULL = zeros; each finite and >= 0.  first_id >= 0 and
+ * first_id + B <= 2^31.  Anything else is MPCB_ERR_INVALID before any CUDA call.  Takes effect from the next step.  The
+ * first call that switches noise on allocates the measured states and the noise history (synchronises the device's
+ * default stream); MPCB_ERR_NOMEM if that fails, noise then stays off. */
+int mpcb_sim_set_noise(mpcb_sim_handle s, unsigned long long seed, int first_id, const double* sigma_meas,
+                       const double* sigma_act, const double* sigma_proc);
+/* The disturbances added in the first history_steps steps, HOST hist_w [n_recorded][B][12] (may be NULL): measurement
+ * 5, actuation 2, process 5, each the value added (sigma z; 0.0 for a component whose sigma is 0).  NaN for steps where
+ * the vehicle had arrived or noise was off. */
+int mpcb_sim_noise_history(mpcb_sim_handle s, int* n_recorded, double* hist_w, void* cuda_stream);
 /* number of vehicles still driving (synchronises the stream) */
 int mpcb_sim_alive(mpcb_sim_handle s, int* n_alive, void* cuda_stream);
 /* HOST outputs (any may be NULL): current states [B][5], steps driven [B], steps whose solve was not MPCB_SOLVED [B] */

@@ -8,7 +8,8 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.environ.get("MPCB_LIB") or os.path.join(HERE, "libmpcb200.so")   # MPCB_LIB: development variants
 SOURCES = ["mpcb_api.cu", "mpcb_planner.cu", "mpcb_sim.cu"]
-HEADERS = ["mpcb_device.cuh", "mpcb_solver.cuh", "mpcb_planner.cuh", "mpcb_internal.h", "mpcb_coop.cuh", "mpcb_params.h"]
+HEADERS = ["mpcb_device.cuh", "mpcb_solver.cuh", "mpcb_planner.cuh", "mpcb_internal.h", "mpcb_coop.cuh", "mpcb_params.h",
+           "mpcb_philox.cuh"]
 
 
 def nvcc_path():

@@ -109,6 +109,8 @@ SYMBOLS = {
     "mpcb_sim_set_follow": (C.c_int, [C.c_void_p, C.c_int, C.c_double]),
     "mpcb_sim_follow_history": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.c_void_p, C.c_void_p, C.c_void_p]),
     "mpcb_sim_follow_check": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mpcb_sim_set_noise": (C.c_int, [C.c_void_p, C.c_ulonglong, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mpcb_sim_noise_history": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.c_void_p, C.c_void_p]),
     "mpcb_sim_alive":(C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.c_void_p]),
     "mpcb_sim_state": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mpcb_sim_check": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

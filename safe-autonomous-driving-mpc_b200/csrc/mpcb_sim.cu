@@ -7,7 +7,9 @@
 // One simulation object holds B vehicles (each with its own scenario constants and FSM state).  A step is three
 // launches on one stream -- FSM kernel -> mpcb_solve_batch -> plant kernel -- with no host round trip, so a
 // Monte-Carlo of whole drives never leaves the GPU; histories are recorded into device buffers when asked for.  With
-// following on (mpcb_sim_set_follow), a key kernel, two radix sorts and a leader kernel come first.
+// following on (mpcb_sim_set_follow), a key kernel, two radix sorts and a leader kernel come first.  With noise on
+// (mpcb_sim_set_noise), the FSM kernel also writes the measured state the solve reads and the plant kernel disturbs the
+// control it applies and the state it produces; the step keeps its launches.
 #include <cuda_runtime.h>
 #include <math.h>
 #include <string.h>
@@ -20,6 +22,7 @@
 
 #include "mpcb200.h"
 #include "mpcb_internal.h"
+#include "mpcb_philox.cuh"
 
 namespace mpcb {
 
@@ -29,23 +32,27 @@ struct DevScenario {          // per vehicle, mirrors ObstaclesFSM.__init__ (:28
   int dynamic_obstacle, traffic_light;
 };
 
-// The device arrays of a simulation, in four groups: the loop state and the histories are one block made at create,
-// following and its histories one block made by the first mpcb_sim_set_follow(on).  The layout of a block, every copy
-// and every fill is derived from SIM_BYTES.
+// The device arrays of a simulation, in five groups: the loop state and the histories are one block made at create,
+// following and its histories one block made by the first mpcb_sim_set_follow(on), the measured states and the noise
+// history one block made by the first mpcb_sim_set_noise that switches noise on.  The layout of a block, every copy and
+// every fill is derived from SIM_BYTES.
 enum SimRegion {
   R_SCEN, R_X, R_FSM_F, R_OBS_SV, R_U, R_FSM_I, R_ALIVE, R_N_OBS, R_STATUS, R_STEPS, R_N_UNSOLVED, R_ALIVE_IDX,
   R_ALIVE_CNT, R_COUNT, R_ROUTE,                                                         // loop state
   R_HIST_X, R_HIST_U, R_HIST_OBS, R_HIST_STATUS, R_HIST_TL, R_VERDICT, R_METRICS,         // histories
   R_F_KEY, R_F_TAG, R_F_TEMP, R_LEAD_IDX, R_LEAD_SV,                                      // following
   R_HIST_LEAD_IDX, R_HIST_LEAD_SV, R_FOLLOW_OK, R_MIN_GAP,                                // following histories
+  R_X_MEAS, R_HIST_NOISE,                                                                 // noise
   N_SIM
 };
-constexpr unsigned sim_span(int lo, int hi) { return ((1u << hi) - 1u) & ~((1u << lo) - 1u); }   // regions lo .. hi-1
-constexpr unsigned SIM_LOOP = sim_span(R_SCEN, R_ROUTE);          // R_ROUTE only on a routed simulation
-constexpr unsigned SIM_HIST = sim_span(R_HIST_X, R_F_KEY);
-constexpr unsigned SIM_FOLLOW = sim_span(R_F_KEY, R_HIST_LEAD_IDX);
-constexpr unsigned SIM_FOLLOW_HIST = sim_span(R_HIST_LEAD_IDX, N_SIM);
-static_assert(N_SIM < 32, "regions are selected by the bits of an unsigned");
+typedef unsigned long long SimMask;                                 // bit r selects region r
+constexpr SimMask sim_bit(int r) { return 1ull << r; }
+constexpr SimMask sim_span(int lo, int hi) { return (sim_bit(hi) - 1ull) & ~(sim_bit(lo) - 1ull); }   // regions lo .. hi-1
+constexpr SimMask SIM_LOOP = sim_span(R_SCEN, R_ROUTE);          // R_ROUTE only on a routed simulation
+constexpr SimMask SIM_HIST = sim_span(R_HIST_X, R_F_KEY);
+constexpr SimMask SIM_FOLLOW = sim_span(R_F_KEY, R_HIST_LEAD_IDX);
+constexpr SimMask SIM_FOLLOW_HIST = sim_span(R_HIST_LEAD_IDX, R_X_MEAS);
+static_assert(N_SIM < 64, "regions are selected by the bits of a SimMask");
 
 enum SimPer { PER_VEHICLE, PER_STEP, FIXED };   // bytes per vehicle, per vehicle and recorded step, or in all
 struct SimBytes { SimPer per; size_t bytes; };
@@ -81,6 +88,8 @@ static const SimBytes SIM_BYTES[N_SIM] = {
   /* hist_lead_sv  */ {PER_STEP, 2 * 8},         // NaN where not recorded
   /* follow_ok     */ {PER_VEHICLE, 4},          // mpcb_sim_follow_check
   /* min_gap       */ {PER_VEHICLE, 8},
+  /* x_meas        */ {PER_VEHICLE, 5 * 8},      // the state the solve sees
+  /* hist_noise    */ {PER_STEP, 12 * 8},        // [cap][B][12]: measurement 5, actuation 2, process 5; NaN where not recorded
 };
 
 // Bytes of region r for B vehicles and T recorded steps (R_F_TEMP: see sim_layout).
@@ -92,9 +101,9 @@ static size_t sim_bytes(int r, size_t B, size_t T) {
 // Layout of the regions in mask of a simulation of B vehicles and T recorded steps, with a radix-sort workspace of temp
 // bytes: region r at off[r] (no bytes when it is not in mask), off[N_SIM] bytes in all.  Each region starts on 256
 // bytes, which also keeps U 16-byte aligned for the solve's 128-bit stores into it.
-static void sim_layout(size_t B, size_t T, unsigned mask, size_t temp, size_t (&off)[N_SIM + 1]) {
+static void sim_layout(size_t B, size_t T, SimMask mask, size_t temp, size_t (&off)[N_SIM + 1]) {
   size_t bytes[N_SIM];
-  for (int r = 0; r < N_SIM; ++r) bytes[r] = !((mask >> r) & 1u) ? 0 : r == R_F_TEMP ? temp : sim_bytes(r, B, T);
+  for (int r = 0; r < N_SIM; ++r) bytes[r] = !((mask >> r) & 1ull) ? 0 : r == R_F_TEMP ? temp : sim_bytes(r, B, T);
   region_offsets(bytes, N_SIM, off);
 }
 
@@ -108,16 +117,17 @@ struct SimArrays {
   double* hist_x; double* hist_u; double* hist_obs; int* hist_status; int* hist_tl; int* verdict; double* metrics;
   unsigned long long* f_key; unsigned* f_tag; void* f_temp; int* lead_idx; double* lead_sv;
   int* hist_lead_idx; double* hist_lead_sv; int* follow_ok; double* min_gap;
+  double* x_meas; double* hist_noise;
 };
 
 // One block holding the regions in mask, laid out by sim_layout; points their arrays in d into it and leaves the others.
 // nullptr (and no error left pending) when it cannot be allocated.
-static char* sim_alloc(SimArrays& d, size_t B, size_t T, unsigned mask, size_t temp, size_t (&off)[N_SIM + 1]) {
+static char* sim_alloc(SimArrays& d, size_t B, size_t T, SimMask mask, size_t temp, size_t (&off)[N_SIM + 1]) {
   sim_layout(B, T, mask, temp, off);
   char* base = nullptr;
   if (cudaMalloc((void**)&base, off[N_SIM]) != cudaSuccess) { cudaGetLastError(); return nullptr; }
   auto at = [&](auto*& p, int r) {
-    if ((mask >> r) & 1u) p = (std::remove_reference_t<decltype(p)>)(base + off[r]);
+    if ((mask >> r) & 1ull) p = (std::remove_reference_t<decltype(p)>)(base + off[r]);
   };
   at(d.scen, R_SCEN); at(d.x, R_X); at(d.fsm_f, R_FSM_F); at(d.obs_sv, R_OBS_SV); at(d.U, R_U);
   at(d.fsm_i, R_FSM_I); at(d.alive, R_ALIVE); at(d.n_obs, R_N_OBS); at(d.status, R_STATUS); at(d.steps, R_STEPS);
@@ -129,6 +139,7 @@ static char* sim_alloc(SimArrays& d, size_t B, size_t T, unsigned mask, size_t t
   at(d.lead_sv, R_LEAD_SV);
   at(d.hist_lead_idx, R_HIST_LEAD_IDX); at(d.hist_lead_sv, R_HIST_LEAD_SV); at(d.follow_ok, R_FOLLOW_OK);
   at(d.min_gap, R_MIN_GAP);
+  at(d.x_meas, R_X_MEAS); at(d.hist_noise, R_HIST_NOISE);
   return base;
 }
 
@@ -153,6 +164,46 @@ __device__ __forceinline__ const DevTable& vehicle_table(const DevTables& Ts, co
 __device__ __forceinline__ double stop_s(const DevTables& Ts, const int* __restrict__ route, int b) {
   return vehicle_table(Ts, route, b).s_max - 1.0;
 }
+
+// ---- noise (mpcb_sim_set_noise): seeded Gaussian disturbances, a draw a function of (seed, id, t, j) only -------------
+// sigma[0..4] measurement, [5..6] actuation, [7..11] process; a channel is on when one of its sigmas is > 0, and a
+// component whose sigma is 0 is left untouched.  With every channel off the kernels compute what they computed without
+// noise, bit for bit.
+struct SimNoise {
+  unsigned long long seed;
+  int first_id;                 // id of vehicle b is first_id + b (first_id + B <= 2^31)
+  int on, meas, act, proc;      // on = meas | act | proc
+  double sigma[12];
+};
+constexpr int NOISE_W = 12;     // values recorded per vehicle and step: measurement 5, actuation 2, process 5
+constexpr int NOISE_ACT = 5, NOISE_PROC = 7;
+
+__device__ __forceinline__ unsigned vehicle_id(const SimNoise& nz, int b) {
+  const long long id = (long long)nz.first_id + b;
+  MPCB_ASSERT(nz.first_id >= 0 && b >= 0 && id <= 0x7fffffffLL);
+  return (unsigned)id;
+}
+
+// w[i] = sigma[c0 + i] z_i for the n components of the channel whose first Philox call is j0 (component i is output
+// i mod 2 of call j0 + i / 2), 0.0 where that sigma is 0.  Rounded product, no contraction into the addition that
+// applies it, so that a replay adds the recorded w and gets the same bits.
+template <int N>
+__device__ __forceinline__ void draw_channel(const SimNoise& nz, unsigned id, unsigned t, unsigned j0, int c0,
+                                             double (&w)[N]) {
+#pragma unroll
+  for (int i = 0; i < N; i += 2) {
+    double z[2];
+    sim_normal_pair(nz.seed, id, t, j0 + i / 2, z);
+#pragma unroll
+    for (int k = 0; k < 2 && i + k < N; ++k) {
+      const double sg = nz.sigma[c0 + i + k];
+      w[i + k] = sg > 0.0 ? __dmul_rn(sg, z[k]) : 0.0;
+    }
+  }
+}
+
+// v + w where sigma > 0, v untouched where it is 0
+__device__ __forceinline__ double disturb(double v, double sigma, double w) { return sigma > 0.0 ? __dadd_rn(v, w) : v; }
 
 // ---- following (mpcb_sim_set_follow): the nearest vehicle ahead on the same route is a moving obstacle ---------------
 // Each step, before the FSM kernel and from the states the loop condition is evaluated on, the vehicles are ordered by
@@ -216,10 +267,12 @@ mpcb_follow_leader_kernel(const __grid_constant__ SimArrays sim, int B, double r
 // ObstaclesFSM.update for every vehicle that is still driving (:330-374); car first, then light (:349, :362).
 // alive_cnt / next_cnt: this step's and the next step's counter of the pair sim.alive_cnt.  With following on, the car
 // slot takes the nearer of the scripted car and the leader (lead_idx / lead_sv of mpcb_follow_leader_kernel), which is
-// recorded into hist_lead_idx / hist_lead_sv.
+// recorded into hist_lead_idx / hist_lead_sv.  With measurement noise on, x_meas = x + w_meas is the state step t's solve
+// sees; everything here uses the true x.  With noise on, w_meas is recorded into hist_noise.
 __global__ void __launch_bounds__(128)
 mpcb_fsm_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ SimArrays sim, int B, double dt, int rec_t,
-                int* __restrict__ alive_cnt, int* __restrict__ next_cnt, int follow) {
+                int* __restrict__ alive_cnt, int* __restrict__ next_cnt, int follow, const __grid_constant__ SimNoise nz,
+                unsigned t) {
   const int* __restrict__ route = sim.route;
   const double* __restrict__ x = sim.x;
   const DevScenario* __restrict__ scen = sim.scen;
@@ -300,12 +353,28 @@ mpcb_fsm_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ Si
     hist_lead_sv[2 * i] = lead >= 0 ? __ldg(lead_sv + 2 * b) : nan("");
     hist_lead_sv[2 * i + 1] = lead >= 0 ? __ldg(lead_sv + 2 * b + 1) : nan("");
   }
+  if (nz.on) {
+    double w[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
+    if (live && nz.meas) {
+      double* __restrict__ x_meas = sim.x_meas;
+      draw_channel(nz, vehicle_id(nz, b), t, 0u, 0, w);
+#pragma unroll
+      for (int c = 0; c < 5; ++c) x_meas[(size_t)b * 5 + c] = disturb(__ldg(x + (size_t)b * 5 + c), nz.sigma[c], w[c]);
+    }
+    double* __restrict__ hist_noise = sim.hist_noise;
+    if (hist_noise && rec_t >= 0) {
+#pragma unroll
+      for (int c = 0; c < 5; ++c) hist_noise[((size_t)rec_t * B + b) * NOISE_W + c] = live ? w[c] : nan("");
+    }
+  }
 }
 
-// plant step (:404-406) for the vehicles that were alive at the start of the step
+// plant step (:404-406) for the vehicles that were alive at the start of the step.  With noise on, the step applies
+// U*[0] + w_act and adds w_proc to the state it produces (hist_u keeps the commanded U*[0]); both are recorded into
+// hist_noise.
 __global__ void __launch_bounds__(128)
 mpcb_plant_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ SimArrays sim, int B, double dt,
-                  int rec_t) {
+                  int rec_t, const __grid_constant__ SimNoise nz, unsigned t) {
   const int* __restrict__ route = sim.route;
   double* __restrict__ x = sim.x;
   const double* __restrict__ U = sim.U;
@@ -330,17 +399,34 @@ mpcb_plant_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ 
     hist_u[((size_t)rec_t * B + b) * 2 + 1] = live ? u2 : nan("");
     hist_status[(size_t)rec_t * B + b] = live ? __ldg(status + b) : -1;
   }
+  double wa[2] = {0.0, 0.0}, wp[5] = {0.0, 0.0, 0.0, 0.0, 0.0};   // actuation and process noise added, 0 where sigma is 0
+  if (nz.on) {
+    if (live && (nz.act | nz.proc)) {
+      const unsigned id = vehicle_id(nz, b);
+      if (nz.act) draw_channel(nz, id, t, 3u, NOISE_ACT, wa);
+      if (nz.proc) draw_channel(nz, id, t, 4u, NOISE_PROC, wp);
+    }
+    double* __restrict__ hist_noise = sim.hist_noise;
+    if (hist_noise && rec_t >= 0) {
+      double* __restrict__ h = hist_noise + ((size_t)rec_t * B + b) * NOISE_W;
+#pragma unroll
+      for (int c = 0; c < 2; ++c) h[NOISE_ACT + c] = live ? wa[c] : nan("");
+#pragma unroll
+      for (int c = 0; c < 5; ++c) h[NOISE_PROC + c] = live ? wp[c] : nan("");
+    }
+  }
   if (!live) return;
   double val[4], slope[4];
   lookup_state(vehicle_table(Ts, route, b), xs[0], val, slope);   // k_ref = get_state(current_s)[3]  (:404)
   const double kref = val[2];
   const double s = xs[0], o = xs[2], k = xs[3], v = xs[4];
-  // x + dt * [v, v o, v (k - k_ref), u1, u2]   (:50-67, :406); no FMA contraction: same rounding as numpy
-  x[(size_t)b * 5 + 0] = __dadd_rn(s, __dmul_rn(dt, v));
-  x[(size_t)b * 5 + 1] = __dadd_rn(xs[1], __dmul_rn(dt, __dmul_rn(v, o)));
-  x[(size_t)b * 5 + 2] = __dadd_rn(o, __dmul_rn(dt, __dmul_rn(v, __dadd_rn(k, -kref))));
-  x[(size_t)b * 5 + 3] = __dadd_rn(k, __dmul_rn(dt, u1));
-  x[(size_t)b * 5 + 4] = __dadd_rn(v, __dmul_rn(dt, u2));
+  const double a1 = disturb(u1, nz.sigma[NOISE_ACT], wa[0]), a2 = disturb(u2, nz.sigma[NOISE_ACT + 1], wa[1]);
+  // x + dt * [v, v o, v (k - k_ref), a1, a2]   (:50-67, :406); no FMA contraction: same rounding as numpy
+  const double xn[5] = {__dadd_rn(s, __dmul_rn(dt, v)), __dadd_rn(xs[1], __dmul_rn(dt, __dmul_rn(v, o))),
+                        __dadd_rn(o, __dmul_rn(dt, __dmul_rn(v, __dadd_rn(k, -kref)))), __dadd_rn(k, __dmul_rn(dt, a1)),
+                        __dadd_rn(v, __dmul_rn(dt, a2))};
+#pragma unroll
+  for (int c = 0; c < 5; ++c) x[(size_t)b * 5 + c] = disturb(xn[c], nz.sigma[NOISE_PROC + c], wp[c]);
   steps[b] += 1;
   if (__ldg(status + b) != MPCB_SOLVED) n_unsolved[b] += 1;
 }
@@ -444,11 +530,13 @@ struct mpcb_sim {
   int hot_start = 0;          // first pass of step t > 0 starts from step t - 1's plans advanced by one step (mpcb_sim_set_hot_start)
   double dt;
   SimArrays d = {};           // the device arrays: loop state and histories in block[0] (made at create), following and
-  char* block[2] = {};        // its histories in block[1] (made the first time following is switched on)
+  char* block[3] = {};        // its histories in block[1] (made the first time following is switched on), the measured
+                              // states and the noise history in block[2] (made the first time noise is switched on)
   // following (mpcb_sim_set_follow)
   int follow = 0;
   double follow_range = 0.0;
   size_t f_temp_bytes = 0;    // bytes of d.f_temp
+  SimNoise noise = {};        // mpcb_sim_set_noise; off: every sigma 0
 };
 
 static DevScenario to_dev_scenario(const mpcb_scenario& c) {
@@ -512,7 +600,7 @@ int mpcb_sim_create_routes(mpcb_sim_handle* out, mpcb_handle h, int B, const mpc
   s->h = h; s->B = B; s->cap = history_steps; s->t = 0;
   s->dt = h->params.dt;
   const size_t nb = (size_t)B;
-  const unsigned mask = SIM_LOOP | (route ? 1u << R_ROUTE : 0u) | (history_steps > 0 ? SIM_HIST : 0u);
+  const SimMask mask = SIM_LOOP | (route ? sim_bit(R_ROUTE) : 0ull) | (history_steps > 0 ? SIM_HIST : 0ull);
   size_t off[N_SIM + 1];
   if (!(s->block[0] = sim_alloc(s->d, nb, (size_t)history_steps, mask, 0, off))) { delete s; return MPCB_ERR_NOMEM; }
   auto fail = [&](int code) { mpcb_sim_destroy(s); return code; };
@@ -561,13 +649,14 @@ int mpcb_sim_step(mpcb_sim_handle s, int n_steps, void* cuda_stream) {
       CK(cudaGetLastError());
       s->h->launches += 2;                                   // the radix sorts' own kernels are not counted
     }
-    mpcb_fsm_kernel<<<grid, 128, 0, st>>>(s->h->dt, d, s->B, s->dt, rec, cnt, d.alive_cnt + ((s->t + 1) & 1), s->follow);
+    mpcb_fsm_kernel<<<grid, 128, 0, st>>>(s->h->dt, d, s->B, s->dt, rec, cnt, d.alive_cnt + ((s->t + 1) & 1), s->follow,
+                                          s->noise, (unsigned)s->t);
     CK(cudaGetLastError());
     // the solve runs over the list of vehicles still driving (arrived vehicles are frozen and cost nothing)
-    int rc = mpcb_solve_list_internal(s->h, s->B, d.alive_idx, cnt, d.x, d.obs_sv, d.n_obs, d.route, d.U, d.status, st,
-                                      (s->hot_start && s->t > 0) ? d.U : nullptr);
+    int rc = mpcb_solve_list_internal(s->h, s->B, d.alive_idx, cnt, s->noise.meas ? d.x_meas : d.x, d.obs_sv, d.n_obs,
+                                      d.route, d.U, d.status, st, (s->hot_start && s->t > 0) ? d.U : nullptr);
     if (rc != MPCB_OK) return rc;
-    mpcb_plant_kernel<<<grid, 128, 0, st>>>(s->h->dt, d, s->B, s->dt, rec);
+    mpcb_plant_kernel<<<grid, 128, 0, st>>>(s->h->dt, d, s->B, s->dt, rec, s->noise, (unsigned)s->t);
     CK(cudaGetLastError());
     s->h->launches += 2;
     s->t += 1;
@@ -594,7 +683,7 @@ int mpcb_sim_set_follow(mpcb_sim_handle s, int on, double follow_range) {
     CK(cub::DeviceRadixSort::SortKeys(nullptr, t2, (unsigned*)nullptr, (unsigned*)nullptr, s->B, FOLLOW_IDX_BITS, 32));
     const size_t temp = t1 > t2 ? t1 : t2;
     size_t off[N_SIM + 1];
-    if (!(s->block[1] = sim_alloc(s->d, nb, T, SIM_FOLLOW | (T > 0 ? SIM_FOLLOW_HIST : 0u), temp, off)))
+    if (!(s->block[1] = sim_alloc(s->d, nb, T, SIM_FOLLOW | (T > 0 ? SIM_FOLLOW_HIST : 0ull), temp, off)))
       return MPCB_ERR_NOMEM;
     s->f_temp_bytes = temp;
     // rows of steps taken with following off stay -1 / NaN (all-ones bytes: int -1, a double NaN)
@@ -606,6 +695,57 @@ int mpcb_sim_set_follow(mpcb_sim_handle s, int on, double follow_range) {
   }
   s->follow = 1;
   s->follow_range = follow_range;
+  return MPCB_OK;
+}
+
+int mpcb_sim_set_noise(mpcb_sim_handle s, unsigned long long seed, int first_id, const double* sigma_meas,
+                       const double* sigma_act, const double* sigma_proc) {
+  if (!s || first_id < 0 || (long long)first_id + s->B > (1ll << 31)) return MPCB_ERR_INVALID;
+  SimNoise nz = {};
+  nz.seed = seed;
+  nz.first_id = first_id;
+  const struct { const double* sigma; int n, c0; int* on; } ch[] = {
+      {sigma_meas, 5, 0, &nz.meas}, {sigma_act, 2, NOISE_ACT, &nz.act}, {sigma_proc, 5, NOISE_PROC, &nz.proc}};
+  for (const auto& c : ch)
+    for (int i = 0; i < c.n; ++i) {
+      const double v = c.sigma ? c.sigma[i] : 0.0;
+      if (!(v >= 0.0) || !isfinite(v)) return MPCB_ERR_INVALID;
+      nz.sigma[c.c0 + i] = v;
+      if (v > 0.0) *c.on = 1;
+    }
+  nz.on = nz.meas | nz.act | nz.proc;
+  if (nz.on && !s->block[2]) {
+    CK(cudaSetDevice(s->h->device));
+    const size_t nb = (size_t)s->B, T = (size_t)s->cap;
+    SimArrays d = s->d;
+    size_t off[N_SIM + 1];
+    char* base = sim_alloc(d, nb, T, sim_bit(R_X_MEAS) | (T > 0 ? sim_bit(R_HIST_NOISE) : 0ull), 0, off);
+    if (!base) return MPCB_ERR_NOMEM;
+    // rows of steps taken with noise off stay NaN (all-ones bytes)
+    cudaError_t e = T > 0 ? cudaMemset(d.hist_noise, 0xff, sim_bytes(R_HIST_NOISE, nb, T)) : cudaSuccess;
+    if (e == cudaSuccess) e = cudaStreamSynchronize(0);
+    if (e != cudaSuccess) { cudaFree(base); return cuda_fail(e, "mpcb_sim_set_noise"); }
+    s->block[2] = base;
+    s->d = d;
+  }
+  s->noise = nz;
+  return MPCB_OK;
+}
+
+int mpcb_sim_noise_history(mpcb_sim_handle s, int* n_recorded, double* hist_w, void* cuda_stream) {
+  if (!s) return MPCB_ERR_INVALID;
+  const int nt = s->t < s->cap ? s->t : s->cap;
+  if (n_recorded) *n_recorded = nt;
+  const size_t n = (size_t)nt * s->B * NOISE_W;
+  if (n == 0 || !hist_w) return MPCB_OK;
+  if (!s->d.hist_noise) {                                    // noise never switched on: nothing recorded
+    for (size_t i = 0; i < n; ++i) hist_w[i] = nan("");
+    return MPCB_OK;
+  }
+  CK(cudaSetDevice(s->h->device));
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  CK(cudaMemcpyAsync(hist_w, s->d.hist_noise, sim_bytes(R_HIST_NOISE, s->B, nt), cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
   return MPCB_OK;
 }
 
@@ -701,8 +841,8 @@ int mpcb_check_histories(mpcb_handle h, int B, int T, double s_total, const mpcb
   const struct { int r; const void* src; } in[] = {{R_SCEN, hs.data()}, {R_X, x_final}, {R_STEPS, steps},
                                                    {R_HIST_X, hist_x}, {R_HIST_U, hist_u}, {R_HIST_OBS, hist_obs},
                                                    {R_HIST_TL, hist_tl}};
-  unsigned mask = 1u << R_VERDICT | 1u << R_METRICS;
-  for (const auto& c : in) mask |= 1u << c.r;
+  SimMask mask = sim_bit(R_VERDICT) | sim_bit(R_METRICS);
+  for (const auto& c : in) mask |= sim_bit(c.r);
   SimArrays d = {};
   size_t off[N_SIM + 1];
   char* base = sim_alloc(d, nb, (size_t)T, mask, 0, off);

@@ -108,7 +108,8 @@ def gather_device(U_shard, status_shard, B, group=None):
 def simulate_sharded(make_sim, B, max_steps=200000, check_every=64, group=None, device=None):
     """Closed-loop Monte-Carlo sharded by scenario (SURVEY 8e: "shards the same way by scenario"): rank g drives the
     vehicles [g*B//G, (g+1)*B//G) to their destination on its own GPU -- ``make_sim(lo, hi)`` returns the
-    ``BatchedSimulation`` of that shard (its scenarios, its start states) -- with no exchange between ranks while the
+    ``BatchedSimulation`` of that shard (its scenarios, its start states; with ``noise=dict(..., first_id=lo)`` it draws
+    the unsharded fleet's disturbances) -- with no exchange between ranks while the
     vehicles drive (run_simulation's loop, trajectory_tracking.py:395-410, is per vehicle).  Afterwards the final states
     [B,5], step counts [B] and unsolved-step counts [B] are all-gathered, so every rank returns the whole fleet's
     result; the slowest rank's number of enqueued steps comes back with it (MAX).  Returns a dict."""

@@ -73,15 +73,37 @@ def _follow_range(r):
     return r
 
 
+NOISE_CHANNELS = (("meas", 5), ("act", 2), ("proc", 5))
+
+
+def _noise_args(B, seed, meas, act, proc, first_id):
+    """Checked arguments of mpcb_sim_set_noise: (seed, first_id, three float64 arrays or None); ValueError otherwise."""
+    if isinstance(seed, bool) or not isinstance(seed, (int, np.integer)) or not 0 <= int(seed) < 2 ** 64:
+        raise ValueError(f"seed must be an integer in [0, 2^64), got {seed!r}")
+    if isinstance(first_id, bool) or not isinstance(first_id, (int, np.integer)) or not 0 <= int(first_id) <= 2 ** 31 - B:
+        raise ValueError(f"first_id must be an integer in [0, 2^31 - B] (B = {B}), got {first_id!r}")
+    sig = []
+    for (name, n), v in zip(NOISE_CHANNELS, (meas, act, proc)):
+        if v is None:
+            sig.append(None)
+            continue
+        a = np.array(np.broadcast_to(np.asarray(v, dtype=np.float64), (n,)))
+        if not (np.all(np.isfinite(a)) and np.all(a >= 0.0)):
+            raise ValueError(f"{name} sigmas must be finite and >= 0, got {v!r}")
+        sig.append(a)
+    return int(seed), int(first_id), sig
+
+
 class BatchedSimulation:
     def __init__(self, tracker, scenarios, B=None, x_init=None, history_steps=0, hot_start=False, route=None,
-                 follow_range=None):
+                 follow_range=None, noise=None):
         """tracker: BatchedTracker; scenarios: one Scenario (shared) or a list of B; x_init: [B,5] or None for the
         reference's start state.  hot_start: from its second step on a vehicle's solve starts from its previous plan
         advanced by one step (mpcb_sim_set_hot_start) instead of the reference's table-based warm start.
         route: one int or an int array [B], vehicle b driving ``tracker.routes[route[b]]`` (None: route 0).
         follow_range: None (off) or a positive distance: the nearest vehicle ahead on the same route within that
-        distance is a moving obstacle (``set_follow``)."""
+        distance is a moving obstacle (``set_follow``).
+        noise: None (off) or a dict of ``set_noise``'s arguments (seed, meas, act, proc, first_id)."""
         self._lib = tracker._lib
         self._t = tracker
         if follow_range is not None:
@@ -89,6 +111,13 @@ class BatchedSimulation:
         scen = list(scenarios) if isinstance(scenarios, (list, tuple)) else [scenarios]
         if B is None:
             B = len(scen) if len(scen) > 1 else (len(x_init) if x_init is not None else 1)
+        if noise is not None:
+            noise = dict(noise)
+            unknown = set(noise) - {"seed", "meas", "act", "proc", "first_id"}
+            if unknown or "seed" not in noise:
+                raise ValueError(f"noise takes seed, meas, act, proc and first_id, got {sorted(noise)}")
+            nz = _noise_args(int(B), noise["seed"], noise.get("meas"), noise.get("act"), noise.get("proc"),
+                             noise.get("first_id", 0))
         arr = (Scenario * len(scen))(*scen)
         xi = None
         if x_init is not None:
@@ -113,6 +142,8 @@ class BatchedSimulation:
             check(self._lib.mpcb_sim_set_hot_start(h, 1), "mpcb_sim_set_hot_start")
         if follow_range is not None:
             self.set_follow(follow_range)
+        if noise is not None:
+            self._set_noise(*nz)
 
     def __del__(self):
         h = getattr(self, "_h", None)
@@ -151,6 +182,26 @@ class BatchedSimulation:
             check(self._lib.mpcb_sim_set_follow(self._h, 0, 0.0), "mpcb_sim_set_follow")
             return
         check(self._lib.mpcb_sim_set_follow(self._h, 1, _follow_range(follow_range)), "mpcb_sim_set_follow")
+
+    def set_noise(self, seed, meas=None, act=None, proc=None, first_id=0):
+        """Seeded Gaussian disturbances from the next step on (mpcb_sim_set_noise; include/mpcb200.h has the rules):
+        meas [5] sigmas of the state the solve sees, act [2] of the applied control, proc [5] added to the state after
+        each step; a scalar stands for every component, None for zeros.  Vehicle b draws as vehicle first_id + b, so a
+        shard [lo, hi) of a fleet with first_id=lo draws the whole fleet's noise.  No sigma > 0: noise off."""
+        self._set_noise(*_noise_args(self.B, seed, meas, act, proc, first_id))
+
+    def _set_noise(self, seed, first_id, sig):
+        check(self._lib.mpcb_sim_set_noise(self._h, seed, first_id, *(None if a is None else _dp(a) for a in sig)),
+              "mpcb_sim_set_noise")
+
+    def noise_history(self):
+        """The disturbances added in the recorded steps, sigma * z (0.0 where sigma is 0): meas [T,B,5], act [T,B,2],
+        proc [T,B,5]; NaN where the vehicle had arrived or noise was off."""
+        n = C.c_int()
+        check(self._lib.mpcb_sim_noise_history(self._h, C.byref(n), None, None), "mpcb_sim_noise_history")
+        w = np.empty((n.value, self.B, 12))
+        check(self._lib.mpcb_sim_noise_history(self._h, C.byref(n), _dp(w), None), "mpcb_sim_noise_history")
+        return dict(meas=w[..., :5], act=w[..., 5:7], proc=w[..., 7:])
 
     def follow_history(self):
         """Leaders of the recorded steps: lead [T,B] (vehicle index, -1: none, arrived, or following off), lead_s and
