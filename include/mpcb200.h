@@ -347,6 +347,23 @@ int mpcb_sim_history(mpcb_sim_handle s, int* n_recorded, double* hist_x, double*
  * within limits (+-0.1), 4 moving obstacle avoided (gap >= 1 m), 5 red light respected, 6 history covers the whole drive
  * (1 = passed).  metrics [B][4] HOST (may be NULL): max |d|, min gap to the car (1e30 if never present), final s, steps. */
 int mpcb_sim_check(mpcb_sim_handle s, int* verdict, double* metrics, void* cuda_stream);
+/* trajectory_tracking_check from the accumulators the loop keeps, without histories (history_steps may be 0).
+ * verdict [B] and metrics [B][4] HOST, same layout as mpcb_sim_check; bit 6 is always set.  On a simulation whose
+ * history covers every vehicle's whole drive, bits 0-5 and metrics equal mpcb_sim_check's bit for bit.  The FSM and
+ * plant kernels update the accumulators of the vehicles still driving, with the check's own expressions, inside the
+ * step's launches; metrics[b][0] (max |d| so far, the current state included) never decreases while b drives. */
+int mpcb_sim_running_check(mpcb_sim_handle s, int* verdict, double* metrics, void* cuda_stream);
+/* Vehicle b takes over the whole state of vehicle parent[b], for every b at once (a gather: a vehicle may be the parent
+ * of several, and a vehicle nobody names is dropped).  parent: HOST [B], each in [0, B); anything else, or following
+ * on, is MPCB_ERR_INVALID before any CUDA call.  Ordered on cuda_stream like mpcb_sim_step; parent may be reused when
+ * the call returns.  Copied: state, scenario, route, FSM state, previous plan (hot start), steps, unsolved count,
+ * running-verdict accumulators, and the recorded rows of every history (states, controls, car, status, light,
+ * leaders, disturbances).  After the call vehicle b keeps drawing noise as id first_id + b.  An identity parent
+ * changes nothing, bit for bit.  The first call allocates the workspace (synchronises the device's default stream;
+ * MPCB_ERR_NOMEM leaves the simulation as it was): B ints, then the larger of the loop state and a window of
+ * W = min(history_steps, max(1, floor(2^26 / (188 B)))) history rows (188 bytes: every history a vehicle can record).
+ * mpcb_launch_count counts 2 kernels for the loop state and 2 per window of the n_recorded rows: 2 + 2 ceil(n_recorded / W). */
+int mpcb_sim_branch(mpcb_sim_handle s, const int* parent, void* cuda_stream);
 
 /* The same checks on histories the caller supplies (HOST arrays laid out like mpcb_sim_history returns them: hist_x
  * [T][B][5] = state BEFORE each step, hist_u [T][B][2], hist_obs [T][B] (NaN: no car), hist_tl [T][B] (0 red, 1 green);

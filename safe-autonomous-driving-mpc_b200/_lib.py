@@ -114,6 +114,8 @@ SYMBOLS = {
     "mpcb_sim_alive":(C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.c_void_p]),
     "mpcb_sim_state": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mpcb_sim_check": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mpcb_sim_running_check": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mpcb_sim_branch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "mpcb_check_histories": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_double, C.POINTER(Scenario)] + [C.c_void_p] * 8),
     "mpcb_sim_history": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)] + [C.c_void_p] * 5 + [C.c_void_p]),
     "mpcb_strerror": (C.c_char_p, [C.c_int]),

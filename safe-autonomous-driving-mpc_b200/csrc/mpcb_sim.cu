@@ -9,7 +9,9 @@
 // Monte-Carlo of whole drives never leaves the GPU; histories are recorded into device buffers when asked for.  With
 // following on (mpcb_sim_set_follow), a key kernel, two radix sorts and a leader kernel come first.  With noise on
 // (mpcb_sim_set_noise), the FSM kernel also writes the measured state the solve reads and the plant kernel disturbs the
-// control it applies and the state it produces; the step keeps its launches.
+// control it applies and the state it produces; the step keeps its launches.  The FSM and plant kernels also keep each
+// vehicle's trajectory_tracking_check accumulators up to date (mpcb_sim_running_check), and mpcb_sim_branch copies
+// whole vehicles onto others for splitting estimators of rare failures.
 #include <cuda_runtime.h>
 #include <math.h>
 #include <string.h>
@@ -32,13 +34,19 @@ struct DevScenario {          // per vehicle, mirrors ObstaclesFSM.__init__ (:28
   int dynamic_obstacle, traffic_light;
 };
 
+// The accumulators of trajectory_tracking_check (mpcb_sim_check_kernel) that the FSM and plant kernels keep per vehicle
+// while it drives (R_RUN, [B][RUN_W] doubles), so that a verdict needs no history: max |d| over the states before each
+// step (NaN before the first; the check folds in the final state), the commanded control's extremes, the least gap to
+// the scripted car, and the light colour at the first step past tl_pos (-1: not passed yet).
+enum { RUN_DEV, RUN_U1LO, RUN_U1HI, RUN_U2LO, RUN_U2HI, RUN_GAP, RUN_TL, RUN_W };
+
 // The device arrays of a simulation, in five groups: the loop state and the histories are one block made at create,
 // following and its histories one block made by the first mpcb_sim_set_follow(on), the measured states and the noise
 // history one block made by the first mpcb_sim_set_noise that switches noise on.  The layout of a block, every copy and
-// every fill is derived from SIM_BYTES.
+// every fill, and what mpcb_sim_branch gathers, is derived from SIM_BYTES.
 enum SimRegion {
   R_SCEN, R_X, R_FSM_F, R_OBS_SV, R_U, R_FSM_I, R_ALIVE, R_N_OBS, R_STATUS, R_STEPS, R_N_UNSOLVED, R_ALIVE_IDX,
-  R_ALIVE_CNT, R_COUNT, R_ROUTE,                                                         // loop state
+  R_ALIVE_CNT, R_COUNT, R_RUN, R_RUN_VERDICT, R_RUN_METRICS, R_ROUTE,                     // loop state
   R_HIST_X, R_HIST_U, R_HIST_OBS, R_HIST_STATUS, R_HIST_TL, R_VERDICT, R_METRICS,         // histories
   R_F_KEY, R_F_TAG, R_F_TEMP, R_LEAD_IDX, R_LEAD_SV,                                      // following
   R_HIST_LEAD_IDX, R_HIST_LEAD_SV, R_FOLLOW_OK, R_MIN_GAP,                                // following histories
@@ -55,42 +63,55 @@ constexpr SimMask SIM_FOLLOW_HIST = sim_span(R_HIST_LEAD_IDX, R_X_MEAS);
 static_assert(N_SIM < 64, "regions are selected by the bits of a SimMask");
 
 enum SimPer { PER_VEHICLE, PER_STEP, FIXED };   // bytes per vehicle, per vehicle and recorded step, or in all
-struct SimBytes { SimPer per; size_t bytes; };
-static const SimBytes SIM_BYTES[N_SIM] = {
-  /* scen          */ {PER_VEHICLE, sizeof(DevScenario)},
-  /* x             */ {PER_VEHICLE, 5 * 8},
-  /* fsm_f         */ {PER_VEHICLE, 2 * 8},      // car position, light timer
-  /* obs_sv        */ {PER_VEHICLE, 4 * 8},
-  /* U             */ {PER_VEHICLE, NV * 8},
-  /* fsm_i         */ {PER_VEHICLE, 4},
-  /* alive         */ {PER_VEHICLE, 4},
-  /* n_obs         */ {PER_VEHICLE, 4},
-  /* status        */ {PER_VEHICLE, 4},
-  /* steps         */ {PER_VEHICLE, 4},
-  /* n_unsolved    */ {PER_VEHICLE, 4},
-  /* alive_idx     */ {PER_VEHICLE, 4},          // list of the vehicles still driving
-  /* alive_cnt     */ {FIXED, 2 * 4},            // its length, double-buffered
-  /* count         */ {FIXED, 4},                // mpcb_sim_alive
-  /* route         */ {PER_VEHICLE, 4},
-  /* hist_x        */ {PER_STEP, 5 * 8},         // [cap][B][5]
-  /* hist_u        */ {PER_STEP, 2 * 8},
-  /* hist_obs      */ {PER_STEP, 8},
-  /* hist_status   */ {PER_STEP, 4},
-  /* hist_tl       */ {PER_STEP, 4},
-  /* verdict       */ {PER_VEHICLE, 4},          // mpcb_sim_check
-  /* metrics       */ {PER_VEHICLE, 4 * 8},
-  /* f_key         */ {PER_VEHICLE, 2 * 8},      // [2][B]: s keys, then sorted
-  /* f_tag         */ {PER_VEHICLE, 3 * 4},      // [3][B]: tags, sorted by s, then by route
-  /* f_temp        */ {FIXED, 0},                // radix-sort workspace: its size query's bytes (sim_layout)
-  /* lead_idx      */ {PER_VEHICLE, 4},          // leader of this step (-1: none)
-  /* lead_sv       */ {PER_VEHICLE, 2 * 8},      // its (s, v) (NaN: none)
-  /* hist_lead_idx */ {PER_STEP, 4},             // -1 where not recorded
-  /* hist_lead_sv  */ {PER_STEP, 2 * 8},         // NaN where not recorded
-  /* follow_ok     */ {PER_VEHICLE, 4},          // mpcb_sim_follow_check
-  /* min_gap       */ {PER_VEHICLE, 8},
-  /* x_meas        */ {PER_VEHICLE, 5 * 8},      // the state the solve sees
-  /* hist_noise    */ {PER_STEP, 12 * 8},        // [cap][B][12]: measurement 5, actuation 2, process 5; NaN where not recorded
+// What mpcb_sim_branch does with a region: STATE, per vehicle, and HIST, [row][B][w], are gathered by the parent index of
+// every vehicle; SCRATCH is rebuilt before it is next read (by the next step, or by the call that returns it).
+enum SimBranch { STATE, HIST, SCRATCH };
+struct SimBytes { SimPer per; size_t bytes; SimBranch branch; };
+static constexpr SimBytes SIM_BYTES[N_SIM] = {
+  /* scen          */ {PER_VEHICLE, sizeof(DevScenario), STATE},
+  /* x             */ {PER_VEHICLE, 5 * 8, STATE},
+  /* fsm_f         */ {PER_VEHICLE, 2 * 8, STATE},      // car position, light timer
+  /* obs_sv        */ {PER_VEHICLE, 4 * 8, STATE},
+  /* U             */ {PER_VEHICLE, NV * 8, STATE},     // this step's plans; the next one's hot start
+  /* fsm_i         */ {PER_VEHICLE, 4, STATE},
+  /* alive         */ {PER_VEHICLE, 4, STATE},
+  /* n_obs         */ {PER_VEHICLE, 4, STATE},
+  /* status        */ {PER_VEHICLE, 4, STATE},
+  /* steps         */ {PER_VEHICLE, 4, STATE},
+  /* n_unsolved    */ {PER_VEHICLE, 4, STATE},
+  /* alive_idx     */ {PER_VEHICLE, 4, SCRATCH},        // list of the vehicles still driving
+  /* alive_cnt     */ {FIXED, 2 * 4, SCRATCH},          // its length, double-buffered
+  /* count         */ {FIXED, 4, SCRATCH},              // mpcb_sim_alive
+  /* run           */ {PER_VEHICLE, RUN_W * 8, STATE},  // running verdict accumulators (RunAcc)
+  /* run_verdict   */ {PER_VEHICLE, 4, SCRATCH},        // mpcb_sim_running_check
+  /* run_metrics   */ {PER_VEHICLE, 4 * 8, SCRATCH},
+  /* route         */ {PER_VEHICLE, 4, STATE},
+  /* hist_x        */ {PER_STEP, 5 * 8, HIST},          // [cap][B][5]
+  /* hist_u        */ {PER_STEP, 2 * 8, HIST},
+  /* hist_obs      */ {PER_STEP, 8, HIST},
+  /* hist_status   */ {PER_STEP, 4, HIST},
+  /* hist_tl       */ {PER_STEP, 4, HIST},
+  /* verdict       */ {PER_VEHICLE, 4, SCRATCH},        // mpcb_sim_check
+  /* metrics       */ {PER_VEHICLE, 4 * 8, SCRATCH},
+  /* f_key         */ {PER_VEHICLE, 2 * 8, SCRATCH},    // [2][B]: s keys, then sorted
+  /* f_tag         */ {PER_VEHICLE, 3 * 4, SCRATCH},    // [3][B]: tags, sorted by s, then by route
+  /* f_temp        */ {FIXED, 0, SCRATCH},              // radix-sort workspace: its size query's bytes (sim_layout)
+  /* lead_idx      */ {PER_VEHICLE, 4, SCRATCH},        // leader of this step (-1: none)
+  /* lead_sv       */ {PER_VEHICLE, 2 * 8, SCRATCH},    // its (s, v) (NaN: none)
+  /* hist_lead_idx */ {PER_STEP, 4, HIST},              // -1 where not recorded
+  /* hist_lead_sv  */ {PER_STEP, 2 * 8, HIST},          // NaN where not recorded
+  /* follow_ok     */ {PER_VEHICLE, 4, SCRATCH},        // mpcb_sim_follow_check
+  /* min_gap       */ {PER_VEHICLE, 8, SCRATCH},
+  /* x_meas        */ {PER_VEHICLE, 5 * 8, SCRATCH},    // the state the solve sees
+  /* hist_noise    */ {PER_STEP, 12 * 8, HIST},         // [cap][B][12]: measurement 5, actuation 2, process 5; NaN where not recorded
 };
+// A gathered region is copied in 4-byte words, vehicle-major (STATE) or [row][B][w] (HIST).
+constexpr bool sim_branch_classes_hold(int r = 0) {
+  return r == N_SIM || ((SIM_BYTES[r].branch == HIST) == (SIM_BYTES[r].per == PER_STEP) &&
+                        (SIM_BYTES[r].branch != STATE || SIM_BYTES[r].per == PER_VEHICLE) &&
+                        (SIM_BYTES[r].branch == SCRATCH || SIM_BYTES[r].bytes % 4 == 0) && sim_branch_classes_hold(r + 1));
+}
+static_assert(sim_branch_classes_hold(), "every recorded region is a history, every gathered one whole words");
 
 // Bytes of region r for B vehicles and T recorded steps (R_F_TEMP: see sim_layout).
 static size_t sim_bytes(int r, size_t B, size_t T) {
@@ -113,26 +134,30 @@ static void sim_layout(size_t B, size_t T, SimMask mask, size_t temp, size_t (&o
 struct SimArrays {
   DevScenario* scen; double* x; double* fsm_f; double* obs_sv; double* U;
   int* fsm_i; int* alive; int* n_obs; int* status; int* steps; int* n_unsolved; int* alive_idx; int* alive_cnt;
-  int* count; int* route;
+  int* count; double* run; int* run_verdict; double* run_metrics; int* route;
   double* hist_x; double* hist_u; double* hist_obs; int* hist_status; int* hist_tl; int* verdict; double* metrics;
   unsigned long long* f_key; unsigned* f_tag; void* f_temp; int* lead_idx; double* lead_sv;
   int* hist_lead_idx; double* hist_lead_sv; int* follow_ok; double* min_gap;
   double* x_meas; double* hist_noise;
 };
 
-// One block holding the regions in mask, laid out by sim_layout; points their arrays in d into it and leaves the others.
-// nullptr (and no error left pending) when it cannot be allocated.
-static char* sim_alloc(SimArrays& d, size_t B, size_t T, SimMask mask, size_t temp, size_t (&off)[N_SIM + 1]) {
+// One block holding the regions in mask, laid out by sim_layout; points their arrays in d (and, when given, their
+// addresses in ptr) into it and leaves the others.  nullptr (and no error left pending) when it cannot be allocated.
+static char* sim_alloc(SimArrays& d, size_t B, size_t T, SimMask mask, size_t temp, size_t (&off)[N_SIM + 1],
+                       char** ptr = nullptr) {
   sim_layout(B, T, mask, temp, off);
   char* base = nullptr;
   if (cudaMalloc((void**)&base, off[N_SIM]) != cudaSuccess) { cudaGetLastError(); return nullptr; }
+  if (ptr)
+    for (int r = 0; r < N_SIM; ++r)
+      if ((mask >> r) & 1ull) ptr[r] = base + off[r];
   auto at = [&](auto*& p, int r) {
     if ((mask >> r) & 1ull) p = (std::remove_reference_t<decltype(p)>)(base + off[r]);
   };
   at(d.scen, R_SCEN); at(d.x, R_X); at(d.fsm_f, R_FSM_F); at(d.obs_sv, R_OBS_SV); at(d.U, R_U);
   at(d.fsm_i, R_FSM_I); at(d.alive, R_ALIVE); at(d.n_obs, R_N_OBS); at(d.status, R_STATUS); at(d.steps, R_STEPS);
   at(d.n_unsolved, R_N_UNSOLVED); at(d.alive_idx, R_ALIVE_IDX); at(d.alive_cnt, R_ALIVE_CNT); at(d.count, R_COUNT);
-  at(d.route, R_ROUTE);
+  at(d.run, R_RUN); at(d.run_verdict, R_RUN_VERDICT); at(d.run_metrics, R_RUN_METRICS); at(d.route, R_ROUTE);
   at(d.hist_x, R_HIST_X); at(d.hist_u, R_HIST_U); at(d.hist_obs, R_HIST_OBS); at(d.hist_status, R_HIST_STATUS);
   at(d.hist_tl, R_HIST_TL); at(d.verdict, R_VERDICT); at(d.metrics, R_METRICS);
   at(d.f_key, R_F_KEY); at(d.f_tag, R_F_TAG); at(d.f_temp, R_F_TEMP); at(d.lead_idx, R_LEAD_IDX);
@@ -337,6 +362,11 @@ mpcb_fsm_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ Si
     fsm_f[2 * b] = obs_s;
     fsm_f[2 * b + 1] = timer;
     fsm_i[b] = f;
+    // running verdicts, with mpcb_sim_check_kernel's expressions: the gap to the scripted car (hist_obs - hist_x's s)
+    // and the colour recorded into hist_tl at the first step past the light
+    double* __restrict__ run = sim.run + (size_t)b * RUN_W;
+    if (!isnan(car_s)) run[RUN_GAP] = fmin(run[RUN_GAP], car_s - s);
+    if (s > sc.tl_pos && run[RUN_TL] < 0.0) run[RUN_TL] = (f & F_TL_GREEN) ? 1.0 : 0.0;
   }
 #pragma unroll
   for (int k = 0; k < 4; ++k) obs_sv[(size_t)b * 4 + k] = o[k];
@@ -416,6 +446,11 @@ mpcb_plant_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ 
     }
   }
   if (!live) return;
+  // running verdicts, with mpcb_sim_check_kernel's expressions: |d| of the state before the step, the commanded control
+  double* __restrict__ run = sim.run + (size_t)b * RUN_W;
+  run[RUN_DEV] = fmax(run[RUN_DEV], fabs(xs[1]));
+  run[RUN_U1LO] = fmin(run[RUN_U1LO], u1); run[RUN_U1HI] = fmax(run[RUN_U1HI], u1);
+  run[RUN_U2LO] = fmin(run[RUN_U2LO], u2); run[RUN_U2HI] = fmax(run[RUN_U2HI], u2);
   double val[4], slope[4];
   lookup_state(vehicle_table(Ts, route, b), xs[0], val, slope);   // k_ref = get_state(current_s)[3]  (:404)
   const double kref = val[2];
@@ -448,6 +483,22 @@ __global__ void mpcb_count_alive_kernel(const __grid_constant__ DevTables Ts, co
 // avoided, gap >= 1 m (:142-164), 5 red light respected (:167-181), 6 history covers the whole drive.  route == nullptr:
 // every vehicle's route is s_total long; else vehicle b's route's s_max.
 // (The reference's CPU-time item :134-139 is a property of the host, not of the trajectory; it is not evaluated here.)
+// Bits 0-5 from the accumulators, shared with mpcb_sim_running_check_kernel:
+__device__ __forceinline__ int tracking_verdict(const DevScenario& sc, double s_final, double s_end, double max_dev,
+                                                double u1lo, double u1hi, double u2lo, double u2hi, double min_gap,
+                                                bool ran_red, double u1_min, double u1_max, double u2_min,
+                                                double u2_max) {
+  const double tol = 0.1, lateral = 1.5, safety = 1.0;
+  int v = 0;
+  if (!(s_final < s_end - 1.0)) v |= 1;
+  if (!(max_dev > lateral)) v |= 2;
+  if (!(u1lo < u1_min - tol || u1hi > u1_max + tol)) v |= 4;
+  if (!(u2lo < u2_min - tol || u2hi > u2_max + tol)) v |= 8;
+  if (!(sc.dynamic_obstacle && min_gap < safety)) v |= 16;
+  if (!ran_red) v |= 32;
+  return v;
+}
+
 __global__ void __launch_bounds__(128)
 mpcb_sim_check_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ SimArrays sim, int B, int n_rec,
                       double s_total, double u1_min, double u1_max, double u2_min, double u2_max) {
@@ -465,7 +516,6 @@ mpcb_sim_check_kernel(const __grid_constant__ DevTables Ts, const __grid_constan
   if (b >= B) return;
   const DevScenario sc = scen[b];
   const int n = min(steps[b], n_rec);
-  const double tol = 0.1, lateral = 1.5, safety = 1.0;
   double max_dev = fabs(x_final[(size_t)b * 5 + 1]);
   double u1lo = BIG, u1hi = -BIG, u2lo = BIG, u2hi = -BIG, min_gap = BIG;
   int first_pass = -1;
@@ -480,15 +530,10 @@ mpcb_sim_check_kernel(const __grid_constant__ DevTables Ts, const __grid_constan
     if (first_pass < 0 && s > sc.tl_pos) first_pass = t;
   }
   const double s_final = x_final[(size_t)b * 5];
-  int v = 0;
   const double s_end = route ? vehicle_table(Ts, route, b).s_max : s_total;
-  if (!(s_final < s_end - 1.0)) v |= 1;
-  if (!(max_dev > lateral)) v |= 2;
-  if (!(u1lo < u1_min - tol || u1hi > u1_max + tol)) v |= 4;
-  if (!(u2lo < u2_min - tol || u2hi > u2_max + tol)) v |= 8;
-  if (!(sc.dynamic_obstacle && min_gap < safety)) v |= 16;
   const bool ran_red = sc.traffic_light && first_pass >= 0 && hist_tl[(size_t)first_pass * B + b] == 0;
-  if (!ran_red) v |= 32;
+  int v = tracking_verdict(sc, s_final, s_end, max_dev, u1lo, u1hi, u2lo, u2hi, min_gap, ran_red, u1_min, u1_max, u2_min,
+                           u2_max);
   if (steps[b] <= n_rec) v |= 64;
   verdict[b] = v;
   metrics[(size_t)b * 4 + 0] = max_dev;
@@ -520,6 +565,58 @@ mpcb_follow_check_kernel(const __grid_constant__ SimArrays sim, int B, int n_rec
   min_gap[b] = g;
 }
 
+// trajectory_tracking_check from the accumulators the FSM and plant kernels keep (R_RUN), into run_verdict and
+// run_metrics; bit 6 is always set.  max |d| folds in the current state as the check folds in the final one.
+__global__ void __launch_bounds__(128)
+mpcb_sim_running_check_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ SimArrays sim, int B,
+                              double s_total, double u1_min, double u1_max, double u2_min, double u2_max) {
+  const int* __restrict__ route = sim.route;
+  const double* __restrict__ x = sim.x;
+  const int* __restrict__ steps = sim.steps;
+  const DevScenario* __restrict__ scen = sim.scen;
+  const double* __restrict__ run = sim.run;
+  int* __restrict__ verdict = sim.run_verdict;
+  double* __restrict__ metrics = sim.run_metrics;
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  const DevScenario sc = scen[b];
+  const double* r = run + (size_t)b * RUN_W;
+  const double max_dev = fmax(fabs(x[(size_t)b * 5 + 1]), r[RUN_DEV]);
+  const double s_final = x[(size_t)b * 5];
+  const double s_end = route ? vehicle_table(Ts, route, b).s_max : s_total;
+  const bool ran_red = sc.traffic_light && r[RUN_TL] == 0.0;
+  verdict[b] = 64 | tracking_verdict(sc, s_final, s_end, max_dev, r[RUN_U1LO], r[RUN_U1HI], r[RUN_U2LO], r[RUN_U2HI],
+                                     r[RUN_GAP], ran_red, u1_min, u1_max, u2_min, u2_max);
+  metrics[(size_t)b * 4 + 0] = max_dev;
+  metrics[(size_t)b * 4 + 1] = r[RUN_GAP];
+  metrics[(size_t)b * 4 + 2] = s_final;
+  metrics[(size_t)b * 4 + 3] = (double)steps[b];
+}
+
+// ---- branching (mpcb_sim_branch): vehicle b takes over the whole state of vehicle parent[b] -------------------------
+// A pass copies up to N_SIM arrays of n 4-byte words, one per blockIdx.y.  With parent, a gather: dst is laid out
+// [rows][B][w] (one row for the loop state) and word (r, b, k) comes from word (r, parent[b], k) of src; without it a
+// straight copy.  Consecutive threads take consecutive words of dst and of a row of src: coalesced on both sides.
+struct BranchCopy { const unsigned* src; unsigned* dst; unsigned long long n; unsigned w; };
+struct BranchPass { BranchCopy c[N_SIM]; };
+constexpr int BRANCH_THREADS = 256;
+
+__global__ void __launch_bounds__(BRANCH_THREADS)
+mpcb_branch_gather_kernel(const __grid_constant__ BranchPass g, const int* __restrict__ parent, int B) {
+  const BranchCopy& c = g.c[blockIdx.y];
+  const unsigned* __restrict__ src = c.src;
+  unsigned* __restrict__ dst = c.dst;
+  const unsigned long long row = (unsigned long long)B * c.w;
+  for (unsigned long long e = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; e < c.n;
+       e += (unsigned long long)gridDim.x * blockDim.x) {
+    if (!parent) { dst[e] = src[e]; continue; }
+    const unsigned long long r = e / row, i = e - r * row, b = i / c.w;
+    const int p = __ldg(parent + b);
+    MPCB_ASSERT(p >= 0 && p < B);
+    dst[e] = src[r * row + (unsigned long long)p * c.w + (i - b * c.w)];
+  }
+}
+
 }  // namespace mpcb
 
 using namespace mpcb;
@@ -537,7 +634,30 @@ struct mpcb_sim {
   double follow_range = 0.0;
   size_t f_temp_bytes = 0;    // bytes of d.f_temp
   SimNoise noise = {};        // mpcb_sim_set_noise; off: every sigma 0
+  char* region[N_SIM] = {};   // address of every allocated region (nullptr: not allocated), for mpcb_sim_branch
+  // branching (mpcb_sim_branch), made by its first call: the device workspace (the parent indices, then the gathered
+  // loop state or one window of history rows), the pinned staging of the parent indices and the event of their copy
+  char* branch_ws = nullptr;
+  int* branch_parent = nullptr;
+  cudaEvent_t branch_copied = nullptr;
+  int branch_rows = 0;        // history rows per window
 };
+
+// Rows of the history window of mpcb_sim_branch: as many as fit BRANCH_WINDOW_BYTES with every history a simulation
+// can have (following and noise may be switched on after the first branch), at least one, at most the capacity.
+constexpr size_t BRANCH_WINDOW_BYTES = size_t(1) << 26;
+static int branch_window_rows(size_t B, int cap) {
+  size_t row = 0;
+  for (int r = 0; r < N_SIM; ++r) if (SIM_BYTES[r].branch == HIST) row += SIM_BYTES[r].bytes;
+  const size_t w = BRANCH_WINDOW_BYTES / (row * B);
+  return (int)(w < 1 ? 1 : w > (size_t)cap ? (size_t)cap : w);
+}
+
+static SimMask sim_branch_mask(SimBranch k) {
+  SimMask m = 0;
+  for (int r = 0; r < N_SIM; ++r) if (SIM_BYTES[r].branch == k) m |= sim_bit(r);
+  return m;
+}
 
 static DevScenario to_dev_scenario(const mpcb_scenario& c) {
   return DevScenario{c.obs_trigger_s, c.obs_start_s, c.obs_v, c.obs_end_s, c.tl_pos, c.tl_trigger_s,
@@ -578,6 +698,9 @@ int mpcb_sim_destroy(mpcb_sim_handle s) {
   if (!s) return MPCB_ERR_INVALID;
   cudaSetDevice(s->h->device);
   for (char* p : s->block) if (p) cudaFree(p);
+  if (s->branch_ws) cudaFree(s->branch_ws);
+  if (s->branch_parent) cudaFreeHost(s->branch_parent);
+  if (s->branch_copied) cudaEventDestroy(s->branch_copied);
   delete s;
   return MPCB_OK;
 }
@@ -602,11 +725,16 @@ int mpcb_sim_create_routes(mpcb_sim_handle* out, mpcb_handle h, int B, const mpc
   const size_t nb = (size_t)B;
   const SimMask mask = SIM_LOOP | (route ? sim_bit(R_ROUTE) : 0ull) | (history_steps > 0 ? SIM_HIST : 0ull);
   size_t off[N_SIM + 1];
-  if (!(s->block[0] = sim_alloc(s->d, nb, (size_t)history_steps, mask, 0, off))) { delete s; return MPCB_ERR_NOMEM; }
+  if (!(s->block[0] = sim_alloc(s->d, nb, (size_t)history_steps, mask, 0, off, s->region))) {
+    delete s;
+    return MPCB_ERR_NOMEM;
+  }
   auto fail = [&](int code) { mpcb_sim_destroy(s); return code; };
   std::vector<DevScenario> hs(nb);
-  std::vector<double> hx(nb * 5), hf(nb * 2);
+  std::vector<double> hx(nb * 5), hf(nb * 2), hr(nb * RUN_W);
   for (size_t b = 0; b < nb; ++b) {
+    double* r = &hr[b * RUN_W];                                         // the check kernel's start values
+    r[RUN_DEV] = nan(""); r[RUN_U1LO] = r[RUN_U2LO] = r[RUN_GAP] = BIG; r[RUN_U1HI] = r[RUN_U2HI] = -BIG; r[RUN_TL] = -1.0;
     const mpcb_scenario& c = scen[n_scen == 1 ? 0 : b];
     hs[b] = to_dev_scenario(c);
     if (x_init) for (int k = 0; k < 5; ++k) hx[b * 5 + k] = x_init[b * 5 + k];
@@ -616,7 +744,7 @@ int mpcb_sim_create_routes(mpcb_sim_handle* out, mpcb_handle h, int B, const mpc
   }
   // start values, synchronous on the default stream: from the host, then zeros
   const struct { int r; const void* src; } start[] = {{R_ROUTE, route}, {R_SCEN, hs.data()}, {R_X, hx.data()},
-                                                      {R_FSM_F, hf.data()}};
+                                                      {R_FSM_F, hf.data()}, {R_RUN, hr.data()}};
   char* base = s->block[0];
   cudaError_t e;
   for (const auto& c : start)
@@ -683,7 +811,7 @@ int mpcb_sim_set_follow(mpcb_sim_handle s, int on, double follow_range) {
     CK(cub::DeviceRadixSort::SortKeys(nullptr, t2, (unsigned*)nullptr, (unsigned*)nullptr, s->B, FOLLOW_IDX_BITS, 32));
     const size_t temp = t1 > t2 ? t1 : t2;
     size_t off[N_SIM + 1];
-    if (!(s->block[1] = sim_alloc(s->d, nb, T, SIM_FOLLOW | (T > 0 ? SIM_FOLLOW_HIST : 0ull), temp, off)))
+    if (!(s->block[1] = sim_alloc(s->d, nb, T, SIM_FOLLOW | (T > 0 ? SIM_FOLLOW_HIST : 0ull), temp, off, s->region)))
       return MPCB_ERR_NOMEM;
     s->f_temp_bytes = temp;
     // rows of steps taken with following off stay -1 / NaN (all-ones bytes: int -1, a double NaN)
@@ -719,7 +847,8 @@ int mpcb_sim_set_noise(mpcb_sim_handle s, unsigned long long seed, int first_id,
     const size_t nb = (size_t)s->B, T = (size_t)s->cap;
     SimArrays d = s->d;
     size_t off[N_SIM + 1];
-    char* base = sim_alloc(d, nb, T, sim_bit(R_X_MEAS) | (T > 0 ? sim_bit(R_HIST_NOISE) : 0ull), 0, off);
+    char* region[N_SIM] = {};
+    char* base = sim_alloc(d, nb, T, sim_bit(R_X_MEAS) | (T > 0 ? sim_bit(R_HIST_NOISE) : 0ull), 0, off, region);
     if (!base) return MPCB_ERR_NOMEM;
     // rows of steps taken with noise off stay NaN (all-ones bytes)
     cudaError_t e = T > 0 ? cudaMemset(d.hist_noise, 0xff, sim_bytes(R_HIST_NOISE, nb, T)) : cudaSuccess;
@@ -727,6 +856,7 @@ int mpcb_sim_set_noise(mpcb_sim_handle s, unsigned long long seed, int first_id,
     if (e != cudaSuccess) { cudaFree(base); return cuda_fail(e, "mpcb_sim_set_noise"); }
     s->block[2] = base;
     s->d = d;
+    for (int r = 0; r < N_SIM; ++r) if (region[r]) s->region[r] = region[r];
   }
   s->noise = nz;
   return MPCB_OK;
@@ -822,6 +952,90 @@ int mpcb_sim_check(mpcb_sim_handle s, int* verdict, double* metrics, void* cuda_
   CK(launch_check(s->h, s->d, s->B, nt, s->h->dt.t[0].s_max, verdict, metrics, st));
   CK(cudaStreamSynchronize(st));
   s->h->launches += 1;
+  return MPCB_OK;
+}
+
+int mpcb_sim_running_check(mpcb_sim_handle s, int* verdict, double* metrics, void* cuda_stream) {
+  if (!s || !verdict) return MPCB_ERR_INVALID;
+  CK(cudaSetDevice(s->h->device));
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  const mpcb_params& p = s->h->params;
+  const size_t nb = (size_t)s->B;
+  mpcb_sim_running_check_kernel<<<(s->B + 127) / 128, 128, 0, st>>>(s->h->dt, s->d, s->B, s->h->dt.t[0].s_max, p.u_min[0],
+                                                                    p.u_max[0], p.u_min[1], p.u_max[1]);
+  CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(verdict, s->d.run_verdict, sim_bytes(R_RUN_VERDICT, nb, 0), cudaMemcpyDeviceToHost, st));
+  if (metrics) CK(cudaMemcpyAsync(metrics, s->d.run_metrics, sim_bytes(R_RUN_METRICS, nb, 0), cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  s->h->launches += 1;
+  return MPCB_OK;
+}
+
+int mpcb_sim_branch(mpcb_sim_handle s, const int* parent, void* cuda_stream) {
+  if (!s || !parent || s->follow) return MPCB_ERR_INVALID;   // a copy would follow its parent at gap 0
+  for (int b = 0; b < s->B; ++b)
+    if (parent[b] < 0 || parent[b] >= s->B) return MPCB_ERR_INVALID;
+  CK(cudaSetDevice(s->h->device));
+  const size_t nb = (size_t)s->B;
+  SimMask have = 0;
+  for (int r = 0; r < N_SIM; ++r) if (s->region[r]) have |= sim_bit(r);
+  // workspace: the parent indices, then room for the gathered loop state or one window of every history there can be
+  const SimMask state = sim_branch_mask(STATE) & have, hist = sim_branch_mask(HIST);
+  size_t soff[N_SIM + 1], hoff[N_SIM + 1];
+  const size_t pbytes = (nb * sizeof(int) + 255) & ~(size_t)255;
+  if (!s->branch_ws) {
+    const int rows = s->cap > 0 ? branch_window_rows(nb, s->cap) : 0;
+    sim_layout(nb, 0, state, 0, soff);
+    sim_layout(nb, (size_t)rows, rows > 0 ? hist : 0ull, 0, hoff);
+    char* ws = nullptr;
+    int* hp = nullptr;
+    cudaEvent_t ev = nullptr;
+    if (cudaMalloc((void**)&ws, pbytes + (soff[N_SIM] > hoff[N_SIM] ? soff[N_SIM] : hoff[N_SIM])) != cudaSuccess ||
+        cudaMallocHost((void**)&hp, nb * sizeof(int)) != cudaSuccess ||
+        cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) != cudaSuccess) {
+      cudaGetLastError();
+      if (ws) cudaFree(ws);
+      if (hp) cudaFreeHost(hp);
+      return MPCB_ERR_NOMEM;
+    }
+    s->branch_ws = ws; s->branch_parent = hp; s->branch_copied = ev; s->branch_rows = rows;
+    CK(cudaStreamSynchronize(0));
+  }
+  sim_layout(nb, 0, state, 0, soff);
+  sim_layout(nb, (size_t)s->branch_rows, s->branch_rows > 0 ? hist : 0ull, 0, hoff);
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  // the caller's parent is read here; the staging is reused once the previous call's copy has left it
+  CK(cudaEventSynchronize(s->branch_copied));
+  memcpy(s->branch_parent, parent, nb * sizeof(int));
+  const int* dpar = (const int*)s->branch_ws;
+  CK(cudaMemcpyAsync((void*)dpar, s->branch_parent, nb * sizeof(int), cudaMemcpyHostToDevice, st));
+  CK(cudaEventRecord(s->branch_copied, st));
+  char* ws = s->branch_ws + pbytes;
+  // one pass: gather regions of mask (rows from row0 on) into the workspace at off, then copy them back
+  auto pass = [&](SimMask mask, const size_t (&off)[N_SIM + 1], size_t row0, size_t rows) -> cudaError_t {
+    BranchPass g = {}, back = {};
+    int n = 0;
+    unsigned long long most = 0;
+    for (int r = 0; r < N_SIM; ++r) {
+      if (!((mask >> r) & 1ull)) continue;
+      const size_t bytes = SIM_BYTES[r].bytes, at = row0 * nb * bytes, words = rows * nb * bytes / 4;
+      g.c[n] = BranchCopy{(const unsigned*)(s->region[r] + at), (unsigned*)(ws + off[r]), words, (unsigned)(bytes / 4)};
+      back.c[n] = BranchCopy{(const unsigned*)(ws + off[r]), (unsigned*)(s->region[r] + at), words, g.c[n].w};
+      if (words > most) most = words;
+      ++n;
+    }
+    if (n == 0) return cudaSuccess;
+    const unsigned long long blocks = (most + BRANCH_THREADS - 1) / BRANCH_THREADS;
+    const dim3 grid((unsigned)(blocks < 2048 ? blocks : 2048), (unsigned)n);
+    mpcb_branch_gather_kernel<<<grid, BRANCH_THREADS, 0, st>>>(g, dpar, s->B);
+    mpcb_branch_gather_kernel<<<grid, BRANCH_THREADS, 0, st>>>(back, nullptr, s->B);
+    s->h->launches += 2;
+    return cudaGetLastError();
+  };
+  CK(pass(state, soff, 0, 1));
+  const int nt = s->t < s->cap ? s->t : s->cap;
+  for (int row0 = 0; row0 < nt; row0 += s->branch_rows)
+    CK(pass(hist & have, hoff, (size_t)row0, (size_t)(nt - row0 < s->branch_rows ? nt - row0 : s->branch_rows)));
   return MPCB_OK;
 }
 

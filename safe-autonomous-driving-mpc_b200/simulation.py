@@ -231,6 +231,28 @@ class BatchedSimulation:
         check(self._lib.mpcb_sim_check(self._h, _dp(v), _dp(m), None), "mpcb_sim_check")
         return _verdict_dict(v, m)
 
+    def running_check(self):
+        """The same dict as ``check``, from the accumulators the loop keeps per vehicle (mpcb_sim_running_check): needs
+        no history, and history_complete is always True.  Equal to ``check`` bit for bit when the history covers every
+        drive; max_dev includes the current state, so it never decreases while a vehicle drives."""
+        v = np.empty(self.B, np.int32)
+        m = np.empty((self.B, 4))
+        check(self._lib.mpcb_sim_running_check(self._h, _dp(v), _dp(m), None), "mpcb_sim_running_check")
+        return _verdict_dict(v, m)
+
+    def branch(self, parent, stream=None):
+        """Vehicle b takes over the whole state of vehicle parent[b], histories and running verdicts included
+        (mpcb_sim_branch; include/mpcb200.h has the rules).  parent: integer array [B] with values in [0, B), else
+        ValueError before any device call.  Vehicle b keeps drawing noise as vehicle first_id + b, so copies of one
+        parent draw independent futures.  Refused (MpcbError) while following is on."""
+        p = np.asarray(parent)
+        if p.shape != (self.B,) or not np.issubdtype(p.dtype, np.integer):
+            raise ValueError(f"parent must be an int array of shape ({self.B},), got {p.dtype} {p.shape}")
+        if p.size and (p.min() < 0 or p.max() >= self.B):
+            raise ValueError(f"parent values must be in [0, {self.B})")
+        p = np.ascontiguousarray(p, dtype=np.int32)
+        check(self._lib.mpcb_sim_branch(self._h, _dp(p), C.c_void_p(stream or 0)), "mpcb_sim_branch")
+
     def run(self, max_steps=200000, check_every=64):
         """Drive until every vehicle has passed s_max - 1 (or max_steps).  Returns the number of steps enqueued."""
         done = 0

@@ -10,4 +10,5 @@ from .environment import ObstaclesFSM, run_simulation  # noqa: E402,F401
 from .planner import PlannerEvaluator  # noqa: E402,F401
 from . import planner_driver  # noqa: E402,F401
 from .simulation import BatchedSimulation, make_scenario, FLEET_SOLVER_CAPS  # noqa: E402,F401
+from . import rare_events  # noqa: E402,F401
 from . import _lib, sharding  # noqa: E402,F401
