@@ -276,7 +276,7 @@ int mpcb_sim_create_routes(mpcb_sim_handle* out, mpcb_handle h, int B, const mpc
                            const int* route, const double* x_init, int history_steps);
 int mpcb_sim_destroy(mpcb_sim_handle s);
 /* n_steps closed-loop steps, asynchronous on cuda_stream (3 + the solver's launches per step, no host round trip; with
- * following on, 2 more plus the kernels of two radix sorts).
+ * following on, 2 more plus the kernels of two radix sorts, or 1 more when worlds are set, mpcb_sim_set_worlds).
  * Vehicles that have passed s_max - 1 are frozen. */
 int mpcb_sim_step(mpcb_sim_handle s, int n_steps, void* cuda_stream);
 /* Hot start (off by default): from its second step on, a vehicle's first pass starts from its previous plan advanced by
@@ -357,13 +357,36 @@ int mpcb_sim_running_check(mpcb_sim_handle s, int* verdict, double* metrics, voi
  * of several, and a vehicle nobody names is dropped).  parent: HOST [B], each in [0, B); anything else, or following
  * on, is MPCB_ERR_INVALID before any CUDA call.  Ordered on cuda_stream like mpcb_sim_step; parent may be reused when
  * the call returns.  Copied: state, scenario, route, FSM state, previous plan (hot start), steps, unsolved count,
- * running-verdict accumulators, and the recorded rows of every history (states, controls, car, status, light,
- * leaders, disturbances).  After the call vehicle b keeps drawing noise as id first_id + b.  An identity parent
+ * running-verdict accumulators, running follower gap, and the recorded rows of every history (states, controls, car,
+ * status, light, leaders, disturbances).  After the call vehicle b keeps drawing noise as id first_id + b.  An identity parent
  * changes nothing, bit for bit.  The first call allocates the workspace (synchronises the device's default stream;
  * MPCB_ERR_NOMEM leaves the simulation as it was): B ints, then the larger of the loop state and a window of
  * W = min(history_steps, max(1, floor(2^26 / (188 B)))) history rows (188 bytes: every history a vehicle can record).
  * mpcb_launch_count counts 2 kernels for the loop state and 2 per window of the n_recorded rows: 2 + 2 ceil(n_recorded / W). */
 int mpcb_sim_branch(mpcb_sim_handle s, const int* parent, void* cuda_stream);
+/* Worlds (off by default): with world_size M, world w is vehicles [w M, (w + 1) M), W = B / M worlds, and a vehicle's
+ * leader is searched for only inside its own world: among the vehicles of b's world still driving on b's route, ordered
+ * by (s, index) with -0.0 equal to +0.0, the leader of b is the next one if s_leader - s_b <= follow_range.  So W
+ * independent platoons, or W copies of one traffic situation, share one simulation.  M = B is mpcb_sim_set_follow's
+ * rule for the whole fleet, bit for bit.  1 <= M <= 1024 with B % M == 0, or 0 for one world (every entry point then
+ * behaves and launches as without this call); anything else is MPCB_ERR_INVALID before any CUDA call.  Takes effect
+ * from the next step and may be changed at any time.  With worlds set and following on, following adds 1 kernel per
+ * step (one CTA holds whole worlds and finds their leaders in shared memory) instead of 2 plus two radix sorts. */
+int mpcb_sim_set_worlds(mpcb_sim_handle s, int world_size);
+/* mpcb_sim_follow_check without histories (history_steps may be 0): same layout, ok [B] HOST, min_gap [B] HOST (may be
+ * NULL), from the least gap to the leader that the FSM kernel keeps per vehicle while following is on, with the check's
+ * expression.  On a simulation whose history covers every vehicle's whole drive it equals mpcb_sim_follow_check bit for
+ * bit; if following was never switched on, min_gap is 1e30 and ok 1.  The gap is copied with its vehicle by
+ * mpcb_sim_branch and mpcb_sim_branch_worlds.  Synchronises the stream; launches no kernel. */
+int mpcb_sim_running_follow_check(mpcb_sim_handle s, int* ok, double* min_gap, void* cuda_stream);
+/* World w takes over the whole state of world parent_world[w]: vehicle w M + i takes over everything mpcb_sim_branch
+ * copies from vehicle parent_world[w] M + i, running accumulators and histories included, and recorded leader indices
+ * j >= 0 are moved into the copy's world (j + (w - parent_world[w]) M).  parent_world: HOST [W], each in [0, W); worlds
+ * must be set (mpcb_sim_set_worlds); anything else is MPCB_ERR_INVALID before any CUDA call.  Following may be on: a
+ * copy only sees the vehicles of its own world.  Ordered on cuda_stream like mpcb_sim_step; vehicle b keeps drawing
+ * noise as id first_id + b.  Workspace and launch count are mpcb_sim_branch's (the two share it), with its window of
+ * rows = min(history_steps, max(1, floor(2^26 / (188 B)))) history rows: 2 + 2 ceil(n_recorded / rows) kernels. */
+int mpcb_sim_branch_worlds(mpcb_sim_handle s, const int* parent_world, void* cuda_stream);
 
 /* The same checks on histories the caller supplies (HOST arrays laid out like mpcb_sim_history returns them: hist_x
  * [T][B][5] = state BEFORE each step, hist_u [T][B][2], hist_obs [T][B] (NaN: no car), hist_tl [T][B] (0 red, 1 green);

@@ -116,6 +116,9 @@ SYMBOLS = {
     "mpcb_sim_check": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mpcb_sim_running_check": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mpcb_sim_branch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mpcb_sim_set_worlds": (C.c_int, [C.c_void_p, C.c_int]),
+    "mpcb_sim_running_follow_check": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mpcb_sim_branch_worlds": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "mpcb_check_histories": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_double, C.POINTER(Scenario)] + [C.c_void_p] * 8),
     "mpcb_sim_history": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)] + [C.c_void_p] * 5 + [C.c_void_p]),
     "mpcb_strerror": (C.c_char_p, [C.c_int]),

@@ -7,11 +7,12 @@
 // One simulation object holds B vehicles (each with its own scenario constants and FSM state).  A step is three
 // launches on one stream -- FSM kernel -> mpcb_solve_batch -> plant kernel -- with no host round trip, so a
 // Monte-Carlo of whole drives never leaves the GPU; histories are recorded into device buffers when asked for.  With
-// following on (mpcb_sim_set_follow), a key kernel, two radix sorts and a leader kernel come first.  With noise on
+// following on (mpcb_sim_set_follow), a key kernel, two radix sorts and a leader kernel come first, or one world kernel
+// when the fleet is split into worlds (mpcb_sim_set_worlds).  With noise on
 // (mpcb_sim_set_noise), the FSM kernel also writes the measured state the solve reads and the plant kernel disturbs the
 // control it applies and the state it produces; the step keeps its launches.  The FSM and plant kernels also keep each
 // vehicle's trajectory_tracking_check accumulators up to date (mpcb_sim_running_check), and mpcb_sim_branch copies
-// whole vehicles onto others for splitting estimators of rare failures.
+// whole vehicles (mpcb_sim_branch_worlds: whole worlds) onto others for splitting estimators of rare failures.
 #include <cuda_runtime.h>
 #include <math.h>
 #include <string.h>
@@ -48,7 +49,7 @@ enum SimRegion {
   R_SCEN, R_X, R_FSM_F, R_OBS_SV, R_U, R_FSM_I, R_ALIVE, R_N_OBS, R_STATUS, R_STEPS, R_N_UNSOLVED, R_ALIVE_IDX,
   R_ALIVE_CNT, R_COUNT, R_RUN, R_RUN_VERDICT, R_RUN_METRICS, R_ROUTE,                     // loop state
   R_HIST_X, R_HIST_U, R_HIST_OBS, R_HIST_STATUS, R_HIST_TL, R_VERDICT, R_METRICS,         // histories
-  R_F_KEY, R_F_TAG, R_F_TEMP, R_LEAD_IDX, R_LEAD_SV,                                      // following
+  R_F_KEY, R_F_TAG, R_F_TEMP, R_LEAD_IDX, R_LEAD_SV, R_RUN_FOLLOW,                        // following
   R_HIST_LEAD_IDX, R_HIST_LEAD_SV, R_FOLLOW_OK, R_MIN_GAP,                                // following histories
   R_X_MEAS, R_HIST_NOISE,                                                                 // noise
   N_SIM
@@ -98,6 +99,7 @@ static constexpr SimBytes SIM_BYTES[N_SIM] = {
   /* f_temp        */ {FIXED, 0, SCRATCH},              // radix-sort workspace: its size query's bytes (sim_layout)
   /* lead_idx      */ {PER_VEHICLE, 4, SCRATCH},        // leader of this step (-1: none)
   /* lead_sv       */ {PER_VEHICLE, 2 * 8, SCRATCH},    // its (s, v) (NaN: none)
+  /* run_follow    */ {PER_VEHICLE, 8, STATE},          // least gap to the leader so far (mpcb_sim_running_follow_check)
   /* hist_lead_idx */ {PER_STEP, 4, HIST},              // -1 where not recorded
   /* hist_lead_sv  */ {PER_STEP, 2 * 8, HIST},          // NaN where not recorded
   /* follow_ok     */ {PER_VEHICLE, 4, SCRATCH},        // mpcb_sim_follow_check
@@ -136,7 +138,7 @@ struct SimArrays {
   int* fsm_i; int* alive; int* n_obs; int* status; int* steps; int* n_unsolved; int* alive_idx; int* alive_cnt;
   int* count; double* run; int* run_verdict; double* run_metrics; int* route;
   double* hist_x; double* hist_u; double* hist_obs; int* hist_status; int* hist_tl; int* verdict; double* metrics;
-  unsigned long long* f_key; unsigned* f_tag; void* f_temp; int* lead_idx; double* lead_sv;
+  unsigned long long* f_key; unsigned* f_tag; void* f_temp; int* lead_idx; double* lead_sv; double* run_follow;
   int* hist_lead_idx; double* hist_lead_sv; int* follow_ok; double* min_gap;
   double* x_meas; double* hist_noise;
 };
@@ -161,7 +163,7 @@ static char* sim_alloc(SimArrays& d, size_t B, size_t T, SimMask mask, size_t te
   at(d.hist_x, R_HIST_X); at(d.hist_u, R_HIST_U); at(d.hist_obs, R_HIST_OBS); at(d.hist_status, R_HIST_STATUS);
   at(d.hist_tl, R_HIST_TL); at(d.verdict, R_VERDICT); at(d.metrics, R_METRICS);
   at(d.f_key, R_F_KEY); at(d.f_tag, R_F_TAG); at(d.f_temp, R_F_TEMP); at(d.lead_idx, R_LEAD_IDX);
-  at(d.lead_sv, R_LEAD_SV);
+  at(d.lead_sv, R_LEAD_SV); at(d.run_follow, R_RUN_FOLLOW);
   at(d.hist_lead_idx, R_HIST_LEAD_IDX); at(d.hist_lead_sv, R_HIST_LEAD_SV); at(d.follow_ok, R_FOLLOW_OK);
   at(d.min_gap, R_MIN_GAP);
   at(d.x_meas, R_X_MEAS); at(d.hist_noise, R_HIST_NOISE);
@@ -243,6 +245,13 @@ constexpr int FOLLOW_ROUTE_BITS = 5;                    // route keys 0 .. MPCB_
 static_assert(MPCB_MAX_ROUTES < (1 << FOLLOW_ROUTE_BITS), "route key does not fit its bits");
 static_assert(FOLLOW_IDX_BITS + FOLLOW_ROUTE_BITS == 32, "tag layout");
 
+// order-preserving key of s (pass s + 0.0: -0.0 -> +0.0, so that equal positions get equal keys): unsigned order of
+// keys = order of s
+__device__ __forceinline__ unsigned long long follow_key(double s) {
+  const unsigned long long u = (unsigned long long)__double_as_longlong(s);
+  return (u >> 63) ? ~u : (u | (1ull << 63));
+}
+
 __global__ void __launch_bounds__(128)
 mpcb_follow_key_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ SimArrays sim, int B) {
   const int* __restrict__ route = sim.route;
@@ -253,8 +262,7 @@ mpcb_follow_key_kernel(const __grid_constant__ DevTables Ts, const __grid_consta
   if (b >= B) return;
   const double s = x[(size_t)b * 5] + 0.0;              // -0.0 -> +0.0: equal positions get equal keys
   const bool live = s <= stop_s(Ts, route, b);          // loop condition (:395), as the FSM kernel evaluates it
-  const unsigned long long u = (unsigned long long)__double_as_longlong(s);
-  key[b] = (u >> 63) ? ~u : (u | (1ull << 63));         // order-preserving: unsigned order of keys = order of s
+  key[b] = follow_key(s);
   const unsigned r = live ? (unsigned)problem_route(route, b, Ts.n) : (unsigned)MPCB_MAX_ROUTES;
   MPCB_ASSERT(r <= (unsigned)MPCB_MAX_ROUTES);
   tag[b] = (r << FOLLOW_IDX_BITS) | (unsigned)b;
@@ -289,10 +297,68 @@ mpcb_follow_leader_kernel(const __grid_constant__ SimArrays sim, int B, double r
   lead_sv[2 * b + 1] = lv;
 }
 
+// ---- worlds (mpcb_sim_set_worlds): with world size M, a leader is searched for only among the vehicles [w M, (w+1) M)
+// of b's world w.  One launch replaces the key kernel, the two sorts and the leader kernel.  A CTA holds whole worlds
+// (blockDim.x a multiple of M): it stages the s keys and route keys of the key kernel in shared memory, and each thread
+// scans its world for the successor of (s key, b) among the vehicles with its route key, which is the next tag of the
+// sorted route segment.  No workspace; at most M shared-memory reads of each array per thread.
+constexpr int WORLD_MAX = 1024;
+
+__global__ void __launch_bounds__(WORLD_MAX)
+mpcb_follow_world_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ SimArrays sim, int B, int M,
+                         double range) {
+  __shared__ unsigned long long skey[WORLD_MAX];
+  __shared__ unsigned sroute[WORLD_MAX];
+  const int* __restrict__ route = sim.route;
+  const double* __restrict__ x = sim.x;
+  int* __restrict__ lead_idx = sim.lead_idx;
+  double* __restrict__ lead_sv = sim.lead_sv;
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  const bool in = b < B;                                 // a CTA past B holds whole worlds past B
+  unsigned long long k = 0;
+  unsigned r = (unsigned)MPCB_MAX_ROUTES;
+  double s = 0.0;
+  if (in) {
+    s = x[(size_t)b * 5];
+    const double s0 = s + 0.0;
+    k = follow_key(s0);
+    if (s0 <= stop_s(Ts, route, b)) r = (unsigned)problem_route(route, b, Ts.n);   // the key kernel's live test
+  }
+  skey[threadIdx.x] = k;
+  sroute[threadIdx.x] = r;
+  __syncthreads();
+  if (!in) return;
+  const int i = threadIdx.x % M, t0 = threadIdx.x - i;   // b's place in its world, the world's first slot in the CTA
+  int best = -1;
+  unsigned long long bk = 0;
+  if (r < (unsigned)MPCB_MAX_ROUTES)
+    for (int j = 0; j < M; ++j) {
+      MPCB_ASSERT((b - i + j) / M == b / M && b - i + j < B);
+      const unsigned long long kj = skey[t0 + j];
+      // after (k, i) in the order of (s key, index), and before the best so far (j rises: equal keys keep the first)
+      if (sroute[t0 + j] == r && (kj > k || (kj == k && j > i)) && (best < 0 || kj < bk)) { best = j; bk = kj; }
+    }
+  int lead = -1;
+  double ls = nan(""), lv = nan("");
+  if (best >= 0) {
+    const int j = b - i + best;
+    MPCB_ASSERT(j / M == b / M && j != b && j < B);
+    const double sj = x[(size_t)j * 5];
+    if (sj - s <= range) { lead = j; ls = sj; lv = x[(size_t)j * 5 + 4]; }
+  }
+  lead_idx[b] = lead;
+  lead_sv[2 * b] = ls;
+  lead_sv[2 * b + 1] = lv;
+}
+
+// CTA width of the world kernel: whole worlds, about 256 threads when worlds are small, one world of M when M >= 256
+static int world_threads(int M) { return M >= 256 ? M : (256 / M) * M; }
+
 // ObstaclesFSM.update for every vehicle that is still driving (:330-374); car first, then light (:349, :362).
 // alive_cnt / next_cnt: this step's and the next step's counter of the pair sim.alive_cnt.  With following on, the car
-// slot takes the nearer of the scripted car and the leader (lead_idx / lead_sv of mpcb_follow_leader_kernel), which is
-// recorded into hist_lead_idx / hist_lead_sv.  With measurement noise on, x_meas = x + w_meas is the state step t's solve
+// slot takes the nearer of the scripted car and the leader (lead_idx / lead_sv of mpcb_follow_leader_kernel or
+// mpcb_follow_world_kernel), which is recorded into hist_lead_idx / hist_lead_sv, and the gap to the leader is folded
+// into run_follow.  With measurement noise on, x_meas = x + w_meas is the state step t's solve
 // sees; everything here uses the true x.  With noise on, w_meas is recorded into hist_noise.
 __global__ void __launch_bounds__(128)
 mpcb_fsm_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ SimArrays sim, int B, double dt, int rec_t,
@@ -346,7 +412,12 @@ mpcb_fsm_kernel(const __grid_constant__ DevTables Ts, const __grid_constant__ Si
       // route the farther car is behind the nearer one, and the nearer car is itself constrained by it, so keeping
       // clear of the nearer one is enough; one car slot keeps n_obs <= MPCB_MAX_OBS with the light after it.
       const double ls = __ldg(lead_sv + 2 * b);
-      if (!isnan(ls) && !(n == 1 && o[0] <= ls)) { o[0] = ls; o[1] = __ldg(lead_sv + 2 * b + 1); n = 1; }
+      if (!isnan(ls)) {
+        // running follower gap, with mpcb_follow_check_kernel's expression (hist_lead_sv's s - hist_x's s)
+        double* __restrict__ run_follow = sim.run_follow;
+        run_follow[b] = fmin(run_follow[b], ls - s);
+        if (!(n == 1 && o[0] <= ls)) { o[0] = ls; o[1] = __ldg(lead_sv + 2 * b + 1); n = 1; }
+      }
     }
     if (sc.traffic_light && !(f & F_TL_GREEN)) {
       const double gap = sc.tl_pos - s;
@@ -597,7 +668,9 @@ mpcb_sim_running_check_kernel(const __grid_constant__ DevTables Ts, const __grid
 // A pass copies up to N_SIM arrays of n 4-byte words, one per blockIdx.y.  With parent, a gather: dst is laid out
 // [rows][B][w] (one row for the loop state) and word (r, b, k) comes from word (r, parent[b], k) of src; without it a
 // straight copy.  Consecutive threads take consecutive words of dst and of a row of src: coalesced on both sides.
-struct BranchCopy { const unsigned* src; unsigned* dst; unsigned long long n; unsigned w; };
+// leaders: the words are vehicle indices (-1: none), moved with their vehicle: j >= 0 becomes j + b - parent[b]
+// (mpcb_sim_branch_worlds, where b - parent[b] is the distance between the two worlds).
+struct BranchCopy { const unsigned* src; unsigned* dst; unsigned long long n; unsigned w, leaders; };
 struct BranchPass { BranchCopy c[N_SIM]; };
 constexpr int BRANCH_THREADS = 256;
 
@@ -613,7 +686,8 @@ mpcb_branch_gather_kernel(const __grid_constant__ BranchPass g, const int* __res
     const unsigned long long r = e / row, i = e - r * row, b = i / c.w;
     const int p = __ldg(parent + b);
     MPCB_ASSERT(p >= 0 && p < B);
-    dst[e] = src[r * row + (unsigned long long)p * c.w + (i - b * c.w)];
+    const unsigned v = src[r * row + (unsigned long long)p * c.w + (i - b * c.w)];
+    dst[e] = (c.leaders && (int)v >= 0) ? (unsigned)((int)v + (int)b - p) : v;
   }
 }
 
@@ -633,6 +707,7 @@ struct mpcb_sim {
   int follow = 0;
   double follow_range = 0.0;
   size_t f_temp_bytes = 0;    // bytes of d.f_temp
+  int world_size = 0;         // mpcb_sim_set_worlds; 0: one world
   SimNoise noise = {};        // mpcb_sim_set_noise; off: every sigma 0
   char* region[N_SIM] = {};   // address of every allocated region (nullptr: not allocated), for mpcb_sim_branch
   // branching (mpcb_sim_branch), made by its first call: the device workspace (the parent indices, then the gathered
@@ -765,7 +840,12 @@ int mpcb_sim_step(mpcb_sim_handle s, int n_steps, void* cuda_stream) {
   for (int k = 0; k < n_steps; ++k) {
     const int rec = (s->t < s->cap) ? s->t : -1;
     int* cnt = d.alive_cnt + (s->t & 1);
-    if (s->follow) {                                         // leaders of this step, from the states before it
+    if (s->follow && s->world_size > 0) {                    // leaders of this step within each world
+      const int wt = world_threads(s->world_size);
+      mpcb_follow_world_kernel<<<(s->B + wt - 1) / wt, wt, 0, st>>>(s->h->dt, d, s->B, s->world_size, s->follow_range);
+      CK(cudaGetLastError());
+      s->h->launches += 1;
+    } else if (s->follow) {                                  // leaders of this step, from the states before it
       const size_t nb = (size_t)s->B;
       mpcb_follow_key_kernel<<<grid, 128, 0, st>>>(s->h->dt, d, s->B);
       CK(cudaGetLastError());
@@ -814,7 +894,10 @@ int mpcb_sim_set_follow(mpcb_sim_handle s, int on, double follow_range) {
     if (!(s->block[1] = sim_alloc(s->d, nb, T, SIM_FOLLOW | (T > 0 ? SIM_FOLLOW_HIST : 0ull), temp, off, s->region)))
       return MPCB_ERR_NOMEM;
     s->f_temp_bytes = temp;
-    // rows of steps taken with following off stay -1 / NaN (all-ones bytes: int -1, a double NaN)
+    // the running gap starts at the check's 1e30; rows of steps taken with following off stay -1 / NaN (all-ones
+    // bytes: int -1, a double NaN)
+    const std::vector<double> big(nb, BIG);
+    CK(cudaMemcpy(s->d.run_follow, big.data(), sim_bytes(R_RUN_FOLLOW, nb, 0), cudaMemcpyHostToDevice));
     if (T > 0) {
       CK(cudaMemset(s->d.hist_lead_idx, 0xff, sim_bytes(R_HIST_LEAD_IDX, nb, T)));
       CK(cudaMemset(s->d.hist_lead_sv, 0xff, sim_bytes(R_HIST_LEAD_SV, nb, T)));
@@ -971,21 +1054,23 @@ int mpcb_sim_running_check(mpcb_sim_handle s, int* verdict, double* metrics, voi
   return MPCB_OK;
 }
 
-int mpcb_sim_branch(mpcb_sim_handle s, const int* parent, void* cuda_stream) {
-  if (!s || !parent || s->follow) return MPCB_ERR_INVALID;   // a copy would follow its parent at gap 0
-  for (int b = 0; b < s->B; ++b)
-    if (parent[b] < 0 || parent[b] >= s->B) return MPCB_ERR_INVALID;
+}  // extern "C"
+
+// mpcb_sim_branch and mpcb_sim_branch_worlds on checked parents: vehicle b takes over the whole state of parent[b];
+// leaders: the recorded leader indices are moved with their vehicle (BranchCopy::leaders).
+static int sim_gather(mpcb_sim* s, const int* parent, bool leaders, void* cuda_stream) {
   CK(cudaSetDevice(s->h->device));
   const size_t nb = (size_t)s->B;
   SimMask have = 0;
   for (int r = 0; r < N_SIM; ++r) if (s->region[r]) have |= sim_bit(r);
   // workspace: the parent indices, then room for the gathered loop state or one window of every history there can be
+  // (following, whose block holds loop state too, may be switched on after the first call)
   const SimMask state = sim_branch_mask(STATE) & have, hist = sim_branch_mask(HIST);
   size_t soff[N_SIM + 1], hoff[N_SIM + 1];
   const size_t pbytes = (nb * sizeof(int) + 255) & ~(size_t)255;
   if (!s->branch_ws) {
     const int rows = s->cap > 0 ? branch_window_rows(nb, s->cap) : 0;
-    sim_layout(nb, 0, state, 0, soff);
+    sim_layout(nb, 0, sim_branch_mask(STATE), 0, soff);
     sim_layout(nb, (size_t)rows, rows > 0 ? hist : 0ull, 0, hoff);
     char* ws = nullptr;
     int* hp = nullptr;
@@ -1019,8 +1104,9 @@ int mpcb_sim_branch(mpcb_sim_handle s, const int* parent, void* cuda_stream) {
     for (int r = 0; r < N_SIM; ++r) {
       if (!((mask >> r) & 1ull)) continue;
       const size_t bytes = SIM_BYTES[r].bytes, at = row0 * nb * bytes, words = rows * nb * bytes / 4;
-      g.c[n] = BranchCopy{(const unsigned*)(s->region[r] + at), (unsigned*)(ws + off[r]), words, (unsigned)(bytes / 4)};
-      back.c[n] = BranchCopy{(const unsigned*)(ws + off[r]), (unsigned*)(s->region[r] + at), words, g.c[n].w};
+      g.c[n] = BranchCopy{(const unsigned*)(s->region[r] + at), (unsigned*)(ws + off[r]), words, (unsigned)(bytes / 4),
+                          leaders && r == R_HIST_LEAD_IDX ? 1u : 0u};
+      back.c[n] = BranchCopy{(const unsigned*)(ws + off[r]), (unsigned*)(s->region[r] + at), words, g.c[n].w, 0u};
       if (words > most) most = words;
       ++n;
     }
@@ -1036,6 +1122,50 @@ int mpcb_sim_branch(mpcb_sim_handle s, const int* parent, void* cuda_stream) {
   const int nt = s->t < s->cap ? s->t : s->cap;
   for (int row0 = 0; row0 < nt; row0 += s->branch_rows)
     CK(pass(hist & have, hoff, (size_t)row0, (size_t)(nt - row0 < s->branch_rows ? nt - row0 : s->branch_rows)));
+  return MPCB_OK;
+}
+
+extern "C" {
+
+int mpcb_sim_branch(mpcb_sim_handle s, const int* parent, void* cuda_stream) {
+  if (!s || !parent || s->follow) return MPCB_ERR_INVALID;   // a copy would follow its parent at gap 0
+  for (int b = 0; b < s->B; ++b)
+    if (parent[b] < 0 || parent[b] >= s->B) return MPCB_ERR_INVALID;
+  return sim_gather(s, parent, false, cuda_stream);
+}
+
+int mpcb_sim_set_worlds(mpcb_sim_handle s, int world_size) {
+  if (!s || world_size < 0 || world_size > WORLD_MAX || (world_size > 0 && s->B % world_size != 0))
+    return MPCB_ERR_INVALID;
+  s->world_size = world_size;
+  return MPCB_OK;
+}
+
+int mpcb_sim_branch_worlds(mpcb_sim_handle s, const int* parent_world, void* cuda_stream) {
+  if (!s || !parent_world || s->world_size < 1) return MPCB_ERR_INVALID;
+  const int M = s->world_size, W = s->B / M;
+  for (int w = 0; w < W; ++w)
+    if (parent_world[w] < 0 || parent_world[w] >= W) return MPCB_ERR_INVALID;
+  std::vector<int> parent((size_t)s->B);
+  for (int w = 0; w < W; ++w)
+    for (int i = 0; i < M; ++i) parent[(size_t)w * M + i] = parent_world[w] * M + i;
+  return sim_gather(s, parent.data(), true, cuda_stream);
+}
+
+int mpcb_sim_running_follow_check(mpcb_sim_handle s, int* ok, double* min_gap, void* cuda_stream) {
+  if (!s || !ok) return MPCB_ERR_INVALID;
+  const size_t nb = (size_t)s->B;
+  std::vector<double> own(min_gap ? 0 : nb);
+  double* g = min_gap ? min_gap : own.data();
+  if (!s->d.run_follow) {                                    // following never switched on: no leader, ever
+    for (size_t b = 0; b < nb; ++b) g[b] = BIG;
+  } else {
+    CK(cudaSetDevice(s->h->device));
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    CK(cudaMemcpyAsync(g, s->d.run_follow, sim_bytes(R_RUN_FOLLOW, nb, 0), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+  }
+  for (size_t b = 0; b < nb; ++b) ok[b] = g[b] < 1.0 ? 0 : 1;   // mpcb_follow_check_kernel's safety test
   return MPCB_OK;
 }
 

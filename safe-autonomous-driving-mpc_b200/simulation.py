@@ -73,6 +73,20 @@ def _follow_range(r):
     return r
 
 
+WORLD_MAX = 1024       # largest world of mpcb_sim_set_worlds
+
+
+def _world_size(B, m):
+    """Checked world size of mpcb_sim_set_worlds: 0 (one world) for None or 0, else an integer in [1, 1024] that divides
+    B; ValueError otherwise."""
+    if m is None:
+        return 0
+    if isinstance(m, bool) or not isinstance(m, (int, np.integer)) or not 0 <= int(m) <= WORLD_MAX or (m and B % int(m)):
+        raise ValueError(f"world_size must be an integer in [1, {WORLD_MAX}] that divides B = {B} (or None / 0 for "
+                         f"one world), got {m!r}")
+    return int(m)
+
+
 NOISE_CHANNELS = (("meas", 5), ("act", 2), ("proc", 5))
 
 
@@ -96,14 +110,16 @@ def _noise_args(B, seed, meas, act, proc, first_id):
 
 class BatchedSimulation:
     def __init__(self, tracker, scenarios, B=None, x_init=None, history_steps=0, hot_start=False, route=None,
-                 follow_range=None, noise=None):
+                 follow_range=None, noise=None, world_size=None):
         """tracker: BatchedTracker; scenarios: one Scenario (shared) or a list of B; x_init: [B,5] or None for the
         reference's start state.  hot_start: from its second step on a vehicle's solve starts from its previous plan
         advanced by one step (mpcb_sim_set_hot_start) instead of the reference's table-based warm start.
         route: one int or an int array [B], vehicle b driving ``tracker.routes[route[b]]`` (None: route 0).
         follow_range: None (off) or a positive distance: the nearest vehicle ahead on the same route within that
         distance is a moving obstacle (``set_follow``).
-        noise: None (off) or a dict of ``set_noise``'s arguments (seed, meas, act, proc, first_id)."""
+        noise: None (off) or a dict of ``set_noise``'s arguments (seed, meas, act, proc, first_id).
+        world_size: None (one world) or M: vehicles [w M, (w + 1) M) form world w and follow only each other
+        (``set_worlds``)."""
         self._lib = tracker._lib
         self._t = tracker
         if follow_range is not None:
@@ -118,6 +134,7 @@ class BatchedSimulation:
                 raise ValueError(f"noise takes seed, meas, act, proc and first_id, got {sorted(noise)}")
             nz = _noise_args(int(B), noise["seed"], noise.get("meas"), noise.get("act"), noise.get("proc"),
                              noise.get("first_id", 0))
+        world_size = _world_size(int(B), world_size)
         arr = (Scenario * len(scen))(*scen)
         xi = None
         if x_init is not None:
@@ -138,12 +155,15 @@ class BatchedSimulation:
         self._h = h
         self.B = int(B)
         self.history_steps = int(history_steps)
+        self.world_size, self.W = None, 1
         if hot_start:
             check(self._lib.mpcb_sim_set_hot_start(h, 1), "mpcb_sim_set_hot_start")
         if follow_range is not None:
             self.set_follow(follow_range)
         if noise is not None:
             self._set_noise(*nz)
+        if world_size:
+            self.set_worlds(world_size)
 
     def __del__(self):
         h = getattr(self, "_h", None)
@@ -182,6 +202,15 @@ class BatchedSimulation:
             check(self._lib.mpcb_sim_set_follow(self._h, 0, 0.0), "mpcb_sim_set_follow")
             return
         check(self._lib.mpcb_sim_set_follow(self._h, 1, _follow_range(follow_range)), "mpcb_sim_set_follow")
+
+    def set_worlds(self, world_size):
+        """Worlds from the next step on (mpcb_sim_set_worlds; include/mpcb200.h has the rules): world w is vehicles
+        [w M, (w + 1) M) for M = world_size, and a vehicle's leader is searched for only inside its own world.  M must
+        be in [1, 1024] and divide B, else ValueError before any device call; None or 0 returns to one world.  Sets
+        ``world_size`` (None: one world) and ``W`` (the number of worlds)."""
+        m = _world_size(self.B, world_size)
+        check(self._lib.mpcb_sim_set_worlds(self._h, m), "mpcb_sim_set_worlds")
+        self.world_size, self.W = (m, self.B // m) if m else (None, 1)
 
     def set_noise(self, seed, meas=None, act=None, proc=None, first_id=0):
         """Seeded Gaussian disturbances from the next step on (mpcb_sim_set_noise; include/mpcb200.h has the rules):
@@ -222,6 +251,15 @@ class BatchedSimulation:
         check(self._lib.mpcb_sim_follow_check(self._h, _dp(ok), _dp(g), None), "mpcb_sim_follow_check")
         return dict(ok=ok.astype(bool), min_gap=g)
 
+    def running_follow_check(self):
+        """The same dict as ``follow_check``, from the least gap to the leader the loop keeps per vehicle
+        (mpcb_sim_running_follow_check): needs no history.  Equal to ``follow_check`` bit for bit when the history
+        covers every drive; min_gap 1e30 and ok True if following was never on."""
+        ok = np.empty(self.B, np.int32)
+        g = np.empty(self.B)
+        check(self._lib.mpcb_sim_running_follow_check(self._h, _dp(ok), _dp(g), None), "mpcb_sim_running_follow_check")
+        return dict(ok=ok.astype(bool), min_gap=g)
+
     CHECKS = CHECKS
 
     def check(self):
@@ -252,6 +290,21 @@ class BatchedSimulation:
             raise ValueError(f"parent values must be in [0, {self.B})")
         p = np.ascontiguousarray(p, dtype=np.int32)
         check(self._lib.mpcb_sim_branch(self._h, _dp(p), C.c_void_p(stream or 0)), "mpcb_sim_branch")
+
+    def branch_worlds(self, parent_world, stream=None):
+        """World w takes over the whole state of world parent_world[w], vehicle by vehicle, histories and running
+        verdicts included; recorded leaders are moved into the copy's world (mpcb_sim_branch_worlds; include/mpcb200.h
+        has the rules).  Needs worlds (``set_worlds``); parent_world: integer array [W] with values in [0, W), else
+        ValueError before any device call.  Following may be on."""
+        if not self.world_size:
+            raise ValueError("branch_worlds needs worlds: set_worlds(M) or BatchedSimulation(world_size=M)")
+        p = np.asarray(parent_world)
+        if p.shape != (self.W,) or not np.issubdtype(p.dtype, np.integer):
+            raise ValueError(f"parent_world must be an int array of shape ({self.W},), got {p.dtype} {p.shape}")
+        if p.min() < 0 or p.max() >= self.W:
+            raise ValueError(f"parent_world values must be in [0, {self.W})")
+        p = np.ascontiguousarray(p, dtype=np.int32)
+        check(self._lib.mpcb_sim_branch_worlds(self._h, _dp(p), C.c_void_p(stream or 0)), "mpcb_sim_branch_worlds")
 
     def run(self, max_steps=200000, check_every=64):
         """Drive until every vehicle has passed s_max - 1 (or max_steps).  Returns the number of steps enqueued."""
